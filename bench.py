@@ -22,8 +22,10 @@ retire query by query and the predictions are real token sequences.  The default
 
 The timed batches are drawn from ONE queue shared by all ranks and in-flight engines (`distributed.BatchQueue`): nobody
 owns a static shard.  `--scaling weak` (default) times N*K batches on N GPUs, `--scaling strong` a fixed set of
-`--queries` queries whatever N is.  Every GPU output is checked: against the reference goldens of the same batch
-(tests/golden/bench_configs.npz) and against the reference run live on the host for a few queries (`parity`).
+`--queries` queries whatever N is.  The side workloads of the default line time `--steps` batches each as well.  Every
+GPU output is checked: against the reference goldens of the same batch (tests/golden/bench_configs.npz) and against the
+reference run live on the host for a few queries (`parity`).  `--dump-outputs DIR` saves the prediction of each workload's
+last timed step; the inputs depend only on the arguments, so two builds run with the same arguments compare file by file.
 Prints ONE JSON line on rank 0.
 """
 from __future__ import annotations
@@ -91,7 +93,13 @@ def parse():
                          "for the random-init greedy workload (every batch keeps all its queries to the end), 8 for the trained-like greedy "
                          "workload whose batches thin out while they decode, 12 for the beam searches (measured: DESIGN.md section 4c)")
     ap.add_argument("--clock-period-ms", type=int, default=200, help="nvidia-smi sampling period; 0 disables the sampler")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the prediction of the last timed step of every measured workload to "
+                         "DIR/<workload>_<weights>.npy (token ids as float32), to compare two builds output for output")
+    args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 1:
+        ap.error("--steps and --warmup must be at least 1 (the warm-up batches size every workspace and feed the parity check)")
+    return args
 
 
 # ------------------------------------------------------------------------------------------------
@@ -618,6 +626,8 @@ def measure_workload(wl, args, local_rank, world, rank, n_fly, steps, warmup, n_
         sampler.start()
     ms, mine, nfail = R.timed(first, n_timed_batches, False)
     clocks = sampler.stop() if (rank == 0 and full) else None
+    last = R.last_gathered[-1]          # None when the last batch ended in a reference failure mode
+    res["last"] = None if last is None else last.cpu()
     c1 = R.counters()
     e2e_ms, _, e2e_fail = R.timed(first, n_timed_batches, True)
     insitu = None
@@ -706,6 +716,18 @@ def roofline_tables(wl, args, m, peaks):
     return roof, table
 
 
+def dump_outputs(out_dir, outputs):
+    """`--dump-outputs`: {name: (batch, n_best, width) int64 prediction or None} -> out_dir/<name>.npy as float32 (token ids are
+    exact in float32).  A step that ended in one of the reference's failure modes returned no prediction and writes no file."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    for name, pred in outputs.items():
+        if pred is None:
+            print(f"bench.py: the last timed step of {name} returned no prediction; {name}.npy not written", file=sys.stderr)
+            continue
+        np.save(d / f"{name}.npy", pred.numpy().astype(np.float32))
+
+
 def main():
     args = parse()
     rank = int(os.environ.get("RANK", "0"))
@@ -740,6 +762,7 @@ def main():
     else:
         n_batches = world * args.steps
     m = measure_workload(wl, args, local_rank, world, rank, n_fly, args.steps, args.warmup, n_batches, full=True)
+    outputs = {f"{wl.key}_{wl.weights}": m["last"]}
     peaks = measured_peaks()
 
     line = None
@@ -785,13 +808,15 @@ def main():
         todo = []
         if args.workload == "greedy":
             other = "copy" if args.weights == "random" else "random"
-            todo.append(("trained_like" if other == "copy" else "random_init_worst_case", Workload("greedy", other, args), 32 if other == "copy" else 6, True))
+            todo.append(("trained_like" if other == "copy" else "random_init_worst_case", Workload("greedy", other, args), True))
         if args.workload == "greedy":
-            todo += [("beam", Workload("beam", "copy", args), 24, False), ("retro", Workload("retro", "copy", args), 24, False)]
-        for key, w2, k2, full in todo:
+            todo += [("beam", Workload("beam", "copy", args), False), ("retro", Workload("retro", "copy", args), False)]
+        k2 = args.steps
+        for key, w2, full in todo:
             try:
                 n_fly2 = fly_for(w2)
-                m2 = measure_workload(w2, args, local_rank, 1, 0, n_fly2, k2, 2, k2, full=full)
+                m2 = measure_workload(w2, args, local_rank, 1, 0, n_fly2, k2, args.warmup, k2, full=full)
+                outputs[f"{w2.key}_{w2.weights}"] = m2["last"]
                 blk = {"workload": w2.describe(), "metric": w2.w["metric"], "value": m2["value"], "unit": "SMILES/s", "steps": k2,
                        "ms_per_step": m2["ms"] / k2, "batches_in_flight": n_fly2,
                        "e2e": {"value": m2["e2e_value"], "unit": "SMILES/s", "h2d_bytes_per_step": m2["h2d"], "d2h_bytes_per_step": m2["d2h"]},
@@ -817,6 +842,8 @@ def main():
                     if g and g.get("checked") and g["top1_identical"] != g["queries"]:
                         line["parity_ok"] = False
     if rank == 0:
+        if args.dump_outputs:
+            dump_outputs(args.dump_outputs, outputs)
         print(json.dumps(line), flush=True)
     if world > 1:
         dist.destroy_process_group()

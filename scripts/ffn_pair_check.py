@@ -3,6 +3,7 @@ full-size bf16 forward on the golden inputs and on a larger random batch, each m
 import os
 import subprocess
 import sys
+import tempfile
 from pathlib import Path
 
 import numpy as np
@@ -44,14 +45,16 @@ if __name__ == "__main__":
         child(sys.argv[1])
         sys.exit(0)
     outs = {}
-    for mode in ("0", "1"):
-        env = dict(os.environ, TTB_FFN_PAIR=mode, TTB_DEBUG="1")
-        f = f"/tmp/ffn_pair_{mode}.npz"
-        r = subprocess.run(["timeout", "120", sys.executable, __file__, f], env=env)
-        print("mode", mode, "rc", r.returncode, flush=True)
-        if r.returncode != 0:
-            sys.exit(1)
-        outs[mode] = np.load(f)
+    with tempfile.TemporaryDirectory() as tmp:      # private to this run: several users may share the machine
+        for mode in ("0", "1"):
+            env = dict(os.environ, TTB_FFN_PAIR=mode, TTB_DEBUG="1")
+            f = os.path.join(tmp, f"ffn_pair_{mode}.npz")
+            r = subprocess.run(["timeout", "120", sys.executable, __file__, f], env=env)
+            print("mode", mode, "rc", r.returncode, flush=True)
+            if r.returncode != 0:
+                sys.exit(1)
+            with np.load(f) as z:
+                outs[mode] = dict(z)
     worst = 0.0
     for k in ("a", "b", "c"):
         d = np.abs(outs["0"][k] - outs["1"][k])

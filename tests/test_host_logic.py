@@ -347,6 +347,28 @@ def test_bench_workloads_are_the_golden_cases():
     assert abs(f / 4 - (4.0 * rows * 256 * 2048 + 2.0 * rows * 256 * 256 + 16.0 * rows * 256)) < 1.0
 
 
+def test_bench_dump_outputs_and_step_arguments(tmp_path, monkeypatch):
+    """bench.py --dump-outputs: one float32 .npy per workload that holds its token ids exactly, no file for a step that returned
+    no prediction; --steps / --warmup below 1 are refused."""
+    import importlib.util
+    import numpy as np
+    spec = importlib.util.spec_from_file_location("bench_mod", REPO / "bench.py")
+    bench = importlib.util.module_from_spec(spec)
+    spec.loader.exec_module(bench)
+    pred = torch.randint(0, 288, (4, 5, 214), generator=torch.Generator().manual_seed(0))
+    bench.dump_outputs(tmp_path / "d", {"beam_copy": pred, "greedy_random": None})
+    assert sorted(p.name for p in (tmp_path / "d").iterdir()) == ["beam_copy.npy"]
+    a = np.load(tmp_path / "d" / "beam_copy.npy")
+    assert a.dtype == np.float32 and np.array_equal(a.astype(np.int64), pred.numpy())
+    monkeypatch.setattr(sys, "argv", ["bench.py", "--steps", "5", "--warmup", "2", "--dump-outputs", str(tmp_path)])
+    args = bench.parse()
+    assert (args.steps, args.warmup, args.dump_outputs) == (5, 2, str(tmp_path))
+    for bad in (["--steps", "0"], ["--warmup", "0"]):
+        monkeypatch.setattr(sys, "argv", ["bench.py", *bad])
+        with pytest.raises(SystemExit):
+            bench.parse()
+
+
 def test_committed_bench_line_keeps_the_driver_contract():
     """profiles/r2_bench_1gpu.json is the line `python bench.py` printed on the B200 for the committed build: the keys the
     driver and the judge read must be there and consistent with each other (BASELINE.json metric, roofline = achieved / peak,
