@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define TTB_ABI_VERSION 2
+#define TTB_ABI_VERSION 3
 
 #define TTB_PRECISION_FP32 0 /* fp32 FMA GEMMs, exact-parity path (1e-5 logits)            */
 #define TTB_PRECISION_BF16 1 /* tcgen05 bf16 GEMMs, fp32 accumulate (1e-2 logits)          */
@@ -94,6 +94,23 @@ int ttb_greedy_speculative_generate(ttb_engine* e, const int64_t* src_dev, int32
                                     int32_t bos_token, int32_t eos_token, int32_t replace_token,
                                     int32_t tie_break, int64_t* out_dev, int32_t* trace_dev,
                                     ttb_generate_stats* stats, void* stream);
+
+/* ---- continuous batching of speculative_decoding.py:39 generate(): n_batches independent batches share `slots`
+ * query slots of ONE device loop.  Batch i is admitted (in list order) as soon as `batch_sizes[i]` slots are free;
+ * its queries keep the width / stop / error rules of their own batch, so out_devs[i], trace_devs[i] and stats[i]
+ * are exactly what ttb_greedy_speculative_generate returns for that batch alone.  A reference failure of one batch
+ * (stats[i].error = TTB_ERR_REF_*) ends that batch only; the call returns 0 unless something else failed.
+ * src_devs[i] is (batch_sizes[i], src_lens[i]) int64, out_devs[i] (batch_sizes[i], max_len) int64, trace_devs[i]
+ * (max_len + 1, batch_sizes[i], 4) int32 like trace_dev above (query ids are indices within the batch).
+ * slots >= max(batch_sizes).  trace_devs may be NULL, or hold NULL entries.  total (may be NULL): launches / ms of the
+ * call, model_calls = decoder iterations of the shared loop.  The loop runs the default attention kernels (not the
+ * opt-in tcgen05 attention).  ttb_engine_get_history afterwards gives the live slots of every iteration. */
+int ttb_greedy_speculative_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs,
+                                            const int32_t* batch_sizes, const int32_t* src_lens, int32_t slots, int32_t max_len,
+                                            int32_t draft_len, int32_t n_drafts, int32_t pad_token, int32_t bos_token,
+                                            int32_t eos_token, int32_t replace_token, int32_t tie_break, int64_t* const* out_devs,
+                                            int32_t* const* trace_devs, ttb_generate_stats* stats, ttb_generate_stats* total,
+                                            void* stream);
 
 /* ---- standard_decoding.py:29 TranslationInferenceGreedy.generate(src)
  * Plain greedy decoding, one token per row and step, on the same KV-cached device loop (no drafts).  Like the

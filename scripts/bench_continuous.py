@@ -1,0 +1,171 @@
+"""Continuous batching vs. one batch at a time vs. engines in flight, on the greedy workload of bench.py.
+
+Weights and batches are exactly the ones `bench.py --workload greedy` times (bench.Workload): product-prediction model,
+vocab 288, seed 1234, batches synthetic_sources(32, 288, seed=100003 + j), bs 32, draft_len 10, n_drafts 23,
+max_len 200, bf16.  Legs, all on the same batches in one process:
+  (a) sequential            one engine, generate() per batch
+  (b) continuous            one engine, generate_batches() for every value of --slots
+  (c) in flight             k engines (InFlightDecoder), generate() per batch
+  (d) continuous in flight  k engines, generate_batches() over a contiguous share of the batches each, best slots of (b)
+Every leg's outputs must equal leg (a) tensor for tensor before any timing is reported.  Rates are SMILES/s from the host
+clock around work that ends in a device synchronise; every shape is warmed up first (graphs are captured lazily).
+
+    python scripts/bench_continuous.py --weights copy --batches 24 --out profiles/continuous_copy.json
+"""
+from __future__ import annotations
+
+import argparse
+import ctypes as C
+import json
+import subprocess
+import sys
+import threading
+import time
+from pathlib import Path
+
+import torch
+
+REPO = Path(__file__).resolve().parent.parent
+sys.path.insert(0, str(REPO))
+
+import bench  # noqa: E402
+from translation_transformer_b200.model import B200Transformer  # noqa: E402
+from translation_transformer_b200.pipeline import InFlightDecoder  # noqa: E402
+
+
+def gpu_info():
+    q = subprocess.run(["nvidia-smi", "--query-gpu=name,power.limit,clocks.max.sm,clocks.sm", "--format=csv,noheader"],
+                       capture_output=True, text=True)
+    name, power, max_sm, sm = [x.strip() for x in q.stdout.splitlines()[0].split(",")]
+    return {"card": name, "power_limit": power, "sm_clock_max": max_sm, "sm_clock_at_start": sm}
+
+
+def history(eng):
+    buf = (C.c_int32 * 200000)()
+    n = eng.lib.ttb_engine_get_history(eng._h, buf, len(buf))
+    return list(buf[:n])
+
+
+def timed(fn):
+    torch.cuda.synchronize()
+    t0 = time.perf_counter()
+    res = fn()
+    torch.cuda.synchronize()
+    return res, time.perf_counter() - t0
+
+
+def main():
+    ap = argparse.ArgumentParser()
+    ap.add_argument("--weights", default="copy", choices=["copy", "random"])
+    ap.add_argument("--batches", type=int, default=24)
+    ap.add_argument("--slots", default="32,48,64,96,128")
+    ap.add_argument("--inflight", default="3,8")
+    ap.add_argument("--cont-inflight", default="2,4")
+    ap.add_argument("--out", required=True)
+    a = ap.parse_args()
+    argv, sys.argv = sys.argv, ["bench.py", "--workload", "greedy", "--weights", a.weights]
+    bargs = bench.parse()
+    sys.argv = argv
+    wl = bench.Workload("greedy", a.weights, bargs)
+    dev = torch.device("cuda", 0)
+    batches = [wl.batch(j).to(dev) for j in range(a.batches)]
+    n_smiles = sum(b.shape[0] for b in batches)
+    res = {"workload": wl.describe(), "batches": a.batches, "bs": wl.bs, "weights": a.weights, **gpu_info()}
+
+    def engine():
+        return B200Transformer(wl.cfg, wl.sd, precision="bf16", device=0)
+
+    def mem_of(make):   # device memory an engine holds after a warm run
+        torch.cuda.synchronize()
+        free0 = torch.cuda.mem_get_info(0)[0]
+        eng = make()
+        return eng, free0
+
+    # (a) sequential
+    eng0, free0 = mem_of(engine)
+    gen0 = wl.generator(eng0)
+    for b in batches[:2]:
+        gen0.generate(b)
+    ref, t = timed(lambda: [gen0.generate(b) for b in batches])
+    h = []
+    for b in batches[:4]:
+        gen0.generate(b)
+        h += history(eng0)
+    torch.cuda.synchronize()
+    res["a_sequential"] = {"smiles_per_s": n_smiles / t, "s": t, "mean_live": sum(h) / len(h), "max_live": max(h),
+                           "engine_bytes": free0 - torch.cuda.mem_get_info(0)[0]}
+
+    # (b) continuous, one engine per slots value (memory per engine then includes that slots value's workspace)
+    res["b_continuous"] = []
+    best = None
+    for slots in [int(x) for x in a.slots.split(",")]:
+        eng, free0 = mem_of(engine)
+        gen = wl.generator(eng)
+        gen.generate_batches(batches[:6], slots=slots)        # warm-up: graphs of every bucket this slots value uses
+        out, t = timed(lambda: gen.generate_batches(batches, slots=slots))
+        assert all(torch.equal(x, y) for x, y in zip(ref, out)), f"continuous slots={slots} differs from generate()"
+        h = history(eng)
+        r = {"slots": slots, "smiles_per_s": n_smiles / t, "s": t, "mean_live": sum(h) / len(h), "max_live": max(h),
+             "iterations": len(h), "engine_bytes": free0 - torch.cuda.mem_get_info(0)[0]}
+        res["b_continuous"].append(r)
+        if best is None or r["smiles_per_s"] > best["smiles_per_s"]:
+            best = r
+        eng.close()
+        del eng, gen
+        torch.cuda.empty_cache()
+        print(json.dumps(r), flush=True)
+
+    # (c) engines in flight
+    res["c_in_flight"] = []
+    for k in [int(x) for x in a.inflight.split(",")]:
+        engs = [engine() for _ in range(k)]
+        dec = InFlightDecoder([wl.generator(e) for e in engs], device=dev)
+        list(dec.map(batches[:2 * k]))
+        out, t = timed(lambda: list(dec.map(batches)))
+        assert all(torch.equal(x, y) for x, y in zip(ref, out)), f"in-flight k={k} differs from generate()"
+        res["c_in_flight"].append({"engines": k, "smiles_per_s": n_smiles / t, "s": t})
+        dec.close()
+        for e in engs:
+            e.close()
+        torch.cuda.empty_cache()
+
+    # (d) continuous loops in flight: each engine decodes a contiguous share of the batches on its own stream
+    res["d_continuous_in_flight"] = []
+    for k in [int(x) for x in a.cont_inflight.split(",")]:
+        engs = [engine() for _ in range(k)]
+        gens = [wl.generator(e) for e in engs]
+        streams = [torch.cuda.Stream(device=dev) for _ in range(k)]
+        share = (len(batches) + k - 1) // k
+        parts = [batches[i * share:(i + 1) * share] for i in range(k)]
+
+        def run(i, outs):
+            torch.cuda.set_device(dev)
+            with torch.cuda.stream(streams[i]):
+                outs[i] = gens[i].generate_batches(parts[i], slots=best["slots"]) if parts[i] else []
+                streams[i].synchronize()
+
+        def all_parts():
+            outs = [None] * k
+            th = [threading.Thread(target=run, args=(i, outs)) for i in range(k)]
+            for x in th:
+                x.start()
+            for x in th:
+                x.join()
+            return [o for part in outs for o in part]
+
+        all_parts()
+        out, t = timed(all_parts)
+        assert all(torch.equal(x, y) for x, y in zip(ref, out)), f"continuous in flight k={k} differs from generate()"
+        res["d_continuous_in_flight"].append({"engines": k, "slots": best["slots"], "smiles_per_s": n_smiles / t, "s": t})
+        for e in engs:
+            e.close()
+        torch.cuda.empty_cache()
+
+    res["best_slots"] = best["slots"]
+    Path(a.out).parent.mkdir(parents=True, exist_ok=True)
+    Path(a.out).write_text(json.dumps(res, indent=1) + "\n")
+    print(json.dumps(res))
+
+
+if __name__ == "__main__":
+    main()

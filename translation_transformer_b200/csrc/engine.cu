@@ -163,7 +163,7 @@ struct ttb_engine {
     cudaEvent_t join_ev{};
     static constexpr int kBuckets = 10;
     cudaGraphExec_t graph_exec[kBuckets][2] = {};   // greedy iteration graphs per live-query bucket (grids sized for the bucket) x {long, short}
-    long long graph_key[12] = {};
+    long long graph_key[13] = {};
     long long graph_launches = 0;
     static constexpr int kBeamBuckets = 8;
     cudaGraphExec_t beam_graph[2][kBeamBuckets] = {};   // steady-state iteration of the speculative beam search, per ping-pong parity and live-candidate bucket
@@ -171,6 +171,8 @@ struct ttb_engine {
     long long beam_graph_launches = 0;
     DevBuf beam;                 // arena of the beam-search state
     DevBuf hist;                 // per-iteration live-query count of the last generate()
+    DevBuf cb;                   // continuous batching: slot / batch tables and the staging buffers of an admitted batch
+    DevBuf cb_work;              // continuous batching: encoder workspace of an admitted batch (the loop's own must stay intact)
     std::vector<int> h_hist;
 
     int E() const { return d.embedding_dim; }
@@ -181,7 +183,7 @@ struct ttb_engine {
     // different host threads, translation_transformer_b200/pipeline.py)
     long long alloc_signature() const {
         const DevBuf* bufs[] = {&x, &xh, &y, &qkv, &att, &q2, &hid, &logits, &tok32, &keytok32, &pred, &src32, &srclen, &desc, &memory, &memh,
-                                &crosskv, &crossvt, &kcache, &vcache, &kcache2, &vcache2, &drafts, &gen, &front, &active, &ctrl, &sel, &out64, &beam, &hist};
+                                &crosskv, &crossvt, &kcache, &vcache, &kcache2, &vcache2, &drafts, &gen, &front, &active, &ctrl, &sel, &out64, &beam, &hist, &cb, &cb_work};
         unsigned long long h = 1469598103934665603ull;
         for (const DevBuf* b : bufs) {
             h = (h ^ (unsigned long long)reinterpret_cast<uintptr_t>(b->p)) * 1099511628211ull;
@@ -451,17 +453,44 @@ static int ensure_work(ttb_engine* e, long long T, int qkv_layers) {
     return rc;
 }
 
+// Workspace of the encoder stack (rows = tokens): the engine's forward workspace unless the caller brings its own.
+template <typename ActT> struct EncWork { float* x; ActT* xh; float* y; ActT* qkv; ActT* att; ActT* hid; };
+template <typename ActT>
+static size_t enc_work_bytes(const ttb_engine* e, long long T) {
+    const long long E = e->E(), F = e->d.feedforward_dim;
+    const long long elems[6] = {T * E * 4, Prec<ActT>::lowp ? T * E * (long long)sizeof(ActT) : 0, T * E * 4, T * 3 * E * (long long)sizeof(ActT),
+                                T * E * (long long)sizeof(ActT), T * F * (long long)sizeof(ActT)};
+    size_t n = 0;
+    for (long long b : elems) n += (size_t)(b + 255) / 256 * 256;
+    return n;
+}
+template <typename ActT>
+static EncWork<ActT> enc_work_carve(const ttb_engine* e, long long T, void* base) {
+    const long long E = e->E(), F = e->d.feedforward_dim;
+    char* p = static_cast<char*>(base);
+    auto take = [&](long long bytes) { char* q = p; p += (bytes + 255) / 256 * 256; return q; };
+    EncWork<ActT> w;
+    w.x = reinterpret_cast<float*>(take(T * E * 4));
+    w.xh = Prec<ActT>::lowp ? reinterpret_cast<ActT*>(take(T * E * sizeof(ActT))) : nullptr;
+    w.y = reinterpret_cast<float*>(take(T * E * 4));
+    w.qkv = reinterpret_cast<ActT*>(take(T * 3 * E * sizeof(ActT)));
+    w.att = reinterpret_cast<ActT*>(take(T * E * sizeof(ActT)));
+    w.hid = reinterpret_cast<ActT*>(take(T * F * sizeof(ActT)));
+    return w;
+}
+
 // Encoder stack on tokens src32 (B, Ls); writes memory (fp32) and, on the bf16 path, memh.
 template <typename ActT>
-static int encode_impl(ttb_engine* e, const int* src32, const int* key_tok, int B, int Ls, float* mem_out, ActT* memh_out, cudaStream_t s) {
+static int encode_impl(ttb_engine* e, const int* src32, const int* key_tok, int B, int Ls, float* mem_out, ActT* memh_out, cudaStream_t s,
+                       const EncWork<ActT>* work = nullptr) {
     const int E = e->E(), T = B * Ls, H = e->d.num_heads, HD = e->HD();
-    if (ensure_work<ActT>(e, T, 1)) return 1;
-    float* x = e->x.as<float>();
-    ActT* xh = Prec<ActT>::lowp ? e->xh.as<ActT>() : nullptr;
-    float* y = e->y.as<float>();
-    ActT* qkv = e->qkv.as<ActT>();
-    ActT* att = e->att.as<ActT>();
-    ActT* hid = e->hid.as<ActT>();
+    if (!work && ensure_work<ActT>(e, T, 1)) return 1;
+    float* x = work ? work->x : e->x.as<float>();
+    ActT* xh = work ? work->xh : (Prec<ActT>::lowp ? e->xh.as<ActT>() : nullptr);
+    float* y = work ? work->y : e->y.as<float>();
+    ActT* qkv = work ? work->qkv : e->qkv.as<ActT>();
+    ActT* att = work ? work->att : e->att.as<ActT>();
+    ActT* hid = work ? work->hid : e->hid.as<ActT>();
     RowCount rows(T);
     e->prof.override_kc = KC_ENCODER;
     struct Reset { ttb_engine* e; ~Reset() { e->prof.override_kc = -1; } } reset{e};
@@ -593,10 +622,23 @@ static int decode_api(ttb_engine* e, const int64_t* tgt_dev, int B, int Lt, cons
     return 0;
 }
 
+// Continuous batching (ttb_greedy_speculative_generate_batches): the batches that share the slots of one loop.
+struct CbArgs {
+    int n;                              // batches, admitted in list order
+    const int64_t* const* src;          // [n] (B_i, Ls_i) int64 sources
+    const int32_t* bs;                  // [n] B_i
+    const int32_t* ls;                  // [n] Ls_i
+    int64_t* const* out;                // [n] (B_i, max_len) int64 predictions
+    int32_t* const* trace;              // [n] optional (max_len + 1, B_i, 4) traces, or NULL
+    ttb_generate_stats* stats;          // [n]
+};
+
+// Speculative greedy loop.  With `cb` the loop is the continuous one: B is the number of query slots, Ls the longest
+// source of all batches, and the batches of `cb` are admitted into free slots between two graph launches.
 template <typename ActT>
 static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int max_len, int draft_len, int N,
                       int pad, int bos, int eos, int replace, int tie_break, int64_t* out_dev, int32_t* trace_dev,
-                      ttb_generate_stats* stats, cudaStream_t user_stream, bool standard = false) {
+                      ttb_generate_stats* stats, cudaStream_t user_stream, bool standard = false, const CbArgs* cb = nullptr) {
     const int E = e->E(), H = e->d.num_heads, HD = e->HD(), V = e->d.tgt_vocab_size;
     const int n_dec = (int)e->dec.size();
     // the loop runs on the engine's own stream (graph capture is not allowed on the legacy default
@@ -618,16 +660,26 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     const int gen_ld = max_len + D + 2;
     const int P = gen_ld;  // cache positions per query
     const long long launches0 = e->launches;
-    const int max_iters = max_len + 1;
+    const bool cont = cb != nullptr;
+    // continuous loop: every batch takes part in at most max_len + 1 iterations; the host stays at most (LAG + 1) graph
+    // launches ahead of the control words it reads, i.e. a few no-op iterations per admission
+    const long long max_iters = cont ? (long long)cb->n * (max_len + 1) + (long long)(cb->n + 1) * 3 * 16 : max_len + 1;
+    // staging of an admitted batch (continuous loop): its encoder runs on the largest batch shape
+    int B_stage = 0;
+    long long TS_stage = 0;
+    if (cont)
+        for (int i = 0; i < cb->n; ++i) { B_stage = std::max(B_stage, (int)cb->bs[i]); TS_stage = std::max(TS_stage, (long long)cb->bs[i] * cb->ls[i]); }
+    const long long TS_enc = cont ? TS_stage : TS_cap;
 
     // encoder + cross-attention K/V (computed once per query, not once per draft row and iteration)
-    if (e->src32.ensure(TS_cap * sizeof(int)) || e->memory.ensure(TS_cap * E * sizeof(float)) || e->srclen.ensure((size_t)B * sizeof(int))) return 1;
-    if (Prec<ActT>::lowp && e->memh.ensure(TS_cap * E * sizeof(ActT))) return 1;
+    if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float)) || e->srclen.ensure((size_t)B * sizeof(int))) return 1;
+    if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
     if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
     // tcgen05 attention inside the loop (bf16, head_dim 32, key counts within its tensor-memory budget): the value caches
-    // are kept transposed ([dim][position], pitch VT_PITCH) so that both products read K-major operands
+    // are kept transposed ([dim][position], pitch VT_PITCH) so that both products read K-major operands.  The continuous
+    // loop runs the default attention kernels.
     constexpr int VT_PITCH = 256;
-    const bool tc_attn = Prec<ActT>::lowp && !attn_simt_forced() && attention_tc_supported(HD, per_q, std::max(P, Ls), D + 1);
+    const bool tc_attn = !cont && Prec<ActT>::lowp && !attn_simt_forced() && attention_tc_supported(HD, per_q, std::max(P, Ls), D + 1);
     const size_t vcache_bytes = tc_attn ? (size_t)n_dec * B * E * VT_PITCH * sizeof(ActT) : (size_t)n_dec * B * P * E * sizeof(ActT);
     if (e->kcache.ensure((size_t)n_dec * B * P * E * sizeof(ActT)) || e->vcache.ensure(vcache_bytes)) return 1;
     if (tc_attn && e->crossvt.ensure((size_t)n_dec * B * E * VT_PITCH * sizeof(ActT))) return 1;
@@ -636,19 +688,79 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     if (e->sel.ensure((size_t)B * 4 * sizeof(int)) || e->out64.ensure((size_t)B * max_len * sizeof(long long))) return 1;
     if (e->desc.ensure((size_t)B * sizeof(int4))) return 1;
     if (e->hist.ensure((size_t)(max_iters + 1) * sizeof(int))) return 1;
-    if (ensure_work<ActT>(e, std::max(T, TS_cap), n_dec)) return 1;
+    if (ensure_work<ActT>(e, cont ? T : std::max(T, TS_cap), n_dec)) return 1;
+    // continuous loop: tables, staging of an admitted batch, slot-major source tokens, encoder workspace
+    CbTable cbt{};
+    int* stage_drafts = nullptr;
+    int* stage_srclen = nullptr;
+    ActT* stage_kv = nullptr;
+    EncWork<ActT> enc_work{};
+    if (cont) {
+        TTB_CHECK((2 * E * sizeof(ActT)) % 16 == 0, "continuous batching needs 16-byte cross-attention K/V rows");
+        TTB_CHECK(B <= 2048, "continuous batching supports at most 2048 slots");
+        // the captured graphs bake the table addresses: their offsets depend on the slot count only (part of the graph
+        // key); the staging buffers of the call's batches come behind them
+        const size_t grp_off = ((size_t)3 * B * sizeof(int) + 255) / 256 * 256;
+        const size_t stage_off = grp_off + ((size_t)cb->n * sizeof(CbGroup) + 255) / 256 * 256;
+        const size_t kv_off = stage_off + (((size_t)2 * B_stage + (size_t)B_stage * N * D) * sizeof(int) + 255) / 256 * 256;
+        if (e->cb.ensure(kv_off + (size_t)n_dec * TS_stage * 2 * E * sizeof(ActT))) return 1;
+        if (e->keytok32.ensure((size_t)TS_cap * sizeof(int))) return 1;
+        if (e->cb_work.ensure(enc_work_bytes<ActT>(e, TS_stage))) return 1;
+        int* base = e->cb.as<int>();
+        cbt.slot_group = base; cbt.slot_q = base + B; cbt.adm_slots = base + 2 * B;
+        cbt.groups = reinterpret_cast<CbGroup*>(e->cb.as<char>() + grp_off);
+        stage_srclen = reinterpret_cast<int*>(e->cb.as<char>() + stage_off);
+        stage_drafts = stage_srclen + B_stage;
+        stage_kv = reinterpret_cast<ActT*>(e->cb.as<char>() + kv_off);
+        enc_work = enc_work_carve<ActT>(e, TS_stage, e->cb_work.p);
+    }
+    // nothing is allocated from here on: the captured graphs bake these addresses
+    const long long sig0 = e->alloc_signature();
 
     TTB_CUDA_OK(cudaEventRecord(e->t0, s));
     int* src32 = e->src32.as<int>();
+    float* mem = e->memory.as<float>();
+    ActT* memh = Prec<ActT>::lowp ? e->memh.as<ActT>() : nullptr;
+    ActT* crosskv = e->crosskv.as<ActT>();
+    GreedyState st{};
+    st.B = B; st.N = N; st.D = D; st.max_len = max_len; st.gen_ld = gen_ld; st.pad = pad; st.bos = bos; st.eos = eos; st.Ls = Ls;
+    st.gen = e->gen.as<int>(); st.front = e->front.as<int>(); st.active = e->active.as<int>(); st.ctrl = e->ctrl.as<int>();
+    st.drafts = e->drafts.as<int>(); st.pred = e->pred.as<int>(); st.out = cont ? nullptr : e->out64.as<long long>();
+    st.sel = e->sel.as<int>(); st.trace = cont ? nullptr : trace_dev; st.tie_break = tie_break; st.hist = e->hist.as<int>();
+    st.desc = e->desc.as<int4>(); st.src_len = e->srclen.as<int>();
+    // admission of batch i (continuous loop): encoder, cross K/V and drafts of the batch alone, as below for one batch,
+    // then the kernels that move it into free slots
+    auto admit = [&](int i) -> int {
+        const int Bi = cb->bs[i], Li = cb->ls[i];
+        const long long TSi = (long long)Bi * Li;
+        { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(cb->src[i]), src32, TSi, s); }
+        { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, Bi, Li, e->d.src_pad_token_idx, stage_srclen, s); }
+        if (encode_impl<ActT>(e, src32, src32, Bi, Li, mem, memh, s, &enc_work)) return 1;
+        if (cross_kv_impl<ActT>(e, mem, memh, (int)TSi, stage_kv, s, TS_stage * 2 * E)) return 1;
+        { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Li, Bi, Li - 1, D, N, eos, pad, replace, stage_drafts, s); }
+        {
+            Scope sc(e, KC_MISC, s);
+            launch_greedy_admit(st, cbt, i, Bi, stage_drafts, stage_srclen, reinterpret_cast<long long*>(cb->out[i]), cb->trace ? cb->trace[i] : nullptr,
+                                Ls_cap, s);
+        }
+        {
+            Scope sc(e, KC_MISC, s);
+            launch_greedy_admit_kv<ActT>(cbt, Bi, Li, Ls_cap, n_dec, E, stage_kv, TS_stage * 2 * E, crosskv, TS_cap * 2 * E, src32, e->keytok32.as<int>(),
+                                         e->d.src_pad_token_idx, s);
+        }
+        TTB_CUDA_OK(cudaGetLastError());
+        TTB_CHECK(e->alloc_signature() == sig0, "a workspace buffer moved while decoding graphs of the continuous loop exist");
+        return 0;
+    };
+    const long long vt_q_stride = (long long)E * VT_PITCH, vt_l_stride = (long long)B * E * VT_PITCH;
+    if (cont) {
+        TTB_CUDA_OK(cudaMemsetAsync(st.ctrl, 0, CTRL_COUNT * sizeof(int), s));
+    } else {
     { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(src_dev), src32, TS, s); }
     // per-query source length: the cross-attention kernels skip the padding behind it
     { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
-    float* mem = e->memory.as<float>();
-    ActT* memh = Prec<ActT>::lowp ? e->memh.as<ActT>() : nullptr;
     if (encode_impl<ActT>(e, src32, src32, B, Ls, mem, memh, s)) return 1;
-    ActT* crosskv = e->crosskv.as<ActT>();
     if (cross_kv_impl<ActT>(e, mem, memh, (int)TS, crosskv, s, TS_cap * 2 * E)) return 1;
-    const long long vt_q_stride = (long long)E * VT_PITCH, vt_l_stride = (long long)B * E * VT_PITCH;
     if constexpr (Prec<ActT>::lowp) {
         if (tc_attn) {
             // every position a product can touch must hold a finite number (masked keys get probability 0, and 0 x NaN = NaN)
@@ -662,14 +774,8 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     }
     // drafts from the source without its BOS column (speculative_decoding.py:64-73)
     if (!standard) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Ls, B, Ls - 1, D, N, eos, pad, replace, e->drafts.as<int>(), s); }
-
-    GreedyState st{};
-    st.B = B; st.N = N; st.D = D; st.max_len = max_len; st.gen_ld = gen_ld; st.pad = pad; st.bos = bos; st.eos = eos; st.Ls = Ls;
-    st.gen = e->gen.as<int>(); st.front = e->front.as<int>(); st.active = e->active.as<int>(); st.ctrl = e->ctrl.as<int>();
-    st.drafts = e->drafts.as<int>(); st.pred = e->pred.as<int>(); st.out = e->out64.as<long long>();
-    st.sel = e->sel.as<int>(); st.trace = trace_dev; st.tie_break = tie_break; st.hist = e->hist.as<int>();
-    st.desc = e->desc.as<int4>(); st.src_len = e->srclen.as<int>();
     { Scope sc(e, KC_MISC, s); launch_greedy_init(st, s); }
+    }
 
     float* x = e->x.as<float>();
     ActT* xh = Prec<ActT>::lowp ? e->xh.as<ActT>() : nullptr;
@@ -699,6 +805,11 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     };
     auto cross_attn = [&](int l, ActT* q2, ActT* att) {
         const ActT* kv = crosskv + (long long)l * TS_cap * 2 * E;
+        if (cont) {   // slot-major K/V rows and key tokens, row stride Ls_cap (= CTRL_LS) per slot
+            attn(q2, E, kv, kv + E, 2 * E, att, E, Bq, n_active, per_q, Ls_cap, Ls_cap, st.active, e->keytok32.as<int>(), Ls_cap,
+                 e->d.src_pad_token_idx, false, H, HD, s, st.ctrl + CTRL_LS, e->srclen.as<int>(), st.desc);
+            return;
+        }
         if constexpr (Prec<ActT>::lowp) {
             if (tc_attn) {
                 // the K/V rows of a query start at row query * Ls of the layer's block (the batch's own source length, read on the
@@ -737,14 +848,22 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
             if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, e->logits.as<float>(), V, rows, false, s)) return 1;
             { Scope sc(e, KC_ARGMAX, s); launch_argmax_rows(e->logits.as<float>(), V, V, st.pred, rows, s); }
         }
-        { Scope sc(e, KC_ACCEPT, s); if (standard) launch_greedy_std_step(st, s); else launch_greedy_accept(st, s); }
+        {
+            Scope sc(e, KC_ACCEPT, s);
+            if (standard) launch_greedy_std_step(st, s);
+            else if (cont) launch_greedy_accept_groups(st, cbt, s);
+            else launch_greedy_accept(st, s);
+        }
         return 0;
     };
 
     // One decoding iteration is a fixed kernel sequence on fixed buffers (all sizes that change while
     // decoding live in device memory), so it is captured once into a CUDA graph and replayed.
     static const bool no_graph = [] { const char* v = getenv("TTB_NO_GRAPH"); return v && v[0] == '1'; }();
-    const bool use_graph = !no_graph && !trace_dev && e->prof.mask == 0;
+    bool traced = trace_dev != nullptr;
+    if (cont && cb->trace)
+        for (int i = 0; i < cb->n; ++i) traced |= cb->trace[i] != nullptr;
+    const bool use_graph = !no_graph && !traced && e->prof.mask == 0;
     // Several iterations per graph: back-to-back graph launches of one stream leave the GPU idle for ~12 us (launch latency
     // plus the control-word copy in between), a graph edge costs ~2 us.  Iterations behind the end of the loop are no-ops
     // (every kernel reads a live count of zero), so a longer graph only adds a few of those per batch.
@@ -765,8 +884,8 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
         }
     }
     if (use_graph) {
-        const long long key[12] = {B, N, D, standard ? 1 : 0, max_len, pad, bos, eos, tie_break, e->alloc_signature(),
-                                   (long long)sizeof(ActT) + 16 * K_it + (tc_attn ? 1024 : 0), replace};
+        const long long key[13] = {B, N, D, standard ? 1 : (cont ? 2 : 0), max_len, pad, bos, eos, tie_break, e->alloc_signature(),
+                                   (long long)sizeof(ActT) + 16 * K_it + (tc_attn ? 1024 : 0), replace, cont ? Ls_cap : 0};
         if (memcmp(key, e->graph_key, sizeof(key)) != 0) {
             for (auto& gb : e->graph_exec) for (auto& g : gb) if (g) { cudaGraphExecDestroy(g); g = nullptr; }
             memcpy(e->graph_key, key, sizeof(key));
@@ -802,6 +921,89 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     // to `it` are already queued, so the GPU never waits for it.
     constexpr int RING = 4;
     const int LAG = K_it > 1 ? 1 : 2;   // launches (of K_it iterations each) the host stays ahead of the control words it reads
+    if (cont) {
+        // Continuous loop.  `bound` is an upper bound of the live slots of every iteration enqueued from now on: the count of
+        // the newest control words read plus every query admitted after the launch they belong to (the device only retires
+        // queries).  It picks the bucket -- a bucket below the true live count would drop queries -- and B - bound is a
+        // lower bound of the free slots: a batch is admitted at a graph boundary once they suffice.
+        long long admitted = 0, adm_at[RING] = {};
+        long long iters_enq = 0;
+        int next = 0, bound = 0, it = 0;
+        while (true) {
+            while (next < cb->n && B - bound >= cb->bs[next]) {
+                if (admit(next)) return 1;
+                bound += cb->bs[next];
+                admitted += cb->bs[next];
+                ++next;
+            }
+            if (bound == 0) break;   // nothing live and nothing pending (every batch fits the slots)
+            TTB_CHECK(iters_enq < max_iters, "continuous decoding loop did not terminate within max_len + 1 iterations per batch");
+            const int known_live = std::max(1, bound);
+            int bi = 0;
+            while (bi + 1 < n_buckets && bucket_q[bi + 1] >= known_live) ++bi;
+            Bq = bucket_q[bi];
+            if (use_graph) {
+                const int sh = (known_live < B && K_short < K_it) ? 1 : 0;
+                if (graph_for(bi, sh)) return 1;
+                TTB_CUDA_OK(cudaGraphLaunch(e->graph_exec[bi][sh], s));
+                e->launches += e->graph_launches * (sh ? K_short : K_it);
+                iters_enq += sh ? K_short : K_it;
+            } else if (enqueue_iteration()) {
+                return 1;
+            } else {
+                ++iters_enq;
+            }
+            TTB_CUDA_OK(cudaMemcpyAsync(e->h_ctrl + (it % RING) * CTRL_COUNT, st.ctrl, CTRL_COUNT * sizeof(int), cudaMemcpyDeviceToHost, s));
+            TTB_CUDA_OK(cudaEventRecord(e->poll_ev[it % RING], s));
+            adm_at[it % RING] = admitted;
+            if (it >= LAG) {
+                const int j = (it - LAG) % RING;
+                TTB_CUDA_OK(cudaEventSynchronize(e->poll_ev[j]));
+                const int* cj = e->h_ctrl + j * CTRL_COUNT;
+                TTB_CHECK(cj[CTRL_ERROR] != 3, "continuous batching admitted a batch without enough free slots");
+                const int live = cj[CTRL_DONE] ? 0 : cj[CTRL_N_ACTIVE];
+                bound = std::min(bound, live + (int)(admitted - adm_at[j]));
+            }
+            ++it;
+        }
+        TTB_CUDA_OK(cudaMemcpyAsync(e->h_ctrl, st.ctrl, CTRL_COUNT * sizeof(int), cudaMemcpyDeviceToHost, s));
+        TTB_CUDA_OK(cudaEventRecord(e->t1, s));
+        TTB_CUDA_OK(cudaStreamSynchronize(s));
+        TTB_CUDA_OK(cudaGetLastError());
+        prof_collect(e);
+        const int* c = e->h_ctrl;
+        TTB_CHECK(c[CTRL_ERROR] != 3, "continuous batching admitted a batch without enough free slots");
+        TTB_CHECK(c[CTRL_DONE] == 1 && c[CTRL_N_ACTIVE] == 0, "continuous decoding loop ended with live queries");
+        std::vector<CbGroup> groups((size_t)cb->n);
+        TTB_CUDA_OK(cudaMemcpy(groups.data(), cbt.groups, groups.size() * sizeof(CbGroup), cudaMemcpyDeviceToHost));
+        e->h_hist.assign((size_t)c[CTRL_ITERS], 0);
+        if (c[CTRL_ITERS] > 0)
+            TTB_CUDA_OK(cudaMemcpy(e->h_hist.data(), st.hist, (size_t)c[CTRL_ITERS] * sizeof(int), cudaMemcpyDeviceToHost));
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, e->t0, e->t1);
+        ttb_generate_stats sum{};
+        for (int i = 0; i < cb->n; ++i) {
+            const CbGroup& g = groups[(size_t)i];
+            TTB_CHECK(g.closed == 1 && g.B == cb->bs[i], "continuous decoding loop ended before every batch was finished");
+            ttb_generate_stats& o = cb->stats[i];
+            o = ttb_generate_stats{};
+            o.model_calls = g.iter;
+            o.accepted_tokens = g.accepted;
+            o.produced_tokens = g.tokens;
+            o.unfinished = g.n_left;
+            o.error = g.error == 1 ? TTB_ERR_REF_INDEX : (g.error == 2 ? TTB_ERR_REF_SHAPE : 0);
+            sum.accepted_tokens += g.accepted;
+            sum.produced_tokens += g.tokens;
+            sum.unfinished += g.n_left;
+        }
+        if (stats) {
+            sum.model_calls = c[CTRL_ITERS];
+            sum.gpu_launches = (int32_t)(e->launches - launches0);
+            sum.gpu_ms = ms;
+            *stats = sum;
+        }
+        return 0;
+    }
     int it = 0, iters_enq = 0;
     bool done = false;
     int known_live = B;                 // live queries in the newest control words read: an upper bound from then on
@@ -1482,7 +1684,8 @@ void ttb_engine_destroy(ttb_engine* e) {
     }
     DevBuf* bufs[] = {&e->x, &e->xh, &e->y, &e->qkv, &e->att, &e->q2, &e->hid, &e->logits, &e->tok32, &e->keytok32, &e->pred,
                       &e->src32, &e->memory, &e->memh, &e->crosskv, &e->kcache, &e->vcache, &e->drafts, &e->gen, &e->front,
-                      &e->active, &e->ctrl, &e->sel, &e->out64, &e->hist, &e->beam, &e->srclen, &e->desc, &e->kcache2, &e->vcache2, &e->crossvt};
+                      &e->active, &e->ctrl, &e->sel, &e->out64, &e->hist, &e->beam, &e->srclen, &e->desc, &e->kcache2, &e->vcache2, &e->crossvt,
+                      &e->cb, &e->cb_work};
     for (DevBuf* b : bufs) b->release();
     if (e->h_ctrl) cudaFreeHost(e->h_ctrl);
     for (auto& ev : e->poll_ev) if (ev) cudaEventDestroy(ev);
@@ -1646,6 +1849,37 @@ int ttb_greedy_speculative_generate(ttb_engine* e, const int64_t* src_dev, int32
                                              replace_token, tie_break, out_dev, trace_dev, stats, s),
                         greedy_api<__nv_bfloat16>(e, src_dev, B, Ls, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token,
                                                   replace_token, tie_break, out_dev, trace_dev, stats, s)));
+}
+
+int ttb_greedy_speculative_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs, const int32_t* batch_sizes,
+                                            const int32_t* src_lens, int32_t slots, int32_t max_len, int32_t draft_len, int32_t n_drafts,
+                                            int32_t pad_token, int32_t bos_token, int32_t eos_token, int32_t replace_token, int32_t tie_break,
+                                            int64_t* const* out_devs, int32_t* const* trace_devs, ttb_generate_stats* stats,
+                                            ttb_generate_stats* total, void* stream) {
+    TTB_CHECK(e && e->finalized, "engine not finalized");
+    TTB_CHECK(n_batches >= 0 && max_len > 1 && slots > 0, "bad arguments");
+    TTB_CHECK(n_batches == 0 || (src_devs && batch_sizes && src_lens && out_devs && stats), "bad arguments");
+    TTB_CHECK(n_drafts > 0, "The number of drafts must be greater than 0");
+    TTB_CHECK(pad_token != replace_token, "The pad token and the replace token must be different");
+    TTB_CHECK(eos_token != replace_token, "The eos token and the replace token must be different");
+    TTB_CHECK(eos_token != pad_token, "The eos token and the pad token must be different");
+    TTB_CHECK(max_len + draft_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
+    int Ls_max = 2;
+    for (int i = 0; i < n_batches; ++i) {
+        TTB_CHECK(src_devs[i] && out_devs[i] && batch_sizes[i] > 0 && src_lens[i] > 1, "bad arguments");
+        TTB_CHECK(batch_sizes[i] <= slots, "slots must be at least the largest batch size");
+        TTB_CHECK(src_lens[i] <= e->d.max_positions, "sequence longer than the positional table");
+        Ls_max = std::max(Ls_max, (int)src_lens[i]);
+    }
+    if (total) *total = ttb_generate_stats{};
+    if (n_batches == 0) return 0;
+    TTB_CUDA_OK(cudaSetDevice(e->device));
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const CbArgs cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, trace_devs, stats};
+    return drained(e, TTB_DISPATCH(e, greedy_api<float>(e, nullptr, slots, Ls_max, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token,
+                                                        replace_token, tie_break, nullptr, nullptr, total, s, false, &cb),
+                                   greedy_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token,
+                                                             replace_token, tie_break, nullptr, nullptr, total, s, false, &cb)));
 }
 
 int ttb_greedy_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len, int32_t pad_token,

@@ -162,6 +162,32 @@ void launch_greedy_accept(const GreedyState& st, cudaStream_t s);
 // standard greedy decoding (no drafts: N = 1, D = 0): appends the predicted token of every row, stop test
 void launch_greedy_std_step(const GreedyState& st, cudaStream_t s);
 
+// Continuous batching of the speculative loop (GreedyState::B = number of slots; every per-query array is per slot).
+// One record per batch: what the reference couples across the queries of a batch (width, stop, errors) plus its counters.
+struct CbGroup {
+    long long* out;    // [B][max_len] the batch's predictions
+    int* trace;        // optional [max_len + 1][B][4], rows indexed by the batch's own iteration and live position
+    int B, W;          // batch size; token-matrix width of the batch's coming iteration
+    int iter, live;    // decoder iterations the batch took part in; its live queries
+    int accepted, tokens, error, n_left, closed;   // counters; error 0 / 1 (splice index) / 2 (shape); unfinished queries
+    int reserved;
+};
+struct CbTable {
+    int* slot_group;   // [slots] batch of the query in the slot
+    int* slot_q;       // [slots] index of that query in its batch
+    int* adm_slots;    // [max batch size] slots given to the batch admitted last
+    CbGroup* groups;   // [n_batches]
+};
+// admission of batch `grp` between two iterations (drafts_in [Bi][N][D], srclen_in [Bi] computed for the batch alone)
+void launch_greedy_admit(const GreedyState& st, const CbTable& cb, int grp, int Bi, const int* drafts_in, const int* srclen_in, long long* out,
+                         int* trace, int Ls_cap, cudaStream_t s);
+// cross-attention K/V rows [layer][Bi * Ls][2E] and source tokens [Bi][Ls] of the batch admitted last -> its slots
+template <typename ActT>
+void launch_greedy_admit_kv(const CbTable& cb, int Bi, int Ls, int Ls_cap, int n_layers, int E, const ActT* stage_kv, long long stage_layer_stride,
+                            ActT* kv, long long layer_stride, const int* src32, int* keytok, int pad, cudaStream_t s);
+// accept kernel of the continuous loop: per-query step of launch_greedy_accept, per-batch retirement / width plan / closing
+void launch_greedy_accept_groups(const GreedyState& st, const CbTable& cb, cudaStream_t s);
+
 // ---- beam.cu --------------------------------------------------------------------------------------
 struct BeamState {
     int B, K, N, dl0, V, pad, bos, eos, ldw, tie_break;

@@ -8,11 +8,22 @@ GPU without a host round-trip per step; the host only polls a completion word.
 from __future__ import annotations
 
 import ctypes as C
+from typing import Callable, Sequence
 
 import torch
 
 from .. import _lib
 from ..model import B200Transformer
+
+# generate_batches(): default query slots per query of the largest batch.  Greedy bench workload (bs 32, trained-like
+# weights, 24 batches) on one B200 at 1000 W: 1908 SMILES/s one batch at a time; 1964 / 3221 / 3681 / 4151 / 4378 with
+# 32 / 48 / 64 / 96 / 128 slots (profiles/r3_continuous_copy.json, DESIGN.md section 10)
+DEFAULT_SLOTS_PER_BATCH = 4
+# messages of the reference failures a batch of generate_batches() can end with (as raised by generate())
+_REF_ERRORS = {
+    _lib.ERR_REF_INDEX: "index out of bounds while splicing drafts into the token matrix (reference scatter, speculative_decoding.py:111)",
+    _lib.ERR_REF_SHAPE: "shape mismatch: a finished row is wider than max_len (reference speculative_decoding.py:158)",
+}
 
 
 class TranslationInferenceGreedySpeculative:
@@ -64,14 +75,80 @@ class TranslationInferenceGreedySpeculative:
         self.gpu_launches += stats.gpu_launches
         self.gpu_ms += stats.gpu_ms
         if trace is not None:
-            t = trace[:stats.model_calls].cpu()
-            for it in range(t.shape[0]):
-                rows = t[it][t[it, :, 0] >= 0]
-                self.trace.append({"rows": rows[:, 0].tolist(), "n_accepted": rows[:, 1].tolist(),
-                                   "draft_index": rows[:, 2].tolist(), "width": int(rows[0, 3]) if len(rows) else 0})
+            self._append_trace(trace, stats.model_calls)
         _lib.check(rc, "ttb_greedy_speculative_generate")
         out = out.unsqueeze(1)
         return out if src.is_cuda else out.to(src.device)
+
+    def generate_batches(self, batches: Sequence[torch.Tensor], slots: int | None = None,
+                         on_error: Callable[[int, Exception], object] | None = None) -> list:
+        """Continuous batching: decode `batches` in ONE device loop whose `slots` query slots are refilled with the
+        queries of the next batch as soon as enough of them are free (batches are admitted in list order).
+
+        Returns `[self.generate(b) for b in batches]` bit for bit, and advances the counters and `trace` exactly as those
+        calls would: a batch keeps the width, stop and error rules of its own batch in the shared loop.  A reference
+        failure of batch i raises its RuntimeError when position i is reached, unless `on_error(i, exc)` is given,
+        whose return value then stands in for that batch's result (the contract of `InFlightDecoder.map`).
+        `slots` defaults to DEFAULT_SLOTS_PER_BATCH times the largest batch size."""
+        batches = list(batches)
+        if not batches:
+            return []
+        m = self.model
+        for b in batches:
+            if b.dim() != 2 or b.shape[0] < 1 or b.shape[1] < 2:
+                raise ValueError(f"every batch must be a (B >= 1, Ls >= 2) tensor of token ids, got shape {tuple(b.shape)}")
+        if len({b.device for b in batches}) != 1:
+            raise ValueError("all batches must be on the same device")
+        bmax = max(int(b.shape[0]) for b in batches)
+        if slots is None:
+            slots = DEFAULT_SLOTS_PER_BATCH * bmax
+        if slots < bmax:
+            raise ValueError(f"slots ({slots}) must be at least the largest batch size ({bmax})")
+        n = len(batches)
+        srcs = [b.to(device=m.device, dtype=torch.int64, non_blocking=True).contiguous() for b in batches]
+        outs = [torch.empty(s.shape[0], self.max_len, dtype=torch.int64, device=m.device) for s in srcs]
+        traces = None
+        if self.keep_trace:
+            traces = [torch.full((self.max_len + 1, s.shape[0], 4), -1, dtype=torch.int32, device=m.device) for s in srcs]
+        ptrs = lambda ts: (C.c_void_p * n)(*[t.data_ptr() for t in ts])
+        sizes = (C.c_int32 * n)(*[s.shape[0] for s in srcs])
+        lens = (C.c_int32 * n)(*[s.shape[1] for s in srcs])
+        stats = (_lib.GenerateStats * n)()
+        total = _lib.GenerateStats()
+        with torch.cuda.device(m.device):
+            rc = m.lib.ttb_greedy_speculative_generate_batches(
+                m._h, n, ptrs(srcs), sizes, lens, slots, self.max_len, self.draft_len, self.n_drafts, self.pad_token,
+                self.bos_token, self.eos_token, self.replace_token, self.tie_break, ptrs(outs),
+                ptrs(traces) if traces is not None else None, stats, C.byref(total),
+                torch.cuda.current_stream(m.device).cuda_stream)
+        _lib.check(rc, "ttb_greedy_speculative_generate_batches")
+        self.last_stats = total
+        self.gpu_launches += total.gpu_launches
+        self.gpu_ms += total.gpu_ms
+        results = []
+        for i in range(n):
+            st = stats[i]
+            self.model_calls_num += st.model_calls
+            self.accepted_tokens_num += st.accepted_tokens
+            self.produced_tokens_num += st.produced_tokens
+            if traces is not None:
+                self._append_trace(traces[i], st.model_calls)
+            if st.error:
+                exc = RuntimeError(_REF_ERRORS[st.error])
+                if on_error is None:
+                    raise exc
+                results.append(on_error(i, exc))
+                continue
+            out = outs[i].unsqueeze(1)
+            results.append(out if batches[i].is_cuda else out.to(batches[i].device))
+        return results
+
+    def _append_trace(self, trace: torch.Tensor, model_calls: int) -> None:
+        t = trace[:model_calls].cpu()
+        for it in range(t.shape[0]):
+            rows = t[it][t[it, :, 0] >= 0]
+            self.trace.append({"rows": rows[:, 0].tolist(), "n_accepted": rows[:, 1].tolist(),
+                               "draft_index": rows[:, 2].tolist(), "width": int(rows[0, 3]) if len(rows) else 0})
 
 
 class TranslationInferenceBeamSearchSpeculative:
