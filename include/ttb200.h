@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define TTB_ABI_VERSION 3
+#define TTB_ABI_VERSION 4
 
 #define TTB_PRECISION_FP32 0 /* fp32 FMA GEMMs, exact-parity path (1e-5 logits)            */
 #define TTB_PRECISION_BF16 1 /* tcgen05 bf16 GEMMs, fp32 accumulate (1e-2 logits)          */
@@ -141,6 +141,26 @@ int ttb_beam_speculative_generate(ttb_engine* e, const int64_t* src_dev, int32_t
                                   int32_t* out_width, int32_t* trace_nacc_dev, int32_t* trace_pick_dev, ttb_generate_stats* stats,
                                   void* stream);
 
+/* ---- continuous batching of speculative_decoding.py:422 generate(): n_batches independent batches share `slots` query
+ * slots of ONE device loop, each slot holding n_best candidate rows.  Batch i is admitted (in list order) between two
+ * iterations as soon as `batch_sizes[i]` slots are free; its queries keep the width / draft length / stop / error rules of
+ * their own batch, so out_devs[i], out_widths[i], the traces and stats[i] are exactly what ttb_beam_speculative_generate
+ * returns for that batch alone.  A reference failure of one batch (stats[i].error = TTB_ERR_REF_*) ends that batch only;
+ * the call returns 0 unless something else failed.  src_devs[i] is (batch_sizes[i], src_lens[i]) int64, out_devs[i] holds
+ * batch_sizes[i] * n_best * (max_len + clamp(draft_len,5,200) + 4) int64 and receives (batch_sizes[i], n_best,
+ * out_widths[i]) densely; trace_nacc_devs[i] / trace_pick_devs[i] are laid out as in ttb_beam_speculative_generate with
+ * B = batch_sizes[i] (the arrays may be NULL or hold NULL entries).  slots >= max(batch_sizes).  total (may be NULL):
+ * launches / ms of the call, model_calls = decoder iterations of the shared loop.  Needs the KV-cached decoder pass
+ * (TTB_BEAM_NO_CACHE unset); iterations are not replayed as graphs.  ttb_engine_get_history afterwards gives the query
+ * slots in use at every iteration. */
+int ttb_beam_speculative_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs,
+                                          const int32_t* batch_sizes, const int32_t* src_lens, int32_t slots, int32_t max_len,
+                                          int32_t n_best, int32_t draft_len, int32_t n_drafts, int32_t smart_drafts_mode,
+                                          int32_t pad_token, int32_t bos_token, int32_t eos_token, int32_t c_token, int32_t tie_break,
+                                          int64_t* const* out_devs, int32_t* out_widths, int32_t* const* trace_nacc_devs,
+                                          int32_t* const* trace_pick_devs, ttb_generate_stats* stats, ttb_generate_stats* total,
+                                          void* stream);
+
 /* ---- instrumentation (bench.py): per-kernel-class CUDA-event timing on the launching stream.
  * class_mask bit i enables class i (names via ttb_kernel_class_name); totals accumulate over
  * generate() calls until the next ttb_engine_set_profiling. */
@@ -148,8 +168,12 @@ int ttb_kernel_class_count(void);
 const char* ttb_kernel_class_name(int32_t id);
 int ttb_engine_set_profiling(ttb_engine* e, uint32_t class_mask);
 int ttb_engine_get_profile(ttb_engine* e, int32_t n_classes, double* ms_out, int64_t* launches_out);
-/* live queries at the start of every decoder iteration of the last generate(); returns their number */
+/* live queries at the start of every decoder iteration of the last generate() (continuous loops: query slots in use);
+ * returns their number */
 int ttb_engine_get_history(ttb_engine* e, int32_t* live_queries_out, int32_t capacity);
+/* last ttb_beam_speculative_generate_batches: per decoder iteration, the draft length the call ran at and the smallest
+ * draft length of the batches in it (smaller when a batch near max_len shares the call); returns the iteration count */
+int ttb_engine_get_draft_history(ttb_engine* e, int32_t* call_dl_out, int32_t* min_dl_out, int32_t capacity);
 
 /* Standalone GEMM entry used by the kernel unit tests and the roofline microbenchmark:
  * C[M,N] = A[M,K] * W[N,K]^T + bias (+ReLU).  precision selects the kernel; A/W are fp32 for

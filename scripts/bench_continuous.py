@@ -1,4 +1,4 @@
-"""Continuous batching vs. one batch at a time vs. engines in flight, on the greedy workload of bench.py.
+"""Continuous batching vs. one batch at a time vs. engines in flight, on the greedy, beam or retro workload of bench.py.
 
 Weights and batches are exactly the ones `bench.py --workload greedy` times (bench.Workload): product-prediction model,
 vocab 288, seed 1234, batches synthetic_sources(32, 288, seed=100003 + j), bs 32, draft_len 10, n_drafts 23,
@@ -11,6 +11,14 @@ Every leg's outputs must equal leg (a) tensor for tensor before any timing is re
 clock around work that ends in a device synchronise; every shape is warmed up first (graphs are captured lazily).
 
     python scripts/bench_continuous.py --weights copy --batches 24 --out profiles/continuous_copy.json
+
+--workload beam / retro runs the speculative beam searches of bench.py (configs[2]: bs 4, n_best 5; configs[3]: 6+6 layers,
+bs 8, n_best 10) with the same legs; their slot sweep and engine counts default to multiples of the batch size and to the
+12 engines bench.py keeps in flight for them, leg (d) is skipped unless --cont-inflight is given.  Every leg also records the
+device memory its engines hold after the run, and leg (b) the mean and maximum query slots in use per iteration; leg (a)
+of a beam search reports the bs slots it holds as `slots_held` (its generate() keeps no per-iteration history).
+
+    python scripts/bench_continuous.py --workload retro --weights copy --batches 48 --out profiles/r4_continuous_beam_retro.json
 """
 from __future__ import annotations
 
@@ -56,21 +64,31 @@ def timed(fn):
 
 def main():
     ap = argparse.ArgumentParser()
+    ap.add_argument("--workload", default="greedy", choices=["greedy", "beam", "retro"])
     ap.add_argument("--weights", default="copy", choices=["copy", "random"])
     ap.add_argument("--batches", type=int, default=24)
-    ap.add_argument("--slots", default="32,48,64,96,128")
-    ap.add_argument("--inflight", default="3,8")
-    ap.add_argument("--cont-inflight", default="2,4")
+    ap.add_argument("--slots", default=None, help="comma-separated slot counts (default greedy: 32,48,64,96,128; beam searches: 1,2,4,8,16 x bs)")
+    ap.add_argument("--inflight", default=None, help="engines in flight (default greedy: 3,8; beam searches: 12)")
+    ap.add_argument("--cont-inflight", default=None, help="continuous loops in flight (default greedy: 2,4; beam searches: none)")
     ap.add_argument("--out", required=True)
     a = ap.parse_args()
-    argv, sys.argv = sys.argv, ["bench.py", "--workload", "greedy", "--weights", a.weights]
+    greedy = a.workload == "greedy"
+    argv, sys.argv = sys.argv, ["bench.py", "--workload", a.workload, "--weights", a.weights]
     bargs = bench.parse()
     sys.argv = argv
-    wl = bench.Workload("greedy", a.weights, bargs)
+    wl = bench.Workload(a.workload, a.weights, bargs)
+    if a.slots is None:
+        a.slots = "32,48,64,96,128" if greedy else ",".join(str(k * wl.bs) for k in (1, 2, 4, 8, 16))
+    if a.inflight is None:
+        a.inflight = "3,8" if greedy else "12"
+    if a.cont_inflight is None:
+        a.cont_inflight = "2,4" if greedy else ""
     dev = torch.device("cuda", 0)
     batches = [wl.batch(j).to(dev) for j in range(a.batches)]
     n_smiles = sum(b.shape[0] for b in batches)
     res = {"workload": wl.describe(), "batches": a.batches, "bs": wl.bs, "weights": a.weights, **gpu_info()}
+    if not greedy:
+        res["n_best"] = wl.n_best
 
     def engine():
         return B200Transformer(wl.cfg, wl.sd, precision="bf16", device=0)
@@ -92,8 +110,12 @@ def main():
         gen0.generate(b)
         h += history(eng0)
     torch.cuda.synchronize()
-    res["a_sequential"] = {"smiles_per_s": n_smiles / t, "s": t, "mean_live": sum(h) / len(h), "max_live": max(h),
-                           "engine_bytes": free0 - torch.cuda.mem_get_info(0)[0]}
+    res["a_sequential"] = {"smiles_per_s": n_smiles / t, "s": t}
+    if greedy:
+        res["a_sequential"].update(mean_live=sum(h) / len(h), max_live=max(h))
+    else:   # generate() of the beam search keeps no per-iteration history: it holds its bs query slots throughout
+        res["a_sequential"]["slots_held"] = wl.bs
+    res["a_sequential"]["engine_bytes"] = free0 - torch.cuda.mem_get_info(0)[0]
 
     # (b) continuous, one engine per slots value (memory per engine then includes that slots value's workspace)
     res["b_continuous"] = []
@@ -117,13 +139,19 @@ def main():
 
     # (c) engines in flight
     res["c_in_flight"] = []
-    for k in [int(x) for x in a.inflight.split(",")]:
+    for k in [int(x) for x in a.inflight.split(",") if x]:
+        torch.cuda.synchronize()
+        free0 = torch.cuda.mem_get_info(0)[0]
         engs = [engine() for _ in range(k)]
         dec = InFlightDecoder([wl.generator(e) for e in engs], device=dev)
         list(dec.map(batches[:2 * k]))
         out, t = timed(lambda: list(dec.map(batches)))
         assert all(torch.equal(x, y) for x, y in zip(ref, out)), f"in-flight k={k} differs from generate()"
-        res["c_in_flight"].append({"engines": k, "smiles_per_s": n_smiles / t, "s": t})
+        torch.cuda.synchronize()
+        r = {"engines": k, "smiles_per_s": n_smiles / t, "s": t}
+        if not greedy:
+            r["engine_bytes"] = free0 - torch.cuda.mem_get_info(0)[0]
+        res["c_in_flight"].append(r)
         dec.close()
         for e in engs:
             e.close()
@@ -131,7 +159,7 @@ def main():
 
     # (d) continuous loops in flight: each engine decodes a contiguous share of the batches on its own stream
     res["d_continuous_in_flight"] = []
-    for k in [int(x) for x in a.cont_inflight.split(",")]:
+    for k in [int(x) for x in a.cont_inflight.split(",") if x]:
         engs = [engine() for _ in range(k)]
         gens = [wl.generator(e) for e in engs]
         streams = [torch.cuda.Stream(device=dev) for _ in range(k)]

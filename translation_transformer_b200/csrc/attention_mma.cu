@@ -195,8 +195,14 @@ __device__ __forceinline__ void process_block(const Tile<HD>& t, int kb, const u
     }
 }
 
-template <int HD>
-__global__ void __launch_bounds__(THREADS, 2)
+// GRP (speculative self-attention of the continuous beam-search loop): the draft rows of the call are p.row_len positions
+// long, but group g's own draft length gives it rows of desc[g].w positions.  The kernel then works on the group's compact
+// rows -- query tiles, key blocks and their columns exactly as a call with D + 1 = desc[g].w would lay them out -- and maps a
+// compact row r to the call's row (r / desc[g].w) * p.row_len + r % desc[g].w for its loads and stores.  So a group's
+// outputs do not depend on the draft length of the other groups in the call; the positions behind its own are not written.
+// (the row mapping needs a few more registers than two CTAs per SM leave: the GRP form runs one CTA per SM without spills)
+template <int HD, bool GRP>
+__global__ void __launch_bounds__(THREADS, GRP ? 1 : 2)
 attn_mma_kernel(Params p) {
     const int g = blockIdx.y, h = blockIdx.x;
     pdl_launch_dependents();
@@ -212,6 +218,11 @@ attn_mma_kernel(Params p) {
     const int dynLk = p.lk_dev ? *p.lk_dev : 0;
     const int n_groups_live = p.n_groups_dev ? *p.n_groups_dev : 0x7fffffff;
     if (g >= n_groups_live) return;
+    const int RLp = p.spec ? p.row_len : 1;                          // positions per draft row of the call
+    const int RL = GRP ? dsc.w : RLp;                                // ... of this group
+    const int Lq = GRP ? (p.Lq / p.row_len) * RL : p.Lq;             // query rows of this group (compact)
+    auto prow = [&](int r) { return GRP ? (r / RL) * RLp + r % RL : r; };
+    if (GRP && (int)blockIdx.z * ROWS_PER_CTA >= Lq) return;
     extern __shared__ __align__(16) uint8_t attn_smem[];
     constexpr int PITCH = Tile<HD>::PITCH;
     Tile<HD> tileA, tileB;
@@ -236,12 +247,12 @@ attn_mma_kernel(Params p) {
     {   // one block of ROWS_PER_CTA query rows per CTA (blockIdx.z): more, smaller CTAs balance the 148 SMs better
         const int blk0 = blockIdx.z * ROWS_PER_CTA;
         const int wrow0 = blk0 + warp * ROWS_PER_WARP;       // first query row of this warp
-        const bool warp_live = wrow0 < p.Lq;
-        const int wrow_last = min(p.Lq, wrow0 + ROWS_PER_WARP) - 1;
+        const bool warp_live = wrow0 < Lq;
+        const int wrow_last = min(Lq, wrow0 + ROWS_PER_WARP) - 1;
 
         // ---- staging (asynchronous; the Q fragments are fetched while the copies are in flight) ----
         // phase A window [j0, j0 + KTA): keys shared by the whole group
-        const int kA_end = p.causal ? min(Lk, min(p.Lq, blk0 + ROWS_PER_CTA)) : Lk;
+        const int kA_end = p.causal ? min(Lk, min(Lq, blk0 + ROWS_PER_CTA)) : Lk;
         // keys behind the last unmasked one (source padding) contribute exactly nothing: s_last_key bounds the scan
         __shared__ int s_last_key;
         if (threadIdx.x == 0) s_last_key = 0;
@@ -260,8 +271,7 @@ attn_mma_kernel(Params p) {
             if (last) atomicMax(&s_last_key, last);
         };
         // phase B window [u0, u0 + KTB): freshly projected keys of the draft rows this CTA's queries belong to
-        const int RL = p.spec ? p.row_len : 1;
-        const int endB = p.spec ? min(p.Lq, blk0 + ROWS_PER_CTA) : 0;
+        const int endB = p.spec ? min(Lq, blk0 + ROWS_PER_CTA) : 0;
         const int firstB = (blk0 / RL) * RL;   // start of the draft row that contains the CTA's first query
         const __nv_bfloat16* nkb = p.spec ? p.newk + (long long)g * p.Lq * p.new_ld + h * HD : nullptr;
         const __nv_bfloat16* nvb = p.spec ? p.newv + (long long)g * p.Lq * p.new_ld + h * HD : nullptr;
@@ -272,7 +282,24 @@ attn_mma_kernel(Params p) {
             const int nk = min(KTB, endB - u0);
             if (nk <= 0) return;
             const int nfill = fastB ? KTB : ((nk + 31) & ~31);
-            stage_rows<HD>(tileB, nkb + (long long)u0 * p.new_ld, nvb + (long long)u0 * p.new_ld, p.new_ld, nk, nfill);
+            if constexpr (GRP) {   // compact key row u0 + j lives in the call's row prow(u0 + j)
+                constexpr int CH = HD / 8;
+                for (int idx = threadIdx.x; idx < nfill * CH; idx += THREADS) {
+                    const int j = idx / CH, c = idx % CH;
+                    __nv_bfloat16* kd = tileB.k + j * PITCH + c * 8;
+                    __nv_bfloat16* vd = tileB.v + j * PITCH + c * 8;
+                    if (j < nk) {
+                        const long long r = (long long)prow(u0 + j) * p.new_ld + c * 8;
+                        cp_async16(kd, nkb + r);
+                        cp_async16(vd, nvb + r);
+                    } else {
+                        *reinterpret_cast<uint4*>(kd) = make_uint4(0, 0, 0, 0);
+                        *reinterpret_cast<uint4*>(vd) = make_uint4(0, 0, 0, 0);
+                    }
+                }
+            } else {
+                stage_rows<HD>(tileB, nkb + (long long)u0 * p.new_ld, nvb + (long long)u0 * p.new_ld, p.new_ld, nk, nfill);
+            }
             for (int j = threadIdx.x; j < nfill; j += THREADS) {
                 const bool bad = j >= nk || (first_new_masked && ((u0 + j) % RL) == 0);
                 tileB.bias[j] = bad ? -INFINITY : 0.f;
@@ -300,15 +327,15 @@ attn_mma_kernel(Params p) {
 #pragma unroll
             for (int nd = 0; nd < HD / 8; ++nd) o[mt][nd][0] = o[mt][nd][1] = o[mt][nd][2] = o[mt][nd][3] = 0.f;
             const int rowA = wrow0 + mt * 16 + rA, rowB = rowA + 8;
-            const __nv_bfloat16* qA = p.q + ((long long)g * p.Lq + rowA) * p.q_ld + h * HD;
-            const __nv_bfloat16* qB = p.q + ((long long)g * p.Lq + rowB) * p.q_ld + h * HD;
+            const __nv_bfloat16* qA = p.q + ((long long)g * p.Lq + prow(rowA)) * p.q_ld + h * HD;
+            const __nv_bfloat16* qB = p.q + ((long long)g * p.Lq + prow(rowB)) * p.q_ld + h * HD;
 #pragma unroll
             for (int ks = 0; ks < HD / 16; ++ks) {
                 const int d = ks * 16 + c0;
-                qa[mt][ks][0] = rowA < p.Lq ? *reinterpret_cast<const uint32_t*>(qA + d) : 0u;
-                qa[mt][ks][1] = rowB < p.Lq ? *reinterpret_cast<const uint32_t*>(qB + d) : 0u;
-                qa[mt][ks][2] = rowA < p.Lq ? *reinterpret_cast<const uint32_t*>(qA + d + 8) : 0u;
-                qa[mt][ks][3] = rowB < p.Lq ? *reinterpret_cast<const uint32_t*>(qB + d + 8) : 0u;
+                qa[mt][ks][0] = rowA < Lq ? *reinterpret_cast<const uint32_t*>(qA + d) : 0u;
+                qa[mt][ks][1] = rowB < Lq ? *reinterpret_cast<const uint32_t*>(qB + d) : 0u;
+                qa[mt][ks][2] = rowA < Lq ? *reinterpret_cast<const uint32_t*>(qA + d + 8) : 0u;
+                qa[mt][ks][3] = rowB < Lq ? *reinterpret_cast<const uint32_t*>(qB + d + 8) : 0u;
             }
         }
         cp_async_wait_all();
@@ -350,7 +377,7 @@ attn_mma_kernel(Params p) {
 #pragma unroll
                 for (int mt = 0; mt < 2; ++mt) {
                     const int row0 = wrow0 + mt * 16;
-                    if (row0 >= p.Lq) continue;
+                    if (row0 >= Lq) continue;
                     const int kstart = (row0 / RL) * RL;      // first key row the tile can see
                     const int rowA = row0 + rA;
                     const int startA = (rowA / RL) * RL, startB = ((rowA + 8) / RL) * RL;
@@ -363,7 +390,7 @@ attn_mma_kernel(Params p) {
             }
         } else if (p.spec) {
             const int lo = warp_live ? (wrow0 / RL) * RL : 0;
-            const int hi = warp_live ? min(p.Lq, (wrow_last / RL + 1) * RL) : 0;
+            const int hi = warp_live ? min(Lq, (wrow_last / RL + 1) * RL) : 0;
             for (int u0 = firstB; u0 < endB; u0 += KTB) {
                 if (u0 > firstB) {
                     __syncthreads();
@@ -405,14 +432,14 @@ attn_mma_kernel(Params p) {
                 const float nanv = __int_as_float(0x7fc00000);
                 const float iA = 1.0f / lA, iB = 1.0f / lB;
                 const int rowA = wrow0 + mt * 16 + rA, rowB = rowA + 8;
-                __nv_bfloat16* oA = p.out + ((long long)g * p.Lq + rowA) * p.out_ld + h * HD;
-                __nv_bfloat16* oB = p.out + ((long long)g * p.Lq + rowB) * p.out_ld + h * HD;
+                __nv_bfloat16* oA = p.out + ((long long)g * p.Lq + prow(rowA)) * p.out_ld + h * HD;
+                __nv_bfloat16* oB = p.out + ((long long)g * p.Lq + prow(rowB)) * p.out_ld + h * HD;
 #pragma unroll
                 for (int nd = 0; nd < HD / 8; ++nd) {
                     const int d = nd * 8 + c0;
-                    if (rowA < p.Lq)
+                    if (rowA < Lq)
                         *reinterpret_cast<uint32_t*>(oA + d) = lA == 0.f ? pack_bf16(nanv, nanv) : pack_bf16(o[mt][nd][0] * iA, o[mt][nd][1] * iA);
-                    if (rowB < p.Lq)
+                    if (rowB < Lq)
                         *reinterpret_cast<uint32_t*>(oB + d) = lB == 0.f ? pack_bf16(nanv, nanv) : pack_bf16(o[mt][nd][2] * iB, o[mt][nd][3] * iB);
                 }
             }
@@ -420,11 +447,12 @@ attn_mma_kernel(Params p) {
     }
 }
 
+template <bool GRP>
 static void launch(const Params& p, int heads, int head_dim, int n_groups_max, cudaStream_t s) {
     dim3 grid(heads, n_groups_max, (p.Lq + ROWS_PER_CTA - 1) / ROWS_PER_CTA);
-    if (head_dim == 16) { if (!ensure_dyn_smem(attn_mma_kernel<16>, (int)smem_bytes<16>())) launch_pdl(attn_mma_kernel<16>, grid, dim3(THREADS), smem_bytes<16>(), s, p); }
-    else if (head_dim == 32) { if (!ensure_dyn_smem(attn_mma_kernel<32>, (int)smem_bytes<32>())) launch_pdl(attn_mma_kernel<32>, grid, dim3(THREADS), smem_bytes<32>(), s, p); }
-    else if (head_dim == 64) { if (!ensure_dyn_smem(attn_mma_kernel<64>, (int)smem_bytes<64>())) launch_pdl(attn_mma_kernel<64>, grid, dim3(THREADS), smem_bytes<64>(), s, p); }
+    if (head_dim == 16) { if (!ensure_dyn_smem(attn_mma_kernel<16, GRP>, (int)smem_bytes<16>())) launch_pdl(attn_mma_kernel<16, GRP>, grid, dim3(THREADS), smem_bytes<16>(), s, p); }
+    else if (head_dim == 32) { if (!ensure_dyn_smem(attn_mma_kernel<32, GRP>, (int)smem_bytes<32>())) launch_pdl(attn_mma_kernel<32, GRP>, grid, dim3(THREADS), smem_bytes<32>(), s, p); }
+    else if (head_dim == 64) { if (!ensure_dyn_smem(attn_mma_kernel<64, GRP>, (int)smem_bytes<64>())) launch_pdl(attn_mma_kernel<64, GRP>, grid, dim3(THREADS), smem_bytes<64>(), s, p); }
 }
 }  // namespace amma
 
@@ -443,14 +471,14 @@ void launch_attention_mma(const __nv_bfloat16* q, int q_ld, const __nv_bfloat16*
     p.key_tok = key_tok; p.key_tok_stride = key_tok_stride; p.pad_id = pad_id; p.causal = causal ? 1 : 0;
     p.scale_log2e = 1.4426950408889634f / sqrtf((float)head_dim);
     p.spec = 0;
-    amma::launch(p, heads, head_dim, n_groups_max, s);
+    amma::launch<false>(p, heads, head_dim, n_groups_max, s);
 }
 
 void launch_spec_self_attention_mma(const __nv_bfloat16* qkv, int qkv_ld, const __nv_bfloat16* kcache, const __nv_bfloat16* vcache,
                                     long long cache_query_stride, int cache_ld, __nv_bfloat16* out, int out_ld,
                                     int B_max, const int* n_active_dev, const int* active, const int* front,
                                     const int* gen, int gen_ld, int pad_id, int N, int D,
-                                    int heads, int head_dim, cudaStream_t s, const int4* desc) {
+                                    int heads, int head_dim, cudaStream_t s, const int4* desc, bool group_row_len) {
     if (B_max <= 0) return;
     const int E = heads * head_dim;
     amma::Params p{};
@@ -462,7 +490,8 @@ void launch_spec_self_attention_mma(const __nv_bfloat16* qkv, int qkv_ld, const 
     p.scale_log2e = 1.4426950408889634f / sqrtf((float)head_dim);
     p.spec = 1; p.active = active; p.front = front; p.gen = gen; p.gen_ld = gen_ld;
     p.newk = qkv + E; p.newv = qkv + 2 * E; p.new_ld = qkv_ld; p.row_len = D + 1;
-    amma::launch(p, heads, head_dim, B_max, s);
+    if (group_row_len && desc) amma::launch<true>(p, heads, head_dim, B_max, s);
+    else amma::launch<false>(p, heads, head_dim, B_max, s);
 }
 
 }  // namespace ttb

@@ -369,21 +369,17 @@ void launch_beam_stats(const BeamState& st, const float* logits, int max_rows, i
 // One CTA per candidate.  "Is draft token a of draft n inside the truncated support of its position?" is evaluated for all
 // (draft, position) pairs in parallel (two dependent global loads each instead of a chain of up to 2 dl per draft); the
 // accepted length of a draft is the length of its leading run of hits.
-__global__ void __launch_bounds__(256) beam_choose_kernel(BeamState st, int C, int beam, int dl, int par) {
-    pdl_wait();   // launched with the programmatic attribute: scheduled while the predecessor drains, starts when it is complete
-    if (st.ctrl[BCX_DONE]) return;   // no-op iteration behind the end of the loop
-    const int iter = st.ctrl[BCX_ITER];
-    const int c = blockIdx.x;
-    __shared__ int s_nacc[64];
-    extern __shared__ unsigned char s_hit[];                 // [m][dl] when par
-    if (c >= C) return;
-    const int q = c / beam, N = st.N, K = st.K;
+// Per-candidate body, shared by the kernel of one batch and the one of the continuous loop: `dl` is the draft length of the
+// candidate's batch, `rs` the scored positions per decoder row of the iteration (dl + 1, or more in the continuous loop),
+// `lmax` the length the tie-break emulation pads to, tr_nacc / tr_pick the candidate's trace entries (or nullptr).
+__device__ __forceinline__ void choose_candidate(const BeamState& st, int c, int q, int dl, int rs, int lmax, int par, unsigned char* s_hit,
+                                                 int* s_nacc, int* tr_nacc, int* tr_pick) {
+    const int N = st.N, K = st.K;
     const bool fin = st.c_fin[c] != 0;
     const int m = cand_n_drafts(st, c);                      // drafts of this candidate
-    const int lmax = st.smart ? st.ctrl[BC_LMAX] : N;        // ragged groups are padded with -1 up to the longest (:206-223)
     const int rb = st.c_rowbase[c];
     auto hit = [&](int n, int a) -> bool {
-        const long long rp = (long long)(rb + n) * (dl + 1) + a;
+        const long long rp = (long long)(rb + n) * rs + a;
         const int keep = st.nkeep[rp];
         const int* ti = st.topi + rp * K;
         const int tok = cand_draft(st, c, q, n)[a];
@@ -406,7 +402,7 @@ __global__ void __launch_bounds__(256) beam_choose_kernel(BeamState st, int C, i
         }
         st.c_nacc[(long long)c * N + n] = a;
         if (n < 64) s_nacc[n] = a;
-        if (st.trace_nacc) st.trace_nacc[((long long)iter * st.B * K + c) * N + n] = a;
+        if (tr_nacc) tr_nacc[n] = a;
     }
     __syncthreads();
     if (threadIdx.x == 0) {
@@ -417,8 +413,21 @@ __global__ void __launch_bounds__(256) beam_choose_kernel(BeamState st, int C, i
             for (int n = 1; n < m; ++n) if (st.c_nacc[(long long)c * N + n] > st.c_nacc[(long long)c * N + pick]) pick = n;
         }
         st.c_pick[c] = pick;
-        if (st.trace_pick) st.trace_pick[(long long)iter * st.B * K + c] = pick;
+        if (tr_pick) *tr_pick = pick;
     }
+}
+__global__ void __launch_bounds__(256) beam_choose_kernel(BeamState st, int C, int beam, int dl, int par) {
+    pdl_wait();   // launched with the programmatic attribute: scheduled while the predecessor drains, starts when it is complete
+    if (st.ctrl[BCX_DONE]) return;   // no-op iteration behind the end of the loop
+    const int iter = st.ctrl[BCX_ITER];
+    const int c = blockIdx.x;
+    __shared__ int s_nacc[64];
+    extern __shared__ unsigned char s_hit[];                 // [m][dl] when par
+    if (c >= C) return;
+    const int lmax = st.smart ? st.ctrl[BC_LMAX] : st.N;     // ragged groups are padded with -1 up to the longest (:206-223)
+    const long long tr = (long long)iter * st.B * st.K + c;
+    choose_candidate(st, c, c / beam, dl, dl + 1, lmax, par, s_hit, s_nacc, st.trace_nacc ? st.trace_nacc + tr * st.N : nullptr,
+                     st.trace_pick ? st.trace_pick + tr : nullptr);
 }
 void launch_beam_choose(const BeamState& st, int C, int beam, int dl, cudaStream_t s) {
     const size_t smem = (size_t)st.N * (dl > 0 ? dl : 1);
@@ -431,16 +440,20 @@ void launch_beam_choose(const BeamState& st, int C, int beam, int dl, cudaStream
 // log softmax exactly as the reference evaluates it: log(exp(x - max) / sum)   (:378)
 __device__ __forceinline__ float ref_logprob(float logit, float mx, float sum) { return logf(expf(logit - mx) / sum); }
 
-__global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam, int dl, const float* __restrict__ logits) {
-    pdl_wait();   // launched with the programmatic attribute: scheduled while the predecessor drains, starts when it is complete
-    if (st.ctrl[BCX_DONE]) return;   // no-op iteration behind the end of the loop (the word of the last real iteration stays posted)
+// Per-query body, shared by the kernel of one batch and the one of the continuous loop: scores the leaves of the
+// continuation trees of the `beam` candidates q * beam .. of query q (draft length dl of its batch, rs scored positions per
+// decoder row, token-matrix width W), keeps the K best and writes them as the query's next candidates.  A candidate with
+// c_fin == 2 is absent (continuous loop: a query's first iteration has one candidate): it has no leaves.  `err` receives
+// error 4, `out` (optional) the new hypotheses at width W; `tally(k, fin, p, pads, has_eos)` feeds the loop control.
+template <typename Tally>
+__device__ __forceinline__ void expand_query(const BeamState& st, int q, int beam, int dl, int rs, int W, const float* __restrict__ logits,
+                                             int* err, long long* out, Tally tally) {
     extern __shared__ float s_score[];                 // [beam][(dl+1)][K] leaf scores, -inf when absent
     __shared__ float s_red_v[256];
     __shared__ int s_red_i[256];
     __shared__ int s_sel[64];
     __shared__ int s_valid;
-    const int q = blockIdx.x, K = st.K, V = st.V, N = st.N;
-    const int W = st.ctrl[BCX_W];                      // rewritten only by the CTA that closes the iteration, after every CTA has arrived
+    const int K = st.K, V = st.V, N = st.N;
     const int per_c = (dl + 1) * K, total = beam * per_c;
     float* s_pre = s_score + total;                    // [beam][dl+2] running log-prob of the accepted path
     if (threadIdx.x == 0) s_valid = 0;
@@ -457,7 +470,7 @@ __global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam
             for (int i0 = 0; i0 < a; i0 += 32) {
                 float term = 0.f;
                 if (i0 + lane < a) {
-                    const long long rp = (long long)r * (dl + 1) + i0 + lane;
+                    const long long rp = (long long)r * rs + i0 + lane;
                     term = ref_logprob(st.tokv ? st.tokv[rp] : logits[rp * V + dr[i0 + lane]], st.lmax[rp], st.lsum[rp]);
                 }
                 const int cnt = min(32, a - i0);
@@ -473,15 +486,18 @@ __global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam
     for (int L = threadIdx.x; L < total; L += blockDim.x) {
         const int cb = L / per_c, p = (L % per_c) / K, j = L % K;
         const int c = q * beam + cb;
+        const int cf = st.c_fin[c];
         float score = -INFINITY;
-        if (st.c_fin[c]) {
+        if (cf == 2) {
+            // absent candidate: no leaves
+        } else if (cf) {
             // finished candidate: the artificial distribution leaves exactly one leaf, PAD at position 0,
             // with log-probability log(1) = 0
             if (p == 0 && j == 0) score = st.logp_cur[c] + 0.f;
         } else {
             const int n = st.c_pick[c], a = st.c_nacc[(long long)c * N + n], r = st.c_rowbase[c] + n;
             if (p <= a) {
-                const long long rp = (long long)r * (dl + 1) + p;
+                const long long rp = (long long)r * rs + p;
                 const int tok = st.topi[rp * K + j];
                 const float lg = st.topv[rp * K + j];
                 const int* dr = cand_draft(st, c, q, n);
@@ -498,7 +514,7 @@ __global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam
     if (my_valid) atomicAdd(&s_valid, my_valid);
     __syncthreads();
     const bool ok = s_valid >= K;
-    if (!ok && threadIdx.x == 0) atomicExch(&st.ctrl[BC_ERROR], 4);   // reference: assert min(group length) >= k (:195)
+    if (!ok && threadIdx.x == 0) atomicExch(err, 4);   // reference: assert min(group length) >= k (:195)
     for (int k = 0; ok && k < K; ++k) {                // K rounds of block-wide argmax (ties: lower leaf index)
         float bv = -INFINITY;
         int bi = 0x7fffffff;
@@ -539,12 +555,13 @@ __global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam
         const int c = q * beam + cb;
         const int* src = st.cand_cur + (long long)c * st.ldw;
         int* dst = st.cand_next + (long long)(q * K + k) * st.ldw;
+        long long* o_row = out ? out + (long long)k * W : nullptr;
         const int slot0 = st.c_slot0[c];
         const bool fin = st.c_fin[c] != 0;
         int n = 0, r = 0;
         if (!fin) { n = st.c_pick[c]; r = st.c_rowbase[c] + n; }
         const int* dr = fin ? st.drafts : cand_draft(st, c, q, n);
-        const int tok = fin ? st.pad : st.topi[((long long)r * (dl + 1) + p) * K + j];
+        const int tok = fin ? st.pad : st.topi[((long long)r * rs + p) * K + j];
         int pads = 0, has_eos = 0;
         for (int col = lane; col < W; col += 32) {
             int t = src[col];
@@ -553,6 +570,7 @@ __global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam
                 t = o < p ? dr[o] : (o == p ? tok : st.pad);
             }
             dst[col] = t;
+            if (o_row) o_row[col] = t;
             pads += t == st.pad;
             has_eos |= t == st.eos;
         }
@@ -566,11 +584,22 @@ __global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam
             st.n_parent[q * K + k] = fin ? -1 : c;
             st.n_keep[q * K + k] = p;
             st.n_row[q * K + k] = r;
-            if (!has_eos) { atomicAnd(&st.ctrl[BCX_ALL_FIN], 0); atomicAdd(&st.ctrl[BCX_NLIVE_NEXT], 1); }
-            atomicMin(&st.ctrl[BCX_MIN_PAD], pads);
-            if (!fin) { atomicAdd(&st.ctrl[BCX_ACC], p); atomicAdd(&st.ctrl[BCX_CNT], 1); }
+            tally(k, fin, p, pads, has_eos);
         }
     }
+}
+
+__global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam, int dl, const float* __restrict__ logits) {
+    pdl_wait();   // launched with the programmatic attribute: scheduled while the predecessor drains, starts when it is complete
+    if (st.ctrl[BCX_DONE]) return;   // no-op iteration behind the end of the loop (the word of the last real iteration stays posted)
+    const int q = blockIdx.x;
+    const int W = st.ctrl[BCX_W];                      // rewritten only by the CTA that closes the iteration, after every CTA has arrived
+    int* ctrl = st.ctrl;
+    expand_query(st, q, beam, dl, dl + 1, W, logits, &st.ctrl[BC_ERROR], nullptr, [ctrl](int, bool fin, int p, int pads, int has_eos) {
+        if (!has_eos) { atomicAnd(&ctrl[BCX_ALL_FIN], 0); atomicAdd(&ctrl[BCX_NLIVE_NEXT], 1); }
+        atomicMin(&ctrl[BCX_MIN_PAD], pads);
+        if (!fin) { atomicAdd(&ctrl[BCX_ACC], p); atomicAdd(&ctrl[BCX_CNT], 1); }
+    });
     // ---- loop control: the CTA that arrives last publishes the control words of the iteration (also into the pinned
     // host mirror, sequence number last) and resets the accumulators
     __syncthreads();
@@ -616,6 +645,316 @@ void launch_beam_expand(const BeamState& st, int beam, int dl, const float* logi
     const size_t smem = ((size_t)beam * (dl + 1) * st.K + (size_t)beam * (dl + 2)) * sizeof(float);
     if (ensure_dyn_smem(beam_expand_kernel, (int)smem)) return;   // error recorded; the launch below fails and cudaGetLastError reports it
     launch_pdl(beam_expand_kernel, dim3(st.B), dim3(256), smem, s, st, beam, dl, logits);
+}
+
+// ---- continuous batching: several batches share the query slots of one loop ----------------------------------------
+// Slot b holds query cb.slot_q[b] of batch cb.slot_group[b] (-1: free) and candidates b K .. b K + K - 1.  A batch keeps
+// in its BcGroup what the reference couples across the queries of a batch: token-matrix width, draft length, iteration,
+// the smart-mode padding length, counters, error and stop rule.  Every decoder call runs at the largest draft length of
+// the open batches; a batch with a shorter one ignores the extra scored positions (the self-attention over the step
+// positions is causal, so its own positions do not see them).  In a query's first iteration only candidate 0 exists (the
+// reference starts from one BOS candidate per query): its other candidates are absent (c_fin = 2), with no rows and no
+// leaves, so the leaf indices and their tie order are those of generate().
+// Loop-level words behind the BCX_* ones: query slots in use; largest draft length of the open batches for the coming
+// iteration; set when an admission found too few free slots (host bookkeeping broken)
+constexpr int BCC_USED = BC_COUNT + 9, BCC_DLMAX = BC_COUNT + 10, BCC_ADM_ERR = BC_COUNT + 11;
+
+// exclusive prefix sums of (a, b) over the threads of the block (blockDim.x a multiple of 32); totals in ta, tb
+__device__ __forceinline__ void block_scan2(int a, int b, int& ea, int& eb, int& ta, int& tb) {
+    __shared__ int s_a[32], s_b[32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    int ia = a, ib = b;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int x = __shfl_up_sync(0xffffffffu, ia, o), y = __shfl_up_sync(0xffffffffu, ib, o);
+        if (lane >= o) { ia += x; ib += y; }
+    }
+    if (lane == 31) { s_a[warp] = ia; s_b[warp] = ib; }
+    __syncthreads();
+    if (warp == 0) {
+        int va = lane < nw ? s_a[lane] : 0, vb = lane < nw ? s_b[lane] : 0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int x = __shfl_up_sync(0xffffffffu, va, o), y = __shfl_up_sync(0xffffffffu, vb, o);
+            if (lane >= o) { va += x; vb += y; }
+        }
+        s_a[lane] = va; s_b[lane] = vb;
+    }
+    __syncthreads();
+    ea = (warp ? s_a[warp - 1] : 0) + ia - a;
+    eb = (warp ? s_b[warp - 1] : 0) + ib - b;
+    ta = s_a[nw - 1];
+    tb = s_b[nw - 1];
+    __syncthreads();
+}
+
+// Admission of batch `grp` (Bi queries) into the first Bi free slots: hypotheses (BOS candidate), scores, drafts or the
+// window library (lib_in windows per query in drafts_in), source lengths and the batch's record.  One CTA, between two
+// iterations.
+__global__ void __launch_bounds__(1024) beam_admit_kernel(BeamState st, BcTable cb, int grp, int Bi, const int* __restrict__ drafts_in, int lib_in,
+                                                          const int* __restrict__ tok_cnt_in, const int* __restrict__ tok_list_in,
+                                                          const int* __restrict__ srclen_in, long long* out, int* trace_nacc, int* trace_pick, int dl_first) {
+    extern __shared__ int s_slots[];   // [Bi] slots taken, in batch order
+    __shared__ int s_nfree;
+    const int S = st.B, K = st.K, N = st.N, V = st.V, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    if (warp == 0) {
+        int taken = 0;
+        for (int i0 = 0; i0 < S && taken < Bi; i0 += 32) {
+            const int i = i0 + lane;
+            const bool fr = i < S && cb.slot_group[i] < 0;
+            const unsigned m = __ballot_sync(0xffffffffu, fr);
+            const int pos = taken + __popc(m & ((1u << lane) - 1u));
+            if (fr && pos < Bi) s_slots[pos] = i;
+            taken += __popc(m);
+        }
+        if (lane == 0) s_nfree = taken;
+    }
+    __syncthreads();
+    if (s_nfree < Bi) {
+        if (threadIdx.x == 0) st.ctrl[BCC_ADM_ERR] = 1;
+        return;
+    }
+    for (int j = threadIdx.x; j < Bi; j += blockDim.x) {
+        const int b = s_slots[j];
+        cb.adm_slots[j] = b;
+        cb.slot_group[b] = grp;
+        cb.slot_q[b] = j;
+        const_cast<int*>(st.src_len)[b] = srclen_in[j];
+    }
+    // both hypothesis buffers (the coming iteration reads one of them and writes the other): BOS row for candidate 0
+    const long long per_slot = (long long)K * st.ldw;
+    for (long long idx = threadIdx.x; idx < (long long)Bi * per_slot; idx += blockDim.x) {
+        const int j = (int)(idx / per_slot);
+        const long long r = idx % per_slot;
+        const int v = r == 0 ? st.bos : st.pad;
+        st.cand_cur[s_slots[j] * per_slot + r] = v;
+        st.cand_next[s_slots[j] * per_slot + r] = v;
+    }
+    for (int idx = threadIdx.x; idx < Bi * K; idx += blockDim.x) {
+        const int c = s_slots[idx / K] * K + idx % K;
+        st.logp_cur[c] = 0.f;
+        st.logp_next[c] = 0.f;
+    }
+    int* drafts = const_cast<int*>(st.drafts);
+    const long long per_in = (long long)(st.smart ? lib_in : N) * st.dl0, per_q = (long long)(st.smart ? st.n_lib : N) * st.dl0;
+    for (long long idx = threadIdx.x; idx < (long long)Bi * per_in; idx += blockDim.x)
+        drafts[s_slots[idx / per_in] * per_q + idx % per_in] = drafts_in[idx];
+    if (st.smart) {
+        for (long long idx = threadIdx.x; idx < (long long)Bi * V; idx += blockDim.x) st.tok_cnt[(long long)s_slots[idx / V] * V + idx % V] = tok_cnt_in[idx];
+        const long long per_l = (long long)V * N;
+        for (long long idx = threadIdx.x; idx < (long long)Bi * per_l; idx += blockDim.x)
+            st.tok_list[s_slots[idx / per_l] * per_l + idx % per_l] = tok_list_in[idx];
+    }
+    if (threadIdx.x == 0) {
+        BcGroup g{};
+        g.out = out; g.trace_nacc = trace_nacc; g.trace_pick = trace_pick;
+        g.B = Bi; g.W = st.w0; g.dl = dl_first;
+        g.all_fin = 1; g.min_pad = 0x7fffffff;
+        cb.groups[grp] = g;
+        st.ctrl[BCC_USED] += Bi;
+    }
+}
+void launch_beam_admit(const BeamState& st, const BcTable& cb, int grp, int Bi, const int* drafts_in, int lib_in, const int* tok_cnt_in,
+                       const int* tok_list_in, const int* srclen_in, long long* out, int* trace_nacc, int* trace_pick, int dl_first, cudaStream_t s) {
+    const size_t smem = (size_t)Bi * sizeof(int);
+    if (ensure_dyn_smem(beam_admit_kernel, (int)smem)) return;   // the launch below then fails loudly
+    beam_admit_kernel<<<1, 1024, smem, s>>>(st, cb, grp, Bi, drafts_in, lib_in, tok_cnt_in, tok_list_in, srclen_in, out, trace_nacc, trace_pick, dl_first);
+}
+
+// Prepare step of the continuous loop: beam_prepare per candidate with the width / draft length of its batch; row bases
+// and live lists by block-wide scans in candidate order.
+__global__ void __launch_bounds__(1024) beam_prepare_groups_kernel(BeamState st, BcTable cb) {
+    const int K = st.K, N = st.N, C = st.B * K;
+    const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, n_warps = blockDim.x >> 5;
+    for (int c = warp; c < C; c += n_warps) {
+        const int g = cb.slot_group[c / K];
+        if (g < 0 || (c % K != 0 && cb.groups[g].iter == 0)) {   // free slot, or a candidate that does not exist yet
+            if (lane == 0) st.c_fin[c] = 2;
+            continue;
+        }
+        const int W = cb.groups[g].W, dl = cb.groups[g].dl;
+        const int* row = st.cand_cur + (long long)c * st.ldw;
+        int first_pad = 0x7fffffff, last_real = -1, fin = 0;
+        for (int j = lane; j < W; j += 32) {
+            const int t = row[j];
+            if (t == st.eos) fin = 1;
+            if (t == st.pad) first_pad = min(first_pad, j); else last_real = max(last_real, j);
+        }
+#pragma unroll
+        for (int o = 16; o > 0; o >>= 1) {
+            first_pad = min(first_pad, __shfl_xor_sync(0xffffffffu, first_pad, o));
+            last_real = max(last_real, __shfl_xor_sync(0xffffffffu, last_real, o));
+            fin |= __shfl_xor_sync(0xffffffffu, fin, o);
+        }
+        if (lane == 0) {
+            const int slot0 = first_pad == 0x7fffffff ? -1 : first_pad;
+            const int hole = slot0 >= 0 && last_real > slot0;
+            st.c_slot0[c] = slot0;
+            st.c_fin[c] = fin;
+            if (hole || slot0 < 1 || slot0 + dl + 1 > W) atomicExch(&cb.groups[g].error, 3);
+        }
+    }
+    __syncthreads();
+    __shared__ int s_rows, s_live;
+    if (threadIdx.x == 0) { s_rows = 0; s_live = 0; }
+    __syncthreads();
+    for (int c0 = 0; c0 < C; c0 += blockDim.x) {
+        const int c = c0 + threadIdx.x, q = c / K;
+        int rows = 0, live = 0, rl = 0;
+        if (c < C && st.c_fin[c] != 2) {
+            const int g = cb.slot_group[q];
+            rl = cb.groups[g].dl + 1;   // positions of the candidate's draft rows (the attention's per-group row length)
+            const int slot0 = st.c_slot0[c];
+            st.c_front[c] = max(0, slot0 - 1);
+            int cnt = N;
+            if (st.smart) {
+                const int W = cb.groups[g].W;
+                const int last = st.cand_cur[(long long)c * st.ldw + (slot0 >= 1 ? slot0 - 1 : (slot0 < 0 ? W - 1 : 0))];
+                st.c_last[c] = last;
+                cnt = st.tok_cnt[(long long)q * st.V + last];
+                st.c_cnt[c] = cnt;
+                atomicMax(&cb.groups[g].lmax, cnt);
+            }
+            if (!st.c_fin[c]) { rows = cnt; live = 1; }
+        }
+        int er, el, tr, tl;
+        block_scan2(rows, live, er, el, tr, tl);
+        if (c < C) st.c_rowbase[c] = s_rows + er;
+        if (live && !st.smart) {
+            const int i = s_live + el, f = st.c_front[c];
+            st.live_cand[i] = c;
+            st.live_query[i] = q;
+            st.desc_self[i] = make_int4(c, f, st.cand_cur[(long long)c * st.ldw + f], rl);
+            st.desc_cross[i] = make_int4(q, 0, 0, st.src_len[q]);
+        }
+        __syncthreads();
+        if (threadIdx.x == 0) { s_rows += tr; s_live += tl; }
+        __syncthreads();
+    }
+    if (threadIdx.x == 0) {
+        st.ctrl[BC_NLIVE_ROWS] = s_rows;
+        st.ctrl[BC_NLIVE_CANDS] = st.smart ? s_rows : s_live;
+    }
+    if (st.smart) {   // every live row is its own attention group: row -> (candidate, query, library window)
+        for (int c = threadIdx.x; c < C; c += blockDim.x) {
+            if (st.c_fin[c]) continue;
+            const int q = c / K, base = st.c_rowbase[c], cnt = st.c_cnt[c];
+            const int* list = st.tok_list + ((long long)q * st.V + st.c_last[c]) * N;
+            const int f = st.c_front[c];
+            const int4 ds = make_int4(c, f, st.cand_cur[(long long)c * st.ldw + f], cb.groups[cb.slot_group[q]].dl + 1);
+            const int4 dc = make_int4(q, 0, 0, st.src_len[q]);
+            for (int j = 0; j < cnt; ++j) {
+                st.live_cand[base + j] = c;
+                st.live_query[base + j] = q;
+                st.row_draft[base + j] = list[j];
+                st.desc_self[base + j] = ds;
+                st.desc_cross[base + j] = dc;
+            }
+        }
+    }
+}
+void launch_beam_prepare_groups(const BeamState& st, const BcTable& cb, cudaStream_t s) { beam_prepare_groups_kernel<<<1, 1024, 0, s>>>(st, cb); }
+
+// Choose step of the continuous loop: beam_choose per candidate with its batch's draft length, padding length and trace
+// rows (indexed by the batch's own iteration and its candidate numbering: query in the first iteration, query * K + k after).
+__global__ void __launch_bounds__(256) beam_choose_groups_kernel(BeamState st, BcTable cb, int rs, int par) {
+    pdl_wait();   // launched with the programmatic attribute: scheduled while the predecessor drains, starts when it is complete
+    const int c = blockIdx.x, K = st.K;
+    __shared__ int s_nacc[64];
+    extern __shared__ unsigned char s_hit[];
+    if (st.c_fin[c] == 2) return;
+    const int q = c / K;
+    const BcGroup& gr = cb.groups[cb.slot_group[q]];
+    const int cl = gr.iter == 0 ? cb.slot_q[q] : cb.slot_q[q] * K + c % K;
+    const long long tr = (long long)gr.iter * gr.B * K + cl;
+    choose_candidate(st, c, q, gr.dl, rs, st.smart ? gr.lmax : st.N, par, s_hit, s_nacc, gr.trace_nacc ? gr.trace_nacc + tr * st.N : nullptr,
+                     gr.trace_pick ? gr.trace_pick + tr : nullptr);
+}
+void launch_beam_choose_groups(const BeamState& st, const BcTable& cb, int dl, cudaStream_t s) {
+    const size_t smem = (size_t)st.N * (dl > 0 ? dl : 1);
+    const int par = smem <= 40 * 1024 ? 1 : 0;
+    launch_pdl(beam_choose_groups_kernel, dim3(st.B * st.K), dim3(256), par ? smem : 0, s, st, cb, dl + 1, par);
+}
+
+// Expand step of the continuous loop: beam_expand per occupied slot with its batch's width and draft length, the new
+// hypotheses also written to the batch's output at its width.  The CTA that arrives last closes the iteration for every
+// open batch with the reference's stop rule (its own counters, error, width and draft length), frees the slots of the
+// batches that closed and posts the loop's word: sequence (24 bits) | slots in use (12) | largest draft length of the open
+// batches (8) | unfinished candidates of the next iteration (16).
+__global__ void __launch_bounds__(256) beam_expand_groups_kernel(BeamState st, BcTable cb, int rs, const float* __restrict__ logits) {
+    pdl_wait();   // launched with the programmatic attribute: scheduled while the predecessor drains, starts when it is complete
+    const int q = blockIdx.x, K = st.K;
+    const int g = cb.slot_group[q];
+    if (g >= 0) {
+        BcGroup* gr = &cb.groups[g];
+        const int W = gr->W;
+        int* ctrl = st.ctrl;
+        expand_query(st, q, K, gr->dl, rs, W, logits, &gr->error, gr->out + (long long)cb.slot_q[q] * K * W,
+                     [gr, ctrl](int, bool fin, int p, int pads, int has_eos) {
+                         if (!has_eos) { atomicAnd(&gr->all_fin, 0); atomicAdd(&ctrl[BCX_NLIVE_NEXT], 1); }
+                         atomicMin(&gr->min_pad, pads);
+                         if (!fin) { atomicAdd(&gr->acc, p); atomicAdd(&gr->cnt, 1); }
+                     });
+    } else {
+        for (int k = threadIdx.x; k < K; k += blockDim.x) st.n_parent[q * K + k] = -1;   // no cache to carry
+    }
+    __shared__ int s_last, s_dlmax, s_dlmin;
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        __threadfence();
+        s_last = atomicAdd(&st.ctrl[BCX_TICKET], 1) == (int)gridDim.x - 1;
+        s_dlmax = 0;
+        s_dlmin = 0x7fffffff;
+    }
+    __syncthreads();
+    if (!s_last) return;
+    __threadfence();
+    for (int gi = threadIdx.x; gi < cb.n_groups; gi += blockDim.x) {
+        BcGroup* gr = &cb.groups[gi];
+        if (gr->closed) continue;
+        const int all_fin = atomicAdd(&gr->all_fin, 0), empty = atomicAdd(&gr->min_pad, 0);
+        const int acc = atomicAdd(&gr->acc, 0), cnt = atomicAdd(&gr->cnt, 0), err = atomicAdd(&gr->error, 0);
+        gr->accepted += acc;
+        gr->produced += acc + cnt;
+        gr->iter += 1;
+        // speculative_decoding.py:452-470 and :570-598, as the CTA that closes an iteration of one batch applies them
+        const int W = gr->W, dl = gr->dl, filled = W - empty, budget = st.max_len - filled - 1;
+        atomicMin(&s_dlmin, dl);
+        if (err != 0 || all_fin != 0 || budget < 1 || filled > st.max_len) {
+            gr->closed = 1;   // W stays the width of the batch's last iteration: the width of its output
+            atomicSub(&st.ctrl[BCC_USED], gr->B);
+        } else {
+            gr->W = W + max(min(budget, dl) + 1 - empty, 0);
+            gr->dl = min(budget, dl);
+            atomicMax(&s_dlmax, gr->dl);
+        }
+        gr->all_fin = 1; gr->min_pad = 0x7fffffff; gr->acc = 0; gr->cnt = 0; gr->lmax = 0;
+    }
+    __syncthreads();
+    for (int b = threadIdx.x; b < st.B; b += blockDim.x) {
+        const int gb = cb.slot_group[b];
+        if (gb >= 0 && cb.groups[gb].closed) cb.slot_group[b] = -1;
+    }
+    __syncthreads();
+    if (threadIdx.x == 0) {
+        const int nlive_next = st.ctrl[BCX_NLIVE_NEXT];
+        st.ctrl[BCX_NLIVE_NEXT] = 0;
+        st.ctrl[BCX_TICKET] = 0;
+        const int seq = st.ctrl[BCX_ITER] + 1;
+        st.ctrl[BCX_ITER] = seq;
+        st.ctrl[BCC_DLMAX] = s_dlmax;
+        if (cb.dl_min) cb.dl_min[seq - 1] = s_dlmin;
+        if (st.host_ctrl) {
+            const unsigned long long word = ((unsigned long long)(seq & 0xffffff) << 40) | ((unsigned long long)(st.ctrl[BCC_USED] & 0xfff) << 28) |
+                                            ((unsigned long long)(s_dlmax & 0xff) << 20) | ((unsigned long long)(nlive_next & 0xffff) << 4);
+            reinterpret_cast<volatile unsigned long long*>(st.host_ctrl)[seq & 3] = word;
+        }
+    }
+}
+void launch_beam_expand_groups(const BeamState& st, const BcTable& cb, int dl, const float* logits, cudaStream_t s) {
+    const size_t smem = ((size_t)st.K * (dl + 1) * st.K + (size_t)st.K * (dl + 2)) * sizeof(float);
+    if (ensure_dyn_smem(beam_expand_groups_kernel, (int)smem)) return;   // error recorded; the launch below fails and cudaGetLastError reports it
+    launch_pdl(beam_expand_groups_kernel, dim3(st.B), dim3(256), smem, s, st, cb, dl + 1, logits);
 }
 
 __global__ void beam_init_kernel(BeamState st) {

@@ -174,6 +174,7 @@ struct ttb_engine {
     DevBuf cb;                   // continuous batching: slot / batch tables and the staging buffers of an admitted batch
     DevBuf cb_work;              // continuous batching: encoder workspace of an admitted batch (the loop's own must stay intact)
     std::vector<int> h_hist;
+    std::vector<int> h_dl, h_dl_min;   // continuous beam-search loop: draft length of every decoder call, smallest of its batches
 
     int E() const { return d.embedding_dim; }
     int HD() const { return d.embedding_dim / d.num_heads; }
@@ -419,16 +420,16 @@ static void attn(const __nv_bfloat16* q, int q_ld, const __nv_bfloat16* k, const
 }
 static void spec_attn(const float* qkv, int ld, const float* kc, const float* vc, long long cqs, int cld, float* out, int old, int B,
                       const int* na, const int* active, const int* front, const int* gen, int gen_ld, int pad, int N, int D, int H,
-                      int HD, int P, cudaStream_t s, const int4* = nullptr) {
+                      int HD, int P, cudaStream_t s, const int4* = nullptr, bool = false) {
     launch_spec_self_attention<float>(qkv, ld, kc, vc, cqs, cld, out, old, B, na, active, front, gen, gen_ld, pad, N, D, H, HD, P, s);
 }
 static void spec_attn(const __nv_bfloat16* qkv, int ld, const __nv_bfloat16* kc, const __nv_bfloat16* vc, long long cqs, int cld,
                       __nv_bfloat16* out, int old, int B, const int* na, const int* active, const int* front, const int* gen,
-                      int gen_ld, int pad, int N, int D, int H, int HD, int P, cudaStream_t s, const int4* desc = nullptr) {
+                      int gen_ld, int pad, int N, int D, int H, int HD, int P, cudaStream_t s, const int4* desc = nullptr, bool group_row_len = false) {
     if (attn_simt_forced())
         launch_spec_self_attention<__nv_bfloat16>(qkv, ld, kc, vc, cqs, cld, out, old, B, na, active, front, gen, gen_ld, pad, N, D, H, HD, P, s);
     else
-        launch_spec_self_attention_mma(qkv, ld, kc, vc, cqs, cld, out, old, B, na, active, front, gen, gen_ld, pad, N, D, H, HD, s, desc);
+        launch_spec_self_attention_mma(qkv, ld, kc, vc, cqs, cld, out, old, B, na, active, front, gen, gen_ld, pad, N, D, H, HD, s, desc, group_row_len);
 }
 
 // GEMM A-operand view of the residual stream: fp32 path reads x itself, bf16 path its bf16 copy
@@ -1066,14 +1067,29 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
 }
 
 
+// Continuous batching (ttb_beam_speculative_generate_batches): the batches that share the query slots of one loop.
+struct BcArgs {
+    int n;                              // batches, admitted in list order
+    const int64_t* const* src;          // [n] (B_i, Ls_i) int64 sources
+    const int32_t* bs;                  // [n] B_i
+    const int32_t* ls;                  // [n] Ls_i
+    int64_t* const* out;                // [n] B_i * n_best * (max_len + draft length + 4) int64 hypotheses
+    int32_t* out_width;                 // [n] width of each batch's hypotheses
+    int32_t* const* trace_nacc;         // [n] optional traces as in ttb_beam_speculative_generate, or NULL
+    int32_t* const* trace_pick;
+    ttb_generate_stats* stats;          // [n]
+};
+
 // ---- speculative beam search (speculative_decoding.py:428-598), host loop + device kernels ---------------
 // The per-iteration shapes (token-matrix width, draft length, live rows) depend on the hypotheses, so the
 // host reads a handful of control words back once per iteration; tokens, scores and logits never leave
-// the device.
+// the device.  With `cb` the loop is the continuous one: B is the number of query slots, Ls the longest source of all
+// batches, and the batches of `cb` are admitted into free slots between two iterations.
 template <typename ActT>
 static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int max_len, int K, int draft_len, int N,
                     int pad, int bos, int eos, int c_token, int tie_break, int64_t* out_dev, int32_t* out_width,
-                    int32_t* trace_nacc, int32_t* trace_pick, ttb_generate_stats* stats, cudaStream_t user_stream, bool smart) {
+                    int32_t* trace_nacc, int32_t* trace_pick, ttb_generate_stats* stats, cudaStream_t user_stream, bool smart,
+                    const BcArgs* cb = nullptr) {
     const int E = e->E(), H = e->d.num_heads, HD = e->HD(), V = e->d.tgt_vocab_size;
     const int n_dec = (int)e->dec.size();
     cudaStream_t s = e->stream;
@@ -1098,14 +1114,22 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     static const bool no_cache = [] { const char* v = getenv("TTB_BEAM_NO_CACHE"); return v && v[0] == '1'; }();
     const bool cached = !no_cache;
     TTB_CHECK(cached || !smart, "smart_drafts_mode needs the KV-cached decoder pass (unset TTB_BEAM_NO_CACHE)");
+    const bool cont = cb != nullptr;
+    TTB_CHECK(cached || !cont, "continuous batching needs the KV-cached decoder pass (unset TTB_BEAM_NO_CACHE)");
+    // continuous loop: the encoder of an admitted batch runs on the largest batch shape, in a workspace of its own
+    int B_stage = 0;
+    long long TS_stage = 0;
+    if (cont)
+        for (int i = 0; i < cb->n; ++i) { B_stage = std::max(B_stage, (int)cb->bs[i]); TS_stage = std::max(TS_stage, (long long)cb->bs[i] * cb->ls[i]); }
     const long long Tc = (long long)Rmax * (D0 + 1);
     const long long Tmax = cached ? Tc : (long long)Rmax * ldw;
 
-    if (e->src32.ensure(TS_cap * sizeof(int)) || e->memory.ensure(TS_cap * E * sizeof(float))) return 1;
-    if (Prec<ActT>::lowp && e->memh.ensure(TS_cap * E * sizeof(ActT))) return 1;
+    const long long TS_enc = cont ? TS_stage : TS_cap;
+    if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float))) return 1;
+    if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
     if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
     if (e->drafts.ensure(smart ? (size_t)B * std::max(n_lib, Ls_cap) * D_lib * sizeof(int) : (size_t)B * N * D0 * sizeof(int))) return 1;
-    if (ensure_work<ActT>(e, std::max(Tmax, TS_cap), cached ? n_dec : 1)) return 1;
+    if (ensure_work<ActT>(e, cont ? Tmax : std::max(Tmax, TS_cap), cached ? n_dec : 1)) return 1;
     const long long cache_c_stride = (long long)ldw * E, cache_l_stride = (long long)Cmax * ldw * E;
     if (cached) {
         const size_t cbytes = (size_t)n_dec * cache_l_stride * sizeof(ActT);
@@ -1128,18 +1152,48 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
                  o_cl = take(Cmax * 4), o_rd = take(Rmax * 4), o_ds = take(Rmax * 16), o_dc = take(Rmax * 16);
     if (bb.ensure(off)) return 1;
     char* base = bb.as<char>();
+    // continuous loop: slot / batch tables, staging of an admitted batch (source lengths, drafts or window library, cross
+    // K/V), slot-major key tokens and source lengths, encoder workspace
+    BcTable cbt{};
+    int *stage_srclen = nullptr, *stage_drafts = nullptr, *stage_tokcnt = nullptr, *stage_toklist = nullptr;
+    ActT* stage_kv = nullptr;
+    EncWork<ActT> enc_work{};
+    if (cont) {
+        TTB_CHECK((2 * E * sizeof(ActT)) % 16 == 0, "continuous batching needs 16-byte cross-attention K/V rows");
+        TTB_CHECK(B <= 2048 && (long long)B * K < 65536, "continuous batching supports at most 2048 slots and 65535 candidates");
+        size_t co = 0;
+        auto ctake = [&](size_t bytes) { size_t o = co; co += (bytes + 255) / 256 * 256; return o; };
+        const size_t c_sg = ctake((size_t)B * 4), c_sq = ctake((size_t)B * 4), c_as = ctake((size_t)B * 4), c_gr = ctake((size_t)cb->n * sizeof(BcGroup));
+        const size_t c_sl = ctake((size_t)B_stage * 4), c_dr = ctake((smart ? (size_t)std::max(n_lib, 1) * D_lib : (size_t)N * D0) * B_stage * 4);
+        const size_t c_tc = ctake(smart ? (size_t)B_stage * V * 4 : 4), c_tl = ctake(smart ? (size_t)B_stage * V * N * 4 : 4);
+        const size_t c_kv = ctake((size_t)n_dec * TS_stage * 2 * E * sizeof(ActT));
+        const size_t c_dm = ctake(((size_t)cb->n * (max_len + 1) + 1) * sizeof(int));
+        if (e->cb.ensure(co) || e->cb_work.ensure(enc_work_bytes<ActT>(e, TS_stage))) return 1;
+        if (e->keytok32.ensure((size_t)TS_cap * sizeof(int)) || e->srclen.ensure((size_t)B * sizeof(int))) return 1;
+        char* cbase = e->cb.as<char>();
+        cbt.slot_group = (int*)(cbase + c_sg); cbt.slot_q = (int*)(cbase + c_sq); cbt.adm_slots = (int*)(cbase + c_as);
+        cbt.groups = (BcGroup*)(cbase + c_gr);
+        cbt.dl_min = (int*)(cbase + c_dm);
+        stage_srclen = (int*)(cbase + c_sl); stage_drafts = (int*)(cbase + c_dr); stage_tokcnt = (int*)(cbase + c_tc); stage_toklist = (int*)(cbase + c_tl);
+        stage_kv = (ActT*)(cbase + c_kv);
+        enc_work = enc_work_carve<ActT>(e, TS_stage, e->cb_work.p);
+    }
+    // nothing is allocated from here on (cudaFree would synchronise the device)
+    const long long sig0 = e->alloc_signature();
 
     TTB_CUDA_OK(cudaEventRecord(e->t0, s));
     int* src32 = e->src32.as<int>();
-    { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(src_dev), src32, TS, s); }
     float* mem = e->memory.as<float>();
     ActT* memh = Prec<ActT>::lowp ? e->memh.as<ActT>() : nullptr;
-    if (encode_impl<ActT>(e, src32, src32, B, Ls, mem, memh, s)) return 1;
     ActT* crosskv = e->crosskv.as<ActT>();
     const long long ckv_l_stride = TS_cap * 2 * E;
-    if (cross_kv_impl<ActT>(e, mem, memh, (int)TS, crosskv, s, ckv_l_stride)) return 1;
-    if (smart) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32, Ls, B, Ls, D_lib, n_lib, eos, pad, c_token, e->drafts.as<int>(), s); }
-    else { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Ls, B, Ls - 1, D0, N, eos, pad, c_token, e->drafts.as<int>(), s); }
+    if (!cont) {
+        { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(src_dev), src32, TS, s); }
+        if (encode_impl<ActT>(e, src32, src32, B, Ls, mem, memh, s)) return 1;
+        if (cross_kv_impl<ActT>(e, mem, memh, (int)TS, crosskv, s, ckv_l_stride)) return 1;
+        if (smart) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32, Ls, B, Ls, D_lib, n_lib, eos, pad, c_token, e->drafts.as<int>(), s); }
+        else { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Ls, B, Ls - 1, D0, N, eos, pad, c_token, e->drafts.as<int>(), s); }
+    }
 
     BeamState st{};
     st.B = B; st.K = K; st.N = N; st.dl0 = smart ? D_lib : D0; st.V = V; st.smart = smart ? 1 : 0; st.n_lib = n_lib; st.pad = pad; st.bos = bos; st.eos = eos; st.ldw = ldw; st.tie_break = tie_break;
@@ -1169,7 +1223,9 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     st.tok_cnt = (int*)(base + o_tc); st.tok_list = (int*)(base + o_tl); st.c_cnt = (int*)(base + o_cc); st.c_last = (int*)(base + o_cl);
     st.row_draft = (int*)(base + o_rd);
     static const bool no_desc = [] { const char* v = getenv("TTB_BEAM_NO_DESC"); return v && v[0] == '1'; }();
-    if (cached && !no_desc) {
+    if (cont) {   // per-slot source lengths, installed by the admission kernel
+        st.desc_self = (int4*)(base + o_ds); st.desc_cross = (int4*)(base + o_dc); st.src_len = e->srclen.as<int>();
+    } else if (cached && !no_desc) {
         // per-query source length: the cross-attention kernels skip the padding behind it
         if (e->srclen.ensure((size_t)B * sizeof(int))) return 1;
         { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
@@ -1183,8 +1239,16 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     float* xg = (float*)(base + o_xg);
     ActT* xgh = Prec<ActT>::lowp ? (ActT*)(base + o_xgh) : nullptr;
     float* logits = (float*)(base + o_lg);
-    { Scope sc(e, KC_MISC, s); launch_beam_init(st, s); }
-    if (smart) { Scope sc(e, KC_MISC, s); launch_beam_build_lib(st, s); }
+    if (cont) {
+        TTB_CHECK(st.host_ctrl, "continuous batching needs mapped pinned host memory for its control word");
+        TTB_CUDA_OK(cudaMemsetAsync(st.ctrl, 0, 32 * sizeof(int), s));
+        TTB_CUDA_OK(cudaMemsetAsync(cbt.slot_group, 0xff, (size_t)B * sizeof(int), s));   // every slot free
+        TTB_CUDA_OK(cudaMemsetAsync(st.n_parent, 0xff, (size_t)Cmax * sizeof(int), s));
+        TTB_CUDA_OK(cudaMemsetAsync(cbt.groups, 0, (size_t)cb->n * sizeof(BcGroup), s));
+    } else {
+        { Scope sc(e, KC_MISC, s); launch_beam_init(st, s); }
+        if (smart) { Scope sc(e, KC_MISC, s); launch_beam_build_lib(st, s); }
+    }
 
     float* x = e->x.as<float>();
     ActT* xh = Prec<ActT>::lowp ? e->xh.as<ActT>() : nullptr;
@@ -1196,7 +1260,7 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     // 5-20 k token rows, not by the ~33 launches per iteration (63.8 ms per batch launched directly, 64.5 ms replayed, the
     // graphs being re-captured whenever the padded source length changes), see DESIGN.md §2b.
     const char* ng = getenv("TTB_BEAM_GRAPH");
-    const bool use_graph = cached && st.host_ctrl && !trace_nacc && !trace_pick && e->prof.mask == 0 && ng && ng[0] == '1';
+    const bool use_graph = !cont && cached && st.host_ctrl && !trace_nacc && !trace_pick && e->prof.mask == 0 && ng && ng[0] == '1';
     if (use_graph) {
         const long long key[20] = {B, K, N, D0, Ls, max_len, V, smart ? 1 : 0, pad, bos, eos, c_token, tie_break, e->alloc_signature(),
                                    (long long)sizeof(ActT), (long long)reinterpret_cast<uintptr_t>(st.host_ctrl), n_dec, 0, 0, 0};
@@ -1236,9 +1300,10 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
             Cb = (C * (ttb_engine::kBeamBuckets - gb) + ttb_engine::kBeamBuckets - 1) / ttb_engine::kBeamBuckets;
         }
         auto body = [&]() -> int {
-        const int R = (smart ? C : std::min(C, std::max(1, Cb))) * N;
+        const int R = (smart && !cont ? C : std::min(C, std::max(1, Cb))) * N;
         bool fused_stats = false;
-        { Scope sc(e, KC_MISC, s); launch_beam_prepare(st, C, beam, dl, s); }
+        if (cont) { Scope sc(e, KC_MISC, s); launch_beam_prepare_groups(st, cbt, s); }
+        else { Scope sc(e, KC_MISC, s); launch_beam_prepare(st, C, beam, dl, s); }
         if (cached) {
             RowCount rows(R * (dl + 1), n_live, dl + 1);
             { Scope sc(e, KC_EMBED, s); launch_beam_embed_cached<ActT>(st, beam, R, dl, e->tgt_emb, e->pe, E, x, xh, s); }
@@ -1246,13 +1311,19 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
             // different number of rows, so every row is a group of its own
             const int G = smart ? R : R / N, n_per_group = smart ? 1 : N;
             auto self_attn = [&](int l, ActT* qkv, ActT* att) {
+                // continuous loop: a candidate's draft rows are its batch's dl + 1 positions long (desc_self.w), whatever the
+                // call's dl, so that the tensor-core kernel lays out its keys as generate() does
                 spec_attn(qkv, 3 * E, kc_cur + l * cache_l_stride, vc_cur + l * cache_l_stride, cache_c_stride, E, att, E, G, n_live_cands,
-                          st.live_cand, st.c_front, st.cand_cur, ldw, e->d.tgt_pad_token_idx, n_per_group, dl, H, HD, ldw, s, st.desc_self);
+                          st.live_cand, st.c_front, st.cand_cur, ldw, e->d.tgt_pad_token_idx, n_per_group, dl, H, HD, ldw, s, st.desc_self, cont);
             };
             auto cross_attn = [&](int l, ActT* q2, ActT* att) {
                 const ActT* kv = crosskv + (long long)l * ckv_l_stride;
-                attn(q2, E, kv, kv + E, 2 * E, att, E, G, n_live_cands, n_per_group * (dl + 1), Ls, Ls, st.live_query,
-                     src32, Ls, e->d.src_pad_token_idx, false, H, HD, s, nullptr, nullptr, st.desc_cross);
+                if (cont)   // slot-major K/V rows and key tokens, row stride Ls_cap per slot
+                    attn(q2, E, kv, kv + E, 2 * E, att, E, G, n_live_cands, n_per_group * (dl + 1), Ls_cap, Ls_cap, st.live_query,
+                         e->keytok32.as<int>(), Ls_cap, e->d.src_pad_token_idx, false, H, HD, s, nullptr, nullptr, st.desc_cross);
+                else
+                    attn(q2, E, kv, kv + E, 2 * E, att, E, G, n_live_cands, n_per_group * (dl + 1), Ls, Ls, st.live_query,
+                         src32, Ls, e->d.src_pad_token_idx, false, H, HD, s, nullptr, nullptr, st.desc_cross);
             };
             if (decoder_stack<ActT>(e, rows, n_dec, Tc * 3 * E, self_attn, cross_attn, s)) return 1;
             // every decoder row is a scored position.  bf16 path: the projection is fused with the statistics the search reads
@@ -1289,10 +1360,12 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
             if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(xg, xgh), E, e->classifier, logits, V, rp_rows, false, s)) return 1;
         }
         if (!fused_stats) { Scope sc(e, KC_ARGMAX, s); launch_beam_stats(st, logits, R, dl, s); }
-        { Scope sc(e, KC_ACCEPT, s); launch_beam_choose(st, C, beam, dl, s); }
+        if (cont) { Scope sc(e, KC_ACCEPT, s); launch_beam_choose_groups(st, cbt, dl, s); }
+        else { Scope sc(e, KC_ACCEPT, s); launch_beam_choose(st, C, beam, dl, s); }
         // the expand kernel also closes the iteration: its last CTA writes the control words and, last, the iteration's
         // sequence number into pinned host memory; the host reads them while the caches are still being re-parented
-        { Scope sc(e, KC_ACCEPT, s); launch_beam_expand(st, beam, dl, logits, s); }
+        if (cont) { Scope sc(e, KC_ACCEPT, s); launch_beam_expand_groups(st, cbt, dl, logits, s); }
+        else { Scope sc(e, KC_ACCEPT, s); launch_beam_expand(st, beam, dl, logits, s); }
         if (cached) {
             Scope sc(e, KC_CACHE_APPEND, s);
             launch_beam_cache_update<ActT>(st, dl, e->qkv.as<ActT>(), Tc * 3 * E, n_dec, 3 * E, E, kc_cur, vc_cur, kc_next, vc_next,
@@ -1326,6 +1399,7 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     // wait for the packed word the expand kernel posts for iteration `seq` (sequence | error | all finished | empty columns)
     static const bool pure_spin = [] { const char* v = getenv("TTB_BEAM_SPIN"); return v && v[0] == '1'; }();
     int live_next = B;      // unfinished candidates entering the next iteration, from the newest word read
+    int cont_used = 0, cont_dl = 0;   // continuous loop: slots in use and largest draft length of the open batches, idem
     auto wait_word = [&](int seq) -> int {
         volatile unsigned long long* word = reinterpret_cast<volatile unsigned long long*>(hc + 16) + (seq & 3);
         unsigned long long w = 0;
@@ -1341,6 +1415,7 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
                 if (q == cudaSuccess) {   // stream drained: the word is there, or the mapping is unavailable: take a copy
                     w = *word;
                     if ((unsigned)((w >> 40) & 0xffffff) != (unsigned)(seq & 0xffffff)) {
+                        TTB_CHECK(!cont, "the control word of the continuous beam-search loop did not arrive");
                         TTB_CUDA_OK(cudaMemcpy(hc, st.ctrl, BC_COUNT * sizeof(int), cudaMemcpyDeviceToHost));
                         w = ((unsigned long long)(seq & 0xffffff) << 40) | ((unsigned long long)(hc[BC_ERROR] & 0xf) << 36) |
                             ((unsigned long long)(hc[BC_ALL_FINISHED] & 1) << 35) | ((unsigned long long)(hc[BC_EMPTY_COLS] & 0xfff) << 23) |
@@ -1351,6 +1426,12 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
                     TTB_CUDA_OK(q);
                 }
             }
+        }
+        if (cont) {   // sequence | slots in use | largest draft length of the open batches | unfinished candidates
+            cont_used = (int)((w >> 28) & 0xfff);
+            cont_dl = (int)((w >> 20) & 0xff);
+            live_next = (int)((w >> 4) & 0xffff);
+            return 0;
         }
         hc[BC_ERROR] = (int)((w >> 36) & 0xf);
         hc[BC_ALL_FINISHED] = (int)((w >> 35) & 1);
@@ -1364,6 +1445,109 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     // word: C = B K and beam = K from the second iteration on, and the draft length stays dl as long as the length budget
     // cannot drop below it (one iteration fills at most dl + 1 more columns).  If the current iteration ends the loop the
     // device has raised BCX_DONE and the iteration enqueued ahead does nothing.
+    if (cont) {
+        // Continuous loop.  Between two iterations the host admits the next batches (whole, in list order) while the free
+        // slots of the newest word suffice, then enqueues one iteration at the largest draft length of the open batches
+        // and waits for its word.  Nothing is enqueued ahead: the coming iteration's draft length and admissions depend
+        // on the word.
+        const int dl_first = std::min(max_len - 2, dl);   // the first iteration's draft length (budget max_len - 2)
+        auto admit = [&](int i) -> int {
+            const int Bi = cb->bs[i], Li = cb->ls[i], lib_i = Li - 5;
+            const long long TSi = (long long)Bi * Li;
+            { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(cb->src[i]), src32, TSi, s); }
+            { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, Bi, Li, e->d.src_pad_token_idx, stage_srclen, s); }
+            if (encode_impl<ActT>(e, src32, src32, Bi, Li, mem, memh, s, &enc_work)) return 1;
+            if (cross_kv_impl<ActT>(e, mem, memh, (int)TSi, stage_kv, s, TS_stage * 2 * E)) return 1;
+            if (smart) {
+                { Scope sc(e, KC_MISC, s); launch_make_drafts(src32, Li, Bi, Li, D_lib, lib_i, eos, pad, c_token, stage_drafts, s); }
+                BeamState lib = st;   // the batch's library alone, as generate() builds it
+                lib.B = Bi; lib.n_lib = lib_i; lib.drafts = stage_drafts; lib.tok_cnt = stage_tokcnt; lib.tok_list = stage_toklist;
+                Scope sc(e, KC_MISC, s);
+                launch_beam_build_lib(lib, s);
+            } else {
+                Scope sc(e, KC_MISC, s);
+                launch_make_drafts(src32 + 1, Li, Bi, Li - 1, D0, N, eos, pad, c_token, stage_drafts, s);
+            }
+            {
+                Scope sc(e, KC_MISC, s);
+                launch_beam_admit(st, cbt, i, Bi, stage_drafts, lib_i, stage_tokcnt, stage_toklist, stage_srclen, reinterpret_cast<long long*>(cb->out[i]),
+                                  cb->trace_nacc ? cb->trace_nacc[i] : nullptr, cb->trace_pick ? cb->trace_pick[i] : nullptr, dl_first, s);
+            }
+            {
+                CbTable kvt{};
+                kvt.adm_slots = cbt.adm_slots;
+                Scope sc(e, KC_MISC, s);
+                launch_greedy_admit_kv<ActT>(kvt, Bi, Li, Ls_cap, n_dec, E, stage_kv, TS_stage * 2 * E, crosskv, ckv_l_stride, src32, e->keytok32.as<int>(),
+                                             e->d.src_pad_token_idx, s);
+            }
+            cbt.n_groups = i + 1;
+            TTB_CUDA_OK(cudaGetLastError());
+            TTB_CHECK(e->alloc_signature() == sig0, "a workspace buffer moved while the continuous beam-search loop was running");
+            return 0;
+        };
+        // every batch takes part in at most max_len iterations
+        const long long max_iters = (long long)cb->n * (max_len + 1);
+        std::vector<int> hist, hist_dl;
+        int next = 0, it = 0;
+        live_next = 0;
+        // TTB_BEAM_CB_FULL_DL=1 (read per call): every decoder call runs at the first iteration's draft length, so that
+        // every batch near max_len runs with a shorter dl than the call's (a check that results do not depend on it)
+        const char* full_dl = getenv("TTB_BEAM_CB_FULL_DL");
+        const bool force_full_dl = full_dl && full_dl[0] == '1';
+        while (true) {
+            int dl_it = force_full_dl ? dl_first : cont_dl;
+            while (next < cb->n && B - cont_used >= cb->bs[next]) {
+                if (admit(next)) return 1;
+                cont_used += cb->bs[next];
+                live_next += cb->bs[next];
+                dl_it = std::max(dl_it, dl_first);
+                ++next;
+            }
+            if (cont_used == 0) break;   // nothing open and nothing pending (every batch fits the slots)
+            TTB_CHECK(it < max_iters, "continuous beam-search loop did not terminate within max_len iterations per batch");
+            hist.push_back(cont_used);
+            hist_dl.push_back(dl_it);
+            if (enqueue_iteration(it, B * K, K, dl_it, std::min(live_next, B * K))) return 1;
+            if (wait_word(it + 1)) return 1;
+            ++it;
+        }
+        TTB_CUDA_OK(cudaEventRecord(e->t1, s));
+        TTB_CUDA_OK(cudaStreamSynchronize(s));
+        TTB_CUDA_OK(cudaGetLastError());
+        prof_collect(e);
+        int ctrl_end[32] = {};
+        TTB_CUDA_OK(cudaMemcpy(ctrl_end, st.ctrl, sizeof(ctrl_end), cudaMemcpyDeviceToHost));
+        TTB_CHECK(ctrl_end[BC_COUNT + 11] == 0, "continuous batching admitted a batch without enough free slots");
+        std::vector<BcGroup> groups((size_t)cb->n);
+        TTB_CUDA_OK(cudaMemcpy(groups.data(), cbt.groups, groups.size() * sizeof(BcGroup), cudaMemcpyDeviceToHost));
+        e->h_hist = hist;
+        e->h_dl = hist_dl;
+        e->h_dl_min.assign(hist_dl.size(), 0);
+        if (it > 0) TTB_CUDA_OK(cudaMemcpy(e->h_dl_min.data(), cbt.dl_min, (size_t)it * sizeof(int), cudaMemcpyDeviceToHost));
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, e->t0, e->t1);
+        ttb_generate_stats sum{};
+        for (int i = 0; i < cb->n; ++i) {
+            const BcGroup& g = groups[(size_t)i];
+            TTB_CHECK(g.closed == 1 && g.B == cb->bs[i], "continuous beam-search loop ended before every batch was finished");
+            ttb_generate_stats& o = cb->stats[i];
+            o = ttb_generate_stats{};
+            o.model_calls = g.iter;
+            o.accepted_tokens = g.accepted;
+            o.produced_tokens = g.produced;
+            o.error = g.error == 3 ? TTB_ERR_REF_SHAPE : (g.error == 4 ? TTB_ERR_REF_ASSERT : 0);
+            cb->out_width[i] = g.W;
+            sum.accepted_tokens += g.accepted;
+            sum.produced_tokens += g.produced;
+        }
+        if (stats) {
+            sum.model_calls = it;
+            sum.gpu_launches = (int32_t)(e->launches - launches0);
+            sum.gpu_ms = ms;
+            *stats = sum;
+        }
+        return 0;
+    }
     static const bool no_ahead = [] { const char* v = getenv("TTB_BEAM_NO_AHEAD"); return v && v[0] == '1'; }();
     const bool ahead_ok = cached && st.host_ctrl && !no_ahead && !trace_nacc && !trace_pick;
     int enq = 0, dl_enq = dl;
@@ -1931,6 +2115,42 @@ int ttb_beam_speculative_generate(ttb_engine* e, const int64_t* src_dev, int32_t
                                                 smart_drafts_mode != 0)));
 }
 
+int ttb_beam_speculative_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs, const int32_t* batch_sizes,
+                                          const int32_t* src_lens, int32_t slots, int32_t max_len, int32_t n_best, int32_t draft_len,
+                                          int32_t n_drafts, int32_t smart_drafts_mode, int32_t pad_token, int32_t bos_token, int32_t eos_token,
+                                          int32_t c_token, int32_t tie_break, int64_t* const* out_devs, int32_t* out_widths,
+                                          int32_t* const* trace_nacc_devs, int32_t* const* trace_pick_devs, ttb_generate_stats* stats,
+                                          ttb_generate_stats* total, void* stream) {
+    TTB_CHECK(e && e->finalized, "engine not finalized");
+    TTB_CHECK(n_batches >= 0 && max_len > 2 && slots > 0, "bad arguments");
+    TTB_CHECK(n_batches == 0 || (src_devs && batch_sizes && src_lens && out_devs && out_widths && stats), "bad arguments");
+    TTB_CHECK(n_best >= 1 && n_best <= 32, "n_best must be in [1, 32]");
+    TTB_CHECK(n_drafts > 0, "The number of drafts must be greater than 0");
+    TTB_CHECK(pad_token != c_token, "The pad token and the replace token must be different");
+    TTB_CHECK(eos_token != c_token, "The eos token and the replace token must be different");
+    TTB_CHECK(eos_token != pad_token, "The eos token and the pad token must be different");
+    TTB_CHECK(max_len + 210 <= e->d.max_positions, "sequence longer than the positional table");
+    TTB_CHECK(e->d.tgt_vocab_size <= 1024, "vocabularies above 1024 tokens are not supported by the beam statistics kernel");
+    int Ls_max = 2;
+    for (int i = 0; i < n_batches; ++i) {
+        TTB_CHECK(src_devs[i] && out_devs[i] && batch_sizes[i] > 0 && src_lens[i] > 1, "bad arguments");
+        TTB_CHECK(batch_sizes[i] <= slots, "slots must be at least the largest batch size");
+        TTB_CHECK(src_lens[i] <= e->d.max_positions, "sequence longer than the positional table");
+        if (smart_drafts_mode) TTB_CHECK(src_lens[i] > 5, "The number of drafts must be greater than 0");
+        Ls_max = std::max(Ls_max, (int)src_lens[i]);
+    }
+    if (total) *total = ttb_generate_stats{};
+    if (n_batches == 0) return 0;
+    TTB_CUDA_OK(cudaSetDevice(e->device));
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const BcArgs cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, out_widths, trace_nacc_devs, trace_pick_devs, stats};
+    return drained(e, TTB_DISPATCH(e, beam_api<float>(e, nullptr, slots, Ls_max, max_len, n_best, draft_len, n_drafts, pad_token, bos_token, eos_token,
+                                                      c_token, tie_break, nullptr, nullptr, nullptr, nullptr, total, s, smart_drafts_mode != 0, &cb),
+                                   beam_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, n_best, draft_len, n_drafts, pad_token, bos_token,
+                                                           eos_token, c_token, tie_break, nullptr, nullptr, nullptr, nullptr, total, s,
+                                                           smart_drafts_mode != 0, &cb)));
+}
+
 int ttb_kernel_class_count(void) { return KC_COUNT; }
 const char* ttb_kernel_class_name(int32_t id) { return (id >= 0 && id < KC_COUNT) ? kKcNames[id] : ""; }
 
@@ -1951,6 +2171,13 @@ int ttb_engine_get_history(ttb_engine* e, int32_t* live_queries_out, int32_t cap
     TTB_CHECK(e && live_queries_out, "null argument");
     const int n = (int)e->h_hist.size();
     for (int i = 0; i < n && i < capacity; ++i) live_queries_out[i] = e->h_hist[i];
+    return n;
+}
+
+int ttb_engine_get_draft_history(ttb_engine* e, int32_t* call_dl_out, int32_t* min_dl_out, int32_t capacity) {
+    TTB_CHECK(e && call_dl_out && min_dl_out, "null argument");
+    const int n = (int)e->h_dl.size();
+    for (int i = 0; i < n && i < capacity; ++i) { call_dl_out[i] = e->h_dl[i]; min_dl_out[i] = e->h_dl_min[i]; }
     return n;
 }
 

@@ -107,7 +107,9 @@ void launch_spec_self_attention_mma(const __nv_bfloat16* qkv, int qkv_ld, const 
                                     long long cache_query_stride, int cache_ld, __nv_bfloat16* out, int out_ld,
                                     int B_max, const int* n_active_dev, const int* active, const int* front,
                                     const int* gen, int gen_ld, int pad_id, int N, int D,
-                                    int heads, int head_dim, cudaStream_t s, const int4* desc = nullptr);
+                                    int heads, int head_dim, cudaStream_t s, const int4* desc = nullptr, bool group_row_len = false);
+// group_row_len (needs desc): group g's draft rows are desc[g].w <= D + 1 positions long (the rest of each row of the call is
+// ignored and not written), and its outputs are the bits a call with D + 1 = desc[g].w gives
 
 // ---- attention_tc.cu : tcgen05 attention of the decoding loops (head_dim 32, S in tensor memory, V caches kept transposed) ----
 bool attention_tc_supported(int head_dim, int Lq, int max_shared_keys, int row_len);
@@ -238,6 +240,33 @@ void launch_beam_stats(const BeamState& st, const float* logits, int max_rows, i
 void launch_beam_choose(const BeamState& st, int C, int beam, int dl, cudaStream_t s);
 void launch_beam_expand(const BeamState& st, int beam, int dl, const float* logits, cudaStream_t s);
 void launch_beam_export(const int* cand, int ldw, int R, int W, long long* out, cudaStream_t s);
+
+// Continuous batching of the speculative beam search (BeamState::B = number of query slots; slot b owns candidates
+// b K .. b K + K - 1).  One record per batch: what the reference couples across the queries of a batch plus its counters.
+struct BcGroup {
+    long long* out;                       // [B][K][W] the batch's hypotheses, rewritten at its width every iteration
+    int* trace_nacc; int* trace_pick;     // optional, indexed by the batch's own iteration and candidate numbering
+    int B, W, dl, iter;                   // batch size; width and draft length of its coming iteration; iterations taken part in
+    int lmax;                             // smart drafts: most drafts of one candidate in the current iteration
+    int accepted, produced, error, closed;   // counters; error 0 / 3 / 4 as BC_ERROR; 1 once the batch has stopped
+    int all_fin, min_pad, acc, cnt;       // accumulators of the iteration in flight
+};
+struct BcTable {
+    int* slot_group;   // [slots] batch of the query in the slot, -1 = free
+    int* slot_q;       // [slots] index of that query in its batch
+    int* adm_slots;    // [max batch size] slots given to the batch admitted last
+    BcGroup* groups;   // [n_batches]
+    int n_groups;      // batches admitted so far
+    int* dl_min;       // [iterations] smallest draft length among the batches of every iteration
+};
+// admission of batch `grp` between two iterations: drafts_in [Bi][N][dl0] (smart: [Bi][lib_in][dl0] window library with
+// tok_cnt_in [Bi][V], tok_list_in [Bi][V][N]), srclen_in [Bi], all computed for the batch alone
+void launch_beam_admit(const BeamState& st, const BcTable& cb, int grp, int Bi, const int* drafts_in, int lib_in, const int* tok_cnt_in,
+                       const int* tok_list_in, const int* srclen_in, long long* out, int* trace_nacc, int* trace_pick, int dl_first, cudaStream_t s);
+// group-aware prepare / choose / expand; `dl` = draft length of the decoder call (the largest of the open batches)
+void launch_beam_prepare_groups(const BeamState& st, const BcTable& cb, cudaStream_t s);
+void launch_beam_choose_groups(const BeamState& st, const BcTable& cb, int dl, cudaStream_t s);
+void launch_beam_expand_groups(const BeamState& st, const BcTable& cb, int dl, const float* logits, cudaStream_t s);
 // ---- std_beam.cu : standard beam search (standard_decoding.py:90-174) -------------------------------------------
 struct StdBeamState {
     int B, K, V, pad, bos, eos, ldw;

@@ -19,11 +19,35 @@ from ..model import B200Transformer
 # weights, 24 batches) on one B200 at 1000 W: 1908 SMILES/s one batch at a time; 1964 / 3221 / 3681 / 4151 / 4378 with
 # 32 / 48 / 64 / 96 / 128 slots (profiles/r3_continuous_copy.json, DESIGN.md section 10)
 DEFAULT_SLOTS_PER_BATCH = 4
+# TranslationInferenceBeamSearchSpeculative.generate_batches(): default query slots per query of the largest batch (each
+# slot holds n_best candidate rows), chosen from the sweep in DESIGN.md section 11
+DEFAULT_BEAM_SLOTS_PER_BATCH = 16
 # messages of the reference failures a batch of generate_batches() can end with (as raised by generate())
 _REF_ERRORS = {
     _lib.ERR_REF_INDEX: "index out of bounds while splicing drafts into the token matrix (reference scatter, speculative_decoding.py:111)",
     _lib.ERR_REF_SHAPE: "shape mismatch: a finished row is wider than max_len (reference speculative_decoding.py:158)",
 }
+_BEAM_REF_ERRORS = {
+    _lib.ERR_REF_SHAPE: (RuntimeError, "PAD predicted inside a hypothesis: draft slots are not contiguous (the reference fails on the "
+                                       "reshape at speculative_decoding.py:524-526)"),
+    _lib.ERR_REF_ASSERT: (AssertionError, "fewer candidate continuations than n_best (reference assert in topk_in_each_group, "
+                                          "speculative_decoding.py:195)"),
+}
+
+
+def _check_batches(batches: list, slots: int | None, per_batch: int) -> int:
+    """Argument rules of generate_batches(), checked before any device work; returns the slot count."""
+    for b in batches:
+        if b.dim() != 2 or b.shape[0] < 1 or b.shape[1] < 2:
+            raise ValueError(f"every batch must be a (B >= 1, Ls >= 2) tensor of token ids, got shape {tuple(b.shape)}")
+    if len({b.device for b in batches}) != 1:
+        raise ValueError("all batches must be on the same device")
+    bmax = max(int(b.shape[0]) for b in batches)
+    if slots is None:
+        slots = per_batch * bmax
+    if slots < bmax:
+        raise ValueError(f"slots ({slots}) must be at least the largest batch size ({bmax})")
+    return slots
 
 
 class TranslationInferenceGreedySpeculative:
@@ -94,16 +118,7 @@ class TranslationInferenceGreedySpeculative:
         if not batches:
             return []
         m = self.model
-        for b in batches:
-            if b.dim() != 2 or b.shape[0] < 1 or b.shape[1] < 2:
-                raise ValueError(f"every batch must be a (B >= 1, Ls >= 2) tensor of token ids, got shape {tuple(b.shape)}")
-        if len({b.device for b in batches}) != 1:
-            raise ValueError("all batches must be on the same device")
-        bmax = max(int(b.shape[0]) for b in batches)
-        if slots is None:
-            slots = DEFAULT_SLOTS_PER_BATCH * bmax
-        if slots < bmax:
-            raise ValueError(f"slots ({slots}) must be at least the largest batch size ({bmax})")
+        slots = _check_batches(batches, slots, DEFAULT_SLOTS_PER_BATCH)
         n = len(batches)
         srcs = [b.to(device=m.device, dtype=torch.int64, non_blocking=True).contiguous() for b in batches]
         outs = [torch.empty(s.shape[0], self.max_len, dtype=torch.int64, device=m.device) for s in srcs]
@@ -215,11 +230,80 @@ class TranslationInferenceBeamSearchSpeculative:
         self.gpu_launches += stats.gpu_launches
         self.gpu_ms += stats.gpu_ms
         if t_nacc is not None:
-            na, pk = t_nacc[:stats.model_calls].cpu(), t_pick[:stats.model_calls].cpu()
-            for it in range(na.shape[0]):
-                live = pk[it] >= 0
-                self.trace.append({"n_accepted": na[it][live].numpy().astype("int64"), "pick": pk[it][live].numpy().astype("int64")})
+            self._append_trace(t_nacc, t_pick, stats.model_calls)
         _lib.check(rc, "ttb_beam_speculative_generate")
         W = width.value
         res = out[:B * K * W].view(B, K, W)
         return res if src.is_cuda else res.to(src.device)
+
+    def generate_batches(self, batches: Sequence[torch.Tensor], slots: int | None = None,
+                         on_error: Callable[[int, Exception], object] | None = None) -> list:
+        """Continuous batching: decode `batches` in ONE device loop whose `slots` query slots (n_best candidate rows each)
+        are refilled with the queries of the next batch as soon as enough of them are free (batches are admitted whole, in
+        list order, between two iterations).
+
+        Returns `[self.generate(b) for b in batches]` bit for bit, each (B_i, n_best, W_i), and advances the counters and
+        `trace` exactly as those calls would: a batch keeps the width, draft length, stop and error rules of its own batch
+        in the shared loop.  A reference failure of batch i raises the exception generate() raises for it when position i
+        is reached, unless `on_error(i, exc)` is given, whose return value then stands in for that batch's result.
+        `slots` defaults to DEFAULT_BEAM_SLOTS_PER_BATCH times the largest batch size."""
+        batches = list(batches)
+        if not batches:
+            return []
+        m = self.model
+        slots = _check_batches(batches, slots, DEFAULT_BEAM_SLOTS_PER_BATCH)
+        if self.smart_drafts_mode:
+            for b in batches:
+                if b.shape[1] <= 5:   # a library of Ls - 5 windows: generate() fails on such a batch as well
+                    raise AssertionError("The number of drafts must be greater than 0")
+        n = len(batches)
+        K, N = self.n_best, self.requested_drafts_num
+        cap = self.max_len + self.draft_len + 4
+        srcs = [b.to(device=m.device, dtype=torch.int64, non_blocking=True).contiguous() for b in batches]
+        outs = [torch.empty(s.shape[0] * K * cap, dtype=torch.int64, device=m.device) for s in srcs]
+        t_nacc = t_pick = None
+        if self.keep_trace:
+            t_nacc = [torch.full((self.max_len, s.shape[0] * K, N), -1, dtype=torch.int32, device=m.device) for s in srcs]
+            t_pick = [torch.full((self.max_len, s.shape[0] * K), -1, dtype=torch.int32, device=m.device) for s in srcs]
+        ptrs = lambda ts: (C.c_void_p * n)(*[t.data_ptr() for t in ts])
+        sizes = (C.c_int32 * n)(*[s.shape[0] for s in srcs])
+        lens = (C.c_int32 * n)(*[s.shape[1] for s in srcs])
+        widths = (C.c_int32 * n)()
+        stats = (_lib.GenerateStats * n)()
+        total = _lib.GenerateStats()
+        with torch.cuda.device(m.device):
+            rc = m.lib.ttb_beam_speculative_generate_batches(
+                m._h, n, ptrs(srcs), sizes, lens, slots, self.max_len, K, self.draft_len, N, int(self.smart_drafts_mode),
+                self.pad_token_idx, self.bos_token_idx, self.eos_token_idx, self.C_token_idx, self.tie_break, ptrs(outs), widths,
+                ptrs(t_nacc) if t_nacc is not None else None, ptrs(t_pick) if t_pick is not None else None, stats, C.byref(total),
+                torch.cuda.current_stream(m.device).cuda_stream)
+        _lib.check(rc, "ttb_beam_speculative_generate_batches")
+        self.last_stats = total
+        self.gpu_launches += total.gpu_launches
+        self.gpu_ms += total.gpu_ms
+        results = []
+        for i in range(n):
+            st, B = stats[i], srcs[i].shape[0]
+            self.n_drafts += B * N
+            self.model_calls_num += st.model_calls
+            self.accepted_tokens_num += st.accepted_tokens
+            self.produced_non_pad_tokens += st.produced_tokens
+            if t_nacc is not None:
+                self._append_trace(t_nacc[i], t_pick[i], st.model_calls)
+            if st.error:
+                kind, msg = _BEAM_REF_ERRORS[st.error]
+                exc = kind(msg)
+                if on_error is None:
+                    raise exc
+                results.append(on_error(i, exc))
+                continue
+            W = widths[i]
+            res = outs[i][:B * K * W].view(B, K, W)
+            results.append(res if batches[i].is_cuda else res.to(batches[i].device))
+        return results
+
+    def _append_trace(self, t_nacc: torch.Tensor, t_pick: torch.Tensor, model_calls: int) -> None:
+        na, pk = t_nacc[:model_calls].cpu(), t_pick[:model_calls].cpu()
+        for it in range(na.shape[0]):
+            live = pk[it] >= 0
+            self.trace.append({"n_accepted": na[it][live].numpy().astype("int64"), "pick": pk[it][live].numpy().astype("int64")})
