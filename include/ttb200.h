@@ -150,9 +150,8 @@ int ttb_beam_speculative_generate(ttb_engine* e, const int64_t* src_dev, int32_t
  * batch_sizes[i] * n_best * (max_len + clamp(draft_len,5,200) + 4) int64 and receives (batch_sizes[i], n_best,
  * out_widths[i]) densely; trace_nacc_devs[i] / trace_pick_devs[i] are laid out as in ttb_beam_speculative_generate with
  * B = batch_sizes[i] (the arrays may be NULL or hold NULL entries).  slots >= max(batch_sizes).  total (may be NULL):
- * launches / ms of the call, model_calls = decoder iterations of the shared loop.  Needs the KV-cached decoder pass
- * (TTB_BEAM_NO_CACHE unset); iterations are not replayed as graphs.  ttb_engine_get_history afterwards gives the query
- * slots in use at every iteration. */
+ * launches / ms of the call, model_calls = decoder iterations of the shared loop.  ttb_engine_get_history afterwards
+ * gives the query slots in use at every iteration. */
 int ttb_beam_speculative_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs,
                                           const int32_t* batch_sizes, const int32_t* src_lens, int32_t slots, int32_t max_len,
                                           int32_t n_best, int32_t draft_len, int32_t n_drafts, int32_t smart_drafts_mode,

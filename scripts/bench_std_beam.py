@@ -1,6 +1,6 @@
 #!/usr/bin/env python
 """Timing of the standard (non-speculative) decoding strategies (standard_decoding.py) on synthetic sources, trained-like weights:
-KV-cached beam search against the full-prefix recomputation (TTB_SBEAM_NO_CACHE=1), plain greedy for reference."""
+beam search, plain greedy for reference."""
 import json
 import os
 import sys
@@ -36,7 +36,7 @@ def main():
         outs[name] = out.cpu()
         print(json.dumps({"strategy": name, "bs": bs, "beam": beam if name == "beam_search" else 1, "smiles_per_s": round(bs * steps / dt, 1),
                           "ms_per_batch": round(1000 * dt / steps, 2), "decoder_calls_per_batch": (gen.model_calls_num - c0) / steps,
-                          "kv_cached": os.environ.get("TTB_SBEAM_NO_CACHE", "0") != "1", "top1_checksum": int(outs[name][:, 0].sum())}), flush=True)
+                          "top1_checksum": int(outs[name][:, 0].sum())}), flush=True)
 
 
 if __name__ == "__main__":

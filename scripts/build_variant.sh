@@ -6,7 +6,7 @@ NAME=$1; shift
 cd "$(dirname "$0")/../translation_transformer_b200"
 mkdir -p csrc/build_$NAME
 pids=()
-for f in elementwise gemm_simt gemm_tcgen05 attention attention_mma attention_tc drafting greedy beam std_beam engine; do
+for f in elementwise gemm_simt gemm_tcgen05 attention attention_mma drafting greedy beam std_beam engine; do
   nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC --expt-relaxed-constexpr "$@" -c csrc/$f.cu -o csrc/build_$NAME/$f.o &
   pids+=($!)
 done

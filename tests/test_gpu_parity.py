@@ -374,7 +374,7 @@ def _beam_cases():
 
 
 @pytest.mark.parametrize("case", _beam_cases(), ids=lambda c: c["id"])
-def test_beam_speculative_fp32_matches_reference_golden(dev, case, monkeypatch):
+def test_beam_speculative_fp32_matches_reference_golden(dev, case):
     from translation_transformer_b200.decoding import TranslationInferenceBeamSearchSpeculative
     z = load_npz("beam_speculative.npz")
     cfg, sd = case_weights(case)
@@ -392,9 +392,8 @@ def test_beam_speculative_fp32_matches_reference_golden(dev, case, monkeypatch):
     pick = np.concatenate([t["pick"] for t in gen.trace])
     assert np.array_equal(nacc, z[case["id"] + "_nacc"].astype(np.int64))               # accepted lengths of every draft
     assert np.array_equal(pick, z[case["id"] + "_pick"].astype(np.int64))               # chosen draft indices
-    # TTB_BEAM_GRAPH=1 and no trace: the steady-state iterations are replayed as CUDA graphs (engine.cu:beam_api): same
-    # hypotheses and counters, also when the graphs of the first call are reused by the second
-    monkeypatch.setenv("TTB_BEAM_GRAPH", "1")
+    # no trace: steady-state iterations are enqueued ahead of the host reading the outcome of the one before
+    # (engine.cu:beam_api): same hypotheses and counters, also on the second call on the same engine
     for _ in range(2):
         gen2 = TranslationInferenceBeamSearchSpeculative(eng, case["max_len"], case["n_best"], case["draft_len"], case["n_drafts"],
                                                          case["vocab"], False, 0, 1, 2, case["C_token"])
@@ -409,7 +408,7 @@ def _beam_smart_cases():
 
 
 @pytest.mark.parametrize("case", _beam_smart_cases(), ids=lambda c: c["id"])
-def test_beam_speculative_smart_drafts_fp32_matches_reference_golden(dev, case, monkeypatch):
+def test_beam_speculative_smart_drafts_fp32_matches_reference_golden(dev, case):
     """smart_drafts_mode=True (speculative_decoding.py:600-845): hypotheses, counters, accepted length of every tried
     draft (ragged groups padded with -1 like the reference's topk_in_each_group) and the chosen drafts, bit-exact."""
     from translation_transformer_b200.decoding import TranslationInferenceBeamSearchSpeculative
@@ -441,8 +440,7 @@ def test_beam_speculative_smart_drafts_fp32_matches_reference_golden(dev, case, 
         assert np.array_equal(t["pick"], ref_pick[o_p:o_p + C])
         o_n += C * L
         o_p += C
-    monkeypatch.setenv("TTB_BEAM_GRAPH", "1")
-    for _ in range(2):   # graph-replayed iterations (no trace), first call capturing and second call reusing the graphs
+    for _ in range(2):   # no trace: iterations enqueued ahead, also on the second call on the same engine
         gen2 = TranslationInferenceBeamSearchSpeculative(eng, case["max_len"], case["n_best"], case["draft_len"], case["n_drafts"],
                                                          case["vocab"], True, 0, 1, 2, case["C_token"])
         assert np.array_equal(gen2.generate(src).cpu().numpy(), ref)

@@ -4,8 +4,8 @@
 //
 // Per iteration the engine runs
 //   beam_prepare  -> per-candidate bookkeeping (first free slot, finished flag, live-row prefix)
-//   beam_fill_rows-> (candidate, draft) decoder input rows, live candidates only
-//   decoder stack on the live rows (full-prefix, causal), gather of the dl+1 scored positions,
+//   beam_embed_cached -> last token + draft tokens of every live (candidate, draft) row
+//   decoder stack on the dl+1 positions of those rows (the prefix comes from the candidate's KV cache),
 //   classifier GEMM
 //   beam_stats    -> per (row, position): softmax max/sum, the n_best largest logits (sorted), size of
 //                    the nucleus-truncated support
@@ -18,9 +18,9 @@
 
 namespace ttb {
 // Accumulators of the loop control behind the BC_COUNT control words (reset by the CTA that finalises an iteration), and the
-// loop state the device carries itself so that an iteration's kernel arguments do not change from one iteration to the next
-// (the iteration is replayed as a CUDA graph): width of the token matrix and number of the CURRENT iteration, advanced by
-// the CTA that closes the iteration with the same rule the host applies (engine.cu:beam_api, speculative_decoding.py:452-470)
+// loop state the device carries itself so that an iteration can be enqueued before the host has read the outcome of the one
+// before it: width of the token matrix and number of the CURRENT iteration, advanced by the CTA that closes the iteration
+// with the same rule the host applies (engine.cu:beam_api, speculative_decoding.py:452-470)
 constexpr int BCX_ALL_FIN = BC_COUNT, BCX_MIN_PAD = BC_COUNT + 1, BCX_ACC = BC_COUNT + 2, BCX_CNT = BC_COUNT + 3, BCX_TICKET = BC_COUNT + 4,
               BCX_W = BC_COUNT + 5, BCX_ITER = BC_COUNT + 6,
               BCX_NLIVE_NEXT = BC_COUNT + 8,   // accumulator: new hypotheses without EOS = live candidates of the next iteration
@@ -115,11 +115,9 @@ __global__ void __launch_bounds__(1024) beam_prepare_kernel(BeamState st, int C,
                 if (!st.smart) {
                     st.live_cand[live] = c;
                     st.live_query[live] = c / beam;
-                    if (st.desc_self) {
-                        const int f = st.c_front[c];
-                        st.desc_self[live] = make_int4(c, f, st.cand_cur[(long long)c * st.ldw + f], 0x7fffffff);
-                        st.desc_cross[live] = make_int4(c / beam, 0, 0, st.src_len ? st.src_len[c / beam] : 0x7fffffff);
-                    }
+                    const int f = st.c_front[c];
+                    st.desc_self[live] = make_int4(c, f, st.cand_cur[(long long)c * st.ldw + f], 0x7fffffff);
+                    st.desc_cross[live] = make_int4(c / beam, 0, 0, st.src_len[c / beam]);
                 }
                 ++live;
             }
@@ -136,12 +134,13 @@ __global__ void __launch_bounds__(1024) beam_prepare_kernel(BeamState st, int C,
             const int* list = st.tok_list + ((long long)q * st.V + st.c_last[c]) * st.N;
             const int f = st.c_front[c];
             const int4 ds = make_int4(c, f, st.cand_cur[(long long)c * st.ldw + f], 0x7fffffff);
-            const int4 dc = make_int4(q, 0, 0, st.src_len ? st.src_len[q] : 0x7fffffff);
+            const int4 dc = make_int4(q, 0, 0, st.src_len[q]);
             for (int j = 0; j < cnt; ++j) {
                 st.live_cand[base + j] = c;
                 st.live_query[base + j] = q;
                 st.row_draft[base + j] = list[j];
-                if (st.desc_self) { st.desc_self[base + j] = ds; st.desc_cross[base + j] = dc; }
+                st.desc_self[base + j] = ds;
+                st.desc_cross[base + j] = dc;
             }
         }
     }
@@ -150,7 +149,7 @@ void launch_beam_prepare(const BeamState& st, int C, int beam, int dl, cudaStrea
     beam_prepare_kernel<<<1, 1024, 0, s>>>(st, C, beam, dl);
 }
 
-// ---- KV-cached decoder pass ---------------------------------------------------------------------------------
+// ---- decoder input: the candidate's prefix is in its KV cache -----------------------------------------------------
 // Row t = (live candidate g, draft n, position i): token = last token of the candidate (i = 0) or draft token i-1,
 // sequence position front + i.  Row order matches c_rowbase (rows of live candidate g start at g * N).
 template <typename ActT>
@@ -173,7 +172,7 @@ __global__ void beam_embed_cached_kernel(BeamState st, int beam, int dl, const f
         f = st.c_front[c];
         tok = (i == 0) ? st.cand_cur[(long long)c * st.ldw + f] : st.drafts[((long long)(c / beam) * st.N + n) * st.dl0 + i - 1];
     }
-    if (lane == 0 && st.row_tok) {   // the draft token at input position i is the "next draft token" of scored position i - 1
+    if (lane == 0) {   // the draft token at input position i is the "next draft token" of scored position i - 1
         if (i >= 1) st.row_tok[t - 1] = tok;
         if (i == dl) st.row_tok[t] = -1;
     }
@@ -242,50 +241,6 @@ template void launch_beam_cache_update<__nv_bfloat16>(const BeamState&, int, con
                                                       const __nv_bfloat16*, const __nv_bfloat16*, __nv_bfloat16*, __nv_bfloat16*, long long,
                                                       long long, cudaStream_t);
 
-__global__ void beam_fill_rows_kernel(BeamState st, int C, int beam, int W, int dl) {
-    const int c = blockIdx.x / st.N, n = blockIdx.x % st.N;
-    if (c >= C || st.c_fin[c]) return;
-    const int q = c / beam;
-    const int r = st.c_rowbase[c] + n;
-    const int slot0 = st.c_slot0[c];
-    const int* src = st.cand_cur + (long long)c * st.ldw;
-    const int* dr = st.drafts + ((long long)q * st.N + n) * st.dl0;
-    int* dst = st.rows_tok + (long long)r * W;
-    for (int j = threadIdx.x; j < W; j += blockDim.x) {
-        int t = src[j];
-        if (j >= slot0 && j < slot0 + dl) t = dr[j - slot0];
-        dst[j] = t;
-    }
-    if (threadIdx.x == 0) { st.row_cand[r] = c; st.row_query[r] = q; st.row_slot0[r] = slot0; }
-}
-void launch_beam_fill_rows(const BeamState& st, int C, int beam, int W, int dl, cudaStream_t s) {
-    beam_fill_rows_kernel<<<C * st.N, 128, 0, s>>>(st, C, beam, W, dl);
-}
-
-// rows of the residual stream that are scored: positions slot0-1 .. slot0+dl-1 of every live row
-template <typename ActT>
-__global__ void beam_gather_kernel(BeamState st, const float* __restrict__ x, const ActT* __restrict__ xh, int W, int dl, int E,
-                                   float* __restrict__ xg, ActT* __restrict__ xgh) {
-    const int t = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (t >= st.ctrl[BC_NLIVE_ROWS] * (dl + 1)) return;
-    const int r = t / (dl + 1), i = t % (dl + 1);
-    const long long src = ((long long)r * W + st.row_slot0[r] - 1 + i) * E, dst = (long long)t * E;
-    for (int c = lane; c < E; c += 32) {
-        if (xg) xg[dst + c] = x[src + c];
-        if (xgh) xgh[dst + c] = xh[src + c];
-    }
-}
-template <typename ActT>
-void launch_beam_gather(const BeamState& st, const float* x, const ActT* xh, int max_rows, int W, int dl, int E,
-                        float* xg, ActT* xgh, cudaStream_t s) {
-    const int T = max_rows * (dl + 1);
-    if (T <= 0) return;
-    beam_gather_kernel<ActT><<<(T + 7) / 8, 256, 0, s>>>(st, x, xh, W, dl, E, xg, xgh);
-}
-template void launch_beam_gather<float>(const BeamState&, const float*, const float*, int, int, int, int, float*, float*, cudaStream_t);
-template void launch_beam_gather<__nv_bfloat16>(const BeamState&, const float*, const __nv_bfloat16*, int, int, int, int, float*, __nv_bfloat16*, cudaStream_t);
-
 // ---- per (row, position) statistics -------------------------------------------------------------------
 // One warp per distribution: softmax max / sum, the K largest logits in descending order (ties: lower
 // token id first) and the size of the truncated support (exclusive cumulative probability < 0.9975,
@@ -300,7 +255,7 @@ __global__ void __launch_bounds__(256) beam_stats_kernel(BeamState st, const flo
     const float* p = logits + (long long)rp * V;
     float v[VPL];
     float mx = -INFINITY;
-    const int want = st.row_tok ? st.row_tok[rp] : -1;
+    const int want = st.row_tok[rp];
 #pragma unroll
     for (int k = 0; k < VPL; ++k) {
         const int c = lane + 32 * k;
@@ -446,14 +401,13 @@ __device__ __forceinline__ float ref_logprob(float logit, float mx, float sum) {
 // c_fin == 2 is absent (continuous loop: a query's first iteration has one candidate): it has no leaves.  `err` receives
 // error 4, `out` (optional) the new hypotheses at width W; `tally(k, fin, p, pads, has_eos)` feeds the loop control.
 template <typename Tally>
-__device__ __forceinline__ void expand_query(const BeamState& st, int q, int beam, int dl, int rs, int W, const float* __restrict__ logits,
-                                             int* err, long long* out, Tally tally) {
+__device__ __forceinline__ void expand_query(const BeamState& st, int q, int beam, int dl, int rs, int W, int* err, long long* out, Tally tally) {
     extern __shared__ float s_score[];                 // [beam][(dl+1)][K] leaf scores, -inf when absent
     __shared__ float s_red_v[256];
     __shared__ int s_red_i[256];
     __shared__ int s_sel[64];
     __shared__ int s_valid;
-    const int K = st.K, V = st.V, N = st.N;
+    const int K = st.K, N = st.N;
     const int per_c = (dl + 1) * K, total = beam * per_c;
     float* s_pre = s_score + total;                    // [beam][dl+2] running log-prob of the accepted path
     if (threadIdx.x == 0) s_valid = 0;
@@ -466,12 +420,11 @@ __device__ __forceinline__ void expand_query(const BeamState& st, int q, int bea
         if (lane == 0) s_pre[cb * (dl + 2)] = 0.f;
         if (!st.c_fin[c]) {
             const int n = st.c_pick[c], a = st.c_nacc[(long long)c * N + n], r = st.c_rowbase[c] + n;
-            const int* dr = cand_draft(st, c, q, n);
             for (int i0 = 0; i0 < a; i0 += 32) {
                 float term = 0.f;
                 if (i0 + lane < a) {
                     const long long rp = (long long)r * rs + i0 + lane;
-                    term = ref_logprob(st.tokv ? st.tokv[rp] : logits[rp * V + dr[i0 + lane]], st.lmax[rp], st.lsum[rp]);
+                    term = ref_logprob(st.tokv[rp], st.lmax[rp], st.lsum[rp]);
                 }
                 const int cnt = min(32, a - i0);
                 for (int i = 0; i < cnt; ++i) {
@@ -589,13 +542,13 @@ __device__ __forceinline__ void expand_query(const BeamState& st, int q, int bea
     }
 }
 
-__global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam, int dl, const float* __restrict__ logits) {
+__global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam, int dl) {
     pdl_wait();   // launched with the programmatic attribute: scheduled while the predecessor drains, starts when it is complete
     if (st.ctrl[BCX_DONE]) return;   // no-op iteration behind the end of the loop (the word of the last real iteration stays posted)
     const int q = blockIdx.x;
     const int W = st.ctrl[BCX_W];                      // rewritten only by the CTA that closes the iteration, after every CTA has arrived
     int* ctrl = st.ctrl;
-    expand_query(st, q, beam, dl, dl + 1, W, logits, &st.ctrl[BC_ERROR], nullptr, [ctrl](int, bool fin, int p, int pads, int has_eos) {
+    expand_query(st, q, beam, dl, dl + 1, W, &st.ctrl[BC_ERROR], nullptr, [ctrl](int, bool fin, int p, int pads, int has_eos) {
         if (!has_eos) { atomicAnd(&ctrl[BCX_ALL_FIN], 0); atomicAdd(&ctrl[BCX_NLIVE_NEXT], 1); }
         atomicMin(&ctrl[BCX_MIN_PAD], pads);
         if (!fin) { atomicAdd(&ctrl[BCX_ACC], p); atomicAdd(&ctrl[BCX_CNT], 1); }
@@ -641,10 +594,10 @@ __global__ void __launch_bounds__(256) beam_expand_kernel(BeamState st, int beam
         }
     }
 }
-void launch_beam_expand(const BeamState& st, int beam, int dl, const float* logits, cudaStream_t s) {
+void launch_beam_expand(const BeamState& st, int beam, int dl, cudaStream_t s) {
     const size_t smem = ((size_t)beam * (dl + 1) * st.K + (size_t)beam * (dl + 2)) * sizeof(float);
     if (ensure_dyn_smem(beam_expand_kernel, (int)smem)) return;   // error recorded; the launch below fails and cudaGetLastError reports it
-    launch_pdl(beam_expand_kernel, dim3(st.B), dim3(256), smem, s, st, beam, dl, logits);
+    launch_pdl(beam_expand_kernel, dim3(st.B), dim3(256), smem, s, st, beam, dl);
 }
 
 // ---- continuous batching: several batches share the query slots of one loop ----------------------------------------
@@ -881,7 +834,7 @@ void launch_beam_choose_groups(const BeamState& st, const BcTable& cb, int dl, c
 // open batch with the reference's stop rule (its own counters, error, width and draft length), frees the slots of the
 // batches that closed and posts the loop's word: sequence (24 bits) | slots in use (12) | largest draft length of the open
 // batches (8) | unfinished candidates of the next iteration (16).
-__global__ void __launch_bounds__(256) beam_expand_groups_kernel(BeamState st, BcTable cb, int rs, const float* __restrict__ logits) {
+__global__ void __launch_bounds__(256) beam_expand_groups_kernel(BeamState st, BcTable cb, int rs) {
     pdl_wait();   // launched with the programmatic attribute: scheduled while the predecessor drains, starts when it is complete
     const int q = blockIdx.x, K = st.K;
     const int g = cb.slot_group[q];
@@ -889,7 +842,7 @@ __global__ void __launch_bounds__(256) beam_expand_groups_kernel(BeamState st, B
         BcGroup* gr = &cb.groups[g];
         const int W = gr->W;
         int* ctrl = st.ctrl;
-        expand_query(st, q, K, gr->dl, rs, W, logits, &gr->error, gr->out + (long long)cb.slot_q[q] * K * W,
+        expand_query(st, q, K, gr->dl, rs, W, &gr->error, gr->out + (long long)cb.slot_q[q] * K * W,
                      [gr, ctrl](int, bool fin, int p, int pads, int has_eos) {
                          if (!has_eos) { atomicAnd(&gr->all_fin, 0); atomicAdd(&ctrl[BCX_NLIVE_NEXT], 1); }
                          atomicMin(&gr->min_pad, pads);
@@ -951,10 +904,10 @@ __global__ void __launch_bounds__(256) beam_expand_groups_kernel(BeamState st, B
         }
     }
 }
-void launch_beam_expand_groups(const BeamState& st, const BcTable& cb, int dl, const float* logits, cudaStream_t s) {
+void launch_beam_expand_groups(const BeamState& st, const BcTable& cb, int dl, cudaStream_t s) {
     const size_t smem = ((size_t)st.K * (dl + 1) * st.K + (size_t)st.K * (dl + 2)) * sizeof(float);
     if (ensure_dyn_smem(beam_expand_groups_kernel, (int)smem)) return;   // error recorded; the launch below fails and cudaGetLastError reports it
-    launch_pdl(beam_expand_groups_kernel, dim3(st.B), dim3(256), smem, s, st, cb, dl + 1, logits);
+    launch_pdl(beam_expand_groups_kernel, dim3(st.B), dim3(256), smem, s, st, cb, dl + 1);
 }
 
 __global__ void beam_init_kernel(BeamState st) {

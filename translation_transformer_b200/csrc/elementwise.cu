@@ -58,29 +58,6 @@ void launch_embed_seq(const int* tok, int T, int L, const float* table, const fl
 template void launch_embed_seq<float>(const int*, int, int, const float*, const float*, int, float*, float*, cudaStream_t);
 template void launch_embed_seq<__nv_bfloat16>(const int*, int, int, const float*, const float*, int, float*, __nv_bfloat16*, cudaStream_t);
 
-template <typename ActT>
-__global__ void embed_seq_rows_kernel(const int* __restrict__ tok, RowCount rows, int L, const float* __restrict__ table,
-                                      const float* __restrict__ pe, int E, float* __restrict__ x, ActT* __restrict__ xh) {
-    int row = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    int lane = threadIdx.x & 31;
-    if (row >= rows.live()) return;
-    const float* e = table + (long long)tok[row] * E;
-    const float* p = pe + (long long)((row % L) + 1) * E;
-    for (int c = lane; c < E; c += 32) {
-        float v = e[c] + p[c];
-        x[(long long)row * E + c] = v;
-        if (xh) xh[(long long)row * E + c] = from_f32<ActT>(v);
-    }
-}
-template <typename ActT>
-void launch_embed_seq_rows(const int* tok, RowCount rows, int L, const float* table, const float* pe, int E,
-                           float* x, ActT* xh, cudaStream_t s) {
-    if (rows.max_rows <= 0) return;
-    embed_seq_rows_kernel<ActT><<<(rows.max_rows + 7) / 8, 256, 0, s>>>(tok, rows, L, table, pe, E, x, xh);
-}
-template void launch_embed_seq_rows<float>(const int*, RowCount, int, const float*, const float*, int, float*, float*, cudaStream_t);
-template void launch_embed_seq_rows<__nv_bfloat16>(const int*, RowCount, int, const float*, const float*, int, float*, __nv_bfloat16*, cudaStream_t);
-
 // ---- residual add + LayerNorm (post-norm layers, modules.py:56-80; eps 1e-5) ----------------
 // Row statistics follow torch's CPU LayerNorm: mean, then biased variance of (x - mean).
 template <typename ActT, int MAXPL>

@@ -152,7 +152,7 @@ struct ttb_engine {
     // forward workspace (typed by the precision's activation type at use)
     DevBuf x, xh, y, qkv, att, q2, hid, logits, tok32, keytok32, pred;
     // encoder products / decoding state
-    DevBuf src32, srclen, desc, memory, memh, crosskv, crossvt, kcache, vcache, kcache2, vcache2, drafts, gen, front, active, ctrl, sel, out64;
+    DevBuf src32, srclen, desc, memory, memh, crosskv, kcache, vcache, kcache2, vcache2, drafts, gen, front, active, ctrl, sel, out64;
     int* h_ctrl = nullptr;  // pinned snapshots of ctrl for lagged polling
     cudaEvent_t poll_ev[4]{};
     cudaEvent_t t0{}, t1{};
@@ -165,10 +165,6 @@ struct ttb_engine {
     cudaGraphExec_t graph_exec[kBuckets][2] = {};   // greedy iteration graphs per live-query bucket (grids sized for the bucket) x {long, short}
     long long graph_key[13] = {};
     long long graph_launches = 0;
-    static constexpr int kBeamBuckets = 8;
-    cudaGraphExec_t beam_graph[2][kBeamBuckets] = {};   // steady-state iteration of the speculative beam search, per ping-pong parity and live-candidate bucket
-    long long beam_graph_key[20] = {};
-    long long beam_graph_launches = 0;
     DevBuf beam;                 // arena of the beam-search state
     DevBuf hist;                 // per-iteration live-query count of the last generate()
     DevBuf cb;                   // continuous batching: slot / batch tables and the staging buffers of an admitted batch
@@ -184,7 +180,7 @@ struct ttb_engine {
     // different host threads, translation_transformer_b200/pipeline.py)
     long long alloc_signature() const {
         const DevBuf* bufs[] = {&x, &xh, &y, &qkv, &att, &q2, &hid, &logits, &tok32, &keytok32, &pred, &src32, &srclen, &desc, &memory, &memh,
-                                &crosskv, &crossvt, &kcache, &vcache, &kcache2, &vcache2, &drafts, &gen, &front, &active, &ctrl, &sel, &out64, &beam, &hist, &cb, &cb_work};
+                                &crosskv, &kcache, &vcache, &kcache2, &vcache2, &drafts, &gen, &front, &active, &ctrl, &sel, &out64, &beam, &hist, &cb, &cb_work};
         unsigned long long h = 1469598103934665603ull;
         for (const DevBuf* b : bufs) {
             h = (h ^ (unsigned long long)reinterpret_cast<uintptr_t>(b->p)) * 1099511628211ull;
@@ -676,14 +672,8 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float)) || e->srclen.ensure((size_t)B * sizeof(int))) return 1;
     if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
     if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
-    // tcgen05 attention inside the loop (bf16, head_dim 32, key counts within its tensor-memory budget): the value caches
-    // are kept transposed ([dim][position], pitch VT_PITCH) so that both products read K-major operands.  The continuous
-    // loop runs the default attention kernels.
-    constexpr int VT_PITCH = 256;
-    const bool tc_attn = !cont && Prec<ActT>::lowp && !attn_simt_forced() && attention_tc_supported(HD, per_q, std::max(P, Ls), D + 1);
-    const size_t vcache_bytes = tc_attn ? (size_t)n_dec * B * E * VT_PITCH * sizeof(ActT) : (size_t)n_dec * B * P * E * sizeof(ActT);
-    if (e->kcache.ensure((size_t)n_dec * B * P * E * sizeof(ActT)) || e->vcache.ensure(vcache_bytes)) return 1;
-    if (tc_attn && e->crossvt.ensure((size_t)n_dec * B * E * VT_PITCH * sizeof(ActT))) return 1;
+    const size_t cache_bytes = (size_t)n_dec * B * P * E * sizeof(ActT);
+    if (e->kcache.ensure(cache_bytes) || e->vcache.ensure(cache_bytes)) return 1;
     if (e->drafts.ensure((size_t)B * N * D * sizeof(int)) || e->gen.ensure((size_t)B * gen_ld * sizeof(int))) return 1;
     if (e->front.ensure(B * sizeof(int)) || e->active.ensure(B * sizeof(int)) || e->ctrl.ensure(CTRL_COUNT * sizeof(int))) return 1;
     if (e->sel.ensure((size_t)B * 4 * sizeof(int)) || e->out64.ensure((size_t)B * max_len * sizeof(long long))) return 1;
@@ -753,7 +743,6 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
         TTB_CHECK(e->alloc_signature() == sig0, "a workspace buffer moved while decoding graphs of the continuous loop exist");
         return 0;
     };
-    const long long vt_q_stride = (long long)E * VT_PITCH, vt_l_stride = (long long)B * E * VT_PITCH;
     if (cont) {
         TTB_CUDA_OK(cudaMemsetAsync(st.ctrl, 0, CTRL_COUNT * sizeof(int), s));
     } else {
@@ -762,17 +751,6 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
     if (encode_impl<ActT>(e, src32, src32, B, Ls, mem, memh, s)) return 1;
     if (cross_kv_impl<ActT>(e, mem, memh, (int)TS, crosskv, s, TS_cap * 2 * E)) return 1;
-    if constexpr (Prec<ActT>::lowp) {
-        if (tc_attn) {
-            // every position a product can touch must hold a finite number (masked keys get probability 0, and 0 x NaN = NaN)
-            TTB_CUDA_OK(cudaMemsetAsync(e->vcache.p, 0, vcache_bytes, s));
-            TTB_CUDA_OK(cudaMemsetAsync(e->crossvt.p, 0, (size_t)n_dec * B * E * VT_PITCH * sizeof(ActT), s));
-            for (int l = 0; l < n_dec; ++l) {
-                Scope sc(e, KC_ENCODER, s);
-                launch_transpose_v(crosskv + (long long)l * TS_cap * 2 * E + E, 2 * E, B, Ls, E, e->crossvt.as<ActT>() + (long long)l * vt_l_stride, VT_PITCH, s);
-            }
-        }
-    }
     // drafts from the source without its BOS column (speculative_decoding.py:64-73)
     if (!standard) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Ls, B, Ls - 1, D, N, eos, pad, replace, e->drafts.as<int>(), s); }
     { Scope sc(e, KC_MISC, s); launch_greedy_init(st, s); }
@@ -793,13 +771,6 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     int Bq = B;
 
     auto self_attn = [&](int l, ActT* qkv, ActT* att) {
-        if constexpr (Prec<ActT>::lowp) {
-            if (tc_attn) {
-                launch_spec_self_attention_tc(qkv, 3 * E, kc + l * cache_l_stride, cache_q_stride, E, vc + l * vt_l_stride, vt_q_stride, VT_PITCH, att, E,
-                                              Bq, n_active, st.gen, gen_ld, e->d.tgt_pad_token_idx, N, D, H, st.desc, s);
-                return;
-            }
-        }
         spec_attn(qkv, 3 * E, kc + l * cache_l_stride, vc + l * cache_l_stride, cache_q_stride, E,
                                          att, E, Bq, n_active, st.active, st.front, st.gen, gen_ld, e->d.tgt_pad_token_idx,
                                          N, D, H, HD, P, s, st.desc);
@@ -810,15 +781,6 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
             attn(q2, E, kv, kv + E, 2 * E, att, E, Bq, n_active, per_q, Ls_cap, Ls_cap, st.active, e->keytok32.as<int>(), Ls_cap,
                  e->d.src_pad_token_idx, false, H, HD, s, st.ctrl + CTRL_LS, e->srclen.as<int>(), st.desc);
             return;
-        }
-        if constexpr (Prec<ActT>::lowp) {
-            if (tc_attn) {
-                // the K/V rows of a query start at row query * Ls of the layer's block (the batch's own source length, read on the
-                // device by the kernel: the row stride of a group is Ls * 2E elements)
-                launch_cross_attention_tc(q2, E, kv, 2 * E, (long long)Ls * 2 * E, e->crossvt.as<ActT>() + (long long)l * vt_l_stride, vt_q_stride, VT_PITCH,
-                                          att, E, Bq, n_active, per_q, src32, Ls, e->d.src_pad_token_idx, st.ctrl + CTRL_LS, H, st.desc, s);
-                return;
-            }
         }
         attn(q2, E, kv, kv + E, 2 * E, att, E, Bq, n_active, per_q, Ls, Ls, st.active,
              src32, Ls, e->d.src_pad_token_idx, false, H, HD, s, st.ctrl + CTRL_LS, e->srclen.as<int>(), st.desc);
@@ -831,7 +793,7 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
             GreedyState stq = st;
             stq.B = Bq;               // grid sizing only: the kernel indexes the live slots, all below the bucket
             launch_greedy_advance<ActT>(stq, e->tgt_emb, e->pe, E, x, xh, e->qkv.as<ActT>(), qkv_l_stride, n_dec, 3 * E, kc, vc,
-                                        cache_l_stride, cache_q_stride, E, s, tc_attn ? vt_l_stride : 0, tc_attn ? vt_q_stride : 0, tc_attn ? VT_PITCH : 0);
+                                        cache_l_stride, cache_q_stride, E, s);
         }
         if (decoder_stack<ActT>(e, rows, n_dec, qkv_l_stride, self_attn, cross_attn, s)) return 1;
         bool fused_cls = false;
@@ -886,7 +848,7 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     }
     if (use_graph) {
         const long long key[13] = {B, N, D, standard ? 1 : (cont ? 2 : 0), max_len, pad, bos, eos, tie_break, e->alloc_signature(),
-                                   (long long)sizeof(ActT) + 16 * K_it + (tc_attn ? 1024 : 0), replace, cont ? Ls_cap : 0};
+                                   (long long)sizeof(ActT) + 16 * K_it, replace, cont ? Ls_cap : 0};
         if (memcmp(key, e->graph_key, sizeof(key)) != 0) {
             for (auto& gb : e->graph_exec) for (auto& g : gb) if (g) { cudaGraphExecDestroy(g); g = nullptr; }
             memcpy(e->graph_key, key, sizeof(key));
@@ -1108,33 +1070,25 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     const long long TS_cap = (long long)B * Ls_cap;
     const int Cmax = B * K, Rmax = Cmax * N;
     const int ldw = max_len + D0 + 4;
-    // KV-cached pass (default): only the dl+1 scored positions of every (candidate, draft) row go through the decoder,
-    // the prefix of a candidate is served from its self-attention cache, which follows the hypotheses through the
-    // re-parenting of every step.  TTB_BEAM_NO_CACHE=1 keeps the full-prefix recomputation (A/B comparisons).
-    static const bool no_cache = [] { const char* v = getenv("TTB_BEAM_NO_CACHE"); return v && v[0] == '1'; }();
-    const bool cached = !no_cache;
-    TTB_CHECK(cached || !smart, "smart_drafts_mode needs the KV-cached decoder pass (unset TTB_BEAM_NO_CACHE)");
+    // only the dl+1 scored positions of every (candidate, draft) row go through the decoder, the prefix of a candidate is
+    // served from its self-attention cache, which follows the hypotheses through the re-parenting of every step
     const bool cont = cb != nullptr;
-    TTB_CHECK(cached || !cont, "continuous batching needs the KV-cached decoder pass (unset TTB_BEAM_NO_CACHE)");
     // continuous loop: the encoder of an admitted batch runs on the largest batch shape, in a workspace of its own
     int B_stage = 0;
     long long TS_stage = 0;
     if (cont)
         for (int i = 0; i < cb->n; ++i) { B_stage = std::max(B_stage, (int)cb->bs[i]); TS_stage = std::max(TS_stage, (long long)cb->bs[i] * cb->ls[i]); }
     const long long Tc = (long long)Rmax * (D0 + 1);
-    const long long Tmax = cached ? Tc : (long long)Rmax * ldw;
 
     const long long TS_enc = cont ? TS_stage : TS_cap;
     if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float))) return 1;
     if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
     if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
     if (e->drafts.ensure(smart ? (size_t)B * std::max(n_lib, Ls_cap) * D_lib * sizeof(int) : (size_t)B * N * D0 * sizeof(int))) return 1;
-    if (ensure_work<ActT>(e, cont ? Tmax : std::max(Tmax, TS_cap), cached ? n_dec : 1)) return 1;
+    if (ensure_work<ActT>(e, cont ? Tc : std::max(Tc, TS_cap), n_dec)) return 1;
     const long long cache_c_stride = (long long)ldw * E, cache_l_stride = (long long)Cmax * ldw * E;
-    if (cached) {
-        const size_t cbytes = (size_t)n_dec * cache_l_stride * sizeof(ActT);
-        if (e->kcache.ensure(cbytes) || e->vcache.ensure(cbytes) || e->kcache2.ensure(cbytes) || e->vcache2.ensure(cbytes)) return 1;
-    }
+    const size_t cbytes = (size_t)n_dec * cache_l_stride * sizeof(ActT);
+    if (e->kcache.ensure(cbytes) || e->vcache.ensure(cbytes) || e->kcache2.ensure(cbytes) || e->vcache2.ensure(cbytes)) return 1;
     DevBuf& bb = e->beam;
     // one arena for the small beam buffers
     size_t off = 0;
@@ -1143,10 +1097,9 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     const size_t o_lp0 = take(Cmax * 4), o_lp1 = take(Cmax * 4);
     const size_t o_slot = take(Cmax * 4), o_fin = take(Cmax * 4), o_base = take(Cmax * 4), o_nacc = take((size_t)Cmax * N * 4);
     const size_t o_pick = take(Cmax * 4), o_acc = take(Cmax * 4), o_ctrl = take(32 * 4);   // control words + loop-control accumulators
-    const size_t o_rows = take((size_t)Rmax * ldw * 4), o_rc = take(Rmax * 4), o_rq = take(Rmax * 4), o_rs = take(Rmax * 4);
     const size_t n_rp = (size_t)Rmax * (D0 + 1);
     const size_t o_topv = take(n_rp * K * 4), o_topi = take(n_rp * K * 4), o_keep = take(n_rp * 4), o_max = take(n_rp * 4), o_sum = take(n_rp * 4);
-    const size_t o_xg = take(n_rp * E * 4), o_xgh = take(n_rp * E * 2), o_lg = take(n_rp * V * 4), o_rt = take(n_rp * 4), o_tv = take(n_rp * 4);
+    const size_t o_lg = take(n_rp * V * 4), o_rt = take(n_rp * 4), o_tv = take(n_rp * 4);
     const size_t o_lc = take(Rmax * 4), o_lq = take(Rmax * 4), o_cf = take(Cmax * 4), o_np = take(Cmax * 4), o_nk = take(Cmax * 4), o_nr = take(Cmax * 4);
     const size_t o_tc = take(smart ? (size_t)B * V * 4 : 4), o_tl = take(smart ? (size_t)B * V * N * 4 : 4), o_cc = take(Cmax * 4),
                  o_cl = take(Cmax * 4), o_rd = take(Rmax * 4), o_ds = take(Rmax * 16), o_dc = take(Rmax * 16);
@@ -1207,7 +1160,6 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     st.drafts = e->drafts.as<int>();
     st.c_slot0 = (int*)(base + o_slot); st.c_fin = (int*)(base + o_fin); st.c_rowbase = (int*)(base + o_base);
     st.c_nacc = (int*)(base + o_nacc); st.c_pick = (int*)(base + o_pick); st.acc_stat = (int*)(base + o_acc); st.ctrl = (int*)(base + o_ctrl);
-    st.rows_tok = (int*)(base + o_rows); st.row_cand = (int*)(base + o_rc); st.row_query = (int*)(base + o_rq); st.row_slot0 = (int*)(base + o_rs);
     st.topv = (float*)(base + o_topv); st.topi = (int*)(base + o_topi); st.nkeep = (int*)(base + o_keep);
     st.lmax = (float*)(base + o_max); st.lsum = (float*)(base + o_sum);
     st.trace_nacc = trace_nacc; st.trace_pick = trace_pick;
@@ -1217,27 +1169,22 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
         st.host_ctrl = cudaHostGetDevicePointer(&dp, e->h_ctrl + 16, 0) == cudaSuccess ? static_cast<int*>(dp) : nullptr;
         (void)cudaGetLastError();
     }
-    if (cached) { st.row_tok = (int*)(base + o_rt); st.tokv = (float*)(base + o_tv); }
+    st.row_tok = (int*)(base + o_rt); st.tokv = (float*)(base + o_tv);
     st.live_cand = (int*)(base + o_lc); st.live_query = (int*)(base + o_lq); st.c_front = (int*)(base + o_cf);
     st.n_parent = (int*)(base + o_np); st.n_keep = (int*)(base + o_nk); st.n_row = (int*)(base + o_nr);
     st.tok_cnt = (int*)(base + o_tc); st.tok_list = (int*)(base + o_tl); st.c_cnt = (int*)(base + o_cc); st.c_last = (int*)(base + o_cl);
     st.row_draft = (int*)(base + o_rd);
-    static const bool no_desc = [] { const char* v = getenv("TTB_BEAM_NO_DESC"); return v && v[0] == '1'; }();
-    if (cont) {   // per-slot source lengths, installed by the admission kernel
-        st.desc_self = (int4*)(base + o_ds); st.desc_cross = (int4*)(base + o_dc); st.src_len = e->srclen.as<int>();
-    } else if (cached && !no_desc) {
+    if (!cont) {   // continuous loop: per-slot source lengths, installed by the admission kernel
         // per-query source length: the cross-attention kernels skip the padding behind it
         if (e->srclen.ensure((size_t)B * sizeof(int))) return 1;
         { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
-        st.desc_self = (int4*)(base + o_ds); st.desc_cross = (int4*)(base + o_dc); st.src_len = e->srclen.as<int>();
     }
-    ActT* kc_cur = cached ? e->kcache.as<ActT>() : nullptr;
-    ActT* vc_cur = cached ? e->vcache.as<ActT>() : nullptr;
-    ActT* kc_next = cached ? e->kcache2.as<ActT>() : nullptr;
-    ActT* vc_next = cached ? e->vcache2.as<ActT>() : nullptr;
+    st.desc_self = (int4*)(base + o_ds); st.desc_cross = (int4*)(base + o_dc); st.src_len = e->srclen.as<int>();
+    ActT* kc_cur = e->kcache.as<ActT>();
+    ActT* vc_cur = e->vcache.as<ActT>();
+    ActT* kc_next = e->kcache2.as<ActT>();
+    ActT* vc_next = e->vcache2.as<ActT>();
     const int* n_live_cands = st.ctrl + BC_NLIVE_CANDS;
-    float* xg = (float*)(base + o_xg);
-    ActT* xgh = Prec<ActT>::lowp ? (ActT*)(base + o_xgh) : nullptr;
     float* logits = (float*)(base + o_lg);
     if (cont) {
         TTB_CHECK(st.host_ctrl, "continuous batching needs mapped pinned host memory for its control word");
@@ -1254,21 +1201,7 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     ActT* xh = Prec<ActT>::lowp ? e->xh.as<ActT>() : nullptr;
     const int* n_live = st.ctrl + BC_NLIVE_ROWS;
     int W = 1, empty_cols = 0, filled = 1, budget = max_len - filled - 1, dl = smart ? D_lib - 1 : D0, C = B, beam = 1, iters = 0;
-    // CUDA graphs of the steady-state iteration (one per parity), kept across calls while nothing they bake in changes
-    const int dl_steady = dl;
-    // Opt-in (TTB_BEAM_GRAPH=1, read per call): measured neutral on one B200 -- the search is bound by the GPU work of its
-    // 5-20 k token rows, not by the ~33 launches per iteration (63.8 ms per batch launched directly, 64.5 ms replayed, the
-    // graphs being re-captured whenever the padded source length changes), see DESIGN.md §2b.
-    const char* ng = getenv("TTB_BEAM_GRAPH");
-    const bool use_graph = !cont && cached && st.host_ctrl && !trace_nacc && !trace_pick && e->prof.mask == 0 && ng && ng[0] == '1';
-    if (use_graph) {
-        const long long key[20] = {B, K, N, D0, Ls, max_len, V, smart ? 1 : 0, pad, bos, eos, c_token, tie_break, e->alloc_signature(),
-                                   (long long)sizeof(ActT), (long long)reinterpret_cast<uintptr_t>(st.host_ctrl), n_dec, 0, 0, 0};
-        if (memcmp(key, e->beam_graph_key, sizeof(key)) != 0) {
-            for (auto& gp : e->beam_graph) for (auto& g : gp) if (g) { cudaGraphExecDestroy(g); g = nullptr; }
-            memcpy(e->beam_graph_key, key, sizeof(key));
-        }
-    }
+    const int dl_steady = dl;   // full draft length: an iteration at it may be enqueued ahead (host loop below)
     int* hc = e->h_ctrl;
     hc[BC_ERROR] = 0;
     // the two hypothesis / score / cache buffer sets: iteration i (0-based) reads set i & 1 and writes the other one
@@ -1279,9 +1212,8 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
 
     // One iteration = a fixed kernel sequence whose arguments depend on (C, beam, dl) and on the ping-pong parity of the
     // hypothesis / cache buffers only: the width of the token matrix and the iteration number live in device memory
-    // (beam.cu: BCX_W, BCX_ITER), so the steady state (C = B K, full draft length) can be replayed as a CUDA graph and
-    // -- because the device also applies the stop rule itself (BCX_DONE) -- be enqueued AHEAD of the host reading the
-    // outcome of the iteration before it.
+    // (beam.cu: BCX_W, BCX_ITER), and the device applies the stop rule itself (BCX_DONE), so the steady state (C = B K,
+    // full draft length) can be enqueued AHEAD of the host reading the outcome of the iteration before it.
     // `Cb`: upper bound of the candidates that are still unfinished in this iteration (exact when the host has read the word
     // of the iteration before, C otherwise): the decoder-side grids are sized for Cb * N rows instead of C * N, so that the
     // no-op CTAs of finished candidates do not queue for SMs that the other batches in flight are using (§4c of DESIGN.md)
@@ -1291,110 +1223,58 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
         st.logp_cur = logp_set[parity]; st.logp_next = logp_set[parity ^ 1];
         kc_cur = kc_set[parity]; kc_next = kc_set[parity ^ 1];
         vc_cur = vc_set[parity]; vc_next = vc_set[parity ^ 1];
-        // replayed iterations bake their grids in: the live-candidate bound is rounded up to one of eight buckets of C
-        const bool graph_it = use_graph && C == B * K && beam == K && dl == dl_steady;
-        int gb = 0;
-        if (graph_it && !smart) {
-            const int want = std::min(C, std::max(1, Cb));
-            while (gb + 1 < ttb_engine::kBeamBuckets && (C * (ttb_engine::kBeamBuckets - gb - 1) + ttb_engine::kBeamBuckets - 1) / ttb_engine::kBeamBuckets >= want) ++gb;
-            Cb = (C * (ttb_engine::kBeamBuckets - gb) + ttb_engine::kBeamBuckets - 1) / ttb_engine::kBeamBuckets;
-        }
-        auto body = [&]() -> int {
         const int R = (smart && !cont ? C : std::min(C, std::max(1, Cb))) * N;
         bool fused_stats = false;
         if (cont) { Scope sc(e, KC_MISC, s); launch_beam_prepare_groups(st, cbt, s); }
         else { Scope sc(e, KC_MISC, s); launch_beam_prepare(st, C, beam, dl, s); }
-        if (cached) {
-            RowCount rows(R * (dl + 1), n_live, dl + 1);
-            { Scope sc(e, KC_EMBED, s); launch_beam_embed_cached<ActT>(st, beam, R, dl, e->tgt_emb, e->pe, E, x, xh, s); }
-            // attention groups: the N rows of a live candidate share its cache prefix; in smart mode candidates own a
-            // different number of rows, so every row is a group of its own
-            const int G = smart ? R : R / N, n_per_group = smart ? 1 : N;
-            auto self_attn = [&](int l, ActT* qkv, ActT* att) {
-                // continuous loop: a candidate's draft rows are its batch's dl + 1 positions long (desc_self.w), whatever the
-                // call's dl, so that the tensor-core kernel lays out its keys as generate() does
-                spec_attn(qkv, 3 * E, kc_cur + l * cache_l_stride, vc_cur + l * cache_l_stride, cache_c_stride, E, att, E, G, n_live_cands,
-                          st.live_cand, st.c_front, st.cand_cur, ldw, e->d.tgt_pad_token_idx, n_per_group, dl, H, HD, ldw, s, st.desc_self, cont);
-            };
-            auto cross_attn = [&](int l, ActT* q2, ActT* att) {
-                const ActT* kv = crosskv + (long long)l * ckv_l_stride;
-                if (cont)   // slot-major K/V rows and key tokens, row stride Ls_cap per slot
-                    attn(q2, E, kv, kv + E, 2 * E, att, E, G, n_live_cands, n_per_group * (dl + 1), Ls_cap, Ls_cap, st.live_query,
-                         e->keytok32.as<int>(), Ls_cap, e->d.src_pad_token_idx, false, H, HD, s, nullptr, nullptr, st.desc_cross);
-                else
-                    attn(q2, E, kv, kv + E, 2 * E, att, E, G, n_live_cands, n_per_group * (dl + 1), Ls, Ls, st.live_query,
-                         src32, Ls, e->d.src_pad_token_idx, false, H, HD, s, nullptr, nullptr, st.desc_cross);
-            };
-            if (decoder_stack<ActT>(e, rows, n_dec, Tc * 3 * E, self_attn, cross_attn, s)) return 1;
-            // every decoder row is a scored position.  bf16 path: the projection is fused with the statistics the search reads
-            // (logits stay in tensor memory); otherwise logits straight from the residual stream + beam_stats below
-            if constexpr (Prec<ActT>::lowp) {
-                const char* nf = getenv("TTB_NO_FUSED_STATS");
-                if (!(nf && nf[0] == '1')) {
-                    Scope sc(e, KC_GEMM_CLASSIFIER, s);
-                    const int rc = launch_classifier_stats(xh, E, e->classifier.wh, e->classifier.b, rows, V, E, K, st.row_tok, st.tokv, st.lmax, st.lsum,
-                                                           st.nkeep, st.topv, st.topi, s);
-                    if (rc > 0) return 1;
-                    fused_stats = rc == 0;
-                    if (!fused_stats) e->launches--;
-                }
+        RowCount rows(R * (dl + 1), n_live, dl + 1);
+        { Scope sc(e, KC_EMBED, s); launch_beam_embed_cached<ActT>(st, beam, R, dl, e->tgt_emb, e->pe, E, x, xh, s); }
+        // attention groups: the N rows of a live candidate share its cache prefix; in smart mode candidates own a
+        // different number of rows, so every row is a group of its own
+        const int G = smart ? R : R / N, n_per_group = smart ? 1 : N;
+        auto self_attn = [&](int l, ActT* qkv, ActT* att) {
+            // continuous loop: a candidate's draft rows are its batch's dl + 1 positions long (desc_self.w), whatever the
+            // call's dl, so that the tensor-core kernel lays out its keys as generate() does
+            spec_attn(qkv, 3 * E, kc_cur + l * cache_l_stride, vc_cur + l * cache_l_stride, cache_c_stride, E, att, E, G, n_live_cands,
+                      st.live_cand, st.c_front, st.cand_cur, ldw, e->d.tgt_pad_token_idx, n_per_group, dl, H, HD, ldw, s, st.desc_self, cont);
+        };
+        auto cross_attn = [&](int l, ActT* q2, ActT* att) {
+            const ActT* kv = crosskv + (long long)l * ckv_l_stride;
+            if (cont)   // slot-major K/V rows and key tokens, row stride Ls_cap per slot
+                attn(q2, E, kv, kv + E, 2 * E, att, E, G, n_live_cands, n_per_group * (dl + 1), Ls_cap, Ls_cap, st.live_query,
+                     e->keytok32.as<int>(), Ls_cap, e->d.src_pad_token_idx, false, H, HD, s, nullptr, nullptr, st.desc_cross);
+            else
+                attn(q2, E, kv, kv + E, 2 * E, att, E, G, n_live_cands, n_per_group * (dl + 1), Ls, Ls, st.live_query,
+                     src32, Ls, e->d.src_pad_token_idx, false, H, HD, s, nullptr, nullptr, st.desc_cross);
+        };
+        if (decoder_stack<ActT>(e, rows, n_dec, Tc * 3 * E, self_attn, cross_attn, s)) return 1;
+        // every decoder row is a scored position.  bf16 path: the projection is fused with the statistics the search reads
+        // (logits stay in tensor memory); otherwise logits straight from the residual stream + beam_stats below
+        if constexpr (Prec<ActT>::lowp) {
+            const char* nf = getenv("TTB_NO_FUSED_STATS");
+            if (!(nf && nf[0] == '1')) {
+                Scope sc(e, KC_GEMM_CLASSIFIER, s);
+                const int rc = launch_classifier_stats(xh, E, e->classifier.wh, e->classifier.b, rows, V, E, K, st.row_tok, st.tokv, st.lmax, st.lsum,
+                                                       st.nkeep, st.topv, st.topi, s);
+                if (rc > 0) return 1;
+                fused_stats = rc == 0;
+                if (!fused_stats) e->launches--;
             }
-            if (!fused_stats && linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, logits, V, rows, false, s)) return 1;
-        } else {
-            const int Wit = W;   // full-prefix recomputation (A/B path): never enqueued ahead, the host's width is exact
-            { Scope sc(e, KC_MISC, s); launch_beam_fill_rows(st, C, beam, Wit, dl, s); }
-            RowCount rows(R * Wit, n_live, Wit);
-            { Scope sc(e, KC_EMBED, s); launch_embed_seq_rows<ActT>(st.rows_tok, rows, Wit, e->tgt_emb, e->pe, E, x, xh, s); }
-            auto self_attn = [&](int, ActT* qkv, ActT* att) {
-                attn(qkv, 3 * E, qkv + E, qkv + 2 * E, 3 * E, att, E, R, n_live, Wit, Wit, Wit, nullptr,
-                     st.rows_tok, Wit, e->d.tgt_pad_token_idx, true, H, HD, s);
-            };
-            auto cross_attn = [&](int l, ActT* q2, ActT* att) {
-                const ActT* kv = crosskv + (long long)l * ckv_l_stride;
-                attn(q2, E, kv, kv + E, 2 * E, att, E, R, n_live, Wit, Ls, Ls, st.row_query,
-                     src32, Ls, e->d.src_pad_token_idx, false, H, HD, s);
-            };
-            if (decoder_stack<ActT>(e, rows, 1, 0, self_attn, cross_attn, s)) return 1;
-            { Scope sc(e, KC_MISC, s); launch_beam_gather<ActT>(st, x, xh, R, Wit, dl, E, Prec<ActT>::lowp ? nullptr : xg, xgh, s); }
-            RowCount rp_rows(R * (dl + 1), n_live, dl + 1);
-            if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(xg, xgh), E, e->classifier, logits, V, rp_rows, false, s)) return 1;
         }
+        if (!fused_stats && linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, logits, V, rows, false, s)) return 1;
         if (!fused_stats) { Scope sc(e, KC_ARGMAX, s); launch_beam_stats(st, logits, R, dl, s); }
         if (cont) { Scope sc(e, KC_ACCEPT, s); launch_beam_choose_groups(st, cbt, dl, s); }
         else { Scope sc(e, KC_ACCEPT, s); launch_beam_choose(st, C, beam, dl, s); }
         // the expand kernel also closes the iteration: its last CTA writes the control words and, last, the iteration's
         // sequence number into pinned host memory; the host reads them while the caches are still being re-parented
-        if (cont) { Scope sc(e, KC_ACCEPT, s); launch_beam_expand_groups(st, cbt, dl, logits, s); }
-        else { Scope sc(e, KC_ACCEPT, s); launch_beam_expand(st, beam, dl, logits, s); }
-        if (cached) {
+        if (cont) { Scope sc(e, KC_ACCEPT, s); launch_beam_expand_groups(st, cbt, dl, s); }
+        else { Scope sc(e, KC_ACCEPT, s); launch_beam_expand(st, beam, dl, s); }
+        {
             Scope sc(e, KC_CACHE_APPEND, s);
             launch_beam_cache_update<ActT>(st, dl, e->qkv.as<ActT>(), Tc * 3 * E, n_dec, 3 * E, E, kc_cur, vc_cur, kc_next, vc_next,
                                            cache_l_stride, cache_c_stride, s);
         }
         return 0;
-        };   // body
-        if (graph_it) {
-            if (!e->beam_graph[parity][gb]) {
-                const long long l0 = e->launches;
-                cudaGraph_t graph = nullptr;
-                TTB_CUDA_OK(cudaStreamBeginCapture(s, cudaStreamCaptureModeRelaxed));
-                const int rc = body();
-                const cudaError_t ce = cudaStreamEndCapture(s, &graph);
-                if (rc || ce != cudaSuccess) {
-                    if (graph) cudaGraphDestroy(graph);
-                    if (!rc) set_last_error(std::string("CUDA graph capture of the beam-search iteration failed: ") + cudaGetErrorString(ce));
-                    return 1;
-                }
-                TTB_CUDA_OK(cudaGraphInstantiate(&e->beam_graph[parity][gb], graph, 0));
-                cudaGraphDestroy(graph);
-                e->beam_graph_launches = e->launches - l0;
-                e->launches = l0;   // capturing did not launch anything
-            }
-            TTB_CUDA_OK(cudaGraphLaunch(e->beam_graph[parity][gb], s));
-            e->launches += e->beam_graph_launches;
-            return 0;
-        }
-        return body();
     };
     // wait for the packed word the expand kernel posts for iteration `seq` (sequence | error | all finished | empty columns)
     static const bool pure_spin = [] { const char* v = getenv("TTB_BEAM_SPIN"); return v && v[0] == '1'; }();
@@ -1549,7 +1429,7 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
         return 0;
     }
     static const bool no_ahead = [] { const char* v = getenv("TTB_BEAM_NO_AHEAD"); return v && v[0] == '1'; }();
-    const bool ahead_ok = cached && st.host_ctrl && !no_ahead && !trace_nacc && !trace_pick;
+    const bool ahead_ok = st.host_ctrl && !no_ahead && !trace_nacc && !trace_pick;
     int enq = 0, dl_enq = dl;
     bool ended = false;
     while (!ended) {
@@ -1627,8 +1507,10 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
 }
 
 // ---- standard beam search (standard_decoding.py:90-174), host loop + device kernels -----------------------------
-// One decoder call per generated column on the hypotheses that have not produced EOS (full prefix, no KV cache yet);
-// tokens, scores and logits stay on the device, the host reads two control words per step for the stop test.
+// One decoder call per generated column on the hypotheses that have not produced EOS, one new token each (the prefix of a
+// hypothesis is served from its self-attention cache, which follows the hypotheses through the re-parenting of every step,
+// in two ping-pong copies); tokens, scores and logits stay on the device, the host reads the control words of the stop
+// test one step behind.
 template <typename ActT>
 static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int max_len, int K, int pad, int bos, int eos,
                         int64_t* out_dev, int32_t* out_width, ttb_generate_stats* stats, cudaStream_t user_stream) {
@@ -1641,36 +1523,23 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
     const long long TS = (long long)B * Ls;
     const long long TS_cap = (long long)B * std::max(256, (Ls + 63) / 64 * 64);   // no reallocation from one batch length to the next
     const int Cmax = B * K, ldw = max_len;
-    const long long Tmax = (long long)Cmax * max_len;
 
     if (e->src32.ensure(TS_cap * sizeof(int)) || e->memory.ensure(TS_cap * E * sizeof(float))) return 1;
     if (Prec<ActT>::lowp && e->memh.ensure(TS_cap * E * sizeof(ActT))) return 1;
     if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
-    {
-        const char* v = getenv("TTB_SBEAM_NO_CACHE");
-        if (ensure_work<ActT>(e, (v && v[0] == '1') ? std::max(Tmax, TS_cap) : std::max<long long>(Cmax, TS_cap), 1)) return 1;
-    }
+    if (ensure_work<ActT>(e, std::max<long long>(Cmax, TS_cap), n_dec)) return 1;
     DevBuf& bb = e->beam;
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
     const size_t o_y0 = take((size_t)Cmax * ldw * 4), o_y1 = take((size_t)Cmax * ldw * 4);
     const size_t o_s0 = take(Cmax * 4), o_s1 = take(Cmax * 4), o_fin = take(Cmax * 4), o_cr = take(Cmax * 4), o_rc = take(Cmax * 4),
-                 o_rq = take(Cmax * 4), o_rows = take((size_t)Cmax * ldw * 4), o_tot = take((size_t)Cmax * V * 4), o_ctrl = take(64),
-                 o_xg = take((size_t)Cmax * E * 4), o_xgh = take((size_t)Cmax * E * 2), o_lg = take((size_t)Cmax * V * 4),
+                 o_rq = take(Cmax * 4), o_tot = take((size_t)Cmax * V * 4), o_ctrl = take(64), o_lg = take((size_t)Cmax * V * 4),
                  o_cf = take(Cmax * 4), o_par = take(Cmax * 4), o_ds = take(Cmax * 16), o_dc = take(Cmax * 16);
     if (bb.ensure(off)) return 1;
-    // KV-cached pass (default): one new token per live hypothesis and step, the prefix of a hypothesis is served from its
-    // self-attention cache, which follows the hypotheses through the re-parenting of every step (two ping-pong copies).
-    // TTB_SBEAM_NO_CACHE=1 keeps the reference-like full-prefix recomputation (A/B runs).
-    static const bool sb_no_cache = [] { const char* v = getenv("TTB_SBEAM_NO_CACHE"); return v && v[0] == '1'; }();
-    const bool cached = !sb_no_cache;
     const long long cache_c_stride = (long long)max_len * E, cache_l_stride = (long long)Cmax * max_len * E;
-    if (cached) {
-        const size_t cbytes = (size_t)n_dec * cache_l_stride * sizeof(ActT);
-        if (e->kcache.ensure(cbytes) || e->vcache.ensure(cbytes) || e->kcache2.ensure(cbytes) || e->vcache2.ensure(cbytes)) return 1;
-        if (e->srclen.ensure((size_t)B * sizeof(int))) return 1;
-        if (ensure_work<ActT>(e, std::max<long long>(Cmax, TS_cap), n_dec)) return 1;
-    }
+    const size_t cbytes = (size_t)n_dec * cache_l_stride * sizeof(ActT);
+    if (e->kcache.ensure(cbytes) || e->vcache.ensure(cbytes) || e->kcache2.ensure(cbytes) || e->vcache2.ensure(cbytes)) return 1;
+    if (e->srclen.ensure((size_t)B * sizeof(int))) return 1;
     char* base = bb.as<char>();
 
     TTB_CUDA_OK(cudaEventRecord(e->t0, s));
@@ -1687,19 +1556,14 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
     st.y_cur = (int*)(base + o_y0); st.y_next = (int*)(base + o_y1);
     st.score_cur = (float*)(base + o_s0); st.score_next = (float*)(base + o_s1);
     st.fin = (int*)(base + o_fin); st.cand_row = (int*)(base + o_cr); st.row_cand = (int*)(base + o_rc); st.row_query = (int*)(base + o_rq);
-    st.rows_tok = (int*)(base + o_rows); st.total = (float*)(base + o_tot); st.ctrl = (int*)(base + o_ctrl);
-    float* xg = (float*)(base + o_xg);
-    ActT* xgh = Prec<ActT>::lowp ? (ActT*)(base + o_xgh) : nullptr;
+    st.total = (float*)(base + o_tot); st.ctrl = (int*)(base + o_ctrl);
     float* logits = (float*)(base + o_lg);
-    ActT *kc_cur = nullptr, *vc_cur = nullptr, *kc_next = nullptr, *vc_next = nullptr;
     int* const y_set[2] = {st.y_cur, st.y_next};
-    if (cached) {
-        st.c_front = (int*)(base + o_cf); st.parent = (int*)(base + o_par);
-        st.desc_self = (int4*)(base + o_ds); st.desc_cross = (int4*)(base + o_dc);
-        { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
-        st.src_len = e->srclen.as<int>();
-        kc_cur = e->kcache.as<ActT>(); vc_cur = e->vcache.as<ActT>(); kc_next = e->kcache2.as<ActT>(); vc_next = e->vcache2.as<ActT>();
-    }
+    st.c_front = (int*)(base + o_cf); st.parent = (int*)(base + o_par);
+    st.desc_self = (int4*)(base + o_ds); st.desc_cross = (int4*)(base + o_dc);
+    { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
+    st.src_len = e->srclen.as<int>();
+    ActT *kc_cur = e->kcache.as<ActT>(), *vc_cur = e->vcache.as<ActT>(), *kc_next = e->kcache2.as<ActT>(), *vc_next = e->vcache2.as<ActT>();
     { Scope sc(e, KC_MISC, s); launch_sbeam_init(st, s); }
 
     float* x = e->x.as<float>();
@@ -1712,87 +1576,54 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
     for (int step = 0; step < max_len - 1; ++step) {
         const int C = B * beam;
         { Scope sc(e, KC_MISC, s); launch_sbeam_prepare(st, C, beam, W, s); }
-        if (cached) {
-            RowCount rows1(C, n_live, 1);
-            { Scope sc(e, KC_EMBED, s); launch_sbeam_embed_last<ActT>(st, C, W, e->tgt_emb, e->pe, E, x, xh, s); }
-            auto self_attn = [&](int l, ActT* qkv, ActT* att) {
-                spec_attn(qkv, 3 * E, kc_cur + l * cache_l_stride, vc_cur + l * cache_l_stride, cache_c_stride, E, att, E, C, n_live, st.row_cand,
-                          st.c_front, st.y_cur, ldw, e->d.tgt_pad_token_idx, 1, 0, H, HD, max_len, s, st.desc_self);
-            };
-            auto cross_attn = [&](int l, ActT* q2, ActT* att) {
-                const ActT* kv = crosskv + (long long)l * TS * 2 * E;
-                attn(q2, E, kv, kv + E, 2 * E, att, E, C, n_live, 1, Ls, Ls, st.row_query, src32, Ls, e->d.src_pad_token_idx, false, H, HD, s,
-                     nullptr, nullptr, st.desc_cross);
-            };
-            if (decoder_stack<ActT>(e, rows1, n_dec, (long long)Cmax * 3 * E, self_attn, cross_attn, s)) return 1;
-            // every live row is the last position of its hypothesis: logits straight from the residual stream
-            if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, logits, V, rows1, false, s)) return 1;
-            { Scope sc(e, KC_ARGMAX, s); launch_sbeam_scores(st, C, logits, s); }
-            {
-                Scope sc(e, KC_ACCEPT, s);
-                TTB_CHECK(launch_sbeam_select(st, beam, W, s) == 0, "beam_size * vocabulary too large for the selection kernel");
-            }
-            {
-                Scope sc(e, KC_CACHE_APPEND, s);
-                launch_sbeam_cache_update<ActT>(st, W, e->qkv.as<ActT>(), (long long)Cmax * 3 * E, n_dec, 3 * E, E, kc_cur, vc_cur, kc_next, vc_next,
-                                                cache_l_stride, cache_c_stride, s);
-            }
-            std::swap(kc_cur, kc_next);
-            std::swap(vc_cur, vc_next);
-            // the stop test runs on the device (std_beam.cu: ctrl[2]); the host reads the control words of step - 1 while
-            // this step is already enqueued (a step behind the end is a no-op), so the GPU never waits for the host
-            TTB_CUDA_OK(cudaMemcpyAsync(hc + 32 + (step & 3) * 8, st.ctrl, 4 * sizeof(int), cudaMemcpyDeviceToHost, s));
-            TTB_CUDA_OK(cudaEventRecord(e->poll_ev[step & 3], s));
-            std::swap(st.y_cur, st.y_next);
-            std::swap(st.score_cur, st.score_next);
-            beam = K;
-            W += 1;
-            if (step >= sb_lag) {
-                const int j = (step - sb_lag) & 3;
-                TTB_CUDA_OK(cudaEventSynchronize(e->poll_ev[j]));
-                if (hc[32 + j * 8 + 2]) break;       // every hypothesis contains EOS (:169)
-            }
-            continue;
-        }
-        RowCount rows(C * W, n_live, W);
-        { Scope sc(e, KC_EMBED, s); launch_embed_seq_rows<ActT>(st.rows_tok, rows, W, e->tgt_emb, e->pe, E, x, xh, s); }
-        auto self_attn = [&](int, ActT* qkv, ActT* att) {
-            attn(qkv, 3 * E, qkv + E, qkv + 2 * E, 3 * E, att, E, C, n_live, W, W, W, nullptr,
-                 st.rows_tok, W, e->d.tgt_pad_token_idx, true, H, HD, s);
+        RowCount rows1(C, n_live, 1);
+        { Scope sc(e, KC_EMBED, s); launch_sbeam_embed_last<ActT>(st, C, W, e->tgt_emb, e->pe, E, x, xh, s); }
+        auto self_attn = [&](int l, ActT* qkv, ActT* att) {
+            spec_attn(qkv, 3 * E, kc_cur + l * cache_l_stride, vc_cur + l * cache_l_stride, cache_c_stride, E, att, E, C, n_live, st.row_cand,
+                      st.c_front, st.y_cur, ldw, e->d.tgt_pad_token_idx, 1, 0, H, HD, max_len, s, st.desc_self);
         };
         auto cross_attn = [&](int l, ActT* q2, ActT* att) {
             const ActT* kv = crosskv + (long long)l * TS * 2 * E;
-            attn(q2, E, kv, kv + E, 2 * E, att, E, C, n_live, W, Ls, Ls, st.row_query,
-                 src32, Ls, e->d.src_pad_token_idx, false, H, HD, s);
+            attn(q2, E, kv, kv + E, 2 * E, att, E, C, n_live, 1, Ls, Ls, st.row_query, src32, Ls, e->d.src_pad_token_idx, false, H, HD, s,
+                 nullptr, nullptr, st.desc_cross);
         };
-        if (decoder_stack<ActT>(e, rows, 1, 0, self_attn, cross_attn, s)) return 1;
-        { Scope sc(e, KC_MISC, s); launch_sbeam_gather_last<ActT>(st, x, xh, C, W, E, Prec<ActT>::lowp ? nullptr : xg, xgh, s); }
-        RowCount last_rows(C, n_live, 1);
-        if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(xg, xgh), E, e->classifier, logits, V, last_rows, false, s)) return 1;
+        if (decoder_stack<ActT>(e, rows1, n_dec, (long long)Cmax * 3 * E, self_attn, cross_attn, s)) return 1;
+        // every live row is the last position of its hypothesis: logits straight from the residual stream
+        if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, logits, V, rows1, false, s)) return 1;
         { Scope sc(e, KC_ARGMAX, s); launch_sbeam_scores(st, C, logits, s); }
         {
             Scope sc(e, KC_ACCEPT, s);
             TTB_CHECK(launch_sbeam_select(st, beam, W, s) == 0, "beam_size * vocabulary too large for the selection kernel");
         }
-        TTB_CUDA_OK(cudaMemcpyAsync(hc, st.ctrl, 2 * sizeof(int), cudaMemcpyDeviceToHost, s));
-        TTB_CUDA_OK(cudaStreamSynchronize(s));
-        ++calls;
+        {
+            Scope sc(e, KC_CACHE_APPEND, s);
+            launch_sbeam_cache_update<ActT>(st, W, e->qkv.as<ActT>(), (long long)Cmax * 3 * E, n_dec, 3 * E, E, kc_cur, vc_cur, kc_next, vc_next,
+                                            cache_l_stride, cache_c_stride, s);
+        }
+        std::swap(kc_cur, kc_next);
+        std::swap(vc_cur, vc_next);
+        // the stop test runs on the device (std_beam.cu: ctrl[2]); the host reads the control words of step - 1 while
+        // this step is already enqueued (a step behind the end is a no-op), so the GPU never waits for the host
+        TTB_CUDA_OK(cudaMemcpyAsync(hc + 32 + (step & 3) * 8, st.ctrl, 4 * sizeof(int), cudaMemcpyDeviceToHost, s));
+        TTB_CUDA_OK(cudaEventRecord(e->poll_ev[step & 3], s));
         std::swap(st.y_cur, st.y_next);
         std::swap(st.score_cur, st.score_next);
         beam = K;
         W += 1;
-        if (step > 0 && hc[1] == B * K) break;   // every hypothesis contains EOS (:169); the first step never breaks (:106-125)
+        if (step >= sb_lag) {
+            const int j = (step - sb_lag) & 3;
+            TTB_CUDA_OK(cudaEventSynchronize(e->poll_ev[j]));
+            if (hc[32 + j * 8 + 2]) break;       // every hypothesis contains EOS (:169)
+        }
     }
-    if (cached) {
-        // steps that really ran (the host may have enqueued one more, a no-op): width, call count, and the hypothesis set
-        // the last real step wrote (step i reads set i & 1 and writes the other one)
-        int fin[4] = {};
-        TTB_CUDA_OK(cudaMemcpyAsync(fin, st.ctrl, sizeof(fin), cudaMemcpyDeviceToHost, s));
-        TTB_CUDA_OK(cudaStreamSynchronize(s));
-        calls = fin[3];
-        W = 1 + calls;
-        st.y_cur = (calls & 1) ? y_set[1] : y_set[0];
-    }
+    // steps that really ran (the host may have enqueued one more, a no-op): width, call count, and the hypothesis set
+    // the last real step wrote (step i reads set i & 1 and writes the other one)
+    int fin[4] = {};
+    TTB_CUDA_OK(cudaMemcpyAsync(fin, st.ctrl, sizeof(fin), cudaMemcpyDeviceToHost, s));
+    TTB_CUDA_OK(cudaStreamSynchronize(s));
+    calls = fin[3];
+    W = 1 + calls;
+    st.y_cur = (calls & 1) ? y_set[1] : y_set[0];
     launch_beam_export(st.y_cur, ldw, B * K, W, reinterpret_cast<long long*>(out_dev), s);
     e->launches++;
     TTB_CUDA_OK(cudaEventRecord(e->t1, s));
@@ -1868,14 +1699,13 @@ void ttb_engine_destroy(ttb_engine* e) {
     }
     DevBuf* bufs[] = {&e->x, &e->xh, &e->y, &e->qkv, &e->att, &e->q2, &e->hid, &e->logits, &e->tok32, &e->keytok32, &e->pred,
                       &e->src32, &e->memory, &e->memh, &e->crosskv, &e->kcache, &e->vcache, &e->drafts, &e->gen, &e->front,
-                      &e->active, &e->ctrl, &e->sel, &e->out64, &e->hist, &e->beam, &e->srclen, &e->desc, &e->kcache2, &e->vcache2, &e->crossvt,
+                      &e->active, &e->ctrl, &e->sel, &e->out64, &e->hist, &e->beam, &e->srclen, &e->desc, &e->kcache2, &e->vcache2,
                       &e->cb, &e->cb_work};
     for (DevBuf* b : bufs) b->release();
     if (e->h_ctrl) cudaFreeHost(e->h_ctrl);
     for (auto& ev : e->poll_ev) if (ev) cudaEventDestroy(ev);
     for (auto& ev : e->prof.pool) cudaEventDestroy(ev);
     for (auto& gb : e->graph_exec) for (auto& g : gb) if (g) cudaGraphExecDestroy(g);
-    for (auto& gp : e->beam_graph) for (auto& g : gp) if (g) cudaGraphExecDestroy(g);
     if (e->stream) cudaStreamDestroy(e->stream);
     if (e->join_ev) cudaEventDestroy(e->join_ev);
     if (e->t0) cudaEventDestroy(e->t0);

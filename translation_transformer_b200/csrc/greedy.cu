@@ -89,8 +89,7 @@ __global__ void greedy_advance_kernel(GreedyState st, const float* __restrict__ 
                                       int E, float* __restrict__ x, ActT* __restrict__ xh, int n_embed_blocks,
                                       const ActT* __restrict__ qkv_all, long long qkv_layer_stride, int n_layers, int qkv_ld,
                                       ActT* __restrict__ kcache, ActT* __restrict__ vcache, long long cache_layer_stride,
-                                      long long cache_query_stride, int cache_ld, long long vt_layer_stride, long long vt_query_stride,
-                                      int vt_pitch) {
+                                      long long cache_query_stride, int cache_ld) {
     // Launched with the programmatic attribute behind the accept kernel (scheduled while it runs, starts when it is
     // complete).  The kernels of the decoding iteration read the control words and descriptor table of the accept kernel
     // ahead of their dependency waits, so none of them may be scheduled before this kernel has SEEN the accept kernel
@@ -115,15 +114,6 @@ __global__ void greedy_advance_kernel(GreedyState st, const float* __restrict__ 
         const int b = sel.x, f = sel.y, pick = sel.z, a = sel.w;
         const ActT* src = qkv_all + (long long)l * qkv_layer_stride + ((long long)g * st.N + pick) * (st.D + 1) * qkv_ld;
         ActT* kd = kcache + (long long)l * cache_layer_stride + (long long)b * cache_query_stride + (long long)f * cache_ld;
-        if (vt_pitch > 0) {   // value cache kept transposed ([dim][position]) for the tcgen05 attention kernel
-            ActT* vt = vcache + (long long)l * vt_layer_stride + (long long)b * vt_query_stride + f;
-            for (int i2 = threadIdx.x; i2 < (a + 1) * E; i2 += blockDim.x) {
-                const int i = i2 / E, c = i2 % E;
-                kd[(long long)i * cache_ld + c] = src[(long long)i * qkv_ld + E + c];
-                vt[(long long)c * vt_pitch + i] = src[(long long)i * qkv_ld + 2 * E + c];
-            }
-            return;
-        }
         ActT* vd = vcache + (long long)l * cache_layer_stride + (long long)b * cache_query_stride + (long long)f * cache_ld;
         for (int i2 = threadIdx.x; i2 < (a + 1) * E; i2 += blockDim.x) {
             const int i = i2 / E, c = i2 % E;
@@ -151,21 +141,19 @@ __global__ void greedy_advance_kernel(GreedyState st, const float* __restrict__ 
 template <typename ActT>
 void launch_greedy_advance(const GreedyState& st, const float* table, const float* pe, int E, float* x, ActT* xh,
                            const ActT* qkv_all, long long qkv_layer_stride, int n_layers, int qkv_ld, ActT* kcache, ActT* vcache,
-                           long long cache_layer_stride, long long cache_query_stride, int cache_ld, cudaStream_t s,
-                           long long vt_layer_stride, long long vt_query_stride, int vt_pitch) {
+                           long long cache_layer_stride, long long cache_query_stride, int cache_ld, cudaStream_t s) {
     const int T = st.B * st.N * (st.D + 1);
     const int n_embed_blocks = (T + 7) / 8;
     // first kernel of the captured iteration: plain launch (its predecessor is the previous graph launch)
     launch_pdl(greedy_advance_kernel<ActT>, dim3(n_embed_blocks + st.B * n_layers), dim3(256), 0, s, st, table, pe, E, x, xh, n_embed_blocks, qkv_all,
                                                                               qkv_layer_stride, n_layers, qkv_ld, kcache, vcache,
-                                                                              cache_layer_stride, cache_query_stride, cache_ld, vt_layer_stride,
-                                                                              vt_query_stride, vt_pitch);
+                                                                              cache_layer_stride, cache_query_stride, cache_ld);
 }
 template void launch_greedy_advance<float>(const GreedyState&, const float*, const float*, int, float*, float*, const float*, long long, int, int,
-                                           float*, float*, long long, long long, int, cudaStream_t, long long, long long, int);
+                                           float*, float*, long long, long long, int, cudaStream_t);
 template void launch_greedy_advance<__nv_bfloat16>(const GreedyState&, const float*, const float*, int, float*, __nv_bfloat16*,
                                                    const __nv_bfloat16*, long long, int, int, __nv_bfloat16*, __nv_bfloat16*, long long,
-                                                   long long, int, cudaStream_t, long long, long long, int);
+                                                   long long, int, cudaStream_t);
 
 // ---- accept / retire / plan ---------------------------------------------------------------------
 // One CTA, one warp per live query: lanes score the drafts in parallel (accepted length = leading

@@ -111,19 +111,6 @@ void launch_spec_self_attention_mma(const __nv_bfloat16* qkv, int qkv_ld, const 
 // group_row_len (needs desc): group g's draft rows are desc[g].w <= D + 1 positions long (the rest of each row of the call is
 // ignored and not written), and its outputs are the bits a call with D + 1 = desc[g].w gives
 
-// ---- attention_tc.cu : tcgen05 attention of the decoding loops (head_dim 32, S in tensor memory, V caches kept transposed) ----
-bool attention_tc_supported(int head_dim, int Lq, int max_shared_keys, int row_len);
-// out[(g * E + c) * pitch + j] = in[(g * L + j) * ld + c]
-void launch_transpose_v(const __nv_bfloat16* in, int ld, int groups, int L, int E, __nv_bfloat16* out, int pitch, cudaStream_t s);
-int launch_cross_attention_tc(const __nv_bfloat16* q, int q_ld, const __nv_bfloat16* k, int k_ld, long long k_group_stride,
-                              const __nv_bfloat16* vt, long long vt_group_stride, int vt_pitch, __nv_bfloat16* out, int out_ld,
-                              int n_groups_max, const int* n_groups_dev, int Lq, const int* key_tok, int key_tok_stride, int pad_id,
-                              const int* lk_dev, int heads, const int4* desc, cudaStream_t s);
-int launch_spec_self_attention_tc(const __nv_bfloat16* qkv, int qkv_ld, const __nv_bfloat16* kcache, long long k_query_stride, int k_ld,
-                                  const __nv_bfloat16* vtcache, long long vt_query_stride, int vt_pitch, __nv_bfloat16* out, int out_ld,
-                                  int B_max, const int* n_active_dev, const int* gen, int gen_ld, int pad_id, int N, int D, int heads,
-                                  const int4* desc, cudaStream_t s);
-
 // ---- drafting.cu ------------------------------------------------------------------------------
 // Mirrors utils/drafting.py::make_drafts on device; src is (B, L) int32 with row stride src_ld (the
 // caller skips the BOS column by passing src + 1, L - 1).  out is (B, N, Deff) int32.
@@ -156,9 +143,7 @@ void launch_greedy_init(const GreedyState& st, cudaStream_t s);
 template <typename ActT>
 void launch_greedy_advance(const GreedyState& st, const float* table, const float* pe, int E, float* x, ActT* xh,
                            const ActT* qkv_all, long long qkv_layer_stride, int n_layers, int qkv_ld, ActT* kcache, ActT* vcache,
-                           long long cache_layer_stride, long long cache_query_stride, int cache_ld, cudaStream_t s,
-                           long long vt_layer_stride = 0, long long vt_query_stride = 0, int vt_pitch = 0);
-// vt_pitch > 0: `vcache` is the TRANSPOSED value cache [layer][query][E][vt_pitch] of the tcgen05 attention kernel
+                           long long cache_layer_stride, long long cache_query_stride, int cache_ld, cudaStream_t s);
 // picks the best draft per live query, appends tokens, retires finished queries, plans next width
 void launch_greedy_accept(const GreedyState& st, cudaStream_t s);
 // standard greedy decoding (no drafts: N = 1, D = 0): appends the predicted token of every row, stop test
@@ -203,13 +188,12 @@ struct BeamState {
     // of the chain live list -> front -> token, and everything the attention kernels may read ahead of their dependency wait
     int4* desc_self; int4* desc_cross; const int* src_len;
     int* host_ctrl;   // pinned host mirror of ctrl (device-accessible): BC_COUNT words + a sequence word written last
-    int* rows_tok; int* row_cand; int* row_query; int* row_slot0;      // live decoder rows
     float* topv; int* topi; int* nkeep; float* lmax; float* lsum;      // per (row, position) statistics
-    // KV-cached pass: token whose logit the accepted-path sums need at (row, position) = the row's next draft token (-1
-    // behind the last one), written by the embedding kernel; its logit, written by the statistics kernel
+    // token whose logit the accepted-path sums need at (row, position) = the row's next draft token (-1 behind the last
+    // one), written by the embedding kernel; its logit, written by the statistics kernel
     int* row_tok; float* tokv;
     int* trace_nacc; int* trace_pick;     // optional [iter][B*K][N] / [iter][B*K]
-    // KV-cached decoder pass: live candidates as attention groups, cache bookkeeping of the new candidates
+    // live candidates as attention groups, cache bookkeeping of the new candidates
     int* live_cand; int* live_query;      // [live candidates] candidate index / query index
     int* c_front;                         // [B*K] cached positions of a candidate = first free slot - 1
     int* n_parent; int* n_keep; int* n_row;   // [B*K] new candidate: parent (-1: finished parent), accepted draft tokens, decoder row
@@ -218,16 +202,12 @@ struct BeamState {
     int smart, n_lib;
     int* tok_cnt; int* tok_list;          // [B][V] number of windows per first token (1..N), [B][V][N] their library indices
     int* c_cnt; int* c_last;              // [B*K] rows (drafts) of a candidate, its last token
-    int* row_draft;                       // [rows] library index of the row's draft (row_cand / row_query: its candidate / query)
+    int* row_draft;                       // [rows] library index of the row's draft
 };
 void launch_beam_build_lib(const BeamState& st, cudaStream_t s);
 void launch_beam_init(const BeamState& st, cudaStream_t s);
 void launch_beam_prepare(const BeamState& st, int C, int beam, int dl, cudaStream_t s);
-void launch_beam_fill_rows(const BeamState& st, int C, int beam, int W, int dl, cudaStream_t s);
-template <typename ActT>
-void launch_beam_gather(const BeamState& st, const float* x, const ActT* xh, int max_rows, int W, int dl, int E,
-                        float* xg, ActT* xgh, cudaStream_t s);
-// KV-cached pass: embeds (last token, draft tokens) of every live (candidate, draft) row at positions front .. front+dl
+// embeds (last token, draft tokens) of every live (candidate, draft) row at positions front .. front+dl
 template <typename ActT>
 void launch_beam_embed_cached(const BeamState& st, int beam, int max_rows, int dl, const float* table, const float* pe, int E,
                               float* x, ActT* xh, cudaStream_t s);
@@ -238,7 +218,7 @@ void launch_beam_cache_update(const BeamState& st, int dl, const ActT* qkv_all, 
                               long long cache_cand_stride, cudaStream_t s);
 void launch_beam_stats(const BeamState& st, const float* logits, int max_rows, int dl, cudaStream_t s);
 void launch_beam_choose(const BeamState& st, int C, int beam, int dl, cudaStream_t s);
-void launch_beam_expand(const BeamState& st, int beam, int dl, const float* logits, cudaStream_t s);
+void launch_beam_expand(const BeamState& st, int beam, int dl, cudaStream_t s);
 void launch_beam_export(const int* cand, int ldw, int R, int W, long long* out, cudaStream_t s);
 
 // Continuous batching of the speculative beam search (BeamState::B = number of query slots; slot b owns candidates
@@ -266,7 +246,7 @@ void launch_beam_admit(const BeamState& st, const BcTable& cb, int grp, int Bi, 
 // group-aware prepare / choose / expand; `dl` = draft length of the decoder call (the largest of the open batches)
 void launch_beam_prepare_groups(const BeamState& st, const BcTable& cb, cudaStream_t s);
 void launch_beam_choose_groups(const BeamState& st, const BcTable& cb, int dl, cudaStream_t s);
-void launch_beam_expand_groups(const BeamState& st, const BcTable& cb, int dl, const float* logits, cudaStream_t s);
+void launch_beam_expand_groups(const BeamState& st, const BcTable& cb, int dl, cudaStream_t s);
 // ---- std_beam.cu : standard beam search (standard_decoding.py:90-174) -------------------------------------------
 struct StdBeamState {
     int B, K, V, pad, bos, eos, ldw;
@@ -274,10 +254,9 @@ struct StdBeamState {
     float* score_cur; float* score_next;  // [B*K]
     int* fin; int* cand_row;              // [B*K] contains EOS / live-row index or -1
     int* row_cand; int* row_query;        // [live rows]
-    int* rows_tok;                        // [live rows][W] decoder input
     float* total;                         // [B*K][V] score + log-softmax
     int* ctrl;                            // [0] live rows, [1] hypotheses with EOS after the selection
-    // KV-cached pass (one new token per live hypothesis and step; nullptr: full-prefix recomputation)
+    // KV cache: one new token per live hypothesis and step
     int* c_front;                         // [B*K] cached positions of a hypothesis (= W - 1 for all of them)
     int* parent;                          // [B*K] hypothesis of the previous step a new hypothesis continues
     int4* desc_self; int4* desc_cross;    // per live row: {hypothesis, front, token at front, -} / {query, -, -, source length}
@@ -285,12 +264,9 @@ struct StdBeamState {
 };
 void launch_sbeam_init(const StdBeamState& st, cudaStream_t s);
 void launch_sbeam_prepare(const StdBeamState& st, int C, int beam, int W, cudaStream_t s);
-template <typename ActT>
-void launch_sbeam_gather_last(const StdBeamState& st, const float* x, const ActT* xh, int max_rows, int W, int E, float* xg, ActT* xgh,
-                              cudaStream_t s);
 void launch_sbeam_scores(const StdBeamState& st, int C, const float* logits, cudaStream_t s);
 int launch_sbeam_select(const StdBeamState& st, int beam, int W, cudaStream_t s);
-// KV-cached pass: embedding of the last token (position W - 1) of every live hypothesis
+// embedding of the last token (position W - 1) of every live hypothesis
 template <typename ActT>
 void launch_sbeam_embed_last(const StdBeamState& st, int max_rows, int W, const float* table, const float* pe, int E, float* x, ActT* xh,
                              cudaStream_t s);
@@ -299,10 +275,5 @@ template <typename ActT>
 void launch_sbeam_cache_update(const StdBeamState& st, int W, const ActT* qkv_all, long long qkv_layer_stride, int n_layers, int qkv_ld, int E,
                                const ActT* kc_cur, const ActT* vc_cur, ActT* kc_next, ActT* vc_next, long long cache_layer_stride,
                                long long cache_cand_stride, cudaStream_t s);
-
-// embedding of (rows, L) token matrices whose live row count is on the device
-template <typename ActT>
-void launch_embed_seq_rows(const int* tok, RowCount rows, int L, const float* table, const float* pe, int E,
-                           float* x, ActT* xh, cudaStream_t s);
 
 }  // namespace ttb

@@ -2,9 +2,10 @@
 // Reference: /root/reference/src/decoding/standard_decoding.py:90-174 (TranslationInferenceBeamSearch.generate).
 //
 // Per step the engine runs
-//   sbeam_prepare -> finished flag of every hypothesis (contains EOS), compact list of live hypotheses, their
-//                    token rows as the decoder input, row -> query map for the cross-attention
-//   decoder stack on the live rows (full prefix, causal), gather of the last position, classifier GEMM
+//   sbeam_prepare -> finished flag of every hypothesis (contains EOS), compact list of live hypotheses,
+//                    row -> query map for the cross-attention
+//   sbeam_embed_last -> embedding of the last token of every live hypothesis
+//   decoder stack on those rows (the prefix comes from the hypothesis' KV cache), classifier GEMM
 //   sbeam_scores  -> log(softmax(logits)) per hypothesis (artificial logits for finished ones: 35 on the PAD
 //                    column, 0 elsewhere, :132-135) added to the hypothesis score
 //   sbeam_select  -> per query: the beam_size best of the (beam x vocab) continuations, sorted, and the new
@@ -18,7 +19,6 @@ namespace ttb {
 // hypothesis contains EOS (raised by the CTA of sbeam_select that finishes last; the reference's stop test, :169) -- a step the
 // host has enqueued ahead of reading [1] is then a no-op --, [3] steps that really ran, [4] ticket of the select CTAs
 __global__ void __launch_bounds__(1024) sbeam_prepare_kernel(StdBeamState st, int C, int beam, int W) {
-    __shared__ int s_run;
     if (st.ctrl[2]) {
         if (threadIdx.x == 0) st.ctrl[0] = 0;   // no live rows: the decoder kernels of this step exit at once
         return;
@@ -37,53 +37,19 @@ __global__ void __launch_bounds__(1024) sbeam_prepare_kernel(StdBeamState st, in
             st.cand_row[c] = run;
             st.row_cand[run] = c;
             st.row_query[run] = c / beam;
-            if (st.desc_self) {   // KV-cached pass: W - 1 cached positions, the token at W - 1 is this step's input
-                st.desc_self[run] = make_int4(c, W - 1, st.y_cur[(long long)c * st.ldw + W - 1], 0x7fffffff);
-                st.desc_cross[run] = make_int4(c / beam, 0, 0, st.src_len ? st.src_len[c / beam] : 0x7fffffff);
-            }
+            // W - 1 cached positions, the token at W - 1 is this step's input
+            st.desc_self[run] = make_int4(c, W - 1, st.y_cur[(long long)c * st.ldw + W - 1], 0x7fffffff);
+            st.desc_cross[run] = make_int4(c / beam, 0, 0, st.src_len[c / beam]);
             ++run;
         }
         st.ctrl[0] = run;
         st.ctrl[1] = 0;       // hypotheses with EOS after the coming selection (sbeam_select counts them)
-        s_run = run;
     }
-    __syncthreads();
-    if (st.c_front) {       // KV-cached pass: no token rows to build
-        for (int c = threadIdx.x; c < C; c += blockDim.x) st.c_front[c] = W - 1;
-        return;
-    }
-    const int R = s_run;
-    for (long long idx = threadIdx.x; idx < (long long)R * W; idx += blockDim.x) {
-        const int r = (int)(idx / W), j = (int)(idx % W);
-        st.rows_tok[idx] = st.y_cur[(long long)st.row_cand[r] * st.ldw + j];
-    }
+    for (int c = threadIdx.x; c < C; c += blockDim.x) st.c_front[c] = W - 1;
 }
 void launch_sbeam_prepare(const StdBeamState& st, int C, int beam, int W, cudaStream_t s) {
     sbeam_prepare_kernel<<<1, 1024, 0, s>>>(st, C, beam, W);
 }
-
-// last position of every live row of the residual stream -> dense (rows, E) classifier input
-template <typename ActT>
-__global__ void sbeam_gather_last_kernel(StdBeamState st, const float* __restrict__ x, const ActT* __restrict__ xh, int W, int E,
-                                         float* __restrict__ xg, ActT* __restrict__ xgh) {
-    const int r = blockIdx.x * (blockDim.x >> 5) + (threadIdx.x >> 5);
-    const int lane = threadIdx.x & 31;
-    if (r >= st.ctrl[0]) return;
-    const long long src = ((long long)r * W + W - 1) * E, dst = (long long)r * E;
-    for (int c = lane; c < E; c += 32) {
-        if (xg) xg[dst + c] = x[src + c];
-        if (xgh) xgh[dst + c] = xh[src + c];
-    }
-}
-template <typename ActT>
-void launch_sbeam_gather_last(const StdBeamState& st, const float* x, const ActT* xh, int max_rows, int W, int E, float* xg, ActT* xgh,
-                              cudaStream_t s) {
-    if (max_rows <= 0) return;
-    sbeam_gather_last_kernel<ActT><<<(max_rows + 7) / 8, 256, 0, s>>>(st, x, xh, W, E, xg, xgh);
-}
-template void launch_sbeam_gather_last<float>(const StdBeamState&, const float*, const float*, int, int, int, float*, float*, cudaStream_t);
-template void launch_sbeam_gather_last<__nv_bfloat16>(const StdBeamState&, const float*, const __nv_bfloat16*, int, int, int, float*,
-                                                      __nv_bfloat16*, cudaStream_t);
 
 // One warp per hypothesis: total[c][v] = score[c] + log(softmax(logits_c)[v])   (softmax first, then log, like
 // `torch.log(torch.softmax(x, -1))` at :111 / :150)
@@ -159,7 +125,7 @@ int launch_sbeam_select(const StdBeamState& st, int beam, int W, cudaStream_t s)
     return 0;
 }
 
-// ---- KV-cached pass ---------------------------------------------------------------------------------------------------
+// ---- KV caches --------------------------------------------------------------------------------------------------------
 template <typename ActT>
 __global__ void sbeam_embed_last_kernel(StdBeamState st, int W, const float* __restrict__ table, const float* __restrict__ pe, int E,
                                         float* __restrict__ x, ActT* __restrict__ xh) {
