@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define TTB_ABI_VERSION 4
+#define TTB_ABI_VERSION 5
 
 #define TTB_PRECISION_FP32 0 /* fp32 FMA GEMMs, exact-parity path (1e-5 logits)            */
 #define TTB_PRECISION_BF16 1 /* tcgen05 bf16 GEMMs, fp32 accumulate (1e-2 logits)          */
@@ -127,6 +127,21 @@ int ttb_greedy_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_
 int ttb_beam_search_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len, int32_t beam_size,
                              int32_t pad_token, int32_t bos_token, int32_t eos_token, int64_t* out_dev, int32_t* out_width,
                              ttb_generate_stats* stats, void* stream);
+
+/* ---- continuous batching of standard_decoding.py:90 generate(): n_batches independent batches share `slots` query slots
+ * of ONE device loop, each slot holding beam_size hypotheses.  Batch i is admitted (whole, in list order) between two steps
+ * as soon as `batch_sizes[i]` slots are free; it keeps the width, first step and stop rule of its own batch and frees its
+ * slots when it stops, so out_devs[i], out_widths[i] and stats[i].model_calls are exactly what ttb_beam_search_generate
+ * returns for that batch alone (the other fields of stats[i] are 0: launches and time belong to the call, in `total`).
+ * src_devs[i] is (batch_sizes[i], src_lens[i]) int64; out_devs[i] holds batch_sizes[i] * beam_size *
+ * max_len int64 and receives (batch_sizes[i], beam_size, out_widths[i]) densely.  slots >= max(batch_sizes).  Arguments
+ * ttb_beam_search_generate rejects are rejected with the same error before any device work.  total (may be NULL):
+ * launches / ms of the call, model_calls = steps of the shared loop.  ttb_engine_get_history afterwards gives the query
+ * slots in use at every step. */
+int ttb_beam_search_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs, const int32_t* batch_sizes,
+                                     const int32_t* src_lens, int32_t slots, int32_t max_len, int32_t beam_size, int32_t pad_token,
+                                     int32_t bos_token, int32_t eos_token, int64_t* const* out_devs, int32_t* out_widths,
+                                     ttb_generate_stats* stats, ttb_generate_stats* total, void* stream);
 
 /* ---- speculative_decoding.py:422 TranslationInferenceBeamSearchSpeculative.generate(src)
  * smart_drafts_mode = 0: "try all the drafts" (:428-598), every candidate tries the n_drafts source windows;

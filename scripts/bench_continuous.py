@@ -19,6 +19,11 @@ device memory its engines hold after the run, and leg (b) the mean and maximum q
 of a beam search reports the bs slots it holds as `slots_held` (its generate() keeps no per-iteration history).
 
     python scripts/bench_continuous.py --workload retro --weights copy --batches 48 --out profiles/r4_continuous_beam_retro.json
+
+--workload std_beam / std_retro run the standard beam search (TranslationInferenceBeamSearch, beam_size = n_best) on the
+model, weights and batches of the beam / retro workloads, with the legs and defaults of those workloads.
+
+    python scripts/bench_continuous.py --workload std_beam --weights copy --batches 48 --out profiles/r5_continuous_std_beam_copy.json
 """
 from __future__ import annotations
 
@@ -37,6 +42,7 @@ REPO = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(REPO))
 
 import bench  # noqa: E402
+from translation_transformer_b200.decoding import TranslationInferenceBeamSearch  # noqa: E402
 from translation_transformer_b200.model import B200Transformer  # noqa: E402
 from translation_transformer_b200.pipeline import InFlightDecoder  # noqa: E402
 
@@ -64,7 +70,7 @@ def timed(fn):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--workload", default="greedy", choices=["greedy", "beam", "retro"])
+    ap.add_argument("--workload", default="greedy", choices=["greedy", "beam", "retro", "std_beam", "std_retro"])
     ap.add_argument("--weights", default="copy", choices=["copy", "random"])
     ap.add_argument("--batches", type=int, default=24)
     ap.add_argument("--slots", default=None, help="comma-separated slot counts (default greedy: 32,48,64,96,128; beam searches: 1,2,4,8,16 x bs)")
@@ -73,10 +79,14 @@ def main():
     ap.add_argument("--out", required=True)
     a = ap.parse_args()
     greedy = a.workload == "greedy"
-    argv, sys.argv = sys.argv, ["bench.py", "--workload", a.workload, "--weights", a.weights]
+    std = a.workload.startswith("std_")
+    base = a.workload[len("std_"):] if std else a.workload
+    argv, sys.argv = sys.argv, ["bench.py", "--workload", base, "--weights", a.weights]
     bargs = bench.parse()
     sys.argv = argv
-    wl = bench.Workload(a.workload, a.weights, bargs)
+    wl = bench.Workload(base, a.weights, bargs)
+    if std:   # the standard beam search on the workload's model and batches
+        wl.generator = lambda eng: TranslationInferenceBeamSearch(eng, wl.n_best, bargs.max_len, bench.PAD, bench.BOS, bench.EOS)
     if a.slots is None:
         a.slots = "32,48,64,96,128" if greedy else ",".join(str(k * wl.bs) for k in (1, 2, 4, 8, 16))
     if a.inflight is None:
@@ -86,7 +96,7 @@ def main():
     dev = torch.device("cuda", 0)
     batches = [wl.batch(j).to(dev) for j in range(a.batches)]
     n_smiles = sum(b.shape[0] for b in batches)
-    res = {"workload": wl.describe(), "batches": a.batches, "bs": wl.bs, "weights": a.weights, **gpu_info()}
+    res = {"workload": ("standard beam search, beam_size = n_best, on: " if std else "") + wl.describe(), "batches": a.batches, "bs": wl.bs, "weights": a.weights, **gpu_info()}
     if not greedy:
         res["n_best"] = wl.n_best
 

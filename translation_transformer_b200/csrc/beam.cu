@@ -612,35 +612,6 @@ void launch_beam_expand(const BeamState& st, int beam, int dl, cudaStream_t s) {
 // iteration; set when an admission found too few free slots (host bookkeeping broken)
 constexpr int BCC_USED = BC_COUNT + 9, BCC_DLMAX = BC_COUNT + 10, BCC_ADM_ERR = BC_COUNT + 11;
 
-// exclusive prefix sums of (a, b) over the threads of the block (blockDim.x a multiple of 32); totals in ta, tb
-__device__ __forceinline__ void block_scan2(int a, int b, int& ea, int& eb, int& ta, int& tb) {
-    __shared__ int s_a[32], s_b[32];
-    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
-    int ia = a, ib = b;
-#pragma unroll
-    for (int o = 1; o < 32; o <<= 1) {
-        const int x = __shfl_up_sync(0xffffffffu, ia, o), y = __shfl_up_sync(0xffffffffu, ib, o);
-        if (lane >= o) { ia += x; ib += y; }
-    }
-    if (lane == 31) { s_a[warp] = ia; s_b[warp] = ib; }
-    __syncthreads();
-    if (warp == 0) {
-        int va = lane < nw ? s_a[lane] : 0, vb = lane < nw ? s_b[lane] : 0;
-#pragma unroll
-        for (int o = 1; o < 32; o <<= 1) {
-            const int x = __shfl_up_sync(0xffffffffu, va, o), y = __shfl_up_sync(0xffffffffu, vb, o);
-            if (lane >= o) { va += x; vb += y; }
-        }
-        s_a[lane] = va; s_b[lane] = vb;
-    }
-    __syncthreads();
-    ea = (warp ? s_a[warp - 1] : 0) + ia - a;
-    eb = (warp ? s_b[warp - 1] : 0) + ib - b;
-    ta = s_a[nw - 1];
-    tb = s_b[nw - 1];
-    __syncthreads();
-}
-
 // Admission of batch `grp` (Bi queries) into the first Bi free slots: hypotheses (BOS candidate), scores, drafts or the
 // window library (lib_in windows per query in drafts_in), source lengths and the batch's record.  One CTA, between two
 // iterations.
@@ -651,15 +622,7 @@ __global__ void __launch_bounds__(1024) beam_admit_kernel(BeamState st, BcTable 
     __shared__ int s_nfree;
     const int S = st.B, K = st.K, N = st.N, V = st.V, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (warp == 0) {
-        int taken = 0;
-        for (int i0 = 0; i0 < S && taken < Bi; i0 += 32) {
-            const int i = i0 + lane;
-            const bool fr = i < S && cb.slot_group[i] < 0;
-            const unsigned m = __ballot_sync(0xffffffffu, fr);
-            const int pos = taken + __popc(m & ((1u << lane) - 1u));
-            if (fr && pos < Bi) s_slots[pos] = i;
-            taken += __popc(m);
-        }
+        const int taken = take_free_slots(cb.slot_group, S, Bi, s_slots);
         if (lane == 0) s_nfree = taken;
     }
     __syncthreads();

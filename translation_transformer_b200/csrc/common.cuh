@@ -51,6 +51,52 @@ __device__ __forceinline__ float warp_max(float v) {
 
 constexpr int kNumSMs = 148;  // B200
 
+// ---- continuous batching (beam.cu, std_beam.cu) --------------------------------------------------------------------
+// exclusive prefix sums of (a, b) over the threads of the block (blockDim.x a multiple of 32); totals in ta, tb
+__device__ __forceinline__ void block_scan2(int a, int b, int& ea, int& eb, int& ta, int& tb) {
+    __shared__ int s_a[32], s_b[32];
+    const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5, nw = blockDim.x >> 5;
+    int ia = a, ib = b;
+#pragma unroll
+    for (int o = 1; o < 32; o <<= 1) {
+        const int x = __shfl_up_sync(0xffffffffu, ia, o), y = __shfl_up_sync(0xffffffffu, ib, o);
+        if (lane >= o) { ia += x; ib += y; }
+    }
+    if (lane == 31) { s_a[warp] = ia; s_b[warp] = ib; }
+    __syncthreads();
+    if (warp == 0) {
+        int va = lane < nw ? s_a[lane] : 0, vb = lane < nw ? s_b[lane] : 0;
+#pragma unroll
+        for (int o = 1; o < 32; o <<= 1) {
+            const int x = __shfl_up_sync(0xffffffffu, va, o), y = __shfl_up_sync(0xffffffffu, vb, o);
+            if (lane >= o) { va += x; vb += y; }
+        }
+        s_a[lane] = va; s_b[lane] = vb;
+    }
+    __syncthreads();
+    ea = (warp ? s_a[warp - 1] : 0) + ia - a;
+    eb = (warp ? s_b[warp - 1] : 0) + ib - b;
+    ta = s_a[nw - 1];
+    tb = s_b[nw - 1];
+    __syncthreads();
+}
+
+// One warp: the first n free slots (slot_group[i] < 0) of S, in slot order, into slots[0 .. n); returns the number of free
+// slots seen (the scan stops once n are found)
+__device__ __forceinline__ int take_free_slots(const int* slot_group, int S, int n, int* slots) {
+    const int lane = threadIdx.x & 31;
+    int taken = 0;
+    for (int i0 = 0; i0 < S && taken < n; i0 += 32) {
+        const int i = i0 + lane;
+        const bool fr = i < S && slot_group[i] < 0;
+        const unsigned m = __ballot_sync(0xffffffffu, fr);
+        const int pos = taken + __popc(m & ((1u << lane) - 1u));
+        if (fr && pos < n) slots[pos] = i;
+        taken += __popc(m);
+    }
+    return taken;
+}
+
 // ---- programmatic dependent launch (PDL) --------------------------------------------------------
 // Kernels of the decoding iteration are launched with the programmatic-stream-serialization attribute:
 // a kernel may be scheduled while its predecessor drains, runs its prologue (barrier init, TMEM

@@ -1029,6 +1029,31 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
 }
 
 
+// Waits for the word the closing CTA of iteration (step) `seq` of a beam-search loop posts into the pinned mapped ring at
+// h_ctrl + 16 (four 64-bit words, sequence number in the top 24 bits).  *arrived = false when the stream drained without it
+// (the mapping is unavailable); `pure_spin`: never give the core away between polls.
+static int wait_posted_word(ttb_engine* e, cudaStream_t s, int seq, unsigned long long* out, bool* arrived, bool pure_spin) {
+    volatile unsigned long long* word = reinterpret_cast<volatile unsigned long long*>(e->h_ctrl + 16) + (seq & 3);
+    auto match = [&](unsigned long long w) { return (unsigned)((w >> 40) & 0xffffff) == (unsigned)(seq & 0xffffff); };
+    *arrived = true;
+    for (long spin = 0;; ++spin) {
+        *out = *word;
+        if (match(*out)) return 0;
+        // the word normally arrives within a few microseconds of the last launch call; past that (long iterations,
+        // several engines per GPU and ranks per box sharing the cores) the thread gives its core away between polls
+        if (spin < 256 || pure_spin) cpu_relax(); else sched_yield();
+        if ((spin & 0x3FFF) == 0x3FFF) {
+            const cudaError_t q = cudaStreamQuery(s);
+            if (q == cudaSuccess) {   // stream drained: the word is there, or the mapping is unavailable
+                *out = *word;
+                *arrived = match(*out);
+                return 0;
+            }
+            if (q != cudaErrorNotReady) TTB_CUDA_OK(q);
+        }
+    }
+}
+
 // Continuous batching (ttb_beam_speculative_generate_batches): the batches that share the query slots of one loop.
 struct BcArgs {
     int n;                              // batches, admitted in list order
@@ -1281,31 +1306,15 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     int live_next = B;      // unfinished candidates entering the next iteration, from the newest word read
     int cont_used = 0, cont_dl = 0;   // continuous loop: slots in use and largest draft length of the open batches, idem
     auto wait_word = [&](int seq) -> int {
-        volatile unsigned long long* word = reinterpret_cast<volatile unsigned long long*>(hc + 16) + (seq & 3);
         unsigned long long w = 0;
-        bool seen = false;
-        for (long spin = 0; !seen; ++spin) {
-            w = *word;
-            seen = (unsigned)((w >> 40) & 0xffffff) == (unsigned)(seq & 0xffffff);
-            // the word normally arrives within a few microseconds of the last launch call; past that (long iterations,
-            // several engines per GPU and ranks per box sharing the cores) the thread gives its core away between polls
-            if (!seen) { if (spin < 256 || pure_spin) cpu_relax(); else sched_yield(); }
-            if (!seen && (spin & 0x3FFF) == 0x3FFF) {
-                const cudaError_t q = cudaStreamQuery(s);
-                if (q == cudaSuccess) {   // stream drained: the word is there, or the mapping is unavailable: take a copy
-                    w = *word;
-                    if ((unsigned)((w >> 40) & 0xffffff) != (unsigned)(seq & 0xffffff)) {
-                        TTB_CHECK(!cont, "the control word of the continuous beam-search loop did not arrive");
-                        TTB_CUDA_OK(cudaMemcpy(hc, st.ctrl, BC_COUNT * sizeof(int), cudaMemcpyDeviceToHost));
-                        w = ((unsigned long long)(seq & 0xffffff) << 40) | ((unsigned long long)(hc[BC_ERROR] & 0xf) << 36) |
-                            ((unsigned long long)(hc[BC_ALL_FINISHED] & 1) << 35) | ((unsigned long long)(hc[BC_EMPTY_COLS] & 0xfff) << 23) |
-                            ((unsigned long long)0xffff << 7);   // live candidates unknown: full grids
-                    }
-                    seen = true;
-                } else if (q != cudaErrorNotReady) {
-                    TTB_CUDA_OK(q);
-                }
-            }
+        bool arrived = true;
+        if (int rc = wait_posted_word(e, s, seq, &w, &arrived, pure_spin)) return rc;
+        if (!arrived) {   // the stream drained without the word (mapping unavailable): take a copy of the control words
+            TTB_CHECK(!cont, "the control word of the continuous beam-search loop did not arrive");
+            TTB_CUDA_OK(cudaMemcpy(hc, st.ctrl, BC_COUNT * sizeof(int), cudaMemcpyDeviceToHost));
+            w = ((unsigned long long)(seq & 0xffffff) << 40) | ((unsigned long long)(hc[BC_ERROR] & 0xf) << 36) |
+                ((unsigned long long)(hc[BC_ALL_FINISHED] & 1) << 35) | ((unsigned long long)(hc[BC_EMPTY_COLS] & 0xfff) << 23) |
+                ((unsigned long long)0xffff << 7);   // live candidates unknown: full grids
         }
         if (cont) {   // sequence | slots in use | largest draft length of the open batches | unfinished candidates
             cont_used = (int)((w >> 28) & 0xfff);
@@ -1511,23 +1520,45 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
 // hypothesis is served from its self-attention cache, which follows the hypotheses through the re-parenting of every step,
 // in two ping-pong copies); tokens, scores and logits stay on the device, the host reads the control words of the stop
 // test one step behind.
+
+// Continuous batching (ttb_beam_search_generate_batches): the batches that share the query slots of one loop.
+struct SbArgs {
+    int n;                              // batches, admitted in list order
+    const int64_t* const* src;          // [n] (B_i, Ls_i) int64 sources
+    const int32_t* bs;                  // [n] B_i
+    const int32_t* ls;                  // [n] Ls_i
+    int64_t* const* out;                // [n] B_i * beam_size * max_len int64 hypotheses
+    int32_t* out_width;                 // [n] width of each batch's hypotheses
+    ttb_generate_stats* stats;          // [n]
+};
+
+// With `cb` the loop is the continuous one: B is the number of query slots, Ls the longest source of all batches, and the
+// batches of `cb` are admitted into free slots between two steps.
 template <typename ActT>
 static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int max_len, int K, int pad, int bos, int eos,
-                        int64_t* out_dev, int32_t* out_width, ttb_generate_stats* stats, cudaStream_t user_stream) {
+                        int64_t* out_dev, int32_t* out_width, ttb_generate_stats* stats, cudaStream_t user_stream, const SbArgs* cb = nullptr) {
     const int E = e->E(), H = e->d.num_heads, HD = e->HD(), V = e->d.tgt_vocab_size;
     const int n_dec = (int)e->dec.size();
     cudaStream_t s = e->stream;
     TTB_CUDA_OK(cudaEventRecord(e->join_ev, user_stream));
     TTB_CUDA_OK(cudaStreamWaitEvent(s, e->join_ev, 0));
     const long long launches0 = e->launches;
+    const bool cont = cb != nullptr;
     const long long TS = (long long)B * Ls;
-    const long long TS_cap = (long long)B * std::max(256, (Ls + 63) / 64 * 64);   // no reallocation from one batch length to the next
+    const int Ls_cap = std::max(256, (Ls + 63) / 64 * 64);
+    const long long TS_cap = (long long)B * Ls_cap;   // no reallocation from one batch length to the next
     const int Cmax = B * K, ldw = max_len;
+    // continuous loop: the encoder of an admitted batch runs on that batch's shape, in a workspace of its own
+    int B_stage = 0;
+    long long TS_stage = 0;
+    if (cont)
+        for (int i = 0; i < cb->n; ++i) { B_stage = std::max(B_stage, (int)cb->bs[i]); TS_stage = std::max(TS_stage, (long long)cb->bs[i] * cb->ls[i]); }
+    const long long TS_enc = cont ? TS_stage : TS_cap;
 
-    if (e->src32.ensure(TS_cap * sizeof(int)) || e->memory.ensure(TS_cap * E * sizeof(float))) return 1;
-    if (Prec<ActT>::lowp && e->memh.ensure(TS_cap * E * sizeof(ActT))) return 1;
+    if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float))) return 1;
+    if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
     if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
-    if (ensure_work<ActT>(e, std::max<long long>(Cmax, TS_cap), n_dec)) return 1;
+    if (ensure_work<ActT>(e, cont ? (long long)Cmax : std::max<long long>(Cmax, TS_cap), n_dec)) return 1;
     DevBuf& bb = e->beam;
     size_t off = 0;
     auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
@@ -1540,51 +1571,92 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
     const size_t cbytes = (size_t)n_dec * cache_l_stride * sizeof(ActT);
     if (e->kcache.ensure(cbytes) || e->vcache.ensure(cbytes) || e->kcache2.ensure(cbytes) || e->vcache2.ensure(cbytes)) return 1;
     if (e->srclen.ensure((size_t)B * sizeof(int))) return 1;
+    // continuous loop: slot / batch tables, staging of an admitted batch (source lengths, cross K/V), slot-major key
+    // tokens, encoder workspace
+    SbTable cbt{};
+    int* stage_srclen = nullptr;
+    ActT* stage_kv = nullptr;
+    EncWork<ActT> enc_work{};
+    if (cont) {
+        TTB_CHECK((2 * E * sizeof(ActT)) % 16 == 0, "continuous batching needs 16-byte cross-attention K/V rows");
+        size_t co = 0;
+        auto ctake = [&](size_t bytes) { size_t o = co; co += (bytes + 255) / 256 * 256; return o; };
+        const size_t c_sg = ctake((size_t)B * 4), c_sq = ctake((size_t)B * 4), c_as = ctake((size_t)B * 4), c_gr = ctake((size_t)cb->n * sizeof(SbGroup));
+        const size_t c_sl = ctake((size_t)B_stage * 4), c_kv = ctake((size_t)n_dec * TS_stage * 2 * E * sizeof(ActT));
+        if (e->cb.ensure(co) || e->cb_work.ensure(enc_work_bytes<ActT>(e, TS_stage))) return 1;
+        if (e->keytok32.ensure((size_t)TS_cap * sizeof(int))) return 1;
+        char* cbase = e->cb.as<char>();
+        cbt.slot_group = (int*)(cbase + c_sg); cbt.slot_q = (int*)(cbase + c_sq); cbt.adm_slots = (int*)(cbase + c_as);
+        cbt.groups = (SbGroup*)(cbase + c_gr);
+        stage_srclen = (int*)(cbase + c_sl);
+        stage_kv = (ActT*)(cbase + c_kv);
+        enc_work = enc_work_carve<ActT>(e, TS_stage, e->cb_work.p);
+    }
+    // nothing is allocated from here on (cudaFree would synchronise the device)
+    const long long sig0 = e->alloc_signature();
     char* base = bb.as<char>();
 
     TTB_CUDA_OK(cudaEventRecord(e->t0, s));
     int* src32 = e->src32.as<int>();
-    { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(src_dev), src32, TS, s); }
     float* mem = e->memory.as<float>();
     ActT* memh = Prec<ActT>::lowp ? e->memh.as<ActT>() : nullptr;
-    if (encode_impl<ActT>(e, src32, src32, B, Ls, mem, memh, s)) return 1;
     ActT* crosskv = e->crosskv.as<ActT>();
-    if (cross_kv_impl<ActT>(e, mem, memh, (int)TS, crosskv, s)) return 1;
+    if (!cont) {
+        { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(src_dev), src32, TS, s); }
+        if (encode_impl<ActT>(e, src32, src32, B, Ls, mem, memh, s)) return 1;
+        if (cross_kv_impl<ActT>(e, mem, memh, (int)TS, crosskv, s)) return 1;
+    }
 
     StdBeamState st{};
-    st.B = B; st.K = K; st.V = V; st.pad = pad; st.bos = bos; st.eos = eos; st.ldw = ldw;
+    st.B = B; st.K = K; st.V = V; st.pad = pad; st.bos = bos; st.eos = eos; st.ldw = ldw; st.max_len = max_len;
     st.y_cur = (int*)(base + o_y0); st.y_next = (int*)(base + o_y1);
     st.score_cur = (float*)(base + o_s0); st.score_next = (float*)(base + o_s1);
     st.fin = (int*)(base + o_fin); st.cand_row = (int*)(base + o_cr); st.row_cand = (int*)(base + o_rc); st.row_query = (int*)(base + o_rq);
     st.total = (float*)(base + o_tot); st.ctrl = (int*)(base + o_ctrl);
     float* logits = (float*)(base + o_lg);
     int* const y_set[2] = {st.y_cur, st.y_next};
+    float* const score_set[2] = {st.score_cur, st.score_next};
     st.c_front = (int*)(base + o_cf); st.parent = (int*)(base + o_par);
     st.desc_self = (int4*)(base + o_ds); st.desc_cross = (int4*)(base + o_dc);
-    { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
+    if (!cont) { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
     st.src_len = e->srclen.as<int>();
     ActT *kc_cur = e->kcache.as<ActT>(), *vc_cur = e->vcache.as<ActT>(), *kc_next = e->kcache2.as<ActT>(), *vc_next = e->vcache2.as<ActT>();
-    { Scope sc(e, KC_MISC, s); launch_sbeam_init(st, s); }
+    if (cont) {
+        void* dp = nullptr;
+        for (int i = 16; i < 24; ++i) e->h_ctrl[i] = 0;   // ring of four 64-bit words the select kernel posts into
+        st.host_ctrl = cudaHostGetDevicePointer(&dp, e->h_ctrl + 16, 0) == cudaSuccess ? static_cast<unsigned long long*>(dp) : nullptr;
+        (void)cudaGetLastError();
+        TTB_CHECK(st.host_ctrl, "continuous batching needs mapped pinned host memory for its control word");
+        TTB_CUDA_OK(cudaMemsetAsync(st.ctrl, 0, 64, s));
+        TTB_CUDA_OK(cudaMemsetAsync(cbt.slot_group, 0xff, (size_t)B * sizeof(int), s));   // every slot free
+        TTB_CUDA_OK(cudaMemsetAsync(cbt.groups, 0, (size_t)cb->n * sizeof(SbGroup), s));
+    } else {
+        Scope sc(e, KC_MISC, s);
+        launch_sbeam_init(st, s);
+    }
 
     float* x = e->x.as<float>();
     ActT* xh = Prec<ActT>::lowp ? e->xh.as<ActT>() : nullptr;
     const int* n_live = st.ctrl;
-    int* hc = e->h_ctrl;
-    int W = 1, beam = 1, calls = 0;
-    constexpr int sb_lag = 1;   // steps the host stays ahead of the control words it reads (blocking-sync events: the wait sleeps)
-    // step 0 on the BOS column (:106), then at most max_len - 2 further columns (:127)
-    for (int step = 0; step < max_len - 1; ++step) {
-        const int C = B * beam;
-        { Scope sc(e, KC_MISC, s); launch_sbeam_prepare(st, C, beam, W, s); }
-        RowCount rows1(C, n_live, 1);
-        { Scope sc(e, KC_EMBED, s); launch_sbeam_embed_last<ActT>(st, C, W, e->tgt_emb, e->pe, E, x, xh, s); }
+    // cross-attention K/V and key tokens: per query (generate()) or slot-major with Ls_cap rows per slot (continuous loop)
+    const int kv_ls = cont ? Ls_cap : Ls;
+    const int* key_tok = cont ? e->keytok32.as<int>() : src32;
+    const long long ckv_l_stride = (cont ? TS_cap : TS) * 2 * E;
+    const int max_beam = max_len > 2 ? K : 1;   // the first step of a query selects among V continuations, later ones among K V
+    // One step: C hypotheses (grid of the per-hypothesis kernels), at most R live rows (grid of the decoder kernels), W and
+    // beam of generate()'s step (the continuous kernels read them per batch)
+    auto enqueue_step = [&](int C, int beam, int W, int R) -> int {
+        if (cont) { Scope sc(e, KC_MISC, s); launch_sbeam_prepare_groups(st, cbt, s); }
+        else { Scope sc(e, KC_MISC, s); launch_sbeam_prepare(st, C, beam, W, s); }
+        RowCount rows1(R, n_live, 1);
+        { Scope sc(e, KC_EMBED, s); launch_sbeam_embed_last<ActT>(st, R, e->tgt_emb, e->pe, E, x, xh, s); }
         auto self_attn = [&](int l, ActT* qkv, ActT* att) {
-            spec_attn(qkv, 3 * E, kc_cur + l * cache_l_stride, vc_cur + l * cache_l_stride, cache_c_stride, E, att, E, C, n_live, st.row_cand,
+            spec_attn(qkv, 3 * E, kc_cur + l * cache_l_stride, vc_cur + l * cache_l_stride, cache_c_stride, E, att, E, R, n_live, st.row_cand,
                       st.c_front, st.y_cur, ldw, e->d.tgt_pad_token_idx, 1, 0, H, HD, max_len, s, st.desc_self);
         };
         auto cross_attn = [&](int l, ActT* q2, ActT* att) {
-            const ActT* kv = crosskv + (long long)l * TS * 2 * E;
-            attn(q2, E, kv, kv + E, 2 * E, att, E, C, n_live, 1, Ls, Ls, st.row_query, src32, Ls, e->d.src_pad_token_idx, false, H, HD, s,
+            const ActT* kv = crosskv + (long long)l * ckv_l_stride;
+            attn(q2, E, kv, kv + E, 2 * E, att, E, R, n_live, 1, kv_ls, kv_ls, st.row_query, key_tok, kv_ls, e->d.src_pad_token_idx, false, H, HD, s,
                  nullptr, nullptr, st.desc_cross);
         };
         if (decoder_stack<ActT>(e, rows1, n_dec, (long long)Cmax * 3 * E, self_attn, cross_attn, s)) return 1;
@@ -1593,52 +1665,143 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
         { Scope sc(e, KC_ARGMAX, s); launch_sbeam_scores(st, C, logits, s); }
         {
             Scope sc(e, KC_ACCEPT, s);
-            TTB_CHECK(launch_sbeam_select(st, beam, W, s) == 0, "beam_size * vocabulary too large for the selection kernel");
+            const int rc = cont ? launch_sbeam_select_groups(st, cbt, max_beam, s) : launch_sbeam_select(st, beam, W, s);
+            TTB_CHECK(rc == 0, "beam_size * vocabulary too large for the selection kernel");
         }
         {
             Scope sc(e, KC_CACHE_APPEND, s);
-            launch_sbeam_cache_update<ActT>(st, W, e->qkv.as<ActT>(), (long long)Cmax * 3 * E, n_dec, 3 * E, E, kc_cur, vc_cur, kc_next, vc_next,
+            launch_sbeam_cache_update<ActT>(st, e->qkv.as<ActT>(), (long long)Cmax * 3 * E, n_dec, 3 * E, E, kc_cur, vc_cur, kc_next, vc_next,
                                             cache_l_stride, cache_c_stride, s);
         }
         std::swap(kc_cur, kc_next);
         std::swap(vc_cur, vc_next);
-        // the stop test runs on the device (std_beam.cu: ctrl[2]); the host reads the control words of step - 1 while
-        // this step is already enqueued (a step behind the end is a no-op), so the GPU never waits for the host
-        TTB_CUDA_OK(cudaMemcpyAsync(hc + 32 + (step & 3) * 8, st.ctrl, 4 * sizeof(int), cudaMemcpyDeviceToHost, s));
-        TTB_CUDA_OK(cudaEventRecord(e->poll_ev[step & 3], s));
-        std::swap(st.y_cur, st.y_next);
-        std::swap(st.score_cur, st.score_next);
-        beam = K;
-        W += 1;
-        if (step >= sb_lag) {
-            const int j = (step - sb_lag) & 3;
-            TTB_CUDA_OK(cudaEventSynchronize(e->poll_ev[j]));
-            if (hc[32 + j * 8 + 2]) break;       // every hypothesis contains EOS (:169)
+        return 0;
+    };
+
+    if (!cont) {
+        int* hc = e->h_ctrl;
+        int W = 1, beam = 1, calls = 0;
+        constexpr int sb_lag = 1;   // steps the host stays ahead of the control words it reads (blocking-sync events: the wait sleeps)
+        // step 0 on the BOS column (:106), then at most max_len - 2 further columns (:127)
+        for (int step = 0; step < max_len - 1; ++step) {
+            const int C = B * beam;
+            if (int rc = enqueue_step(C, beam, W, C)) return rc;
+            // the stop test runs on the device (std_beam.cu: ctrl[2]); the host reads the control words of step - 1 while
+            // this step is already enqueued (a step behind the end is a no-op), so the GPU never waits for the host
+            TTB_CUDA_OK(cudaMemcpyAsync(hc + 32 + (step & 3) * 8, st.ctrl, 4 * sizeof(int), cudaMemcpyDeviceToHost, s));
+            TTB_CUDA_OK(cudaEventRecord(e->poll_ev[step & 3], s));
+            std::swap(st.y_cur, st.y_next);
+            std::swap(st.score_cur, st.score_next);
+            beam = K;
+            W += 1;
+            if (step >= sb_lag) {
+                const int j = (step - sb_lag) & 3;
+                TTB_CUDA_OK(cudaEventSynchronize(e->poll_ev[j]));
+                if (hc[32 + j * 8 + 2]) break;       // every hypothesis contains EOS (:169)
+            }
         }
+        // steps that really ran (the host may have enqueued one more, a no-op): width, call count, and the hypothesis set
+        // the last real step wrote (step i reads set i & 1 and writes the other one)
+        int fin[4] = {};
+        TTB_CUDA_OK(cudaMemcpyAsync(fin, st.ctrl, sizeof(fin), cudaMemcpyDeviceToHost, s));
+        TTB_CUDA_OK(cudaStreamSynchronize(s));
+        calls = fin[3];
+        W = 1 + calls;
+        st.y_cur = (calls & 1) ? y_set[1] : y_set[0];
+        launch_beam_export(st.y_cur, ldw, B * K, W, reinterpret_cast<long long*>(out_dev), s);
+        e->launches++;
+        TTB_CUDA_OK(cudaEventRecord(e->t1, s));
+        TTB_CUDA_OK(cudaStreamSynchronize(s));
+        TTB_CUDA_OK(cudaGetLastError());
+        prof_collect(e);
+        if (out_width) *out_width = W;
+        float ms = 0.f;
+        cudaEventElapsedTime(&ms, e->t0, e->t1);
+        if (stats) {
+            stats->model_calls = calls;
+            stats->accepted_tokens = 0;
+            stats->produced_tokens = 0;
+            stats->unfinished = 0;
+            stats->error = 0;
+            stats->gpu_launches = (int32_t)(e->launches - launches0);
+            stats->gpu_ms = ms;
+        }
+        return 0;
     }
-    // steps that really ran (the host may have enqueued one more, a no-op): width, call count, and the hypothesis set
-    // the last real step wrote (step i reads set i & 1 and writes the other one)
-    int fin[4] = {};
-    TTB_CUDA_OK(cudaMemcpyAsync(fin, st.ctrl, sizeof(fin), cudaMemcpyDeviceToHost, s));
-    TTB_CUDA_OK(cudaStreamSynchronize(s));
-    calls = fin[3];
-    W = 1 + calls;
-    st.y_cur = (calls & 1) ? y_set[1] : y_set[0];
-    launch_beam_export(st.y_cur, ldw, B * K, W, reinterpret_cast<long long*>(out_dev), s);
-    e->launches++;
+
+    // Continuous loop.  Between two steps the host admits the next batches (whole, in list order) while the free slots of
+    // the newest word suffice, then enqueues one step with decoder grids sized for the live rows of the word and waits for
+    // the word of that step (the closing CTA of the select kernel posts it while the caches are still being re-parented).
+    auto admit = [&](int i) -> int {
+        const int Bi = cb->bs[i], Li = cb->ls[i];
+        const long long TSi = (long long)Bi * Li;
+        { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(cb->src[i]), src32, TSi, s); }
+        { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, Bi, Li, e->d.src_pad_token_idx, stage_srclen, s); }
+        if (encode_impl<ActT>(e, src32, src32, Bi, Li, mem, memh, s, &enc_work)) return 1;
+        if (cross_kv_impl<ActT>(e, mem, memh, (int)TSi, stage_kv, s, TS_stage * 2 * E)) return 1;
+        {
+            Scope sc(e, KC_MISC, s);
+            if (launch_sbeam_admit(st, cbt, i, Bi, stage_srclen, reinterpret_cast<long long*>(cb->out[i]), s)) return 1;
+        }
+        {
+            CbTable kvt{};
+            kvt.adm_slots = cbt.adm_slots;
+            Scope sc(e, KC_MISC, s);
+            launch_greedy_admit_kv<ActT>(kvt, Bi, Li, Ls_cap, n_dec, E, stage_kv, TS_stage * 2 * E, crosskv, ckv_l_stride, src32, e->keytok32.as<int>(),
+                                         e->d.src_pad_token_idx, s);
+        }
+        cbt.n_groups = i + 1;
+        TTB_CUDA_OK(cudaGetLastError());
+        TTB_CHECK(e->alloc_signature() == sig0, "a workspace buffer moved while the continuous beam-search loop was running");
+        return 0;
+    };
+    // every batch takes part in at most max_len - 1 steps
+    const long long max_steps = (long long)cb->n * (max_len + 1);
+    std::vector<int> hist;
+    int next = 0, step = 0, used = 0, live_next = 0;
+    while (true) {
+        while (next < cb->n && B - used >= cb->bs[next]) {
+            if (int rc = admit(next)) return rc;
+            used += cb->bs[next];
+            live_next += cb->bs[next];   // one BOS hypothesis per query
+            ++next;
+        }
+        if (used == 0) break;   // nothing open and nothing pending (every batch fits the slots)
+        TTB_CHECK(step < max_steps, "continuous beam-search loop did not terminate within max_len steps per batch");
+        hist.push_back(used);
+        st.y_cur = y_set[step & 1]; st.y_next = y_set[(step & 1) ^ 1];
+        st.score_cur = score_set[step & 1]; st.score_next = score_set[(step & 1) ^ 1];
+        if (int rc = enqueue_step(Cmax, K, 0, std::max(1, std::min(live_next, Cmax)))) return rc;
+        unsigned long long w = 0;
+        bool arrived = true;
+        if (int rc = wait_posted_word(e, s, step + 1, &w, &arrived, false)) return rc;
+        TTB_CHECK(arrived, "the control word of the continuous beam-search loop did not arrive");
+        used = (int)((w >> 24) & 0xffff);
+        live_next = (int)(w & 0xffffff);
+        ++step;
+    }
     TTB_CUDA_OK(cudaEventRecord(e->t1, s));
     TTB_CUDA_OK(cudaStreamSynchronize(s));
     TTB_CUDA_OK(cudaGetLastError());
     prof_collect(e);
-    if (out_width) *out_width = W;
+    int ctrl_end[16] = {};
+    TTB_CUDA_OK(cudaMemcpy(ctrl_end, st.ctrl, sizeof(ctrl_end), cudaMemcpyDeviceToHost));
+    TTB_CHECK(ctrl_end[SBC_ADM_ERR] == 0, "continuous batching admitted a batch without enough free slots");
+    std::vector<SbGroup> groups((size_t)cb->n);
+    TTB_CUDA_OK(cudaMemcpy(groups.data(), cbt.groups, groups.size() * sizeof(SbGroup), cudaMemcpyDeviceToHost));
+    e->h_hist = hist;
     float ms = 0.f;
     cudaEventElapsedTime(&ms, e->t0, e->t1);
+    for (int i = 0; i < cb->n; ++i) {
+        const SbGroup& g = groups[(size_t)i];
+        TTB_CHECK(g.closed == 1 && g.B == cb->bs[i], "continuous beam-search loop ended before every batch was finished");
+        cb->stats[i] = ttb_generate_stats{};
+        cb->stats[i].model_calls = g.steps;
+        cb->out_width[i] = 1 + g.steps;
+    }
     if (stats) {
-        stats->model_calls = calls;
-        stats->accepted_tokens = 0;
-        stats->produced_tokens = 0;
-        stats->unfinished = 0;
-        stats->error = 0;
+        *stats = ttb_generate_stats{};
+        stats->model_calls = step;
         stats->gpu_launches = (int32_t)(e->launches - launches0);
         stats->gpu_ms = ms;
     }
@@ -1919,6 +2082,39 @@ int ttb_beam_search_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, i
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     return drained(e, TTB_DISPATCH(e, std_beam_api<float>(e, src_dev, B, Ls, max_len, beam_size, pad_token, bos_token, eos_token, out_dev, out_width, stats, s),
                         std_beam_api<__nv_bfloat16>(e, src_dev, B, Ls, max_len, beam_size, pad_token, bos_token, eos_token, out_dev, out_width, stats, s)));
+}
+
+int ttb_beam_search_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs, const int32_t* batch_sizes,
+                                     const int32_t* src_lens, int32_t slots, int32_t max_len, int32_t beam_size, int32_t pad_token,
+                                     int32_t bos_token, int32_t eos_token, int64_t* const* out_devs, int32_t* out_widths,
+                                     ttb_generate_stats* stats, ttb_generate_stats* total, void* stream) {
+    TTB_CHECK(e && e->finalized, "engine not finalized");
+    TTB_CHECK(n_batches >= 0 && slots > 0, "bad arguments");
+    TTB_CHECK(n_batches == 0 || (src_devs && batch_sizes && src_lens && out_devs && out_widths && stats), "bad arguments");
+    for (int i = 0; i < n_batches; ++i) TTB_CHECK(src_devs[i] && out_devs[i] && batch_sizes[i] > 0 && src_lens[i] > 0, "bad arguments");
+    // the rules of ttb_beam_search_generate, in its order, before any device work
+    TTB_CHECK(max_len > 1 && beam_size > 0, "max_len must be greater than 1 and beam_size greater than 0");
+    TTB_CHECK(beam_size <= e->d.tgt_vocab_size, "beam_size larger than the vocabulary (the reference's first topk fails as well)");
+    TTB_CHECK(max_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
+    int Ls_max = 1;
+    for (int i = 0; i < n_batches; ++i) {
+        TTB_CHECK(src_lens[i] <= e->d.max_positions, "sequence longer than the positional table");
+        TTB_CHECK(batch_sizes[i] <= slots, "slots must be at least the largest batch size");
+        Ls_max = std::max(Ls_max, (int)src_lens[i]);
+    }
+    // generate() fails in its first step (one hypothesis per query) or its second (beam_size of them)
+    TTB_CHECK(sbeam_select_fits(1, e->d.tgt_vocab_size) && (max_len == 2 || sbeam_select_fits(beam_size, e->d.tgt_vocab_size)),
+              "beam_size * vocabulary too large for the selection kernel");
+    TTB_CHECK(slots <= 65535 && (long long)slots * beam_size < (1 << 24), "continuous batching supports at most 65535 slots and 2^24 - 1 hypotheses");
+    if (total) *total = ttb_generate_stats{};
+    if (n_batches == 0) return 0;
+    TTB_CUDA_OK(cudaSetDevice(e->device));
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const SbArgs cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, out_widths, stats};
+    return drained(e, TTB_DISPATCH(e, std_beam_api<float>(e, nullptr, slots, Ls_max, max_len, beam_size, pad_token, bos_token, eos_token, nullptr, nullptr,
+                                                          total, s, &cb),
+                                   std_beam_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, beam_size, pad_token, bos_token, eos_token, nullptr,
+                                                               nullptr, total, s, &cb)));
 }
 
 int ttb_beam_speculative_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len,

@@ -250,30 +250,59 @@ void launch_beam_expand_groups(const BeamState& st, const BcTable& cb, int dl, c
 // ---- std_beam.cu : standard beam search (standard_decoding.py:90-174) -------------------------------------------
 struct StdBeamState {
     int B, K, V, pad, bos, eos, ldw;
+    int max_len;                          // continuous loop: a batch stops after max_len - 1 steps
     int* y_cur; int* y_next;              // [B*K][ldw] hypotheses (query-major), ping-pong
     float* score_cur; float* score_next;  // [B*K]
-    int* fin; int* cand_row;              // [B*K] contains EOS / live-row index or -1
+    int* fin; int* cand_row;              // [B*K] contains EOS / live-row index, -1 (finished) or -2 (absent)
     int* row_cand; int* row_query;        // [live rows]
     float* total;                         // [B*K][V] score + log-softmax
     int* ctrl;                            // [0] live rows, [1] hypotheses with EOS after the selection
     // KV cache: one new token per live hypothesis and step
-    int* c_front;                         // [B*K] cached positions of a hypothesis (= W - 1 for all of them)
-    int* parent;                          // [B*K] hypothesis of the previous step a new hypothesis continues
+    int* c_front;                         // [B*K] cached positions of a hypothesis (= W - 1 of its batch)
+    int* parent;                          // [B*K] hypothesis of the previous step a new hypothesis continues, -1: none
     int4* desc_self; int4* desc_cross;    // per live row: {hypothesis, front, token at front, -} / {query, -, -, source length}
     const int* src_len;
+    unsigned long long* host_ctrl;        // continuous loop: pinned mapped ring of four words the closing CTA posts into
 };
 void launch_sbeam_init(const StdBeamState& st, cudaStream_t s);
 void launch_sbeam_prepare(const StdBeamState& st, int C, int beam, int W, cudaStream_t s);
 void launch_sbeam_scores(const StdBeamState& st, int C, const float* logits, cudaStream_t s);
 int launch_sbeam_select(const StdBeamState& st, int beam, int W, cudaStream_t s);
-// embedding of the last token (position W - 1) of every live hypothesis
+// shared memory of the selection of a query with `beam` hypotheses fits the kernel
+bool sbeam_select_fits(int beam, int V);
+// embedding of the last token (position front = W - 1 of desc_self) of every live hypothesis
 template <typename ActT>
-void launch_sbeam_embed_last(const StdBeamState& st, int max_rows, int W, const float* table, const float* pe, int E, float* x, ActT* xh,
+void launch_sbeam_embed_last(const StdBeamState& st, int max_rows, const float* table, const float* pe, int E, float* x, ActT* xh,
                              cudaStream_t s);
-// cache of a new hypothesis = cache of its parent [0, W - 1) + K/V of the parent's row of this step (position W - 1)
+// cache of a new hypothesis = cache of its parent [0, W - 1) + K/V of the parent's row of this step (position W - 1, W of
+// the parent's batch)
 template <typename ActT>
-void launch_sbeam_cache_update(const StdBeamState& st, int W, const ActT* qkv_all, long long qkv_layer_stride, int n_layers, int qkv_ld, int E,
+void launch_sbeam_cache_update(const StdBeamState& st, const ActT* qkv_all, long long qkv_layer_stride, int n_layers, int qkv_ld, int E,
                                const ActT* kc_cur, const ActT* vc_cur, ActT* kc_next, ActT* vc_next, long long cache_layer_stride,
                                long long cache_cand_stride, cudaStream_t s);
+
+// Continuous batching of the standard beam search (StdBeamState::B = number of query slots; slot q owns hypotheses
+// q K .. q K + K - 1).  One record per batch: what the reference couples across the queries of a batch.
+struct SbGroup {
+    long long* out;      // [B][K][W + 1] the batch's hypotheses, rewritten at its width every step
+    int B, W, beam;      // batch size; hypothesis width and hypotheses per query of its coming step
+    int steps;           // steps taken part in (model calls)
+    int n_eos, closed;   // hypotheses with EOS after the selection of the step in flight; 1 once the batch has stopped
+};
+struct SbTable {
+    int* slot_group;     // [slots] batch of the query in the slot, -1 = free
+    int* slot_q;         // [slots] index of that query in its batch
+    int* adm_slots;      // [max batch size] slots given to the batch admitted last
+    SbGroup* groups;     // [n_batches]
+    int n_groups;        // batches admitted so far
+};
+// control words of the continuous loop behind the ones of generate()
+constexpr int SBC_TICKET = 4, SBC_USED = 5, SBC_SEQ = 6, SBC_ADM_ERR = 7;
+// admission of batch `grp` (Bi queries, srclen_in [Bi]) into the first Bi free slots, between two steps; 0 or an error code
+int launch_sbeam_admit(const StdBeamState& st, const SbTable& cb, int grp, int Bi, const int* srclen_in, long long* out, cudaStream_t s);
+// group-aware prepare and select; the select kernel's last CTA closes the step of every open batch and posts the word
+// sequence (24 bits) | slots in use (16) | live rows of the next step (24)
+void launch_sbeam_prepare_groups(const StdBeamState& st, const SbTable& cb, cudaStream_t s);
+int launch_sbeam_select_groups(const StdBeamState& st, const SbTable& cb, int max_beam, cudaStream_t s);
 
 }  // namespace ttb

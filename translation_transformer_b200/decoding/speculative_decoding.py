@@ -35,11 +35,12 @@ _BEAM_REF_ERRORS = {
 }
 
 
-def _check_batches(batches: list, slots: int | None, per_batch: int) -> int:
-    """Argument rules of generate_batches(), checked before any device work; returns the slot count."""
+def _check_batches(batches: list, slots: int | None, per_batch: int, min_len: int = 2) -> int:
+    """Argument rules of generate_batches(), checked before any device work; returns the slot count.  `min_len`: the
+    shortest source width the decoder's generate() accepts."""
     for b in batches:
-        if b.dim() != 2 or b.shape[0] < 1 or b.shape[1] < 2:
-            raise ValueError(f"every batch must be a (B >= 1, Ls >= 2) tensor of token ids, got shape {tuple(b.shape)}")
+        if b.dim() != 2 or b.shape[0] < 1 or b.shape[1] < min_len:
+            raise ValueError(f"every batch must be a (B >= 1, Ls >= {min_len}) tensor of token ids, got shape {tuple(b.shape)}")
     if len({b.device for b in batches}) != 1:
         raise ValueError("all batches must be on the same device")
     bmax = max(int(b.shape[0]) for b in batches)

@@ -7,11 +7,19 @@ no draft tokens (one CUDA-graph replay per generated token, no host round-trip p
 from __future__ import annotations
 
 import ctypes as C
+from typing import Sequence
 
 import torch
 
 from .. import _lib
 from ..model import B200Transformer
+from .speculative_decoding import _check_batches
+
+# TranslationInferenceBeamSearch.generate_batches(): default query slots per query of the largest batch (each slot holds
+# beam_size hypotheses).  Trained-like bench batches on one B200 at 1000 W, 1 / 2 / 4 / 8 / 16 x bs slots: 145 / 262 / 473 /
+# 739 / 1051 SMILES/s (bs 4, beam 5) and 281 / 462 / 676 / 897 / 1095 (retro, bs 8, beam 10), against 138 and 261 one batch
+# at a time (profiles/r5_continuous_std_beam_*.json, DESIGN.md section 12)
+DEFAULT_STD_BEAM_SLOTS_PER_BATCH = 16
 
 
 class TranslationInferenceGreedy:
@@ -92,3 +100,42 @@ class TranslationInferenceBeamSearch:
         W = width.value
         res = out[:B * self.beam_size * W].view(B, self.beam_size, W)
         return res if src.is_cuda else res.to(src.device)
+
+    def generate_batches(self, batches: Sequence[torch.Tensor], slots: int | None = None) -> list:
+        """Continuous batching: decode `batches` in ONE device loop whose `slots` query slots (beam_size hypotheses each)
+        are refilled with the queries of the next batch as soon as enough of them are free (batches are admitted whole, in
+        list order, between two steps; a batch frees its slots when it stops).
+
+        Returns `[self.generate(b) for b in batches]` bit for bit, each (B_i, beam_size, W_i), and advances the counters
+        as those calls would: a batch keeps the width, first step and stop rule of its own batch in the shared loop.
+        `slots` defaults to DEFAULT_STD_BEAM_SLOTS_PER_BATCH times the largest batch size."""
+        batches = list(batches)
+        if not batches:
+            return []
+        m = self.model
+        slots = _check_batches(batches, slots, DEFAULT_STD_BEAM_SLOTS_PER_BATCH, min_len=1)   # generate() takes Ls = 1 too
+        n, K = len(batches), self.beam_size
+        srcs = [b.to(device=m.device, dtype=torch.int64, non_blocking=True).contiguous() for b in batches]
+        outs = [torch.empty(s.shape[0] * K * self.max_len, dtype=torch.int64, device=m.device) for s in srcs]
+        ptrs = lambda ts: (C.c_void_p * n)(*[t.data_ptr() for t in ts])
+        sizes = (C.c_int32 * n)(*[s.shape[0] for s in srcs])
+        lens = (C.c_int32 * n)(*[s.shape[1] for s in srcs])
+        widths = (C.c_int32 * n)()
+        stats = (_lib.GenerateStats * n)()
+        total = _lib.GenerateStats()
+        with torch.cuda.device(m.device):
+            rc = m.lib.ttb_beam_search_generate_batches(
+                m._h, n, ptrs(srcs), sizes, lens, slots, self.max_len, K, self.pad_token, self.bos_token, self.eos_token,
+                ptrs(outs), widths, stats, C.byref(total), torch.cuda.current_stream(m.device).cuda_stream)
+        _lib.check(rc, "ttb_beam_search_generate_batches")
+        self.last_stats = total
+        self.gpu_launches += total.gpu_launches
+        self.gpu_ms += total.gpu_ms
+        results = []
+        for i in range(n):
+            B, W = srcs[i].shape[0], widths[i]
+            self.model_calls_num += stats[i].model_calls
+            self.given_tokens += int((srcs[i] != m.src_pad_token_i).sum().item())
+            res = outs[i][:B * K * W].view(B, K, W)
+            results.append(res if batches[i].is_cuda else res.to(batches[i].device))
+        return results
