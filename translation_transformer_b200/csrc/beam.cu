@@ -601,7 +601,7 @@ void launch_beam_expand(const BeamState& st, int beam, int dl, cudaStream_t s) {
 }
 
 // ---- continuous batching: several batches share the query slots of one loop ----------------------------------------
-// Slot b holds query cb.slot_q[b] of batch cb.slot_group[b] (-1: free) and candidates b K .. b K + K - 1.  A batch keeps
+// Slot b holds query cb.slots.slot_q[b] of batch cb.slots.slot_group[b] (-1: free) and candidates b K .. b K + K - 1.  A batch keeps
 // in its BcGroup what the reference couples across the queries of a batch: token-matrix width, draft length, iteration,
 // the smart-mode padding length, counters, error and stop rule.  Every decoder call runs at the largest draft length of
 // the open batches; a batch with a shorter one ignores the extra scored positions (the self-attention over the step
@@ -622,7 +622,7 @@ __global__ void __launch_bounds__(1024) beam_admit_kernel(BeamState st, BcTable 
     __shared__ int s_nfree;
     const int S = st.B, K = st.K, N = st.N, V = st.V, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     if (warp == 0) {
-        const int taken = take_free_slots(cb.slot_group, S, Bi, s_slots);
+        const int taken = take_free_slots(cb.slots.slot_group, S, Bi, s_slots);
         if (lane == 0) s_nfree = taken;
     }
     __syncthreads();
@@ -632,9 +632,9 @@ __global__ void __launch_bounds__(1024) beam_admit_kernel(BeamState st, BcTable 
     }
     for (int j = threadIdx.x; j < Bi; j += blockDim.x) {
         const int b = s_slots[j];
-        cb.adm_slots[j] = b;
-        cb.slot_group[b] = grp;
-        cb.slot_q[b] = j;
+        cb.slots.adm_slots[j] = b;
+        cb.slots.slot_group[b] = grp;
+        cb.slots.slot_q[b] = j;
         const_cast<int*>(st.src_len)[b] = srclen_in[j];
     }
     // both hypothesis buffers (the coming iteration reads one of them and writes the other): BOS row for candidate 0
@@ -670,11 +670,12 @@ __global__ void __launch_bounds__(1024) beam_admit_kernel(BeamState st, BcTable 
         st.ctrl[BCC_USED] += Bi;
     }
 }
-void launch_beam_admit(const BeamState& st, const BcTable& cb, int grp, int Bi, const int* drafts_in, int lib_in, const int* tok_cnt_in,
-                       const int* tok_list_in, const int* srclen_in, long long* out, int* trace_nacc, int* trace_pick, int dl_first, cudaStream_t s) {
+int launch_beam_admit(const BeamState& st, const BcTable& cb, int grp, int Bi, const int* drafts_in, int lib_in, const int* tok_cnt_in,
+                      const int* tok_list_in, const int* srclen_in, long long* out, int* trace_nacc, int* trace_pick, int dl_first, cudaStream_t s) {
     const size_t smem = (size_t)Bi * sizeof(int);
-    if (ensure_dyn_smem(beam_admit_kernel, (int)smem)) return;   // the launch below then fails loudly
+    if (ensure_dyn_smem(beam_admit_kernel, (int)smem)) return 1;   // error recorded by ensure_dyn_smem
     beam_admit_kernel<<<1, 1024, smem, s>>>(st, cb, grp, Bi, drafts_in, lib_in, tok_cnt_in, tok_list_in, srclen_in, out, trace_nacc, trace_pick, dl_first);
+    return 0;
 }
 
 // Prepare step of the continuous loop: beam_prepare per candidate with the width / draft length of its batch; row bases
@@ -683,7 +684,7 @@ __global__ void __launch_bounds__(1024) beam_prepare_groups_kernel(BeamState st,
     const int K = st.K, N = st.N, C = st.B * K;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, n_warps = blockDim.x >> 5;
     for (int c = warp; c < C; c += n_warps) {
-        const int g = cb.slot_group[c / K];
+        const int g = cb.slots.slot_group[c / K];
         if (g < 0 || (c % K != 0 && cb.groups[g].iter == 0)) {   // free slot, or a candidate that does not exist yet
             if (lane == 0) st.c_fin[c] = 2;
             continue;
@@ -718,7 +719,7 @@ __global__ void __launch_bounds__(1024) beam_prepare_groups_kernel(BeamState st,
         const int c = c0 + threadIdx.x, q = c / K;
         int rows = 0, live = 0, rl = 0;
         if (c < C && st.c_fin[c] != 2) {
-            const int g = cb.slot_group[q];
+            const int g = cb.slots.slot_group[q];
             rl = cb.groups[g].dl + 1;   // positions of the candidate's draft rows (the attention's per-group row length)
             const int slot0 = st.c_slot0[c];
             st.c_front[c] = max(0, slot0 - 1);
@@ -757,7 +758,7 @@ __global__ void __launch_bounds__(1024) beam_prepare_groups_kernel(BeamState st,
             const int q = c / K, base = st.c_rowbase[c], cnt = st.c_cnt[c];
             const int* list = st.tok_list + ((long long)q * st.V + st.c_last[c]) * N;
             const int f = st.c_front[c];
-            const int4 ds = make_int4(c, f, st.cand_cur[(long long)c * st.ldw + f], cb.groups[cb.slot_group[q]].dl + 1);
+            const int4 ds = make_int4(c, f, st.cand_cur[(long long)c * st.ldw + f], cb.groups[cb.slots.slot_group[q]].dl + 1);
             const int4 dc = make_int4(q, 0, 0, st.src_len[q]);
             for (int j = 0; j < cnt; ++j) {
                 st.live_cand[base + j] = c;
@@ -780,8 +781,8 @@ __global__ void __launch_bounds__(256) beam_choose_groups_kernel(BeamState st, B
     extern __shared__ unsigned char s_hit[];
     if (st.c_fin[c] == 2) return;
     const int q = c / K;
-    const BcGroup& gr = cb.groups[cb.slot_group[q]];
-    const int cl = gr.iter == 0 ? cb.slot_q[q] : cb.slot_q[q] * K + c % K;
+    const BcGroup& gr = cb.groups[cb.slots.slot_group[q]];
+    const int cl = gr.iter == 0 ? cb.slots.slot_q[q] : cb.slots.slot_q[q] * K + c % K;
     const long long tr = (long long)gr.iter * gr.B * K + cl;
     choose_candidate(st, c, q, gr.dl, rs, st.smart ? gr.lmax : st.N, par, s_hit, s_nacc, gr.trace_nacc ? gr.trace_nacc + tr * st.N : nullptr,
                      gr.trace_pick ? gr.trace_pick + tr : nullptr);
@@ -800,12 +801,12 @@ void launch_beam_choose_groups(const BeamState& st, const BcTable& cb, int dl, c
 __global__ void __launch_bounds__(256) beam_expand_groups_kernel(BeamState st, BcTable cb, int rs) {
     pdl_wait();   // launched with the programmatic attribute: scheduled while the predecessor drains, starts when it is complete
     const int q = blockIdx.x, K = st.K;
-    const int g = cb.slot_group[q];
+    const int g = cb.slots.slot_group[q];
     if (g >= 0) {
         BcGroup* gr = &cb.groups[g];
         const int W = gr->W;
         int* ctrl = st.ctrl;
-        expand_query(st, q, K, gr->dl, rs, W, &gr->error, gr->out + (long long)cb.slot_q[q] * K * W,
+        expand_query(st, q, K, gr->dl, rs, W, &gr->error, gr->out + (long long)cb.slots.slot_q[q] * K * W,
                      [gr, ctrl](int, bool fin, int p, int pads, int has_eos) {
                          if (!has_eos) { atomicAnd(&gr->all_fin, 0); atomicAdd(&ctrl[BCX_NLIVE_NEXT], 1); }
                          atomicMin(&gr->min_pad, pads);
@@ -848,8 +849,8 @@ __global__ void __launch_bounds__(256) beam_expand_groups_kernel(BeamState st, B
     }
     __syncthreads();
     for (int b = threadIdx.x; b < st.B; b += blockDim.x) {
-        const int gb = cb.slot_group[b];
-        if (gb >= 0 && cb.groups[gb].closed) cb.slot_group[b] = -1;
+        const int gb = cb.slots.slot_group[b];
+        if (gb >= 0 && cb.groups[gb].closed) cb.slots.slot_group[b] = -1;
     }
     __syncthreads();
     if (threadIdx.x == 0) {

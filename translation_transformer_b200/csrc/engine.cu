@@ -11,6 +11,8 @@
 #include <map>
 #include <mutex>
 #include <string>
+#include <type_traits>
+#include <utility>
 #include <vector>
 
 namespace ttb {
@@ -619,35 +621,144 @@ static int decode_api(ttb_engine* e, const int64_t* tgt_dev, int B, int Lt, cons
     return 0;
 }
 
-// Continuous batching (ttb_greedy_speculative_generate_batches): the batches that share the slots of one loop.
-struct CbArgs {
+// Encoder and cross-attention K/V of one batch of (B, Ls) int64 sources: tokens into e->src32, per-query source lengths
+// into `srclen` (the cross-attention kernels skip the padding behind them), the K/V of decoder layer l at
+// kv + l * kv_layer_stride.  `work`: the encoder's workspace, nullptr for the engine's forward workspace.
+template <typename ActT>
+static int encode_batch(ttb_engine* e, const int64_t* src, int B, int Ls, int* srclen, ActT* kv, long long kv_layer_stride, cudaStream_t s,
+                        const EncWork<ActT>* work = nullptr) {
+    const long long TS = (long long)B * Ls;
+    int* src32 = e->src32.as<int>();
+    float* mem = e->memory.as<float>();
+    ActT* memh = Prec<ActT>::lowp ? e->memh.as<ActT>() : nullptr;
+    { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(src), src32, TS, s); }
+    { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, srclen, s); }
+    if (encode_impl<ActT>(e, src32, src32, B, Ls, mem, memh, s, work)) return 1;
+    return cross_kv_impl<ActT>(e, mem, memh, (int)TS, kv, s, kv_layer_stride);
+}
+
+// The decoding loops run on the engine's own stream (graph capture is not allowed on the legacy default stream), ordered
+// after the caller's stream and drained before they return.
+static int join_caller_stream(ttb_engine* e, cudaStream_t user_stream) {
+    TTB_CUDA_OK(cudaEventRecord(e->join_ev, user_stream));
+    TTB_CUDA_OK(cudaStreamWaitEvent(e->stream, e->join_ev, 0));
+    return 0;
+}
+// End of a decoding loop: drains the engine's stream and collects the kernel-class timings; ms = time since e->t0.
+static int finish_loop(ttb_engine* e, float& ms) {
+    TTB_CUDA_OK(cudaEventRecord(e->t1, e->stream));
+    TTB_CUDA_OK(cudaStreamSynchronize(e->stream));
+    TTB_CUDA_OK(cudaGetLastError());
+    prof_collect(e);
+    ms = 0.f;
+    cudaEventElapsedTime(&ms, e->t0, e->t1);
+    return 0;
+}
+
+// ---- continuous batching, common to the three loops (DESIGN.md section 10) --------------------------------------------
+// The batches that share the query slots of one loop (ttb_*_generate_batches).
+struct BatchList {
     int n;                              // batches, admitted in list order
     const int64_t* const* src;          // [n] (B_i, Ls_i) int64 sources
     const int32_t* bs;                  // [n] B_i
     const int32_t* ls;                  // [n] Ls_i
-    int64_t* const* out;                // [n] (B_i, max_len) int64 predictions
-    int32_t* const* trace;              // [n] optional (max_len + 1, B_i, 4) traces, or NULL
+    int64_t* const* out;                // [n] outputs, laid out as the loop's generate() writes them
     ttb_generate_stats* stats;          // [n]
+    int32_t* out_width;                 // [n] width of each batch's hypotheses (beam searches), or NULL
+    int32_t* const* trace;              // [n] optional greedy traces, or NULL
+    int32_t* const* trace_nacc;         // [n] optional speculative beam-search traces, or NULL
+    int32_t* const* trace_pick;
 };
+
+// Slot tables of a continuous loop and staging of the batch being admitted, in e->cb; the admitted batch's encoder
+// workspace in e->cb_work (never the loop's x / qkv: the next iteration's first kernel still reads qkv).  Admission of
+// batch i: encode(i), the loop's own staging and admission kernel (which takes the free slots), then scatter(i).
+template <typename ActT>
+struct Staging {
+    const BatchList* cb;
+    int B_stage = 0;             // largest batch; the encoder of an admitted batch runs on the largest batch shape
+    long long TS_stage = 0;
+    int slots = 0, Ls_cap = 0;
+    int* srclen = nullptr;       // [B_stage] source lengths of the batch being admitted
+    ActT* kv = nullptr;          // [layers][TS_stage][2E] its cross-attention K/V
+    EncWork<ActT> work{};
+    long long sig0 = 0;          // e->alloc_signature() once the loop is sized: nothing is allocated after it
+
+    explicit Staging(const BatchList* cb_) : cb(cb_) {
+        for (int i = 0; cb && i < cb->n; ++i) {
+            B_stage = std::max(B_stage, (int)cb->bs[i]);
+            TS_stage = std::max(TS_stage, (long long)cb->bs[i] * cb->ls[i]);
+        }
+    }
+    // Sizes and carves e->cb for B slots: the slot tables and t.groups first, at offsets that depend on the slot count only
+    // (the greedy loop's captured graphs bake them; the slot count is part of the graph key), then the common staging and
+    // the loop's `extra` regions {&pointer, bytes}.  Also sizes cb_work and the slot-major key tokens.
+    template <typename Table>
+    int alloc(ttb_engine* e, Table& t, int B, int Ls_cap_, std::initializer_list<std::pair<int**, size_t>> extra) {
+        using G = std::remove_pointer_t<decltype(t.groups)>;
+        const int E = e->E();
+        TTB_CHECK((2 * E * sizeof(ActT)) % 16 == 0, "continuous batching needs 16-byte cross-attention K/V rows");
+        slots = B;
+        Ls_cap = Ls_cap_;
+        size_t off = 0;
+        auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
+        const size_t o_sg = take((size_t)B * 4), o_sq = take((size_t)B * 4), o_as = take((size_t)B * 4), o_gr = take((size_t)cb->n * sizeof(G));
+        const size_t o_sl = take((size_t)B_stage * 4), o_kv = take(e->dec.size() * TS_stage * 2 * E * sizeof(ActT));
+        std::vector<size_t> o_extra;
+        for (const auto& x : extra) o_extra.push_back(take(x.second));
+        if (e->cb.ensure(off) || e->cb_work.ensure(enc_work_bytes<ActT>(e, TS_stage)) || e->keytok32.ensure((size_t)B * Ls_cap * sizeof(int))) return 1;
+        char* base = e->cb.as<char>();
+        t.slots = SlotTable{(int*)(base + o_sg), (int*)(base + o_sq), (int*)(base + o_as)};
+        t.groups = (G*)(base + o_gr);
+        srclen = (int*)(base + o_sl);
+        kv = (ActT*)(base + o_kv);
+        size_t k = 0;
+        for (const auto& x : extra) *x.first = (int*)(base + o_extra[k++]);
+        work = enc_work_carve<ActT>(e, TS_stage, e->cb_work.p);
+        return 0;
+    }
+    // encoder, source lengths and cross K/V of batch i, for the batch alone; its int32 tokens stay in e->src32
+    int encode(ttb_engine* e, int i, cudaStream_t s) {
+        return encode_batch<ActT>(e, cb->src[i], cb->bs[i], cb->ls[i], srclen, kv, TS_stage * 2 * e->E(), s, &work);
+    }
+    // after the admission kernel: the staged K/V and key tokens of batch i -> its slots (slot-major, Ls_cap rows per slot)
+    int scatter(ttb_engine* e, const SlotTable& t, int i, cudaStream_t s) {
+        const int E = e->E();
+        {
+            Scope sc(e, KC_MISC, s);
+            launch_admit_kv<ActT>(t.adm_slots, cb->bs[i], cb->ls[i], Ls_cap, (int)e->dec.size(), E, kv, TS_stage * 2 * E, e->crosskv.as<ActT>(),
+                                  (long long)slots * Ls_cap * 2 * E, e->src32.as<int>(), e->keytok32.as<int>(), e->d.src_pad_token_idx, s);
+        }
+        TTB_CUDA_OK(cudaGetLastError());
+        TTB_CHECK(e->alloc_signature() == sig0, "a workspace buffer moved while a continuous decoding loop was running");
+        return 0;
+    }
+};
+
+// Per-batch records of a continuous loop that has drained: every batch must have been admitted whole and closed.
+template <typename G>
+static int read_groups(const BatchList* cb, const G* dev, std::vector<G>& groups) {
+    groups.resize((size_t)cb->n);
+    TTB_CUDA_OK(cudaMemcpy(groups.data(), dev, groups.size() * sizeof(G), cudaMemcpyDeviceToHost));
+    for (int i = 0; i < cb->n; ++i)
+        TTB_CHECK(groups[(size_t)i].closed == 1 && groups[(size_t)i].B == cb->bs[i], "continuous decoding loop ended before every batch was finished");
+    return 0;
+}
 
 // Speculative greedy loop.  With `cb` the loop is the continuous one: B is the number of query slots, Ls the longest
 // source of all batches, and the batches of `cb` are admitted into free slots between two graph launches.
 template <typename ActT>
 static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int max_len, int draft_len, int N,
                       int pad, int bos, int eos, int replace, int tie_break, int64_t* out_dev, int32_t* trace_dev,
-                      ttb_generate_stats* stats, cudaStream_t user_stream, bool standard = false, const CbArgs* cb = nullptr) {
+                      ttb_generate_stats* stats, cudaStream_t user_stream, bool standard = false, const BatchList* cb = nullptr) {
     const int E = e->E(), H = e->d.num_heads, HD = e->HD(), V = e->d.tgt_vocab_size;
     const int n_dec = (int)e->dec.size();
-    // the loop runs on the engine's own stream (graph capture is not allowed on the legacy default
-    // stream); it is ordered after the caller's stream and fully synchronised before returning
     cudaStream_t s = e->stream;
-    TTB_CUDA_OK(cudaEventRecord(e->join_ev, user_stream));
-    TTB_CUDA_OK(cudaStreamWaitEvent(s, e->join_ev, 0));
+    if (int rc = join_caller_stream(e, user_stream)) return rc;
     // speculative: make_drafts(min_draft_len=1, max_draft_len=max_len); standard greedy decoding (standard_decoding.py)
     // is the same KV-cached loop with one row per query and no draft tokens
     const int D = standard ? 0 : std::min(std::max(1, draft_len), max_len);
     if (standard) N = 1;
-    const long long TS = (long long)B * Ls;
     // buffers that depend on the source length are sized for a rounded-up capacity so that batches of
     // different length neither reallocate nor invalidate the captured graph
     const int Ls_cap = std::max(256, (Ls + 63) / 64 * 64);
@@ -661,12 +772,8 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     // continuous loop: every batch takes part in at most max_len + 1 iterations; the host stays at most (LAG + 1) graph
     // launches ahead of the control words it reads, i.e. a few no-op iterations per admission
     const long long max_iters = cont ? (long long)cb->n * (max_len + 1) + (long long)(cb->n + 1) * 3 * 16 : max_len + 1;
-    // staging of an admitted batch (continuous loop): its encoder runs on the largest batch shape
-    int B_stage = 0;
-    long long TS_stage = 0;
-    if (cont)
-        for (int i = 0; i < cb->n; ++i) { B_stage = std::max(B_stage, (int)cb->bs[i]); TS_stage = std::max(TS_stage, (long long)cb->bs[i] * cb->ls[i]); }
-    const long long TS_enc = cont ? TS_stage : TS_cap;
+    Staging<ActT> sg(cb);
+    const long long TS_enc = cont ? sg.TS_stage : TS_cap;
 
     // encoder + cross-attention K/V (computed once per query, not once per draft row and iteration)
     if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float)) || e->srclen.ensure((size_t)B * sizeof(int))) return 1;
@@ -680,38 +787,18 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     if (e->desc.ensure((size_t)B * sizeof(int4))) return 1;
     if (e->hist.ensure((size_t)(max_iters + 1) * sizeof(int))) return 1;
     if (ensure_work<ActT>(e, cont ? T : std::max(T, TS_cap), n_dec)) return 1;
-    // continuous loop: tables, staging of an admitted batch, slot-major source tokens, encoder workspace
+    // continuous loop: slot / batch tables, staging of an admitted batch (drafts as well)
     CbTable cbt{};
     int* stage_drafts = nullptr;
-    int* stage_srclen = nullptr;
-    ActT* stage_kv = nullptr;
-    EncWork<ActT> enc_work{};
     if (cont) {
-        TTB_CHECK((2 * E * sizeof(ActT)) % 16 == 0, "continuous batching needs 16-byte cross-attention K/V rows");
         TTB_CHECK(B <= 2048, "continuous batching supports at most 2048 slots");
-        // the captured graphs bake the table addresses: their offsets depend on the slot count only (part of the graph
-        // key); the staging buffers of the call's batches come behind them
-        const size_t grp_off = ((size_t)3 * B * sizeof(int) + 255) / 256 * 256;
-        const size_t stage_off = grp_off + ((size_t)cb->n * sizeof(CbGroup) + 255) / 256 * 256;
-        const size_t kv_off = stage_off + (((size_t)2 * B_stage + (size_t)B_stage * N * D) * sizeof(int) + 255) / 256 * 256;
-        if (e->cb.ensure(kv_off + (size_t)n_dec * TS_stage * 2 * E * sizeof(ActT))) return 1;
-        if (e->keytok32.ensure((size_t)TS_cap * sizeof(int))) return 1;
-        if (e->cb_work.ensure(enc_work_bytes<ActT>(e, TS_stage))) return 1;
-        int* base = e->cb.as<int>();
-        cbt.slot_group = base; cbt.slot_q = base + B; cbt.adm_slots = base + 2 * B;
-        cbt.groups = reinterpret_cast<CbGroup*>(e->cb.as<char>() + grp_off);
-        stage_srclen = reinterpret_cast<int*>(e->cb.as<char>() + stage_off);
-        stage_drafts = stage_srclen + B_stage;
-        stage_kv = reinterpret_cast<ActT*>(e->cb.as<char>() + kv_off);
-        enc_work = enc_work_carve<ActT>(e, TS_stage, e->cb_work.p);
+        if (int rc = sg.alloc(e, cbt, B, Ls_cap, {{&stage_drafts, (size_t)sg.B_stage * N * D * sizeof(int)}})) return rc;
     }
     // nothing is allocated from here on: the captured graphs bake these addresses
-    const long long sig0 = e->alloc_signature();
+    sg.sig0 = e->alloc_signature();
 
     TTB_CUDA_OK(cudaEventRecord(e->t0, s));
     int* src32 = e->src32.as<int>();
-    float* mem = e->memory.as<float>();
-    ActT* memh = Prec<ActT>::lowp ? e->memh.as<ActT>() : nullptr;
     ActT* crosskv = e->crosskv.as<ActT>();
     GreedyState st{};
     st.B = B; st.N = N; st.D = D; st.max_len = max_len; st.gen_ld = gen_ld; st.pad = pad; st.bos = bos; st.eos = eos; st.Ls = Ls;
@@ -723,34 +810,20 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     // then the kernels that move it into free slots
     auto admit = [&](int i) -> int {
         const int Bi = cb->bs[i], Li = cb->ls[i];
-        const long long TSi = (long long)Bi * Li;
-        { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(cb->src[i]), src32, TSi, s); }
-        { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, Bi, Li, e->d.src_pad_token_idx, stage_srclen, s); }
-        if (encode_impl<ActT>(e, src32, src32, Bi, Li, mem, memh, s, &enc_work)) return 1;
-        if (cross_kv_impl<ActT>(e, mem, memh, (int)TSi, stage_kv, s, TS_stage * 2 * E)) return 1;
+        if (int rc = sg.encode(e, i, s)) return rc;
         { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Li, Bi, Li - 1, D, N, eos, pad, replace, stage_drafts, s); }
         {
             Scope sc(e, KC_MISC, s);
-            launch_greedy_admit(st, cbt, i, Bi, stage_drafts, stage_srclen, reinterpret_cast<long long*>(cb->out[i]), cb->trace ? cb->trace[i] : nullptr,
-                                Ls_cap, s);
+            if (int rc = launch_greedy_admit(st, cbt, i, Bi, stage_drafts, sg.srclen, reinterpret_cast<long long*>(cb->out[i]),
+                                             cb->trace ? cb->trace[i] : nullptr, Ls_cap, s))
+                return rc;
         }
-        {
-            Scope sc(e, KC_MISC, s);
-            launch_greedy_admit_kv<ActT>(cbt, Bi, Li, Ls_cap, n_dec, E, stage_kv, TS_stage * 2 * E, crosskv, TS_cap * 2 * E, src32, e->keytok32.as<int>(),
-                                         e->d.src_pad_token_idx, s);
-        }
-        TTB_CUDA_OK(cudaGetLastError());
-        TTB_CHECK(e->alloc_signature() == sig0, "a workspace buffer moved while decoding graphs of the continuous loop exist");
-        return 0;
+        return sg.scatter(e, cbt.slots, i, s);
     };
     if (cont) {
         TTB_CUDA_OK(cudaMemsetAsync(st.ctrl, 0, CTRL_COUNT * sizeof(int), s));
     } else {
-    { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(src_dev), src32, TS, s); }
-    // per-query source length: the cross-attention kernels skip the padding behind it
-    { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
-    if (encode_impl<ActT>(e, src32, src32, B, Ls, mem, memh, s)) return 1;
-    if (cross_kv_impl<ActT>(e, mem, memh, (int)TS, crosskv, s, TS_cap * 2 * E)) return 1;
+    if (encode_batch<ActT>(e, src_dev, B, Ls, e->srclen.as<int>(), crosskv, TS_cap * 2 * E, s)) return 1;
     // drafts from the source without its BOS column (speculative_decoding.py:64-73)
     if (!standard) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Ls, B, Ls - 1, D, N, eos, pad, replace, e->drafts.as<int>(), s); }
     { Scope sc(e, KC_MISC, s); launch_greedy_init(st, s); }
@@ -930,24 +1003,19 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
             ++it;
         }
         TTB_CUDA_OK(cudaMemcpyAsync(e->h_ctrl, st.ctrl, CTRL_COUNT * sizeof(int), cudaMemcpyDeviceToHost, s));
-        TTB_CUDA_OK(cudaEventRecord(e->t1, s));
-        TTB_CUDA_OK(cudaStreamSynchronize(s));
-        TTB_CUDA_OK(cudaGetLastError());
-        prof_collect(e);
+        float ms = 0.f;
+        if (int rc = finish_loop(e, ms)) return rc;
         const int* c = e->h_ctrl;
         TTB_CHECK(c[CTRL_ERROR] != 3, "continuous batching admitted a batch without enough free slots");
         TTB_CHECK(c[CTRL_DONE] == 1 && c[CTRL_N_ACTIVE] == 0, "continuous decoding loop ended with live queries");
-        std::vector<CbGroup> groups((size_t)cb->n);
-        TTB_CUDA_OK(cudaMemcpy(groups.data(), cbt.groups, groups.size() * sizeof(CbGroup), cudaMemcpyDeviceToHost));
+        std::vector<CbGroup> groups;
+        if (int rc = read_groups(cb, cbt.groups, groups)) return rc;
         e->h_hist.assign((size_t)c[CTRL_ITERS], 0);
         if (c[CTRL_ITERS] > 0)
             TTB_CUDA_OK(cudaMemcpy(e->h_hist.data(), st.hist, (size_t)c[CTRL_ITERS] * sizeof(int), cudaMemcpyDeviceToHost));
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, e->t0, e->t1);
         ttb_generate_stats sum{};
         for (int i = 0; i < cb->n; ++i) {
             const CbGroup& g = groups[(size_t)i];
-            TTB_CHECK(g.closed == 1 && g.B == cb->bs[i], "continuous decoding loop ended before every batch was finished");
             ttb_generate_stats& o = cb->stats[i];
             o = ttb_generate_stats{};
             o.model_calls = g.iter;
@@ -997,17 +1065,13 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     }
     TTB_CUDA_OK(cudaMemcpyAsync(out_dev, st.out, (size_t)B * max_len * sizeof(long long), cudaMemcpyDeviceToDevice, s));
     TTB_CUDA_OK(cudaMemcpyAsync(e->h_ctrl, st.ctrl, CTRL_COUNT * sizeof(int), cudaMemcpyDeviceToHost, s));
-    TTB_CUDA_OK(cudaEventRecord(e->t1, s));
-    TTB_CUDA_OK(cudaStreamSynchronize(s));
-    TTB_CUDA_OK(cudaGetLastError());
-    prof_collect(e);
+    float ms = 0.f;
+    if (int rc = finish_loop(e, ms)) return rc;
     const int* c = e->h_ctrl;
     TTB_CHECK(c[CTRL_DONE] == 1, "greedy decoding loop did not terminate within max_len + 1 iterations");
     e->h_hist.assign((size_t)c[CTRL_ITERS], 0);
     if (c[CTRL_ITERS] > 0)
         TTB_CUDA_OK(cudaMemcpy(e->h_hist.data(), st.hist, (size_t)c[CTRL_ITERS] * sizeof(int), cudaMemcpyDeviceToHost));
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, e->t0, e->t1);
     if (stats) {
         stats->model_calls = c[CTRL_ITERS];
         stats->accepted_tokens = c[CTRL_ACCEPTED];
@@ -1054,18 +1118,14 @@ static int wait_posted_word(ttb_engine* e, cudaStream_t s, int seq, unsigned lon
     }
 }
 
-// Continuous batching (ttb_beam_speculative_generate_batches): the batches that share the query slots of one loop.
-struct BcArgs {
-    int n;                              // batches, admitted in list order
-    const int64_t* const* src;          // [n] (B_i, Ls_i) int64 sources
-    const int32_t* bs;                  // [n] B_i
-    const int32_t* ls;                  // [n] Ls_i
-    int64_t* const* out;                // [n] B_i * n_best * (max_len + draft length + 4) int64 hypotheses
-    int32_t* out_width;                 // [n] width of each batch's hypotheses
-    int32_t* const* trace_nacc;         // [n] optional traces as in ttb_beam_speculative_generate, or NULL
-    int32_t* const* trace_pick;
-    ttb_generate_stats* stats;          // [n]
-};
+// Device pointer of that ring, cleared, or nullptr when the mapping is unavailable.
+static void* map_posted_ring(ttb_engine* e) {
+    void* dp = nullptr;
+    for (int i = 16; i < 24; ++i) e->h_ctrl[i] = 0;
+    const bool mapped = cudaHostGetDevicePointer(&dp, e->h_ctrl + 16, 0) == cudaSuccess;
+    (void)cudaGetLastError();
+    return mapped ? dp : nullptr;
+}
 
 // ---- speculative beam search (speculative_decoding.py:428-598), host loop + device kernels ---------------
 // The per-iteration shapes (token-matrix width, draft length, live rows) depend on the hypotheses, so the
@@ -1076,19 +1136,17 @@ template <typename ActT>
 static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int max_len, int K, int draft_len, int N,
                     int pad, int bos, int eos, int c_token, int tie_break, int64_t* out_dev, int32_t* out_width,
                     int32_t* trace_nacc, int32_t* trace_pick, ttb_generate_stats* stats, cudaStream_t user_stream, bool smart,
-                    const BcArgs* cb = nullptr) {
+                    const BatchList* cb = nullptr) {
     const int E = e->E(), H = e->d.num_heads, HD = e->HD(), V = e->d.tgt_vocab_size;
     const int n_dec = (int)e->dec.size();
     cudaStream_t s = e->stream;
-    TTB_CUDA_OK(cudaEventRecord(e->join_ev, user_stream));
-    TTB_CUDA_OK(cudaStreamWaitEvent(s, e->join_ev, 0));
+    if (int rc = join_caller_stream(e, user_stream)) return rc;
     const long long launches0 = e->launches;
     const int D0 = std::min(std::max(5, draft_len), 200);       // speculative_decoding.py:278-284
     // smart_drafts_mode (:600-615): library of Ls - 5 windows of draft_len + 1 tokens (BOS column included), first token = key
     const int D_lib = std::min(std::max(5, D0 + 1), 200);
     const int n_lib = Ls - 5;
     if (smart) TTB_CHECK(n_lib > 0, "The number of drafts must be greater than 0");
-    const long long TS = (long long)B * Ls;
     // buffers that depend on the source length are sized for a rounded-up capacity: batches of different length must not
     // reallocate (cudaFree synchronises the whole device, i.e. every other engine decoding on this GPU as well)
     const int Ls_cap = std::max(256, (Ls + 63) / 64 * 64);
@@ -1098,15 +1156,11 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     // only the dl+1 scored positions of every (candidate, draft) row go through the decoder, the prefix of a candidate is
     // served from its self-attention cache, which follows the hypotheses through the re-parenting of every step
     const bool cont = cb != nullptr;
-    // continuous loop: the encoder of an admitted batch runs on the largest batch shape, in a workspace of its own
-    int B_stage = 0;
-    long long TS_stage = 0;
-    if (cont)
-        for (int i = 0; i < cb->n; ++i) { B_stage = std::max(B_stage, (int)cb->bs[i]); TS_stage = std::max(TS_stage, (long long)cb->bs[i] * cb->ls[i]); }
+    Staging<ActT> sg(cb);
     const long long Tc = (long long)Rmax * (D0 + 1);
 
-    const long long TS_enc = cont ? TS_stage : TS_cap;
-    if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float))) return 1;
+    const long long TS_enc = cont ? sg.TS_stage : TS_cap;
+    if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float)) || e->srclen.ensure((size_t)B * sizeof(int))) return 1;
     if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
     if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
     if (e->drafts.ensure(smart ? (size_t)B * std::max(n_lib, Ls_cap) * D_lib * sizeof(int) : (size_t)B * N * D0 * sizeof(int))) return 1;
@@ -1130,45 +1184,28 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
                  o_cl = take(Cmax * 4), o_rd = take(Rmax * 4), o_ds = take(Rmax * 16), o_dc = take(Rmax * 16);
     if (bb.ensure(off)) return 1;
     char* base = bb.as<char>();
-    // continuous loop: slot / batch tables, staging of an admitted batch (source lengths, drafts or window library, cross
-    // K/V), slot-major key tokens and source lengths, encoder workspace
+    // continuous loop: slot / batch tables, staging of an admitted batch (drafts or window library as well), smallest draft
+    // length of every iteration
     BcTable cbt{};
-    int *stage_srclen = nullptr, *stage_drafts = nullptr, *stage_tokcnt = nullptr, *stage_toklist = nullptr;
-    ActT* stage_kv = nullptr;
-    EncWork<ActT> enc_work{};
+    int *stage_drafts = nullptr, *stage_tokcnt = nullptr, *stage_toklist = nullptr;
     if (cont) {
-        TTB_CHECK((2 * E * sizeof(ActT)) % 16 == 0, "continuous batching needs 16-byte cross-attention K/V rows");
         TTB_CHECK(B <= 2048 && (long long)B * K < 65536, "continuous batching supports at most 2048 slots and 65535 candidates");
-        size_t co = 0;
-        auto ctake = [&](size_t bytes) { size_t o = co; co += (bytes + 255) / 256 * 256; return o; };
-        const size_t c_sg = ctake((size_t)B * 4), c_sq = ctake((size_t)B * 4), c_as = ctake((size_t)B * 4), c_gr = ctake((size_t)cb->n * sizeof(BcGroup));
-        const size_t c_sl = ctake((size_t)B_stage * 4), c_dr = ctake((smart ? (size_t)std::max(n_lib, 1) * D_lib : (size_t)N * D0) * B_stage * 4);
-        const size_t c_tc = ctake(smart ? (size_t)B_stage * V * 4 : 4), c_tl = ctake(smart ? (size_t)B_stage * V * N * 4 : 4);
-        const size_t c_kv = ctake((size_t)n_dec * TS_stage * 2 * E * sizeof(ActT));
-        const size_t c_dm = ctake(((size_t)cb->n * (max_len + 1) + 1) * sizeof(int));
-        if (e->cb.ensure(co) || e->cb_work.ensure(enc_work_bytes<ActT>(e, TS_stage))) return 1;
-        if (e->keytok32.ensure((size_t)TS_cap * sizeof(int)) || e->srclen.ensure((size_t)B * sizeof(int))) return 1;
-        char* cbase = e->cb.as<char>();
-        cbt.slot_group = (int*)(cbase + c_sg); cbt.slot_q = (int*)(cbase + c_sq); cbt.adm_slots = (int*)(cbase + c_as);
-        cbt.groups = (BcGroup*)(cbase + c_gr);
-        cbt.dl_min = (int*)(cbase + c_dm);
-        stage_srclen = (int*)(cbase + c_sl); stage_drafts = (int*)(cbase + c_dr); stage_tokcnt = (int*)(cbase + c_tc); stage_toklist = (int*)(cbase + c_tl);
-        stage_kv = (ActT*)(cbase + c_kv);
-        enc_work = enc_work_carve<ActT>(e, TS_stage, e->cb_work.p);
+        const size_t B_stage = (size_t)sg.B_stage;
+        if (int rc = sg.alloc(e, cbt, B, Ls_cap, {{&stage_drafts, (smart ? (size_t)std::max(n_lib, 1) * D_lib : (size_t)N * D0) * B_stage * 4},
+                                                   {&stage_tokcnt, smart ? B_stage * V * 4 : 4},
+                                                   {&stage_toklist, smart ? B_stage * V * N * 4 : 4},
+                                                   {&cbt.dl_min, ((size_t)cb->n * (max_len + 1) + 1) * sizeof(int)}}))
+            return rc;
     }
     // nothing is allocated from here on (cudaFree would synchronise the device)
-    const long long sig0 = e->alloc_signature();
+    sg.sig0 = e->alloc_signature();
 
     TTB_CUDA_OK(cudaEventRecord(e->t0, s));
     int* src32 = e->src32.as<int>();
-    float* mem = e->memory.as<float>();
-    ActT* memh = Prec<ActT>::lowp ? e->memh.as<ActT>() : nullptr;
     ActT* crosskv = e->crosskv.as<ActT>();
     const long long ckv_l_stride = TS_cap * 2 * E;
     if (!cont) {
-        { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(src_dev), src32, TS, s); }
-        if (encode_impl<ActT>(e, src32, src32, B, Ls, mem, memh, s)) return 1;
-        if (cross_kv_impl<ActT>(e, mem, memh, (int)TS, crosskv, s, ckv_l_stride)) return 1;
+        if (encode_batch<ActT>(e, src_dev, B, Ls, e->srclen.as<int>(), crosskv, ckv_l_stride, s)) return 1;
         if (smart) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32, Ls, B, Ls, D_lib, n_lib, eos, pad, c_token, e->drafts.as<int>(), s); }
         else { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Ls, B, Ls - 1, D0, N, eos, pad, c_token, e->drafts.as<int>(), s); }
     }
@@ -1188,22 +1225,12 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     st.topv = (float*)(base + o_topv); st.topi = (int*)(base + o_topi); st.nkeep = (int*)(base + o_keep);
     st.lmax = (float*)(base + o_max); st.lsum = (float*)(base + o_sum);
     st.trace_nacc = trace_nacc; st.trace_pick = trace_pick;
-    {
-        void* dp = nullptr;
-        for (int i = 16; i < 24; ++i) e->h_ctrl[i] = 0;   // ring of four 64-bit words the expand kernel posts into
-        st.host_ctrl = cudaHostGetDevicePointer(&dp, e->h_ctrl + 16, 0) == cudaSuccess ? static_cast<int*>(dp) : nullptr;
-        (void)cudaGetLastError();
-    }
+    st.host_ctrl = static_cast<int*>(map_posted_ring(e));   // the expand kernel posts into it
     st.row_tok = (int*)(base + o_rt); st.tokv = (float*)(base + o_tv);
     st.live_cand = (int*)(base + o_lc); st.live_query = (int*)(base + o_lq); st.c_front = (int*)(base + o_cf);
     st.n_parent = (int*)(base + o_np); st.n_keep = (int*)(base + o_nk); st.n_row = (int*)(base + o_nr);
     st.tok_cnt = (int*)(base + o_tc); st.tok_list = (int*)(base + o_tl); st.c_cnt = (int*)(base + o_cc); st.c_last = (int*)(base + o_cl);
     st.row_draft = (int*)(base + o_rd);
-    if (!cont) {   // continuous loop: per-slot source lengths, installed by the admission kernel
-        // per-query source length: the cross-attention kernels skip the padding behind it
-        if (e->srclen.ensure((size_t)B * sizeof(int))) return 1;
-        { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
-    }
     st.desc_self = (int4*)(base + o_ds); st.desc_cross = (int4*)(base + o_dc); st.src_len = e->srclen.as<int>();
     ActT* kc_cur = e->kcache.as<ActT>();
     ActT* vc_cur = e->vcache.as<ActT>();
@@ -1214,7 +1241,7 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     if (cont) {
         TTB_CHECK(st.host_ctrl, "continuous batching needs mapped pinned host memory for its control word");
         TTB_CUDA_OK(cudaMemsetAsync(st.ctrl, 0, 32 * sizeof(int), s));
-        TTB_CUDA_OK(cudaMemsetAsync(cbt.slot_group, 0xff, (size_t)B * sizeof(int), s));   // every slot free
+        TTB_CUDA_OK(cudaMemsetAsync(cbt.slots.slot_group, 0xff, (size_t)B * sizeof(int), s));   // every slot free
         TTB_CUDA_OK(cudaMemsetAsync(st.n_parent, 0xff, (size_t)Cmax * sizeof(int), s));
         TTB_CUDA_OK(cudaMemsetAsync(cbt.groups, 0, (size_t)cb->n * sizeof(BcGroup), s));
     } else {
@@ -1342,11 +1369,7 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
         const int dl_first = std::min(max_len - 2, dl);   // the first iteration's draft length (budget max_len - 2)
         auto admit = [&](int i) -> int {
             const int Bi = cb->bs[i], Li = cb->ls[i], lib_i = Li - 5;
-            const long long TSi = (long long)Bi * Li;
-            { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(cb->src[i]), src32, TSi, s); }
-            { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, Bi, Li, e->d.src_pad_token_idx, stage_srclen, s); }
-            if (encode_impl<ActT>(e, src32, src32, Bi, Li, mem, memh, s, &enc_work)) return 1;
-            if (cross_kv_impl<ActT>(e, mem, memh, (int)TSi, stage_kv, s, TS_stage * 2 * E)) return 1;
+            if (int rc = sg.encode(e, i, s)) return rc;
             if (smart) {
                 { Scope sc(e, KC_MISC, s); launch_make_drafts(src32, Li, Bi, Li, D_lib, lib_i, eos, pad, c_token, stage_drafts, s); }
                 BeamState lib = st;   // the batch's library alone, as generate() builds it
@@ -1359,20 +1382,13 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
             }
             {
                 Scope sc(e, KC_MISC, s);
-                launch_beam_admit(st, cbt, i, Bi, stage_drafts, lib_i, stage_tokcnt, stage_toklist, stage_srclen, reinterpret_cast<long long*>(cb->out[i]),
-                                  cb->trace_nacc ? cb->trace_nacc[i] : nullptr, cb->trace_pick ? cb->trace_pick[i] : nullptr, dl_first, s);
-            }
-            {
-                CbTable kvt{};
-                kvt.adm_slots = cbt.adm_slots;
-                Scope sc(e, KC_MISC, s);
-                launch_greedy_admit_kv<ActT>(kvt, Bi, Li, Ls_cap, n_dec, E, stage_kv, TS_stage * 2 * E, crosskv, ckv_l_stride, src32, e->keytok32.as<int>(),
-                                             e->d.src_pad_token_idx, s);
+                if (int rc = launch_beam_admit(st, cbt, i, Bi, stage_drafts, lib_i, stage_tokcnt, stage_toklist, sg.srclen,
+                                               reinterpret_cast<long long*>(cb->out[i]), cb->trace_nacc ? cb->trace_nacc[i] : nullptr,
+                                               cb->trace_pick ? cb->trace_pick[i] : nullptr, dl_first, s))
+                    return rc;
             }
             cbt.n_groups = i + 1;
-            TTB_CUDA_OK(cudaGetLastError());
-            TTB_CHECK(e->alloc_signature() == sig0, "a workspace buffer moved while the continuous beam-search loop was running");
-            return 0;
+            return sg.scatter(e, cbt.slots, i, s);
         };
         // every batch takes part in at most max_len iterations
         const long long max_iters = (long long)cb->n * (max_len + 1);
@@ -1400,25 +1416,20 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
             if (wait_word(it + 1)) return 1;
             ++it;
         }
-        TTB_CUDA_OK(cudaEventRecord(e->t1, s));
-        TTB_CUDA_OK(cudaStreamSynchronize(s));
-        TTB_CUDA_OK(cudaGetLastError());
-        prof_collect(e);
+        float ms = 0.f;
+        if (int rc = finish_loop(e, ms)) return rc;
         int ctrl_end[32] = {};
         TTB_CUDA_OK(cudaMemcpy(ctrl_end, st.ctrl, sizeof(ctrl_end), cudaMemcpyDeviceToHost));
         TTB_CHECK(ctrl_end[BC_COUNT + 11] == 0, "continuous batching admitted a batch without enough free slots");
-        std::vector<BcGroup> groups((size_t)cb->n);
-        TTB_CUDA_OK(cudaMemcpy(groups.data(), cbt.groups, groups.size() * sizeof(BcGroup), cudaMemcpyDeviceToHost));
+        std::vector<BcGroup> groups;
+        if (int rc = read_groups(cb, cbt.groups, groups)) return rc;
         e->h_hist = hist;
         e->h_dl = hist_dl;
         e->h_dl_min.assign(hist_dl.size(), 0);
         if (it > 0) TTB_CUDA_OK(cudaMemcpy(e->h_dl_min.data(), cbt.dl_min, (size_t)it * sizeof(int), cudaMemcpyDeviceToHost));
-        float ms = 0.f;
-        cudaEventElapsedTime(&ms, e->t0, e->t1);
         ttb_generate_stats sum{};
         for (int i = 0; i < cb->n; ++i) {
             const BcGroup& g = groups[(size_t)i];
-            TTB_CHECK(g.closed == 1 && g.B == cb->bs[i], "continuous beam-search loop ended before every batch was finished");
             ttb_generate_stats& o = cb->stats[i];
             o = ttb_generate_stats{};
             o.model_calls = g.iter;
@@ -1486,13 +1497,9 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
         launch_beam_export(st.cand_cur, ldw, B * K, W, reinterpret_cast<long long*>(out_dev), s);
         e->launches++;
     }
-    TTB_CUDA_OK(cudaEventRecord(e->t1, s));
-    TTB_CUDA_OK(cudaStreamSynchronize(s));
-    TTB_CUDA_OK(cudaGetLastError());
-    prof_collect(e);
-    if (out_width) *out_width = W;
     float ms = 0.f;
-    cudaEventElapsedTime(&ms, e->t0, e->t1);
+    if (int rc = finish_loop(e, ms)) return rc;
+    if (out_width) *out_width = W;
     if (stats) {
         int fin_ctrl[BC_COUNT] = {};
         if (iters > 0) TTB_CUDA_OK(cudaMemcpy(fin_ctrl, st.ctrl, sizeof(fin_ctrl), cudaMemcpyDeviceToHost));
@@ -1521,39 +1528,23 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
 // in two ping-pong copies); tokens, scores and logits stay on the device, the host reads the control words of the stop
 // test one step behind.
 
-// Continuous batching (ttb_beam_search_generate_batches): the batches that share the query slots of one loop.
-struct SbArgs {
-    int n;                              // batches, admitted in list order
-    const int64_t* const* src;          // [n] (B_i, Ls_i) int64 sources
-    const int32_t* bs;                  // [n] B_i
-    const int32_t* ls;                  // [n] Ls_i
-    int64_t* const* out;                // [n] B_i * beam_size * max_len int64 hypotheses
-    int32_t* out_width;                 // [n] width of each batch's hypotheses
-    ttb_generate_stats* stats;          // [n]
-};
-
 // With `cb` the loop is the continuous one: B is the number of query slots, Ls the longest source of all batches, and the
 // batches of `cb` are admitted into free slots between two steps.
 template <typename ActT>
 static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int max_len, int K, int pad, int bos, int eos,
-                        int64_t* out_dev, int32_t* out_width, ttb_generate_stats* stats, cudaStream_t user_stream, const SbArgs* cb = nullptr) {
+                        int64_t* out_dev, int32_t* out_width, ttb_generate_stats* stats, cudaStream_t user_stream, const BatchList* cb = nullptr) {
     const int E = e->E(), H = e->d.num_heads, HD = e->HD(), V = e->d.tgt_vocab_size;
     const int n_dec = (int)e->dec.size();
     cudaStream_t s = e->stream;
-    TTB_CUDA_OK(cudaEventRecord(e->join_ev, user_stream));
-    TTB_CUDA_OK(cudaStreamWaitEvent(s, e->join_ev, 0));
+    if (int rc = join_caller_stream(e, user_stream)) return rc;
     const long long launches0 = e->launches;
     const bool cont = cb != nullptr;
     const long long TS = (long long)B * Ls;
     const int Ls_cap = std::max(256, (Ls + 63) / 64 * 64);
     const long long TS_cap = (long long)B * Ls_cap;   // no reallocation from one batch length to the next
     const int Cmax = B * K, ldw = max_len;
-    // continuous loop: the encoder of an admitted batch runs on that batch's shape, in a workspace of its own
-    int B_stage = 0;
-    long long TS_stage = 0;
-    if (cont)
-        for (int i = 0; i < cb->n; ++i) { B_stage = std::max(B_stage, (int)cb->bs[i]); TS_stage = std::max(TS_stage, (long long)cb->bs[i] * cb->ls[i]); }
-    const long long TS_enc = cont ? TS_stage : TS_cap;
+    Staging<ActT> sg(cb);
+    const long long TS_enc = cont ? sg.TS_stage : TS_cap;
 
     if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float))) return 1;
     if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
@@ -1571,41 +1562,18 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
     const size_t cbytes = (size_t)n_dec * cache_l_stride * sizeof(ActT);
     if (e->kcache.ensure(cbytes) || e->vcache.ensure(cbytes) || e->kcache2.ensure(cbytes) || e->vcache2.ensure(cbytes)) return 1;
     if (e->srclen.ensure((size_t)B * sizeof(int))) return 1;
-    // continuous loop: slot / batch tables, staging of an admitted batch (source lengths, cross K/V), slot-major key
-    // tokens, encoder workspace
+    // continuous loop: slot / batch tables, staging of an admitted batch
     SbTable cbt{};
-    int* stage_srclen = nullptr;
-    ActT* stage_kv = nullptr;
-    EncWork<ActT> enc_work{};
-    if (cont) {
-        TTB_CHECK((2 * E * sizeof(ActT)) % 16 == 0, "continuous batching needs 16-byte cross-attention K/V rows");
-        size_t co = 0;
-        auto ctake = [&](size_t bytes) { size_t o = co; co += (bytes + 255) / 256 * 256; return o; };
-        const size_t c_sg = ctake((size_t)B * 4), c_sq = ctake((size_t)B * 4), c_as = ctake((size_t)B * 4), c_gr = ctake((size_t)cb->n * sizeof(SbGroup));
-        const size_t c_sl = ctake((size_t)B_stage * 4), c_kv = ctake((size_t)n_dec * TS_stage * 2 * E * sizeof(ActT));
-        if (e->cb.ensure(co) || e->cb_work.ensure(enc_work_bytes<ActT>(e, TS_stage))) return 1;
-        if (e->keytok32.ensure((size_t)TS_cap * sizeof(int))) return 1;
-        char* cbase = e->cb.as<char>();
-        cbt.slot_group = (int*)(cbase + c_sg); cbt.slot_q = (int*)(cbase + c_sq); cbt.adm_slots = (int*)(cbase + c_as);
-        cbt.groups = (SbGroup*)(cbase + c_gr);
-        stage_srclen = (int*)(cbase + c_sl);
-        stage_kv = (ActT*)(cbase + c_kv);
-        enc_work = enc_work_carve<ActT>(e, TS_stage, e->cb_work.p);
-    }
+    if (cont)
+        if (int rc = sg.alloc(e, cbt, B, Ls_cap, {})) return rc;
     // nothing is allocated from here on (cudaFree would synchronise the device)
-    const long long sig0 = e->alloc_signature();
+    sg.sig0 = e->alloc_signature();
     char* base = bb.as<char>();
 
     TTB_CUDA_OK(cudaEventRecord(e->t0, s));
     int* src32 = e->src32.as<int>();
-    float* mem = e->memory.as<float>();
-    ActT* memh = Prec<ActT>::lowp ? e->memh.as<ActT>() : nullptr;
     ActT* crosskv = e->crosskv.as<ActT>();
-    if (!cont) {
-        { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(src_dev), src32, TS, s); }
-        if (encode_impl<ActT>(e, src32, src32, B, Ls, mem, memh, s)) return 1;
-        if (cross_kv_impl<ActT>(e, mem, memh, (int)TS, crosskv, s)) return 1;
-    }
+    if (!cont && encode_batch<ActT>(e, src_dev, B, Ls, e->srclen.as<int>(), crosskv, TS * 2 * E, s)) return 1;
 
     StdBeamState st{};
     st.B = B; st.K = K; st.V = V; st.pad = pad; st.bos = bos; st.eos = eos; st.ldw = ldw; st.max_len = max_len;
@@ -1618,17 +1586,13 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
     float* const score_set[2] = {st.score_cur, st.score_next};
     st.c_front = (int*)(base + o_cf); st.parent = (int*)(base + o_par);
     st.desc_self = (int4*)(base + o_ds); st.desc_cross = (int4*)(base + o_dc);
-    if (!cont) { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, B, Ls, e->d.src_pad_token_idx, e->srclen.as<int>(), s); }
     st.src_len = e->srclen.as<int>();
     ActT *kc_cur = e->kcache.as<ActT>(), *vc_cur = e->vcache.as<ActT>(), *kc_next = e->kcache2.as<ActT>(), *vc_next = e->vcache2.as<ActT>();
     if (cont) {
-        void* dp = nullptr;
-        for (int i = 16; i < 24; ++i) e->h_ctrl[i] = 0;   // ring of four 64-bit words the select kernel posts into
-        st.host_ctrl = cudaHostGetDevicePointer(&dp, e->h_ctrl + 16, 0) == cudaSuccess ? static_cast<unsigned long long*>(dp) : nullptr;
-        (void)cudaGetLastError();
+        st.host_ctrl = static_cast<unsigned long long*>(map_posted_ring(e));   // the select kernel posts into it
         TTB_CHECK(st.host_ctrl, "continuous batching needs mapped pinned host memory for its control word");
         TTB_CUDA_OK(cudaMemsetAsync(st.ctrl, 0, 64, s));
-        TTB_CUDA_OK(cudaMemsetAsync(cbt.slot_group, 0xff, (size_t)B * sizeof(int), s));   // every slot free
+        TTB_CUDA_OK(cudaMemsetAsync(cbt.slots.slot_group, 0xff, (size_t)B * sizeof(int), s));   // every slot free
         TTB_CUDA_OK(cudaMemsetAsync(cbt.groups, 0, (size_t)cb->n * sizeof(SbGroup), s));
     } else {
         Scope sc(e, KC_MISC, s);
@@ -1710,13 +1674,9 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
         st.y_cur = (calls & 1) ? y_set[1] : y_set[0];
         launch_beam_export(st.y_cur, ldw, B * K, W, reinterpret_cast<long long*>(out_dev), s);
         e->launches++;
-        TTB_CUDA_OK(cudaEventRecord(e->t1, s));
-        TTB_CUDA_OK(cudaStreamSynchronize(s));
-        TTB_CUDA_OK(cudaGetLastError());
-        prof_collect(e);
-        if (out_width) *out_width = W;
         float ms = 0.f;
-        cudaEventElapsedTime(&ms, e->t0, e->t1);
+        if (int rc = finish_loop(e, ms)) return rc;
+        if (out_width) *out_width = W;
         if (stats) {
             stats->model_calls = calls;
             stats->accepted_tokens = 0;
@@ -1733,27 +1693,13 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
     // the newest word suffice, then enqueues one step with decoder grids sized for the live rows of the word and waits for
     // the word of that step (the closing CTA of the select kernel posts it while the caches are still being re-parented).
     auto admit = [&](int i) -> int {
-        const int Bi = cb->bs[i], Li = cb->ls[i];
-        const long long TSi = (long long)Bi * Li;
-        { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(cb->src[i]), src32, TSi, s); }
-        { Scope sc(e, KC_MISC, s); launch_row_lengths(src32, Bi, Li, e->d.src_pad_token_idx, stage_srclen, s); }
-        if (encode_impl<ActT>(e, src32, src32, Bi, Li, mem, memh, s, &enc_work)) return 1;
-        if (cross_kv_impl<ActT>(e, mem, memh, (int)TSi, stage_kv, s, TS_stage * 2 * E)) return 1;
+        if (int rc = sg.encode(e, i, s)) return rc;
         {
             Scope sc(e, KC_MISC, s);
-            if (launch_sbeam_admit(st, cbt, i, Bi, stage_srclen, reinterpret_cast<long long*>(cb->out[i]), s)) return 1;
-        }
-        {
-            CbTable kvt{};
-            kvt.adm_slots = cbt.adm_slots;
-            Scope sc(e, KC_MISC, s);
-            launch_greedy_admit_kv<ActT>(kvt, Bi, Li, Ls_cap, n_dec, E, stage_kv, TS_stage * 2 * E, crosskv, ckv_l_stride, src32, e->keytok32.as<int>(),
-                                         e->d.src_pad_token_idx, s);
+            if (int rc = launch_sbeam_admit(st, cbt, i, cb->bs[i], sg.srclen, reinterpret_cast<long long*>(cb->out[i]), s)) return rc;
         }
         cbt.n_groups = i + 1;
-        TTB_CUDA_OK(cudaGetLastError());
-        TTB_CHECK(e->alloc_signature() == sig0, "a workspace buffer moved while the continuous beam-search loop was running");
-        return 0;
+        return sg.scatter(e, cbt.slots, i, s);
     };
     // every batch takes part in at most max_len - 1 steps
     const long long max_steps = (long long)cb->n * (max_len + 1);
@@ -1780,21 +1726,16 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
         live_next = (int)(w & 0xffffff);
         ++step;
     }
-    TTB_CUDA_OK(cudaEventRecord(e->t1, s));
-    TTB_CUDA_OK(cudaStreamSynchronize(s));
-    TTB_CUDA_OK(cudaGetLastError());
-    prof_collect(e);
+    float ms = 0.f;
+    if (int rc = finish_loop(e, ms)) return rc;
     int ctrl_end[16] = {};
     TTB_CUDA_OK(cudaMemcpy(ctrl_end, st.ctrl, sizeof(ctrl_end), cudaMemcpyDeviceToHost));
     TTB_CHECK(ctrl_end[SBC_ADM_ERR] == 0, "continuous batching admitted a batch without enough free slots");
-    std::vector<SbGroup> groups((size_t)cb->n);
-    TTB_CUDA_OK(cudaMemcpy(groups.data(), cbt.groups, groups.size() * sizeof(SbGroup), cudaMemcpyDeviceToHost));
+    std::vector<SbGroup> groups;
+    if (int rc = read_groups(cb, cbt.groups, groups)) return rc;
     e->h_hist = hist;
-    float ms = 0.f;
-    cudaEventElapsedTime(&ms, e->t0, e->t1);
     for (int i = 0; i < cb->n; ++i) {
         const SbGroup& g = groups[(size_t)i];
-        TTB_CHECK(g.closed == 1 && g.B == cb->bs[i], "continuous beam-search loop ended before every batch was finished");
         cb->stats[i] = ttb_generate_stats{};
         cb->stats[i].model_calls = g.steps;
         cb->out_width[i] = 1 + g.steps;
@@ -2052,7 +1993,7 @@ int ttb_greedy_speculative_generate_batches(ttb_engine* e, int32_t n_batches, co
     if (n_batches == 0) return 0;
     TTB_CUDA_OK(cudaSetDevice(e->device));
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    const CbArgs cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, trace_devs, stats};
+    const BatchList cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, stats, nullptr, trace_devs, nullptr, nullptr};
     return drained(e, TTB_DISPATCH(e, greedy_api<float>(e, nullptr, slots, Ls_max, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token,
                                                         replace_token, tie_break, nullptr, nullptr, total, s, false, &cb),
                                    greedy_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token,
@@ -2110,7 +2051,7 @@ int ttb_beam_search_generate_batches(ttb_engine* e, int32_t n_batches, const int
     if (n_batches == 0) return 0;
     TTB_CUDA_OK(cudaSetDevice(e->device));
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    const SbArgs cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, out_widths, stats};
+    const BatchList cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, stats, out_widths, nullptr, nullptr, nullptr};
     return drained(e, TTB_DISPATCH(e, std_beam_api<float>(e, nullptr, slots, Ls_max, max_len, beam_size, pad_token, bos_token, eos_token, nullptr, nullptr,
                                                           total, s, &cb),
                                    std_beam_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, beam_size, pad_token, bos_token, eos_token, nullptr,
@@ -2169,7 +2110,7 @@ int ttb_beam_speculative_generate_batches(ttb_engine* e, int32_t n_batches, cons
     if (n_batches == 0) return 0;
     TTB_CUDA_OK(cudaSetDevice(e->device));
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    const BcArgs cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, out_widths, trace_nacc_devs, trace_pick_devs, stats};
+    const BatchList cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, stats, out_widths, nullptr, trace_nacc_devs, trace_pick_devs};
     return drained(e, TTB_DISPATCH(e, beam_api<float>(e, nullptr, slots, Ls_max, max_len, n_best, draft_len, n_drafts, pad_token, bos_token, eos_token,
                                                       c_token, tie_break, nullptr, nullptr, nullptr, nullptr, total, s, smart_drafts_mode != 0, &cb),
                                    beam_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, n_best, draft_len, n_drafts, pad_token, bos_token,

@@ -388,7 +388,7 @@ void launch_greedy_accept(const GreedyState& st, cudaStream_t s) {
 }
 
 // ---- continuous batching: several batches share the live slots of one loop -------------------------------------
-// Every slot belongs to the batch it was admitted with (cb.slot_group) and holds that batch's query cb.slot_q.  A batch
+// Every slot belongs to the batch it was admitted with (cb.slots.slot_group) and holds that batch's query cb.slots.slot_q.  A batch
 // keeps its own token-matrix width, iteration count, counters and error (CbGroup): the only quantities of the
 // reference that couple the queries of a batch.  The live list keeps the members of a batch contiguous and in batch
 // order (admission appends, compaction preserves the order), so a batch's live queries are one run of the list.
@@ -421,26 +421,18 @@ __device__ void plan_width_warp(const GreedyState& st, const int* list, const in
 __global__ void __launch_bounds__(1024) greedy_admit_kernel(GreedyState st, CbTable cb, int grp, int Bi, const int* __restrict__ drafts_in,
                                                             const int* __restrict__ srclen_in, long long* out, int* trace, int Ls_cap) {
     extern __shared__ int s_adm[];
-    int* s_occ = s_adm;             // [S] slot in use
+    int* s_occ = s_adm;             // [S] -1 = free: the slots outside the live list (slot_group keeps stale entries)
     int* s_slots = s_adm + st.B;    // [Bi] slots taken, in batch order
     __shared__ int s_nfree;
     __shared__ int s_pick[64];      // scratch of the tie-break emulation
     const int S = st.B, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int n_active = st.ctrl[CTRL_N_ACTIVE];
-    for (int i = threadIdx.x; i < S; i += blockDim.x) s_occ[i] = 0;
+    for (int i = threadIdx.x; i < S; i += blockDim.x) s_occ[i] = -1;
     __syncthreads();
-    for (int g = threadIdx.x; g < n_active; g += blockDim.x) s_occ[st.active[g]] = 1;
+    for (int g = threadIdx.x; g < n_active; g += blockDim.x) s_occ[st.active[g]] = 0;
     __syncthreads();
     if (warp == 0) {
-        int taken = 0;
-        for (int i0 = 0; i0 < S && taken < Bi; i0 += 32) {
-            const int i = i0 + lane;
-            const bool fr = i < S && !s_occ[i];
-            const unsigned m = __ballot_sync(0xffffffffu, fr);
-            const int pos = taken + __popc(m & ((1u << lane) - 1u));
-            if (fr && pos < Bi) s_slots[pos] = i;
-            taken += __popc(m);
-        }
+        const int taken = take_free_slots(s_occ, S, Bi, s_slots);
         if (lane == 0) s_nfree = taken;
     }
     __syncthreads();
@@ -451,9 +443,9 @@ __global__ void __launch_bounds__(1024) greedy_admit_kernel(GreedyState st, CbTa
     const int D = st.D, N = st.N;
     for (int j = threadIdx.x; j < Bi; j += blockDim.x) {
         const int b = s_slots[j];
-        cb.adm_slots[j] = b;
-        cb.slot_group[b] = grp;
-        cb.slot_q[b] = j;
+        cb.slots.adm_slots[j] = b;
+        cb.slots.slot_group[b] = grp;
+        cb.slots.slot_q[b] = j;
         st.front[b] = 0;
         const_cast<int*>(st.src_len)[b] = srclen_in[j];
     }
@@ -500,17 +492,19 @@ __global__ void __launch_bounds__(1024) greedy_admit_kernel(GreedyState st, CbTa
     }
     if (threadIdx.x == 0) { st.ctrl[CTRL_N_ACTIVE] = n_active + Bi; st.ctrl[CTRL_DONE] = 0; }
 }
-void launch_greedy_admit(const GreedyState& st, const CbTable& cb, int grp, int Bi, const int* drafts_in, const int* srclen_in, long long* out,
-                         int* trace, int Ls_cap, cudaStream_t s) {
+int launch_greedy_admit(const GreedyState& st, const CbTable& cb, int grp, int Bi, const int* drafts_in, const int* srclen_in, long long* out,
+                        int* trace, int Ls_cap, cudaStream_t s) {
     const size_t smem = (size_t)(st.B + Bi) * sizeof(int);
-    if (ensure_dyn_smem(greedy_admit_kernel, (int)smem)) return;   // the launch below then fails loudly
+    if (ensure_dyn_smem(greedy_admit_kernel, (int)smem)) return 1;   // error recorded by ensure_dyn_smem
     greedy_admit_kernel<<<1, 1024, smem, s>>>(st, cb, grp, Bi, drafts_in, srclen_in, out, trace, Ls_cap);
+    return 0;
 }
 
-// Cross-attention K/V rows and key tokens of an admitted batch -> its slots (cb.adm_slots, written by the admission
-// kernel just before): rows [0, Ls) of slot b at b * Ls_cap; key tokens PAD behind Ls.  16-byte copies, grid-stride.
+// Cross-attention K/V rows and key tokens of an admitted batch -> its slots (adm_slots, written by the admission kernel of
+// any of the three continuous loops just before): rows [0, Ls) of slot b at b * Ls_cap; key tokens PAD behind Ls.  16-byte
+// copies, grid-stride.
 template <typename ActT>
-__global__ void greedy_admit_kv_kernel(const int* __restrict__ slots, int Bi, int Ls, int Ls_cap, int n_layers, int row_chunks,
+__global__ void admit_kv_kernel(const int* __restrict__ slots, int Bi, int Ls, int Ls_cap, int n_layers, int row_chunks,
                                        const uint4* __restrict__ stage_kv, long long stage_layer_chunks, uint4* __restrict__ kv,
                                        long long layer_chunks, const int* __restrict__ src32, int* __restrict__ keytok, int pad) {
     const long long per_layer = (long long)Bi * Ls * row_chunks;
@@ -528,19 +522,19 @@ __global__ void greedy_admit_kv_kernel(const int* __restrict__ slots, int Bi, in
     }
 }
 template <typename ActT>
-void launch_greedy_admit_kv(const CbTable& cb, int Bi, int Ls, int Ls_cap, int n_layers, int E, const ActT* stage_kv, long long stage_layer_stride,
-                            ActT* kv, long long layer_stride, const int* src32, int* keytok, int pad, cudaStream_t s) {
+void launch_admit_kv(const int* adm_slots, int Bi, int Ls, int Ls_cap, int n_layers, int E, const ActT* stage_kv, long long stage_layer_stride,
+                     ActT* kv, long long layer_stride, const int* src32, int* keytok, int pad, cudaStream_t s) {
     const int row_chunks = (int)(2 * E * sizeof(ActT) / 16);
     const long long total = (long long)n_layers * Bi * Ls * row_chunks;
     const int blocks = (int)std::min<long long>((total + 255) / 256 + 1, 8LL * kNumSMs);
-    greedy_admit_kv_kernel<ActT><<<blocks, 256, 0, s>>>(cb.adm_slots, Bi, Ls, Ls_cap, n_layers, row_chunks, reinterpret_cast<const uint4*>(stage_kv),
-                                                        stage_layer_stride * (long long)sizeof(ActT) / 16, reinterpret_cast<uint4*>(kv),
-                                                        layer_stride * (long long)sizeof(ActT) / 16, src32, keytok, pad);
+    admit_kv_kernel<ActT><<<blocks, 256, 0, s>>>(adm_slots, Bi, Ls, Ls_cap, n_layers, row_chunks, reinterpret_cast<const uint4*>(stage_kv),
+                                                 stage_layer_stride * (long long)sizeof(ActT) / 16, reinterpret_cast<uint4*>(kv),
+                                                 layer_stride * (long long)sizeof(ActT) / 16, src32, keytok, pad);
 }
-template void launch_greedy_admit_kv<float>(const CbTable&, int, int, int, int, int, const float*, long long, float*, long long, const int*, int*, int,
-                                            cudaStream_t);
-template void launch_greedy_admit_kv<__nv_bfloat16>(const CbTable&, int, int, int, int, int, const __nv_bfloat16*, long long, __nv_bfloat16*, long long,
-                                                    const int*, int*, int, cudaStream_t);
+template void launch_admit_kv<float>(const int*, int, int, int, int, int, const float*, long long, float*, long long, const int*, int*, int,
+                                     cudaStream_t);
+template void launch_admit_kv<__nv_bfloat16>(const int*, int, int, int, int, int, const __nv_bfloat16*, long long, __nv_bfloat16*, long long,
+                                             const int*, int*, int, cudaStream_t);
 
 // Accept kernel of the continuous loop: the per-query step of greedy_accept_kernel, then per batch (= run of the live
 // list) retirement into that batch's output, trace rows at the batch's own iteration, its error checks and width plan.
@@ -580,7 +574,7 @@ __global__ void __launch_bounds__(1024) greedy_accept_groups_kernel(GreedyState 
         const int a = st.active[b];
         s_active[b] = a;
         s_front[b] = st.front[b];
-        if (b < n_active) s_grp[b] = cb.slot_group[a];
+        if (b < n_active) s_grp[b] = cb.slots.slot_group[a];
     }
     if (stage_gen) stage_token_matrix(st, s_gen);
     pdl_wait();
@@ -620,7 +614,7 @@ __global__ void __launch_bounds__(1024) greedy_accept_groups_kernel(GreedyState 
         const int f = s_front[b];
         const int k = s_pseg[g];
         const CbGroup& gr = cb.groups[s_seg_grp[k]];
-        const int q = cb.slot_q[b], Wn = s_seg_W[k];
+        const int q = cb.slots.slot_q[b], Wn = s_seg_W[k];
         const AcceptStep r = accept_query(st, g, b, f, Wn, G + (long long)b * st.gen_ld, st.gen + (long long)b * st.gen_ld, stage_gen, keep_pred,
                                           alleq_pick, s_nacc, s_tokw, gr.out + (long long)q * st.max_len);
         if (lane == 0) {

@@ -149,6 +149,20 @@ void launch_greedy_accept(const GreedyState& st, cudaStream_t s);
 // standard greedy decoding (no drafts: N = 1, D = 0): appends the predicted token of every row, stop test
 void launch_greedy_std_step(const GreedyState& st, cudaStream_t s);
 
+// ---- continuous batching, common to the three loops: several batches share the query slots of one loop ----------
+// Slot table of a continuous loop, written by the loop's admission kernel.
+struct SlotTable {
+    int* slot_group;   // [slots] batch of the query in the slot, -1 = free (the greedy loop does not reset it: its free
+                       // slots are the ones outside the live list)
+    int* slot_q;       // [slots] index of that query in its batch
+    int* adm_slots;    // [max batch size] slots given to the batch admitted last
+};
+// cross-attention K/V rows [layer][Bi * Ls][2E] and source tokens [Bi][Ls] of the batch admitted last -> its slots adm_slots
+// (rows [0, Ls) of slot b at b * Ls_cap; key tokens PAD behind Ls); greedy.cu
+template <typename ActT>
+void launch_admit_kv(const int* adm_slots, int Bi, int Ls, int Ls_cap, int n_layers, int E, const ActT* stage_kv, long long stage_layer_stride,
+                     ActT* kv, long long layer_stride, const int* src32, int* keytok, int pad, cudaStream_t s);
+
 // Continuous batching of the speculative loop (GreedyState::B = number of slots; every per-query array is per slot).
 // One record per batch: what the reference couples across the queries of a batch (width, stop, errors) plus its counters.
 struct CbGroup {
@@ -160,18 +174,13 @@ struct CbGroup {
     int reserved;
 };
 struct CbTable {
-    int* slot_group;   // [slots] batch of the query in the slot
-    int* slot_q;       // [slots] index of that query in its batch
-    int* adm_slots;    // [max batch size] slots given to the batch admitted last
+    SlotTable slots;
     CbGroup* groups;   // [n_batches]
 };
-// admission of batch `grp` between two iterations (drafts_in [Bi][N][D], srclen_in [Bi] computed for the batch alone)
-void launch_greedy_admit(const GreedyState& st, const CbTable& cb, int grp, int Bi, const int* drafts_in, const int* srclen_in, long long* out,
-                         int* trace, int Ls_cap, cudaStream_t s);
-// cross-attention K/V rows [layer][Bi * Ls][2E] and source tokens [Bi][Ls] of the batch admitted last -> its slots
-template <typename ActT>
-void launch_greedy_admit_kv(const CbTable& cb, int Bi, int Ls, int Ls_cap, int n_layers, int E, const ActT* stage_kv, long long stage_layer_stride,
-                            ActT* kv, long long layer_stride, const int* src32, int* keytok, int pad, cudaStream_t s);
+// admission of batch `grp` between two iterations (drafts_in [Bi][N][D], srclen_in [Bi] computed for the batch alone); 0 or an
+// error code
+int launch_greedy_admit(const GreedyState& st, const CbTable& cb, int grp, int Bi, const int* drafts_in, const int* srclen_in, long long* out,
+                        int* trace, int Ls_cap, cudaStream_t s);
 // accept kernel of the continuous loop: per-query step of launch_greedy_accept, per-batch retirement / width plan / closing
 void launch_greedy_accept_groups(const GreedyState& st, const CbTable& cb, cudaStream_t s);
 
@@ -232,17 +241,15 @@ struct BcGroup {
     int all_fin, min_pad, acc, cnt;       // accumulators of the iteration in flight
 };
 struct BcTable {
-    int* slot_group;   // [slots] batch of the query in the slot, -1 = free
-    int* slot_q;       // [slots] index of that query in its batch
-    int* adm_slots;    // [max batch size] slots given to the batch admitted last
+    SlotTable slots;
     BcGroup* groups;   // [n_batches]
     int n_groups;      // batches admitted so far
     int* dl_min;       // [iterations] smallest draft length among the batches of every iteration
 };
 // admission of batch `grp` between two iterations: drafts_in [Bi][N][dl0] (smart: [Bi][lib_in][dl0] window library with
-// tok_cnt_in [Bi][V], tok_list_in [Bi][V][N]), srclen_in [Bi], all computed for the batch alone
-void launch_beam_admit(const BeamState& st, const BcTable& cb, int grp, int Bi, const int* drafts_in, int lib_in, const int* tok_cnt_in,
-                       const int* tok_list_in, const int* srclen_in, long long* out, int* trace_nacc, int* trace_pick, int dl_first, cudaStream_t s);
+// tok_cnt_in [Bi][V], tok_list_in [Bi][V][N]), srclen_in [Bi], all computed for the batch alone; 0 or an error code
+int launch_beam_admit(const BeamState& st, const BcTable& cb, int grp, int Bi, const int* drafts_in, int lib_in, const int* tok_cnt_in,
+                      const int* tok_list_in, const int* srclen_in, long long* out, int* trace_nacc, int* trace_pick, int dl_first, cudaStream_t s);
 // group-aware prepare / choose / expand; `dl` = draft length of the decoder call (the largest of the open batches)
 void launch_beam_prepare_groups(const BeamState& st, const BcTable& cb, cudaStream_t s);
 void launch_beam_choose_groups(const BeamState& st, const BcTable& cb, int dl, cudaStream_t s);
@@ -290,9 +297,7 @@ struct SbGroup {
     int n_eos, closed;   // hypotheses with EOS after the selection of the step in flight; 1 once the batch has stopped
 };
 struct SbTable {
-    int* slot_group;     // [slots] batch of the query in the slot, -1 = free
-    int* slot_q;         // [slots] index of that query in its batch
-    int* adm_slots;      // [max batch size] slots given to the batch admitted last
+    SlotTable slots;
     SbGroup* groups;     // [n_batches]
     int n_groups;        // batches admitted so far
 };

@@ -221,7 +221,7 @@ __global__ void sbeam_init_kernel(StdBeamState st) {
 void launch_sbeam_init(const StdBeamState& st, cudaStream_t s) { sbeam_init_kernel<<<8, 256, 0, s>>>(st); }
 
 // ---- continuous batching: several batches share the query slots of one loop ----------------------------------------
-// Slot q holds query cb.slot_q[q] of batch cb.slot_group[q] (-1: free) and hypotheses q K .. q K + K - 1.  A batch keeps in
+// Slot q holds query cb.slots.slot_q[q] of batch cb.slots.slot_group[q] (-1: free) and hypotheses q K .. q K + K - 1.  A batch keeps in
 // its SbGroup what the reference couples across the queries of a batch: width, hypotheses per query, step count and the
 // stop rule.  In a query's first step only hypothesis 0 exists (the reference starts from the BOS column, beam = 1): the
 // others are absent (cand_row -2), with no decoder rows and no continuations, so its selection sees the V scores
@@ -235,7 +235,7 @@ __global__ void __launch_bounds__(1024) sbeam_admit_kernel(StdBeamState st, SbTa
     __shared__ int s_nfree;
     const int K = st.K;
     if ((threadIdx.x >> 5) == 0) {
-        const int taken = take_free_slots(cb.slot_group, st.B, Bi, s_slots);
+        const int taken = take_free_slots(cb.slots.slot_group, st.B, Bi, s_slots);
         if (threadIdx.x == 0) s_nfree = taken;
     }
     __syncthreads();
@@ -246,9 +246,9 @@ __global__ void __launch_bounds__(1024) sbeam_admit_kernel(StdBeamState st, SbTa
     for (int j = threadIdx.x; j < Bi; j += blockDim.x) {
         const int q = s_slots[j];
         const long long c = (long long)q * K;
-        cb.adm_slots[j] = q;
-        cb.slot_group[q] = grp;
-        cb.slot_q[q] = j;
+        cb.slots.adm_slots[j] = q;
+        cb.slots.slot_group[q] = grp;
+        cb.slots.slot_q[q] = j;
         const_cast<int*>(st.src_len)[q] = srclen_in[j];
         st.y_cur[c * st.ldw] = st.bos;
         st.y_next[c * st.ldw] = st.bos;
@@ -276,7 +276,7 @@ __global__ void __launch_bounds__(1024) sbeam_prepare_groups_kernel(StdBeamState
     const int K = st.K, C = st.B * K;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31, n_warps = blockDim.x >> 5;
     for (int c = warp; c < C; c += n_warps) {
-        const int g = cb.slot_group[c / K];
+        const int g = cb.slots.slot_group[c / K];
         if (g < 0 || c % K >= cb.groups[g].beam) {
             if (lane == 0) st.fin[c] = 2;
             continue;
@@ -322,12 +322,12 @@ __global__ void __launch_bounds__(256) sbeam_select_groups_kernel(StdBeamState s
     extern __shared__ __align__(8) unsigned char s_sel_raw[];
     __shared__ int s_last, s_live;
     const int q = blockIdx.x, K = st.K, V = st.V;
-    const int g = cb.slot_group[q];
+    const int g = cb.slots.slot_group[q];
     if (g >= 0) {
         SbGroup* gr = &cb.groups[g];
         const int W = gr->W;
         const int n_fin = sbeam_select_query(st, reinterpret_cast<VF*>(s_sel_raw), st.total + (long long)q * K * V, gr->beam * V, q * K, q * K, W,
-                                             gr->out + (long long)cb.slot_q[q] * K * (W + 1));
+                                             gr->out + (long long)cb.slots.slot_q[q] * K * (W + 1));
         if (threadIdx.x == 0 && n_fin) atomicAdd(&gr->n_eos, n_fin);
     } else {
         for (int k = threadIdx.x; k < K; k += blockDim.x) st.parent[q * K + k] = -1;   // no cache to carry
@@ -358,8 +358,8 @@ __global__ void __launch_bounds__(256) sbeam_select_groups_kernel(StdBeamState s
     }
     __syncthreads();
     for (int b = threadIdx.x; b < st.B; b += blockDim.x) {
-        const int gb = cb.slot_group[b];
-        if (gb >= 0 && cb.groups[gb].closed) cb.slot_group[b] = -1;
+        const int gb = cb.slots.slot_group[b];
+        if (gb >= 0 && cb.groups[gb].closed) cb.slots.slot_group[b] = -1;
     }
     __syncthreads();
     if (threadIdx.x == 0) {

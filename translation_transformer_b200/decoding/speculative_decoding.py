@@ -51,6 +51,32 @@ def _check_batches(batches: list, slots: int | None, per_batch: int, min_len: in
     return slots
 
 
+def _run_batches(dec, fn: str, batches: list, slots: int, params: tuple, per_query: int, traces: tuple = (),
+                 widths: bool = False) -> tuple:
+    """The call of library entry point `fn` common to the generate_batches() methods of decoder `dec`: device copies of the
+    sources, int64 outputs of `per_query` elements per query, `params` (the loop's arguments behind the slot count),
+    per-batch pointer arrays of the outputs, of the widths when `widths`, and of every entry of `traces` (a list of
+    tensors, or None); then the accounting of the call's totals.  Returns (per-batch stats, widths or None, outputs)."""
+    m = dec.model
+    n = len(batches)
+    srcs = [b.to(device=m.device, dtype=torch.int64, non_blocking=True).contiguous() for b in batches]
+    outs = [torch.empty(s.shape[0] * per_query, dtype=torch.int64, device=m.device) for s in srcs]
+    ptrs = lambda ts: None if ts is None else (C.c_void_p * n)(*[t.data_ptr() for t in ts])
+    sizes = (C.c_int32 * n)(*[s.shape[0] for s in srcs])
+    lens = (C.c_int32 * n)(*[s.shape[1] for s in srcs])
+    out_widths = (C.c_int32 * n)() if widths else None
+    stats = (_lib.GenerateStats * n)()
+    total = _lib.GenerateStats()
+    with torch.cuda.device(m.device):
+        rc = getattr(m.lib, fn)(m._h, n, ptrs(srcs), sizes, lens, slots, *params, ptrs(outs), *([out_widths] if widths else []),
+                                *[ptrs(t) for t in traces], stats, C.byref(total), torch.cuda.current_stream(m.device).cuda_stream)
+    _lib.check(rc, fn)
+    dec.last_stats = total
+    dec.gpu_launches += total.gpu_launches
+    dec.gpu_ms += total.gpu_ms
+    return stats, out_widths, outs
+
+
 class TranslationInferenceGreedySpeculative:
     """Mirror of speculative_decoding.py:8-174 (same arguments, same counters, same output)."""
 
@@ -118,31 +144,16 @@ class TranslationInferenceGreedySpeculative:
         batches = list(batches)
         if not batches:
             return []
-        m = self.model
         slots = _check_batches(batches, slots, DEFAULT_SLOTS_PER_BATCH)
-        n = len(batches)
-        srcs = [b.to(device=m.device, dtype=torch.int64, non_blocking=True).contiguous() for b in batches]
-        outs = [torch.empty(s.shape[0], self.max_len, dtype=torch.int64, device=m.device) for s in srcs]
         traces = None
         if self.keep_trace:
-            traces = [torch.full((self.max_len + 1, s.shape[0], 4), -1, dtype=torch.int32, device=m.device) for s in srcs]
-        ptrs = lambda ts: (C.c_void_p * n)(*[t.data_ptr() for t in ts])
-        sizes = (C.c_int32 * n)(*[s.shape[0] for s in srcs])
-        lens = (C.c_int32 * n)(*[s.shape[1] for s in srcs])
-        stats = (_lib.GenerateStats * n)()
-        total = _lib.GenerateStats()
-        with torch.cuda.device(m.device):
-            rc = m.lib.ttb_greedy_speculative_generate_batches(
-                m._h, n, ptrs(srcs), sizes, lens, slots, self.max_len, self.draft_len, self.n_drafts, self.pad_token,
-                self.bos_token, self.eos_token, self.replace_token, self.tie_break, ptrs(outs),
-                ptrs(traces) if traces is not None else None, stats, C.byref(total),
-                torch.cuda.current_stream(m.device).cuda_stream)
-        _lib.check(rc, "ttb_greedy_speculative_generate_batches")
-        self.last_stats = total
-        self.gpu_launches += total.gpu_launches
-        self.gpu_ms += total.gpu_ms
+            traces = [torch.full((self.max_len + 1, b.shape[0], 4), -1, dtype=torch.int32, device=self.model.device) for b in batches]
+        stats, _, outs = _run_batches(
+            self, "ttb_greedy_speculative_generate_batches", batches, slots,
+            (self.max_len, self.draft_len, self.n_drafts, self.pad_token, self.bos_token, self.eos_token, self.replace_token, self.tie_break),
+            self.max_len, (traces,))
         results = []
-        for i in range(n):
+        for i in range(len(batches)):
             st = stats[i]
             self.model_calls_num += st.model_calls
             self.accepted_tokens_num += st.accepted_tokens
@@ -155,7 +166,7 @@ class TranslationInferenceGreedySpeculative:
                     raise exc
                 results.append(on_error(i, exc))
                 continue
-            out = outs[i].unsqueeze(1)
+            out = outs[i].view(-1, 1, self.max_len)
             results.append(out if batches[i].is_cuda else out.to(batches[i].device))
         return results
 
@@ -251,40 +262,24 @@ class TranslationInferenceBeamSearchSpeculative:
         batches = list(batches)
         if not batches:
             return []
-        m = self.model
         slots = _check_batches(batches, slots, DEFAULT_BEAM_SLOTS_PER_BATCH)
         if self.smart_drafts_mode:
             for b in batches:
                 if b.shape[1] <= 5:   # a library of Ls - 5 windows: generate() fails on such a batch as well
                     raise AssertionError("The number of drafts must be greater than 0")
-        n = len(batches)
         K, N = self.n_best, self.requested_drafts_num
-        cap = self.max_len + self.draft_len + 4
-        srcs = [b.to(device=m.device, dtype=torch.int64, non_blocking=True).contiguous() for b in batches]
-        outs = [torch.empty(s.shape[0] * K * cap, dtype=torch.int64, device=m.device) for s in srcs]
         t_nacc = t_pick = None
         if self.keep_trace:
-            t_nacc = [torch.full((self.max_len, s.shape[0] * K, N), -1, dtype=torch.int32, device=m.device) for s in srcs]
-            t_pick = [torch.full((self.max_len, s.shape[0] * K), -1, dtype=torch.int32, device=m.device) for s in srcs]
-        ptrs = lambda ts: (C.c_void_p * n)(*[t.data_ptr() for t in ts])
-        sizes = (C.c_int32 * n)(*[s.shape[0] for s in srcs])
-        lens = (C.c_int32 * n)(*[s.shape[1] for s in srcs])
-        widths = (C.c_int32 * n)()
-        stats = (_lib.GenerateStats * n)()
-        total = _lib.GenerateStats()
-        with torch.cuda.device(m.device):
-            rc = m.lib.ttb_beam_speculative_generate_batches(
-                m._h, n, ptrs(srcs), sizes, lens, slots, self.max_len, K, self.draft_len, N, int(self.smart_drafts_mode),
-                self.pad_token_idx, self.bos_token_idx, self.eos_token_idx, self.C_token_idx, self.tie_break, ptrs(outs), widths,
-                ptrs(t_nacc) if t_nacc is not None else None, ptrs(t_pick) if t_pick is not None else None, stats, C.byref(total),
-                torch.cuda.current_stream(m.device).cuda_stream)
-        _lib.check(rc, "ttb_beam_speculative_generate_batches")
-        self.last_stats = total
-        self.gpu_launches += total.gpu_launches
-        self.gpu_ms += total.gpu_ms
+            t_nacc = [torch.full((self.max_len, b.shape[0] * K, N), -1, dtype=torch.int32, device=self.model.device) for b in batches]
+            t_pick = [torch.full((self.max_len, b.shape[0] * K), -1, dtype=torch.int32, device=self.model.device) for b in batches]
+        stats, widths, outs = _run_batches(
+            self, "ttb_beam_speculative_generate_batches", batches, slots,
+            (self.max_len, K, self.draft_len, N, int(self.smart_drafts_mode), self.pad_token_idx, self.bos_token_idx, self.eos_token_idx,
+             self.C_token_idx, self.tie_break),
+            K * (self.max_len + self.draft_len + 4), (t_nacc, t_pick), widths=True)
         results = []
-        for i in range(n):
-            st, B = stats[i], srcs[i].shape[0]
+        for i in range(len(batches)):
+            st, B = stats[i], batches[i].shape[0]
             self.n_drafts += B * N
             self.model_calls_num += st.model_calls
             self.accepted_tokens_num += st.accepted_tokens

@@ -13,7 +13,7 @@ import torch
 
 from .. import _lib
 from ..model import B200Transformer
-from .speculative_decoding import _check_batches
+from .speculative_decoding import _check_batches, _run_batches
 
 # TranslationInferenceBeamSearch.generate_batches(): default query slots per query of the largest batch (each slot holds
 # beam_size hypotheses).  Trained-like bench batches on one B200 at 1000 W, 1 / 2 / 4 / 8 / 16 x bs slots: 145 / 262 / 473 /
@@ -112,30 +112,15 @@ class TranslationInferenceBeamSearch:
         batches = list(batches)
         if not batches:
             return []
-        m = self.model
         slots = _check_batches(batches, slots, DEFAULT_STD_BEAM_SLOTS_PER_BATCH, min_len=1)   # generate() takes Ls = 1 too
-        n, K = len(batches), self.beam_size
-        srcs = [b.to(device=m.device, dtype=torch.int64, non_blocking=True).contiguous() for b in batches]
-        outs = [torch.empty(s.shape[0] * K * self.max_len, dtype=torch.int64, device=m.device) for s in srcs]
-        ptrs = lambda ts: (C.c_void_p * n)(*[t.data_ptr() for t in ts])
-        sizes = (C.c_int32 * n)(*[s.shape[0] for s in srcs])
-        lens = (C.c_int32 * n)(*[s.shape[1] for s in srcs])
-        widths = (C.c_int32 * n)()
-        stats = (_lib.GenerateStats * n)()
-        total = _lib.GenerateStats()
-        with torch.cuda.device(m.device):
-            rc = m.lib.ttb_beam_search_generate_batches(
-                m._h, n, ptrs(srcs), sizes, lens, slots, self.max_len, K, self.pad_token, self.bos_token, self.eos_token,
-                ptrs(outs), widths, stats, C.byref(total), torch.cuda.current_stream(m.device).cuda_stream)
-        _lib.check(rc, "ttb_beam_search_generate_batches")
-        self.last_stats = total
-        self.gpu_launches += total.gpu_launches
-        self.gpu_ms += total.gpu_ms
+        K = self.beam_size
+        stats, widths, outs = _run_batches(self, "ttb_beam_search_generate_batches", batches, slots,
+                                           (self.max_len, K, self.pad_token, self.bos_token, self.eos_token), K * self.max_len, widths=True)
         results = []
-        for i in range(n):
-            B, W = srcs[i].shape[0], widths[i]
+        for i in range(len(batches)):
+            B, W = batches[i].shape[0], widths[i]
             self.model_calls_num += stats[i].model_calls
-            self.given_tokens += int((srcs[i] != m.src_pad_token_i).sum().item())
+            self.given_tokens += int((batches[i] != self.model.src_pad_token_i).sum().item())
             res = outs[i][:B * K * W].view(B, K, W)
             results.append(res if batches[i].is_cuda else res.to(batches[i].device))
         return results
