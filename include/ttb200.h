@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define TTB_ABI_VERSION 5
+#define TTB_ABI_VERSION 6
 
 #define TTB_PRECISION_FP32 0 /* fp32 FMA GEMMs, exact-parity path (1e-5 logits)            */
 #define TTB_PRECISION_BF16 1 /* tcgen05 bf16 GEMMs, fp32 accumulate (1e-2 logits)          */
@@ -118,6 +118,20 @@ int ttb_greedy_speculative_generate_batches(ttb_engine* e, int32_t n_batches, co
  * out_dev is (B, max_len) int64, PAD behind the last generated column. */
 int ttb_greedy_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len, int32_t pad_token,
                         int32_t bos_token, int32_t eos_token, int64_t* out_dev, ttb_generate_stats* stats, void* stream);
+
+/* ---- continuous batching of standard_decoding.py:29 generate(): n_batches independent batches share `slots` query slots
+ * of ONE device loop.  Batch i is admitted (whole, in list order) between two steps as soon as `batch_sizes[i]` slots are
+ * free; it keeps the step count and stop rule of its own batch (every row predicted EOS or PAD in the same step, or the
+ * rows are full) and frees its slots when it stops, so out_devs[i] and stats[i] are exactly what ttb_greedy_generate
+ * returns for that batch alone (launches and time belong to the call, in `total`).  src_devs[i] is (batch_sizes[i],
+ * src_lens[i]) int64, out_devs[i] (batch_sizes[i], max_len) int64.  max(batch_sizes) <= slots <= 2048.  Arguments
+ * ttb_greedy_generate rejects are rejected with the same error before any device work.  total (may be NULL): launches /
+ * ms of the call, model_calls = steps of the shared loop.  ttb_engine_get_history afterwards gives the query slots in use
+ * at every step. */
+int ttb_greedy_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs, const int32_t* batch_sizes,
+                                const int32_t* src_lens, int32_t slots, int32_t max_len, int32_t pad_token, int32_t bos_token,
+                                int32_t eos_token, int64_t* const* out_devs, ttb_generate_stats* stats, ttb_generate_stats* total,
+                                void* stream);
 
 /* ---- standard_decoding.py:90 TranslationInferenceBeamSearch.generate(src)
  * Standard beam search: one decoder call per generated column on the hypotheses without EOS; scores are

@@ -24,6 +24,12 @@ of a beam search reports the bs slots it holds as `slots_held` (its generate() k
 model, weights and batches of the beam / retro workloads, with the legs and defaults of those workloads.
 
     python scripts/bench_continuous.py --workload std_beam --weights copy --batches 48 --out profiles/r5_continuous_std_beam_copy.json
+
+--workload std_greedy runs the standard greedy decoding (TranslationInferenceGreedy) on the model, weights and batches of
+the greedy workload, with the greedy workload's engines in flight and a slot sweep of 1, 2, 4, 8 and 16 x bs (no leg (d)
+unless --cont-inflight is given).
+
+    python scripts/bench_continuous.py --workload std_greedy --weights copy --batches 24 --out profiles/r6_continuous_std_greedy_copy.json
 """
 from __future__ import annotations
 
@@ -42,7 +48,7 @@ REPO = Path(__file__).resolve().parent.parent
 sys.path.insert(0, str(REPO))
 
 import bench  # noqa: E402
-from translation_transformer_b200.decoding import TranslationInferenceBeamSearch  # noqa: E402
+from translation_transformer_b200.decoding import TranslationInferenceBeamSearch, TranslationInferenceGreedy  # noqa: E402
 from translation_transformer_b200.model import B200Transformer  # noqa: E402
 from translation_transformer_b200.pipeline import InFlightDecoder  # noqa: E402
 
@@ -70,33 +76,36 @@ def timed(fn):
 
 def main():
     ap = argparse.ArgumentParser()
-    ap.add_argument("--workload", default="greedy", choices=["greedy", "beam", "retro", "std_beam", "std_retro"])
+    ap.add_argument("--workload", default="greedy", choices=["greedy", "beam", "retro", "std_greedy", "std_beam", "std_retro"])
     ap.add_argument("--weights", default="copy", choices=["copy", "random"])
     ap.add_argument("--batches", type=int, default=24)
-    ap.add_argument("--slots", default=None, help="comma-separated slot counts (default greedy: 32,48,64,96,128; beam searches: 1,2,4,8,16 x bs)")
-    ap.add_argument("--inflight", default=None, help="engines in flight (default greedy: 3,8; beam searches: 12)")
-    ap.add_argument("--cont-inflight", default=None, help="continuous loops in flight (default greedy: 2,4; beam searches: none)")
+    ap.add_argument("--slots", default=None, help="comma-separated slot counts (default greedy: 32,48,64,96,128; std_greedy and beam searches: 1,2,4,8,16 x bs)")
+    ap.add_argument("--inflight", default=None, help="engines in flight (default greedy and std_greedy: 3,8; beam searches: 12)")
+    ap.add_argument("--cont-inflight", default=None, help="continuous loops in flight (default greedy: 2,4; std_greedy and beam searches: none)")
     ap.add_argument("--out", required=True)
     a = ap.parse_args()
-    greedy = a.workload == "greedy"
     std = a.workload.startswith("std_")
     base = a.workload[len("std_"):] if std else a.workload
+    greedy = base == "greedy"
     argv, sys.argv = sys.argv, ["bench.py", "--workload", base, "--weights", a.weights]
     bargs = bench.parse()
     sys.argv = argv
     wl = bench.Workload(base, a.weights, bargs)
-    if std:   # the standard beam search on the workload's model and batches
+    if std and greedy:   # the standard greedy decoding on the workload's model and batches
+        wl.generator = lambda eng: TranslationInferenceGreedy(eng, bargs.max_len, bench.PAD, bench.BOS, bench.EOS)
+    elif std:   # the standard beam search on the workload's model and batches
         wl.generator = lambda eng: TranslationInferenceBeamSearch(eng, wl.n_best, bargs.max_len, bench.PAD, bench.BOS, bench.EOS)
     if a.slots is None:
-        a.slots = "32,48,64,96,128" if greedy else ",".join(str(k * wl.bs) for k in (1, 2, 4, 8, 16))
+        a.slots = "32,48,64,96,128" if a.workload == "greedy" else ",".join(str(k * wl.bs) for k in (1, 2, 4, 8, 16))
     if a.inflight is None:
         a.inflight = "3,8" if greedy else "12"
     if a.cont_inflight is None:
-        a.cont_inflight = "2,4" if greedy else ""
+        a.cont_inflight = "2,4" if a.workload == "greedy" else ""
     dev = torch.device("cuda", 0)
     batches = [wl.batch(j).to(dev) for j in range(a.batches)]
     n_smiles = sum(b.shape[0] for b in batches)
-    res = {"workload": ("standard beam search, beam_size = n_best, on: " if std else "") + wl.describe(), "batches": a.batches, "bs": wl.bs, "weights": a.weights, **gpu_info()}
+    std_name = "standard greedy decoding, on: " if greedy else "standard beam search, beam_size = n_best, on: "
+    res = {"workload": (std_name if std else "") + wl.describe(), "batches": a.batches, "bs": wl.bs, "weights": a.weights, **gpu_info()}
     if not greedy:
         res["n_best"] = wl.n_best
 

@@ -12,7 +12,7 @@ from pathlib import Path
 # TTB_LIB: file name (inside the package) of an experimental build of the same sources, for A/B runs (scripts/build_variant.sh)
 LIB_PATH = Path(__file__).resolve().parent / os.environ.get("TTB_LIB", "libttb200.so")
 
-ABI_VERSION = 5
+ABI_VERSION = 6
 PRECISION = {"fp32": 0, "bf16": 1}
 ERR_REF_INDEX, ERR_REF_SHAPE, ERR_REF_ASSERT = 10, 11, 12
 
@@ -51,7 +51,9 @@ SIGNATURES = {
                                                 [C.c_void_p, C.c_void_p, C.POINTER(GenerateStats), C.POINTER(GenerateStats), C.c_void_p]),
     "ttb_greedy_generate": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
                                       C.c_void_p, C.POINTER(GenerateStats), C.c_void_p]),
-    "ttb_beam_search_generate": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int32] * 7 +
+    "ttb_greedy_generate_batches": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int32] * 5 +
+                                    [C.c_void_p, C.POINTER(GenerateStats), C.POINTER(GenerateStats), C.c_void_p]),
+    "ttb_beam_search_generate":(C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int32] * 7 +
                                  [C.c_void_p, C.POINTER(C.c_int32), C.POINTER(GenerateStats), C.c_void_p]),
     "ttb_beam_search_generate_batches": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int32] * 6 +
                                          [C.c_void_p, C.c_void_p, C.POINTER(GenerateStats), C.POINTER(GenerateStats), C.c_void_p]),

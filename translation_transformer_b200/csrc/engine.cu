@@ -745,8 +745,9 @@ static int read_groups(const BatchList* cb, const G* dev, std::vector<G>& groups
     return 0;
 }
 
-// Speculative greedy loop.  With `cb` the loop is the continuous one: B is the number of query slots, Ls the longest
-// source of all batches, and the batches of `cb` are admitted into free slots between two graph launches.
+// Speculative greedy loop, and with `standard` the standard greedy decoding (no drafts).  With `cb` the loop is the
+// continuous one: B is the number of query slots, Ls the longest source of all batches, and the batches of `cb` are
+// admitted into free slots between two graph launches.
 template <typename ActT>
 static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int max_len, int draft_len, int N,
                       int pad, int bos, int eos, int replace, int tie_break, int64_t* out_dev, int32_t* trace_dev,
@@ -811,7 +812,7 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     auto admit = [&](int i) -> int {
         const int Bi = cb->bs[i], Li = cb->ls[i];
         if (int rc = sg.encode(e, i, s)) return rc;
-        { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Li, Bi, Li - 1, D, N, eos, pad, replace, stage_drafts, s); }
+        if (!standard) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Li, Bi, Li - 1, D, N, eos, pad, replace, stage_drafts, s); }
         {
             Scope sc(e, KC_MISC, s);
             if (int rc = launch_greedy_admit(st, cbt, i, Bi, stage_drafts, sg.srclen, reinterpret_cast<long long*>(cb->out[i]),
@@ -886,7 +887,8 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
         }
         {
             Scope sc(e, KC_ACCEPT, s);
-            if (standard) launch_greedy_std_step(st, s);
+            if (standard && cont) { if (launch_greedy_std_step_groups(st, cbt, s)) return 1; }
+            else if (standard) launch_greedy_std_step(st, s);
             else if (cont) launch_greedy_accept_groups(st, cbt, s);
             else launch_greedy_accept(st, s);
         }
@@ -915,12 +917,13 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
         cand[8] = (B + 15) / 16;
         cand[9] = 1;
         for (int i = 0; i < ttb_engine::kBuckets; ++i) {
-            if (i > 0 && (no_buckets || standard)) break;
+            // generate() of the standard greedy decoding keeps every row to the end; its continuous loop sheds stopped batches
+            if (i > 0 && (no_buckets || (standard && !cont))) break;
             if (n_buckets == 0 || (cand[i] >= 1 && cand[i] < bucket_q[n_buckets - 1])) bucket_q[n_buckets++] = cand[i];
         }
     }
     if (use_graph) {
-        const long long key[13] = {B, N, D, standard ? 1 : (cont ? 2 : 0), max_len, pad, bos, eos, tie_break, e->alloc_signature(),
+        const long long key[13] = {B, N, D, (standard ? 1 : 0) + (cont ? 2 : 0), max_len, pad, bos, eos, tie_break, e->alloc_signature(),
                                    (long long)sizeof(ActT) + 16 * K_it, replace, cont ? Ls_cap : 0};
         if (memcmp(key, e->graph_key, sizeof(key)) != 0) {
             for (auto& gb : e->graph_exec) for (auto& g : gb) if (g) { cudaGraphExecDestroy(g); g = nullptr; }
@@ -2009,6 +2012,35 @@ int ttb_greedy_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_
     cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     return drained(e, TTB_DISPATCH(e, greedy_api<float>(e, src_dev, B, Ls, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, out_dev, nullptr, stats, s, true),
                         greedy_api<__nv_bfloat16>(e, src_dev, B, Ls, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, out_dev, nullptr, stats, s, true)));
+}
+
+int ttb_greedy_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs, const int32_t* batch_sizes,
+                                const int32_t* src_lens, int32_t slots, int32_t max_len, int32_t pad_token, int32_t bos_token,
+                                int32_t eos_token, int64_t* const* out_devs, ttb_generate_stats* stats, ttb_generate_stats* total,
+                                void* stream) {
+    TTB_CHECK(e && e->finalized, "engine not finalized");
+    TTB_CHECK(n_batches >= 0 && slots > 0, "bad arguments");
+    TTB_CHECK(n_batches == 0 || (src_devs && batch_sizes && src_lens && out_devs && stats), "bad arguments");
+    // the rules of ttb_greedy_generate, in its order, before any device work
+    for (int i = 0; i < n_batches; ++i) TTB_CHECK(src_devs[i] && out_devs[i] && batch_sizes[i] > 0 && src_lens[i] > 0, "bad arguments");
+    TTB_CHECK(max_len > 1, "bad arguments");
+    TTB_CHECK(max_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
+    int Ls_max = 1;
+    for (int i = 0; i < n_batches; ++i) {
+        TTB_CHECK(src_lens[i] <= e->d.max_positions, "sequence longer than the positional table");
+        TTB_CHECK(batch_sizes[i] <= slots, "slots must be at least the largest batch size");
+        Ls_max = std::max(Ls_max, (int)src_lens[i]);
+    }
+    TTB_CHECK(slots <= 2048, "continuous batching supports at most 2048 slots");
+    if (total) *total = ttb_generate_stats{};
+    if (n_batches == 0) return 0;
+    TTB_CUDA_OK(cudaSetDevice(e->device));
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const BatchList cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, stats, nullptr, nullptr, nullptr, nullptr};
+    return drained(e, TTB_DISPATCH(e, greedy_api<float>(e, nullptr, slots, Ls_max, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1,
+                                                        nullptr, nullptr, total, s, true, &cb),
+                                   greedy_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1,
+                                                             nullptr, nullptr, total, s, true, &cb)));
 }
 
 int ttb_beam_search_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len, int32_t beam_size,

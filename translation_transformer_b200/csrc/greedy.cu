@@ -465,7 +465,8 @@ __global__ void __launch_bounds__(1024) greedy_admit_kernel(GreedyState st, CbTa
         int Wn = 1;
         bool oob = false;
         const bool short_loop = st.max_len <= 1;   // the reference's loop does not run at all
-        if (!short_loop) plan_width_warp(st, s_slots, st.front, st.gen, Bi, 1, Wn, oob);
+        // the standard loop (D = 0) has no token-matrix width to plan: with BOS = PAD the plan would close the batch
+        if (!short_loop && D > 0) plan_width_warp(st, s_slots, st.front, st.gen, Bi, 1, Wn, oob);
         if (lane == 0) {
             const bool open = !short_loop && !oob;
             CbGroup gr{};
@@ -753,6 +754,122 @@ __global__ void __launch_bounds__(1024) greedy_std_step_kernel(GreedyState st) {
 }
 void launch_greedy_std_step(const GreedyState& st, cudaStream_t s) {
     launch_pdl(greedy_std_step_kernel, dim3(1), dim3(st.B < 1024 ? ((st.B + 31) / 32 * 32) : 1024), 0, s, st);
+}
+
+// Step kernel of the continuous loop without drafts, in place of greedy_std_step_kernel.  What the reference couples across
+// a batch is kept per batch (CbGroup): its step count (every row of the batch holds 1 + iter tokens, so it is also the
+// front of each of its slots), its stop rule and its output.  A batch's slots are one run of the live list (admission
+// appends them in batch order, compaction preserves the order), and a batch leaves the list whole, when it stops.
+__global__ void __launch_bounds__(1024) greedy_std_step_groups_kernel(GreedyState st, CbTable cb) {
+    __shared__ int s_nseg, s_nstop;
+    extern __shared__ int s_dyn[];
+    const int S = st.B, warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    int* s_active = s_dyn;          // [S] live list of the step
+    int* s_grp = s_active + S;      // [S] per position: batch
+    int* s_pseg = s_grp + S;        // [S] per position: run of the live list it belongs to
+    int* s_stop = s_pseg + S;       // [S] positions of the batches that stop in this step
+    int* s_seg_grp = s_stop + S;    // [S] per run: batch
+    int* s_seg_f = s_seg_grp + S;   // [S] per run: front before the step (the batch's step count)
+    int* s_seg_go = s_seg_f + S;    // [S] per run: a row predicted neither EOS nor PAD; then: the batch stays open
+    pdl_launch_dependents();
+    // loads ahead of the dependency wait: written by the previous step or admission kernel (see greedy_accept_kernel)
+    const int done = st.ctrl[CTRL_DONE];
+    const int n_active = st.ctrl[CTRL_N_ACTIVE];
+    const int iter = st.ctrl[CTRL_ITERS];
+    for (int g = threadIdx.x; g < n_active; g += blockDim.x) {
+        const int b = st.active[g];
+        s_active[g] = b;
+        s_grp[g] = cb.slots.slot_group[b];
+    }
+    pdl_wait();
+    if (done) return;
+    __syncthreads();
+    // runs of the live list (one per open batch): the ballot scan of greedy_accept_groups_kernel
+    if (warp == 0) {
+        int nseg = 0;
+        for (int g0 = 0; g0 < n_active; g0 += 32) {
+            const int g = g0 + lane;
+            const int grp = g < n_active ? s_grp[g] : -1;
+            const bool start = g < n_active && (g == 0 || s_grp[g - 1] != grp);
+            const unsigned m = __ballot_sync(0xffffffffu, start);
+            const int k = nseg + __popc(m & ((2u << lane) - 1u)) - 1;
+            if (g < n_active) s_pseg[g] = k;
+            if (start) s_seg_grp[k] = grp;
+            nseg += __popc(m);
+        }
+        if (lane == 0) s_nseg = nseg;
+    }
+    __syncthreads();
+    const int nseg = s_nseg;
+    for (int k = threadIdx.x; k < nseg; k += blockDim.x) { s_seg_f[k] = cb.groups[s_seg_grp[k]].iter; s_seg_go[k] = 0; }
+    if (threadIdx.x == 0 && st.hist) st.hist[iter] = n_active;
+    __syncthreads();
+    // token append (pred is indexed by live position); the K/V row of the step's input token goes to cache position f
+    for (int g = threadIdx.x; g < n_active; g += blockDim.x) {
+        const int b = s_active[g], k = s_pseg[g], f = s_seg_f[k];
+        const int tok = st.pred[g];
+        st.gen[(long long)b * st.gen_ld + f + 1] = tok;
+        st.front[b] = f + 1;
+        reinterpret_cast<int4*>(st.sel)[g] = make_int4(b, f, 0, 0);
+        if (tok != st.eos && tok != st.pad) s_seg_go[k] = 1;
+    }
+    __syncthreads();
+    // per batch: the stop rule of generate() (every row predicted EOS or PAD in this step, or the rows are full)
+    for (int k = threadIdx.x; k < nseg; k += blockDim.x) {
+        const int f = s_seg_f[k];
+        const bool open = s_seg_go[k] && f + 2 < st.max_len;
+        CbGroup& gr = cb.groups[s_seg_grp[k]];
+        gr.iter = f + 1;
+        gr.tokens += gr.B;
+        gr.live = open ? gr.B : 0;
+        gr.closed = open ? 0 : 1;
+        s_seg_go[k] = open ? 1 : 0;
+    }
+    __syncthreads();
+    // live list and descriptors of the coming step without the stopped batches (order preserved); positions of the stopped
+    if (warp == 0) {
+        int w = 0, n_stop = 0;
+        for (int g0 = 0; g0 < n_active; g0 += 32) {
+            const int g = g0 + lane;
+            const bool keep = g < n_active && s_seg_go[s_pseg[g]];
+            const bool stop = g < n_active && !keep;
+            const unsigned m = __ballot_sync(0xffffffffu, keep), ms = __ballot_sync(0xffffffffu, stop);
+            const unsigned lt = (1u << lane) - 1u;
+            if (keep) {
+                const int pos = w + __popc(m & lt);
+                const int b = s_active[g];
+                st.active[pos] = b;
+                st.desc[pos] = make_int4(b, s_seg_f[s_pseg[g]] + 1, st.pred[g], st.src_len[b]);
+            }
+            if (stop) s_stop[n_stop + __popc(ms & lt)] = g;
+            w += __popc(m);
+            n_stop += __popc(ms);
+        }
+        if (lane == 0) {
+            st.ctrl[CTRL_N_SEL] = n_active;
+            st.ctrl[CTRL_N_ACTIVE] = w;
+            st.ctrl[CTRL_ITERS] = iter + 1;
+            st.ctrl[CTRL_DONE] = w == 0 ? 1 : 0;
+            s_nstop = n_stop;
+        }
+    }
+    __syncthreads();
+    // stopped batches: their slots may be handed out again before the next advance kernel, which skips a < 0; each row goes
+    // to the batch's output at its index in the batch, tokens 0 .. f + 1 and PAD behind them (as greedy_std_step_kernel)
+    const int n_stop = s_nstop;
+    for (int i = threadIdx.x; i < n_stop; i += blockDim.x) st.sel[s_stop[i] * 4 + 3] = -1;
+    for (long long idx = threadIdx.x; idx < (long long)n_stop * st.max_len; idx += blockDim.x) {
+        const int g = s_stop[idx / st.max_len], c = (int)(idx % st.max_len);
+        const int b = s_active[g], f = s_seg_f[s_pseg[g]];
+        long long* out = cb.groups[s_grp[g]].out + (long long)cb.slots.slot_q[b] * st.max_len;
+        out[c] = c <= f + 1 ? st.gen[(long long)b * st.gen_ld + c] : st.pad;
+    }
+}
+int launch_greedy_std_step_groups(const GreedyState& st, const CbTable& cb, cudaStream_t s) {
+    const size_t smem = (size_t)7 * st.B * sizeof(int);
+    if (ensure_dyn_smem(greedy_std_step_groups_kernel, (int)smem)) return 1;   // error recorded by ensure_dyn_smem
+    TTB_CUDA_OK(launch_pdl(greedy_std_step_groups_kernel, dim3(1), dim3(st.B < 1024 ? ((st.B + 31) / 32 * 32) : 1024), smem, s, st, cb));
+    return 0;
 }
 
 }  // namespace ttb

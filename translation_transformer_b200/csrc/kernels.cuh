@@ -165,6 +165,7 @@ void launch_admit_kv(const int* adm_slots, int Bi, int Ls, int Ls_cap, int n_lay
 
 // Continuous batching of the speculative loop (GreedyState::B = number of slots; every per-query array is per slot).
 // One record per batch: what the reference couples across the queries of a batch (width, stop, errors) plus its counters.
+// The standard greedy loop uses the same record without width and errors (W, accepted, error and n_left stay 0 or unused).
 struct CbGroup {
     long long* out;    // [B][max_len] the batch's predictions
     int* trace;        // optional [max_len + 1][B][4], rows indexed by the batch's own iteration and live position
@@ -183,6 +184,9 @@ int launch_greedy_admit(const GreedyState& st, const CbTable& cb, int grp, int B
                         int* trace, int Ls_cap, cudaStream_t s);
 // accept kernel of the continuous loop: per-query step of launch_greedy_accept, per-batch retirement / width plan / closing
 void launch_greedy_accept_groups(const GreedyState& st, const CbTable& cb, cudaStream_t s);
+// step kernel of the continuous loop without drafts (N = 1, D = 0): token append of launch_greedy_std_step with the step
+// count, stop rule and output of each batch; stopped batches leave the live list whole; 0 or an error code
+int launch_greedy_std_step_groups(const GreedyState& st, const CbTable& cb, cudaStream_t s);
 
 // ---- beam.cu --------------------------------------------------------------------------------------
 struct BeamState {

@@ -20,6 +20,10 @@ from .speculative_decoding import _check_batches, _run_batches
 # 739 / 1051 SMILES/s (bs 4, beam 5) and 281 / 462 / 676 / 897 / 1095 (retro, bs 8, beam 10), against 138 and 261 one batch
 # at a time (profiles/r5_continuous_std_beam_*.json, DESIGN.md section 12)
 DEFAULT_STD_BEAM_SLOTS_PER_BATCH = 16
+# TranslationInferenceGreedy.generate_batches(): default query slots per query of the largest batch.  Greedy bench workload's
+# model and batches (bs 32, trained-like weights, 24 batches) on one B200 at 1000 W, 1 / 2 / 4 / 8 / 16 x bs slots: 823 / 1392 /
+# 2018 / 2802 / 3160 SMILES/s, against 780 one batch at a time (profiles/r6_continuous_std_greedy_copy.json, DESIGN.md section 13)
+DEFAULT_GREEDY_SLOTS_PER_BATCH = 16
 
 
 class TranslationInferenceGreedy:
@@ -58,6 +62,28 @@ class TranslationInferenceGreedy:
         self.gpu_ms += stats.gpu_ms
         out = out.unsqueeze(1)
         return out if src.is_cuda else out.to(src.device)
+
+    def generate_batches(self, batches: Sequence[torch.Tensor], slots: int | None = None) -> list:
+        """Continuous batching: decode `batches` in ONE device loop whose `slots` query slots are refilled with the queries
+        of the next batch as soon as enough of them are free (batches are admitted whole, in list order, between two steps;
+        a batch frees its slots when it stops).
+
+        Returns `[self.generate(b) for b in batches]` bit for bit, each (B_i, 1, max_len), and advances the counters as
+        those calls would: a batch keeps the step count and stop rule of its own batch in the shared loop.  `slots`
+        defaults to DEFAULT_GREEDY_SLOTS_PER_BATCH times the largest batch size."""
+        batches = list(batches)
+        if not batches:
+            return []
+        slots = _check_batches(batches, slots, DEFAULT_GREEDY_SLOTS_PER_BATCH, min_len=1)   # generate() takes Ls = 1 too
+        stats, _, outs = _run_batches(self, "ttb_greedy_generate_batches", batches, slots,
+                                      (self.max_len, self.pad_token, self.bos_token, self.eos_token), self.max_len)
+        results = []
+        for i in range(len(batches)):
+            self.model_calls_num += stats[i].model_calls
+            self.given_tokens += int((batches[i] != self.model.src_pad_token_i).sum().item())
+            out = outs[i].view(-1, 1, self.max_len)
+            results.append(out if batches[i].is_cuda else out.to(batches[i].device))
+        return results
 
 
 class TranslationInferenceBeamSearch:
