@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define TTB_ABI_VERSION 6
+#define TTB_ABI_VERSION 7
 
 #define TTB_PRECISION_FP32 0 /* fp32 FMA GEMMs, exact-parity path (1e-5 logits)            */
 #define TTB_PRECISION_BF16 1 /* tcgen05 bf16 GEMMs, fp32 accumulate (1e-2 logits)          */
@@ -188,6 +188,16 @@ int ttb_beam_speculative_generate_batches(ttb_engine* e, int32_t n_batches, cons
                                           int64_t* const* out_devs, int32_t* out_widths, int32_t* const* trace_nacc_devs,
                                           int32_t* const* trace_pick_devs, ttb_generate_stats* stats, ttb_generate_stats* total,
                                           void* stream);
+
+/* ---- teacher-forced scoring of given targets (no reference counterpart; DESIGN.md §14).  src_dev (B, Ls) int64,
+ * tgt_dev (B, K, Lt) int64 with column 0 = start token; candidate (b,k) is tgt[b,k,1:] up to and including its first
+ * eos_token or up to its first pad_token.  logp_out_dev (B*K) f32 sums, ntok_out_dev (B*K) int32 scored positions,
+ * token_logp_out_dev (B*K*(Lt-1)) f32 or NULL.  Encoder and cross-attention K/V once per source.  Whole sources are
+ * processed in chunks of at most 32768 decoder rows; K * Lt > 32768 is rejected.  Token ids must lie in the vocabularies
+ * and no source row may be all padding.  The call returns once the results are written. */
+int ttb_score_targets(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, const int64_t* tgt_dev, int32_t K,
+                      int32_t Lt, int32_t pad_token, int32_t eos_token, float* logp_out_dev, int32_t* ntok_out_dev,
+                      float* token_logp_out_dev, void* stream);
 
 /* ---- instrumentation (bench.py): per-kernel-class CUDA-event timing on the launching stream.
  * class_mask bit i enables class i (names via ttb_kernel_class_name); totals accumulate over

@@ -107,6 +107,18 @@ def load_batches(args):
     return tk, batches
 
 
+def load_weights(args, tk):
+    """State dict of --ckpt, the trained-like weights of --weights copy, or None (random init from --seed)."""
+    if args.ckpt:
+        sd = torch.load(args.ckpt, map_location="cpu", weights_only=True)
+        sd = sd.get("state_dict", sd)
+        return {k[len("model."):] if k.startswith("model.") else k: v for k, v in sd.items() if "positional_encoding" not in k}
+    if args.weights == "copy":
+        from translation_transformer_b200.weights import ModelConfig, copy_task_state_dict
+        return copy_task_state_dict(ModelConfig(src_vocab_size=tk.n_tokens, tgt_vocab_size=tk.n_tokens, **PRODUCT_PREDICTION), args.seed)
+    return None
+
+
 def main_dynamic(args, model, tk, batches, n_best, rank, world, dev):
     """One queue of batch indices shared by all ranks and in-flight engines (distributed.BatchQueue) instead of contiguous
     static shards: a rank that drew long queries draws fewer batches.  Predictions are collected with ONE indexed all-gather
@@ -173,14 +185,7 @@ def main():
         dist.init_process_group("nccl", device_id=dev)
 
     tk, batches = load_batches(args)
-    sd = None
-    if args.ckpt:
-        sd = torch.load(args.ckpt, map_location="cpu", weights_only=True)
-        sd = sd.get("state_dict", sd)
-        sd = {k[len("model."):] if k.startswith("model.") else k: v for k, v in sd.items() if "positional_encoding" not in k}
-    elif args.weights == "copy":
-        from translation_transformer_b200.weights import ModelConfig, copy_task_state_dict
-        sd = copy_task_state_dict(ModelConfig(src_vocab_size=tk.n_tokens, tgt_vocab_size=tk.n_tokens, **PRODUCT_PREDICTION), args.seed)
+    sd = load_weights(args, tk)
     model = VanillaEncoderDecoderTransformerLightning(
         src_tokenizer=tk, tgt_tokenizer=tk, generation=args.generation, beam_size=args.beam_size,
         max_len=args.max_len, n_drafts=args.n_drafts, draft_len=args.draft_len, smart_drafts_mode=args.smart_drafts_mode,

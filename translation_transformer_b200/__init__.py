@@ -8,5 +8,6 @@ in `include/ttb200.h`; PyTorch only owns device memory and `torch.distributed`. 
 CPU fallback: importing the package works anywhere, using it without the CUDA library raises.
 """
 from .weights import ModelConfig, random_init_state_dict, infer_config, PRODUCT_PREDICTION, SINGLE_STEP_RETRO  # noqa: F401
+from .scoring import Scores, TranslationScorer  # noqa: F401
 
 __version__ = "0.1.0"

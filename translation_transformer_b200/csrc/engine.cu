@@ -171,6 +171,7 @@ struct ttb_engine {
     DevBuf hist;                 // per-iteration live-query count of the last generate()
     DevBuf cb;                   // continuous batching: slot / batch tables and the staging buffers of an admitted batch
     DevBuf cb_work;              // continuous batching: encoder workspace of an admitted batch (the loop's own must stay intact)
+    DevBuf score;                // ttb_score_targets: candidate -> source map and per-row statistics of one chunk
     std::vector<int> h_hist;
     std::vector<int> h_dl, h_dl_min;   // continuous beam-search loop: draft length of every decoder call, smallest of its batches
 
@@ -1752,6 +1753,93 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
     return 0;
 }
 
+// ---- teacher-forced scoring of given targets (DESIGN.md section 14) ------------------------------------------------------
+// Decoder rows per chunk (and encoder rows: source tokens of the chunk): bounds the workspace ensure_work grows to, about
+// 10 KB per row at the full architecture.
+constexpr int kScoreMaxRows = 32768;
+
+// Whole sources per chunk: the encoder and the cross-attention K/V of every decoder layer once per source, then one decoder
+// pass over the K * Lt rows of its candidates (cross-attention groups mapped to their source by kvmap), the vocabulary
+// projection reduced per row to (logit of the next target token, soft-max maximum, sum), and one warp per candidate that
+// sums the log-probabilities of its scored columns.
+template <typename ActT>
+static int score_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, const int64_t* tgt_dev, int K, int Lt, int pad, int eos,
+                     float* logp_out, int* ntok_out, float* token_logp_out, cudaStream_t user_stream) {
+    const int E = e->E(), H = e->d.num_heads, HD = e->HD(), V = e->d.tgt_vocab_size;
+    const int n_dec = (int)e->dec.size();
+    cudaStream_t s = e->stream;
+    if (int rc = join_caller_stream(e, user_stream)) return rc;
+    const int Bc = std::max(1, std::min(B, kScoreMaxRows / std::max(K * Lt, Ls)));
+    const long long T_cap = (long long)Bc * K * Lt, TS_cap = (long long)Bc * Ls;
+    if (ensure_work<ActT>(e, std::max(T_cap, TS_cap), 1)) return 1;
+    if (e->src32.ensure(TS_cap * sizeof(int)) || e->memory.ensure(TS_cap * E * sizeof(float)) || e->srclen.ensure((size_t)Bc * sizeof(int))) return 1;
+    if (Prec<ActT>::lowp && e->memh.ensure(TS_cap * E * sizeof(ActT))) return 1;
+    if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
+    // kvmap [Bc K], then per row: tokv, lmax, lsum and the top-1 / support outputs of classifier_stats that nothing reads
+    const size_t G_cap = (size_t)Bc * K, R = (size_t)T_cap;
+    if (e->score.ensure((G_cap + 6 * R) * 4)) return 1;
+    int* kvmap = e->score.as<int>();
+    float* tokv = e->score.as<float>() + G_cap;
+    float* lmax = tokv + R;
+    float* lsum = lmax + R;
+    float* topv = lsum + R;
+    int* nkeep = reinterpret_cast<int*>(topv + R);
+    int* topi = nkeep + R;
+    int* tgt32 = e->tok32.as<int>();
+    int* row_tok = e->pred.as<int>();
+    int* src32 = e->src32.as<int>();
+    int* srclen = e->srclen.as<int>();
+    ActT* crosskv = e->crosskv.as<ActT>();
+    float* x = e->x.as<float>();
+    ActT* xh = Prec<ActT>::lowp ? e->xh.as<ActT>() : nullptr;
+    const char* nf = getenv("TTB_NO_FUSED_STATS");
+    const bool try_fused = Prec<ActT>::lowp && !(nf && nf[0] == '1');
+    TTB_CUDA_OK(cudaEventRecord(e->t0, s));
+
+    for (int b0 = 0; b0 < B; b0 += Bc) {
+        const int nb = std::min(Bc, B - b0), G = nb * K;
+        const long long T = (long long)G * Lt, TS = (long long)nb * Ls;
+        if (encode_batch<ActT>(e, src_dev + (long long)b0 * Ls, nb, Ls, srclen, crosskv, TS * 2 * E, s)) return 1;
+        { Scope sc(e, KC_MISC, s); launch_i64_to_i32(reinterpret_cast<const long long*>(tgt_dev) + (long long)b0 * K * Lt, tgt32, T, s); }
+        { Scope sc(e, KC_MISC, s); launch_score_prepare(tgt32, G, Lt, K, kvmap, row_tok, s); }
+        { Scope sc(e, KC_EMBED, s); launch_embed_seq<ActT>(tgt32, (int)T, Lt, e->tgt_emb, e->pe, E, x, xh, s); }
+        RowCount rows((int)T);
+        auto self_attn = [&](int, ActT* qkv, ActT* att) {
+            attn(qkv, 3 * E, qkv + E, qkv + 2 * E, 3 * E, att, E, G, nullptr, Lt, Lt, Lt, nullptr, tgt32, Lt, e->d.tgt_pad_token_idx, true, H, HD, s);
+        };
+        auto cross_attn = [&](int l, ActT* q2, ActT* att) {
+            const ActT* kv = crosskv + (long long)l * TS * 2 * E;
+            attn(q2, E, kv, kv + E, 2 * E, att, E, G, nullptr, Lt, Ls, Ls, kvmap, src32, Ls, e->d.src_pad_token_idx, false, H, HD, s,
+                 nullptr, srclen);
+        };
+        if (decoder_stack<ActT>(e, rows, 1, 0, self_attn, cross_attn, s)) return 1;
+        bool fused = false;
+        if constexpr (Prec<ActT>::lowp) {
+            if (try_fused) {
+                Scope sc(e, KC_GEMM_CLASSIFIER, s);
+                const int rc = launch_classifier_stats(xh, E, e->classifier.wh, e->classifier.b, rows, V, E, 1, row_tok, tokv, lmax, lsum,
+                                                       nkeep, topv, topi, s);
+                if (rc > 0) return 1;
+                fused = rc == 0;
+                if (!fused) e->launches--;
+            }
+        }
+        if (!fused) {
+            if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, e->logits.as<float>(), V, rows, false, s)) return 1;
+            Scope sc(e, KC_ARGMAX, s);
+            launch_logprob_stats(e->logits.as<float>(), V, V, row_tok, (int)T, tokv, lmax, lsum, s);
+        }
+        {
+            Scope sc(e, KC_ACCEPT, s);
+            launch_score_reduce(tgt32, G, Lt, pad, eos, tokv, lmax, lsum, logp_out + (long long)b0 * K, ntok_out + (long long)b0 * K,
+                                token_logp_out ? token_logp_out + (long long)b0 * K * (Lt - 1) : nullptr, s);
+        }
+        TTB_CUDA_OK(cudaGetLastError());
+    }
+    float ms = 0.f;
+    return finish_loop(e, ms);
+}
+
 }  // namespace ttb
 
 // =================================================================================================
@@ -1807,7 +1895,7 @@ void ttb_engine_destroy(ttb_engine* e) {
     DevBuf* bufs[] = {&e->x, &e->xh, &e->y, &e->qkv, &e->att, &e->q2, &e->hid, &e->logits, &e->tok32, &e->keytok32, &e->pred,
                       &e->src32, &e->memory, &e->memh, &e->crosskv, &e->kcache, &e->vcache, &e->drafts, &e->gen, &e->front,
                       &e->active, &e->ctrl, &e->sel, &e->out64, &e->hist, &e->beam, &e->srclen, &e->desc, &e->kcache2, &e->vcache2,
-                      &e->cb, &e->cb_work};
+                      &e->cb, &e->cb_work, &e->score};
     for (DevBuf* b : bufs) b->release();
     if (e->h_ctrl) cudaFreeHost(e->h_ctrl);
     for (auto& ev : e->poll_ev) if (ev) cudaEventDestroy(ev);
@@ -2148,6 +2236,23 @@ int ttb_beam_speculative_generate_batches(ttb_engine* e, int32_t n_batches, cons
                                    beam_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, n_best, draft_len, n_drafts, pad_token, bos_token,
                                                            eos_token, c_token, tie_break, nullptr, nullptr, nullptr, nullptr, total, s,
                                                            smart_drafts_mode != 0, &cb)));
+}
+
+int ttb_score_targets(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, const int64_t* tgt_dev, int32_t K, int32_t Lt,
+                      int32_t pad_token, int32_t eos_token, float* logp_out_dev, int32_t* ntok_out_dev, float* token_logp_out_dev,
+                      void* stream) {
+    TTB_CHECK(e && e->finalized, "engine not finalized");
+    TTB_CHECK(src_dev && tgt_dev && logp_out_dev && ntok_out_dev, "bad arguments");
+    TTB_CHECK(B > 0 && K > 0 && Ls > 0 && Lt > 1, "bad arguments: B, K, Ls >= 1 and Lt >= 2");
+    TTB_CHECK(Ls <= e->d.max_positions && Lt <= e->d.max_positions, "sequence longer than the positional table");
+    TTB_CHECK((long long)K * Lt <= kScoreMaxRows, "K * Lt above 32768 decoder rows per source");
+    TTB_CHECK(pad_token != eos_token, "The eos token and the pad token must be different");
+    TTB_CUDA_OK(cudaSetDevice(e->device));
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    return drained(e, TTB_DISPATCH(e, score_api<float>(e, src_dev, B, Ls, tgt_dev, K, Lt, pad_token, eos_token, logp_out_dev, ntok_out_dev,
+                                                       token_logp_out_dev, s),
+                                   score_api<__nv_bfloat16>(e, src_dev, B, Ls, tgt_dev, K, Lt, pad_token, eos_token, logp_out_dev, ntok_out_dev,
+                                                            token_logp_out_dev, s)));
 }
 
 int ttb_kernel_class_count(void) { return KC_COUNT; }

@@ -2556,7 +2556,10 @@ int launch_classifier_stats(const __nv_bfloat16* A, int lda, const __nv_bfloat16
     if (rows.max_rows <= 0) return 0;
     const int V_pad = (V + 31) / 32 * 32, KB = Kdim / BK;
     const int smem = KB * A_BYTES + KB * V_pad * 128 + V_pad * 4 + BM * 8 + 8 * 18 + 64 + 1024;
-    const int KT = n_best <= 8 ? 8 : 16;
+    // one-entry list for n_best = 1 (teacher-forced scoring reads only the maximum, the sum and the token logit): the same
+    // outputs as the 8-entry list, without its sift in the column loop.  Which shapes fit is decided with the 8-entry
+    // exchange area either way, so that n_best does not move a shape between the fused and the unfused kernels.
+    const int KT = n_best == 1 ? 1 : (n_best <= 8 ? 8 : 16), KT_fit = KT < 8 ? 8 : KT;
     // n_best > 8 stays on the unfused kernels unless forced (TTB_FUSED_STATS_WIDE=1): a warp runs the sift of the sorted list
     // whenever ANY of its 32 rows inserts, which at 16 entries is nearly every element -- measured on B200 (retrosynthesis,
     // bs 8, n_best 10): 267 SMILES/s fused against 291 unfused, while n_best 5 is on par (253 / 252) with one launch less
@@ -2565,7 +2568,7 @@ int launch_classifier_stats(const __nv_bfloat16* A, int lda, const __nv_bfloat16
         if (!(wide && wide[0] == '1')) return -1;
     }
     if (Kdim % BK != 0 || KB > 16 || V_pad > 512 || smem > 227 * 1024 || lda % 8 != 0 || (reinterpret_cast<uintptr_t>(A) & 15) ||
-        (reinterpret_cast<uintptr_t>(W) & 15) || n_best > 16 || n_best > V || 4096 + 4 * KT * BM * 4 > KB * A_BYTES)
+        (reinterpret_cast<uintptr_t>(W) & 15) || n_best > 16 || n_best > V || 4096 + 4 * KT_fit * BM * 4 > KB * A_BYTES)
         return -1;
     CUtensorMap tmA, tmW, tmWtail;
     if (int rc = get_tensor_map(A, rows.max_rows, Kdim, lda, BM, &tmA)) return rc;
@@ -2573,7 +2576,11 @@ int launch_classifier_stats(const __nv_bfloat16* A, int lda, const __nv_bfloat16
     if (int rc = get_tensor_map(W, V, Kdim, Kdim, V_pad >= 128 ? 128 : tail_rows, &tmW)) return rc;
     if (int rc = get_tensor_map(W, V, Kdim, Kdim, tail_rows, &tmWtail)) return rc;
     const int tiles = (rows.max_rows + BM - 1) / BM;
-    if (KT == 8) {
+    if (KT == 1) {
+        if (int rc = ensure_dyn_smem(classifier_stats_kernel<1>, smem)) return rc;
+        launch_pdl(classifier_stats_kernel<1>, dim3(tiles), dim3(cls::THREADS), (size_t)smem, s, tmA, tmW, tmWtail, bias, rows, V, V_pad, KB, n_best, row_tok,
+                   tokv, lmax, lsum, nkeep, topv, topi);
+    } else if (KT == 8) {
         if (int rc = ensure_dyn_smem(classifier_stats_kernel<8>, smem)) return rc;
         launch_pdl(classifier_stats_kernel<8>, dim3(tiles), dim3(cls::THREADS), (size_t)smem, s, tmA, tmW, tmWtail, bias, rows, V, V_pad, KB, n_best, row_tok,
                    tokv, lmax, lsum, nkeep, topv, topi);

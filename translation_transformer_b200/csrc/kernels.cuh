@@ -314,4 +314,15 @@ int launch_sbeam_admit(const StdBeamState& st, const SbTable& cb, int grp, int B
 void launch_sbeam_prepare_groups(const StdBeamState& st, const SbTable& cb, cudaStream_t s);
 int launch_sbeam_select_groups(const StdBeamState& st, const SbTable& cb, int max_beam, cudaStream_t s);
 
+// ---- scoring.cu : teacher-forced scoring of given targets (G candidates, Lt columns each, int32 tokens tgt [G][Lt]) -----
+// kvmap[g] = g / K (candidate -> source), row_tok[g * Lt + t] = tgt[g][t + 1] (-1 in the last column)
+void launch_score_prepare(const int* tgt, int G, int Lt, int K, int* kvmap, int* row_tok, cudaStream_t s);
+// per row of fp32 logits: logit of token row_tok[row] (0 when -1), soft-max maximum and sum of exp(logit - maximum)
+void launch_logprob_stats(const float* logits, int ld, int V, const int* row_tok, int rows, float* tokv, float* lmax, float* lsum,
+                          cudaStream_t s);
+// per candidate: scored columns n (EOS / PAD rule), sum of tokv - lmax - log(lsum) over rows g * Lt + 0 .. n - 1, optional
+// per-column values token_logp_out [G][Lt - 1] (0 at unscored columns)
+void launch_score_reduce(const int* tgt, int G, int Lt, int pad, int eos, const float* tokv, const float* lmax, const float* lsum,
+                         float* logp_out, int* ntok_out, float* token_logp_out, cudaStream_t s);
+
 }  // namespace ttb
