@@ -22,7 +22,7 @@
 extern "C" {
 #endif
 
-#define TTB_ABI_VERSION 7
+#define TTB_ABI_VERSION 8
 
 #define TTB_PRECISION_FP32 0 /* fp32 FMA GEMMs, exact-parity path (1e-5 logits)            */
 #define TTB_PRECISION_BF16 1 /* tcgen05 bf16 GEMMs, fp32 accumulate (1e-2 logits)          */
@@ -188,6 +188,20 @@ int ttb_beam_speculative_generate_batches(ttb_engine* e, int32_t n_batches, cons
                                           int64_t* const* out_devs, int32_t* out_widths, int32_t* const* trace_nacc_devs,
                                           int32_t* const* trace_pick_devs, ttb_generate_stats* stats, ttb_generate_stats* total,
                                           void* stream);
+
+/* ---- sampling decoding (no reference counterpart; DESIGN.md section 15).  src_dev (B, Ls) int64; out_dev (B, n_samples,
+ * max_len) int64.  Sample s of source b starts from bos_token and appends one token per step drawn by the Gumbel-max rule:
+ * argmax_v (logit_v / temperature + g_v) over the top_k largest logits (top_k = 0: the whole vocabulary; ties at the
+ * boundary and between equal z go to the lower token id), g_v = -log(-log(u)) with u from Philox4x32-10 at counter
+ * (column, s, v >> 2, 0) and key = FNV-1a-64(seed bytes, non-PAD tokens of src[b]).  A row ends at its first drawn
+ * eos_token or pad_token (kept) or when it holds max_len tokens; PAD behind.  The samples of a source depend on its tokens,
+ * the seed and the settings only (identical sources with one seed get identical samples).  Rejected before any device
+ * work: B * n_samples > 2048, n_samples < 1, a temperature that is not finite and > 0, top_k outside [0, V],
+ * max_len < 2, pad_token == eos_token, lengths above the positional table.  stats: model_calls = decoder steps,
+ * produced_tokens = drawn tokens, unfinished = rows that reached max_len without EOS or PAD. */
+int ttb_sample_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len, int32_t n_samples, float temperature,
+                        int32_t top_k, uint64_t seed, int32_t pad_token, int32_t bos_token, int32_t eos_token, int64_t* out_dev,
+                        ttb_generate_stats* stats, void* stream);
 
 /* ---- teacher-forced scoring of given targets (no reference counterpart; DESIGN.md §14).  src_dev (B, Ls) int64,
  * tgt_dev (B, K, Lt) int64 with column 0 = start token; candidate (b,k) is tgt[b,k,1:] up to and including its first

@@ -44,7 +44,7 @@ def parse():
     ap.add_argument("--vocab", type=int, default=288, help="vocabulary size of the synthetic queries")
     ap.add_argument("--ckpt", help="torch file with the reference checkpoint (state_dict under 'state_dict', keys 'model.*')")
     ap.add_argument("--generation", default="greedy_speculative",
-                    choices=["greedy", "beam_search", "greedy_speculative", "beam_search_speculative"])
+                    choices=["greedy", "beam_search", "greedy_speculative", "beam_search_speculative", "sampling"])
     ap.add_argument("--batch-size", type=int, default=32)
     ap.add_argument("--beam-size", type=int, default=5)
     ap.add_argument("--max-len", type=int, default=200)
@@ -52,7 +52,12 @@ def parse():
     ap.add_argument("--n-drafts", type=int, default=23)
     ap.add_argument("--smart-drafts-mode", action="store_true")
     ap.add_argument("--precision", default="bf16", choices=["bf16", "fp32"])
-    ap.add_argument("--seed", type=int, default=1234)
+    ap.add_argument("--seed", type=int, default=1234, help="seed of the random weights (without --ckpt)")
+    ap.add_argument("--n-samples", type=int, default=5, help="--generation sampling: samples per source (CSV prediction_1..n)")
+    ap.add_argument("--temperature", type=float, default=1.0, help="--generation sampling: soft-max temperature")
+    ap.add_argument("--top-k", type=int, default=0, help="--generation sampling: draw from the k most likely tokens (0: all)")
+    ap.add_argument("--sampling-seed", type=int, default=0,
+                    help="--generation sampling: seed of the noise (a query's samples depend on its tokens and this seed only)")
     ap.add_argument("--output", help="prediction CSV (reference format); omitted -> predictions are not saved")
     ap.add_argument("--report-file")
     ap.add_argument("--in-flight", type=int, default=3,
@@ -190,10 +195,11 @@ def main():
         src_tokenizer=tk, tgt_tokenizer=tk, generation=args.generation, beam_size=args.beam_size,
         max_len=args.max_len, n_drafts=args.n_drafts, draft_len=args.draft_len, smart_drafts_mode=args.smart_drafts_mode,
         report_prediction_time=rank == 0, report_prediction_file=args.report_file, state_dict=sd, precision=args.precision,
-        device=local_rank, seed=args.seed, batches_in_flight=max(1, args.in_flight), **PRODUCT_PREDICTION)
+        device=local_rank, seed=args.seed, batches_in_flight=max(1, args.in_flight), n_samples=args.n_samples,
+        temperature=args.temperature, top_k=args.top_k, sampling_seed=args.sampling_seed, **PRODUCT_PREDICTION)
 
     mine = shard_batches(len(batches), rank, world)
-    n_best = 1 if args.generation in ("greedy", "greedy_speculative") else args.beam_size
+    n_best = 1 if args.generation in ("greedy", "greedy_speculative") else (args.n_samples if args.generation == "sampling" else args.beam_size)
     if args.sharding == "dynamic":
         return main_dynamic(args, model, tk, batches, n_best, rank, world, dev)
     failures = 0

@@ -12,7 +12,7 @@ from pathlib import Path
 # TTB_LIB: file name (inside the package) of an experimental build of the same sources, for A/B runs (scripts/build_variant.sh)
 LIB_PATH = Path(__file__).resolve().parent / os.environ.get("TTB_LIB", "libttb200.so")
 
-ABI_VERSION = 7
+ABI_VERSION = 8
 PRECISION = {"fp32": 0, "bf16": 1}
 ERR_REF_INDEX, ERR_REF_SHAPE, ERR_REF_ASSERT = 10, 11, 12
 
@@ -62,6 +62,8 @@ SIGNATURES = {
     "ttb_beam_speculative_generate_batches": (C.c_int, [C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p] + [C.c_int32] * 11 +
                                               [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.POINTER(GenerateStats), C.POINTER(GenerateStats),
                                                C.c_void_p]),
+    "ttb_sample_generate": (C.c_int, [C.c_void_p, C.c_void_p] + [C.c_int32] * 4 + [C.c_float, C.c_int32, C.c_uint64] + [C.c_int32] * 3 +
+                            [C.c_void_p, C.POINTER(GenerateStats), C.c_void_p]),
     "ttb_score_targets": (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int32, C.c_int32, C.c_int32,
                                     C.c_int32, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p]),
     "ttb_engine_get_draft_history": (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32]),

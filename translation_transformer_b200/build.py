@@ -8,7 +8,7 @@ from pathlib import Path
 
 CSRC = Path(__file__).resolve().parent / "csrc"
 LIB = Path(__file__).resolve().parent / "libttb200.so"
-SOURCES = ["elementwise.cu", "gemm_simt.cu", "gemm_tcgen05.cu", "attention.cu", "attention_mma.cu", "drafting.cu", "greedy.cu", "beam.cu", "std_beam.cu", "scoring.cu", "engine.cu"]
+SOURCES = ["elementwise.cu", "gemm_simt.cu", "gemm_tcgen05.cu", "attention.cu", "attention_mma.cu", "drafting.cu", "greedy.cu", "beam.cu", "std_beam.cu", "scoring.cu", "sampling.cu", "engine.cu"]
 NVCC_FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
               "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

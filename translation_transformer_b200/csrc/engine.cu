@@ -165,13 +165,14 @@ struct ttb_engine {
     cudaEvent_t join_ev{};
     static constexpr int kBuckets = 10;
     cudaGraphExec_t graph_exec[kBuckets][2] = {};   // greedy iteration graphs per live-query bucket (grids sized for the bucket) x {long, short}
-    long long graph_key[13] = {};
+    long long graph_key[17] = {};
     long long graph_launches = 0;
     DevBuf beam;                 // arena of the beam-search state
     DevBuf hist;                 // per-iteration live-query count of the last generate()
     DevBuf cb;                   // continuous batching: slot / batch tables and the staging buffers of an admitted batch
     DevBuf cb_work;              // continuous batching: encoder workspace of an admitted batch (the loop's own must stay intact)
     DevBuf score;                // ttb_score_targets: candidate -> source map and per-row statistics of one chunk
+    DevBuf smp;                  // ttb_sample_generate: per-source keys, per-live-row source and cross-attention descriptor
     std::vector<int> h_hist;
     std::vector<int> h_dl, h_dl_min;   // continuous beam-search loop: draft length of every decoder call, smallest of its batches
 
@@ -183,7 +184,7 @@ struct ttb_engine {
     // different host threads, translation_transformer_b200/pipeline.py)
     long long alloc_signature() const {
         const DevBuf* bufs[] = {&x, &xh, &y, &qkv, &att, &q2, &hid, &logits, &tok32, &keytok32, &pred, &src32, &srclen, &desc, &memory, &memh,
-                                &crosskv, &kcache, &vcache, &kcache2, &vcache2, &drafts, &gen, &front, &active, &ctrl, &sel, &out64, &beam, &hist, &cb, &cb_work};
+                                &crosskv, &kcache, &vcache, &kcache2, &vcache2, &drafts, &gen, &front, &active, &ctrl, &sel, &out64, &beam, &hist, &cb, &cb_work, &smp};
         unsigned long long h = 1469598103934665603ull;
         for (const DevBuf* b : bufs) {
             h = (h ^ (unsigned long long)reinterpret_cast<uintptr_t>(b->p)) * 1099511628211ull;
@@ -746,13 +747,24 @@ static int read_groups(const BatchList* cb, const G* dev, std::vector<G>& groups
     return 0;
 }
 
+// Sampling decoding (ttb_sample_generate, DESIGN.md section 15): S sample slots per source, drawn with temperature T from
+// the top_k largest logits (0: all) under the per-source keys of `seed`.
+struct SampleCfg {
+    int S;
+    float temperature;
+    int top_k;
+    unsigned long long seed;
+};
+
 // Speculative greedy loop, and with `standard` the standard greedy decoding (no drafts).  With `cb` the loop is the
 // continuous one: B is the number of query slots, Ls the longest source of all batches, and the batches of `cb` are
-// admitted into free slots between two graph launches.
+// admitted into free slots between two graph launches.  With `smp` (and `standard`) the loop is the sampling decoding:
+// B is the number of sample slots (sources x S), slot b * S + s is sample s of source b, and the draw replaces the arg-max.
 template <typename ActT>
 static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int max_len, int draft_len, int N,
                       int pad, int bos, int eos, int replace, int tie_break, int64_t* out_dev, int32_t* trace_dev,
-                      ttb_generate_stats* stats, cudaStream_t user_stream, bool standard = false, const BatchList* cb = nullptr) {
+                      ttb_generate_stats* stats, cudaStream_t user_stream, bool standard = false, const BatchList* cb = nullptr,
+                      const SampleCfg* smp = nullptr) {
     const int E = e->E(), H = e->d.num_heads, HD = e->HD(), V = e->d.tgt_vocab_size;
     const int n_dec = (int)e->dec.size();
     cudaStream_t s = e->stream;
@@ -764,7 +776,10 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     // buffers that depend on the source length are sized for a rounded-up capacity so that batches of
     // different length neither reallocate nor invalidate the captured graph
     const int Ls_cap = std::max(256, (Ls + 63) / 64 * 64);
-    const long long TS_cap = (long long)B * Ls_cap;
+    // sampling: the encoder and the cross-attention K/V run once per source, shared by its S slots
+    const bool sampling = smp != nullptr;
+    const int S = sampling ? smp->S : 1, B_src = B / S;
+    const long long TS_cap = (long long)B_src * Ls_cap;
     const int per_q = N * (D + 1);
     const long long T = (long long)B * per_q;
     const int gen_ld = max_len + D + 2;
@@ -789,6 +804,17 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     if (e->desc.ensure((size_t)B * sizeof(int4))) return 1;
     if (e->hist.ensure((size_t)(max_iters + 1) * sizeof(int))) return 1;
     if (ensure_work<ActT>(e, cont ? T : std::max(T, TS_cap), n_dec)) return 1;
+    SampleLoop sl{S, nullptr, nullptr};
+    unsigned long long* smp_keys = nullptr;
+    if (sampling) {
+        if (e->smp.ensure((size_t)B_src * 8 + (size_t)B * 20 + 256)) return 1;
+        smp_keys = e->smp.as<unsigned long long>();
+        sl.xdesc = reinterpret_cast<int4*>(e->smp.as<char>() + ((size_t)B_src * 8 + 15) / 16 * 16);
+        sl.kvsrc = reinterpret_cast<int*>(sl.xdesc + B);
+    }
+    // the draw's fused / fallback choice is read per call (part of the graph key), so that one process can compare both
+    const char* nfa = sampling ? getenv("TTB_NO_FUSED_ARGMAX") : nullptr;
+    const bool smp_fused = sampling && Prec<ActT>::lowp && !(nfa && nfa[0] == '1');
     // continuous loop: slot / batch tables, staging of an admitted batch (drafts as well)
     CbTable cbt{};
     int* stage_drafts = nullptr;
@@ -825,10 +851,16 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     if (cont) {
         TTB_CUDA_OK(cudaMemsetAsync(st.ctrl, 0, CTRL_COUNT * sizeof(int), s));
     } else {
-    if (encode_batch<ActT>(e, src_dev, B, Ls, e->srclen.as<int>(), crosskv, TS_cap * 2 * E, s)) return 1;
+    if (encode_batch<ActT>(e, src_dev, B_src, Ls, e->srclen.as<int>(), crosskv, TS_cap * 2 * E, s)) return 1;
     // drafts from the source without its BOS column (speculative_decoding.py:64-73)
     if (!standard) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Ls, B, Ls - 1, D, N, eos, pad, replace, e->drafts.as<int>(), s); }
-    { Scope sc(e, KC_MISC, s); launch_greedy_init(st, s); }
+    if (sampling) {
+        { Scope sc(e, KC_MISC, s); launch_sample_keys(src32, B_src, Ls, e->d.src_pad_token_idx, smp->seed, smp_keys, s); }
+        { Scope sc(e, KC_MISC, s); launch_sample_init(st, sl, s); }
+    } else {
+        Scope sc(e, KC_MISC, s);
+        launch_greedy_init(st, s);
+    }
     }
 
     float* x = e->x.as<float>();
@@ -857,6 +889,11 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
                  e->d.src_pad_token_idx, false, H, HD, s, st.ctrl + CTRL_LS, e->srclen.as<int>(), st.desc);
             return;
         }
+        if (sampling) {   // the K/V rows of the slot's source, not of the slot
+            attn(q2, E, kv, kv + E, 2 * E, att, E, Bq, n_active, per_q, Ls, Ls, sl.kvsrc, src32, Ls, e->d.src_pad_token_idx, false, H, HD, s,
+                 st.ctrl + CTRL_LS, e->srclen.as<int>(), sl.xdesc);
+            return;
+        }
         attn(q2, E, kv, kv + E, 2 * E, att, E, Bq, n_active, per_q, Ls, Ls, st.active,
              src32, Ls, e->d.src_pad_token_idx, false, H, HD, s, st.ctrl + CTRL_LS, e->srclen.as<int>(), st.desc);
     };
@@ -871,6 +908,27 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
                                         cache_l_stride, cache_q_stride, E, s);
         }
         if (decoder_stack<ActT>(e, rows, n_dec, qkv_l_stride, self_attn, cross_attn, s)) return 1;
+        if (sampling) {
+            const SampleArgs sa{st.desc, smp_keys, S, smp->temperature, smp->top_k, st.pred};
+            bool fused = false;
+            if constexpr (Prec<ActT>::lowp) {
+                if (smp_fused) {
+                    Scope sc(e, KC_GEMM_CLASSIFIER, s);
+                    const int rc = launch_classifier_sample(xh, E, e->classifier.wh, e->classifier.b, rows, V, E, sa, s);
+                    if (rc > 0) return 1;
+                    fused = rc == 0;
+                    if (!fused) e->launches--;
+                }
+            }
+            if (!fused) {
+                if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, e->logits.as<float>(), V, rows, false, s)) return 1;
+                Scope sc(e, KC_ARGMAX, s);
+                launch_sample_rows(e->logits.as<float>(), V, V, rows, sa, s);
+            }
+            Scope sc(e, KC_ACCEPT, s);
+            launch_sample_step(st, sl, s);
+            return 0;
+        }
         bool fused_cls = false;
         if constexpr (Prec<ActT>::lowp) {
             static const bool off = [] { const char* v = getenv("TTB_NO_FUSED_ARGMAX"); return v && v[0] == '1'; }();
@@ -919,13 +977,18 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
         cand[9] = 1;
         for (int i = 0; i < ttb_engine::kBuckets; ++i) {
             // generate() of the standard greedy decoding keeps every row to the end; its continuous loop sheds stopped batches
-            if (i > 0 && (no_buckets || (standard && !cont))) break;
+            // and sampling retires every slot on its own
+            if (i > 0 && (no_buckets || (standard && !cont && !sampling))) break;
             if (n_buckets == 0 || (cand[i] >= 1 && cand[i] < bucket_q[n_buckets - 1])) bucket_q[n_buckets++] = cand[i];
         }
     }
     if (use_graph) {
-        const long long key[13] = {B, N, D, (standard ? 1 : 0) + (cont ? 2 : 0), max_len, pad, bos, eos, tie_break, e->alloc_signature(),
-                                   (long long)sizeof(ActT) + 16 * K_it, replace, cont ? Ls_cap : 0};
+        // sampling: everything a call may change that the captured kernels take by value (the keys are in device memory)
+        uint32_t t_bits = 0;
+        if (sampling) memcpy(&t_bits, &smp->temperature, 4);
+        const long long key[17] = {B, N, D, (standard ? 1 : 0) + (cont ? 2 : 0) + (sampling ? 4 : 0), max_len, pad, bos, eos, tie_break,
+                                   e->alloc_signature(), (long long)sizeof(ActT) + 16 * K_it, replace, cont ? Ls_cap : 0, sampling ? S : 0,
+                                   (long long)t_bits, sampling ? smp->top_k : -1, smp_fused ? 1 : 0};
         if (memcmp(key, e->graph_key, sizeof(key)) != 0) {
             for (auto& gb : e->graph_exec) for (auto& g : gb) if (g) { cudaGraphExecDestroy(g); g = nullptr; }
             memcpy(e->graph_key, key, sizeof(key));
@@ -1895,7 +1958,7 @@ void ttb_engine_destroy(ttb_engine* e) {
     DevBuf* bufs[] = {&e->x, &e->xh, &e->y, &e->qkv, &e->att, &e->q2, &e->hid, &e->logits, &e->tok32, &e->keytok32, &e->pred,
                       &e->src32, &e->memory, &e->memh, &e->crosskv, &e->kcache, &e->vcache, &e->drafts, &e->gen, &e->front,
                       &e->active, &e->ctrl, &e->sel, &e->out64, &e->hist, &e->beam, &e->srclen, &e->desc, &e->kcache2, &e->vcache2,
-                      &e->cb, &e->cb_work, &e->score};
+                      &e->cb, &e->cb_work, &e->score, &e->smp};
     for (DevBuf* b : bufs) b->release();
     if (e->h_ctrl) cudaFreeHost(e->h_ctrl);
     for (auto& ev : e->poll_ev) if (ev) cudaEventDestroy(ev);
@@ -2129,6 +2192,28 @@ int ttb_greedy_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t*
                                                         nullptr, nullptr, total, s, true, &cb),
                                    greedy_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1,
                                                              nullptr, nullptr, total, s, true, &cb)));
+}
+
+int ttb_sample_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len, int32_t n_samples, float temperature,
+                        int32_t top_k, uint64_t seed, int32_t pad_token, int32_t bos_token, int32_t eos_token, int64_t* out_dev,
+                        ttb_generate_stats* stats, void* stream) {
+    TTB_CHECK(e && e->finalized, "engine not finalized");
+    TTB_CHECK(src_dev && out_dev && B > 0 && Ls > 0, "bad arguments");
+    TTB_CHECK(n_samples >= 1, "n_samples must be at least 1");
+    TTB_CHECK((long long)B * n_samples <= 2048, "B * n_samples above 2048 sample slots");
+    TTB_CHECK(std::isfinite(temperature) && temperature > 0.f, "temperature must be finite and greater than 0");
+    TTB_CHECK(top_k >= 0 && top_k <= e->d.tgt_vocab_size, "top_k must lie in [0, vocabulary size]");
+    TTB_CHECK(max_len >= 2, "max_len must be at least 2");
+    TTB_CHECK(pad_token != eos_token, "The eos token and the pad token must be different");
+    TTB_CHECK(Ls <= e->d.max_positions && max_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
+    TTB_CUDA_OK(cudaSetDevice(e->device));
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    const SampleCfg smp{n_samples, temperature, top_k, (unsigned long long)seed};
+    const int R = B * n_samples;
+    return drained(e, TTB_DISPATCH(e, greedy_api<float>(e, src_dev, R, Ls, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, out_dev, nullptr,
+                                                        stats, s, true, nullptr, &smp),
+                                   greedy_api<__nv_bfloat16>(e, src_dev, R, Ls, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, out_dev,
+                                                             nullptr, stats, s, true, nullptr, &smp)));
 }
 
 int ttb_beam_search_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len, int32_t beam_size,

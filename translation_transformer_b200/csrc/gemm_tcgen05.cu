@@ -11,6 +11,7 @@
 // of one tile overlaps the main loop of another.  The live row count is read on the device
 // (RowCount): CTAs beyond it exit before touching any barrier.
 #include "kernels.cuh"
+#include "philox.cuh"
 
 #include <cuda.h>
 #include <cstdlib>
@@ -2164,13 +2165,23 @@ gemm_pair_k256_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_cons
 // the whole [V x K] classifier weight and its A tile in shared memory (K = 256: 64 KB + 144 KB for V = 288),
 // accumulates all V_pad <= 512 columns in TMEM (one N <= 256 MMA group plus a tail group), and each row's
 // maximum is found by two threads scanning disjoint column ranges straight out of TMEM.
+//
+// The same kernel draws the sampling decoding's tokens (DESIGN.md section 15) with another epilogue, EPI:
+//   CLS_ARGMAX       the arg-max above (the greedy loops);
+//   CLS_SAMPLE       top_k = 0: one pass, z = (logit + bias) / T + Gumbel noise (one Philox call per 4 columns), running
+//                    arg-max of z; the halves merge as the arg-max does (a strictly larger upper-half z wins);
+//   CLS_SAMPLE_TOPK  1 <= top_k <= 8: the sorted 8-entry list pass of classifier_stats_kernel, the two lists merged in
+//                    shared memory (the A tiles are dead by then), noise for the first top_k entries only.
 namespace cls {
 constexpr int THREADS = 320;
+enum Epi : int { CLS_ARGMAX = 0, CLS_SAMPLE = 1, CLS_SAMPLE_TOPK = 2 };
+constexpr int SAMPLE_KT = 8;
 }
+template <int EPI>
 __global__ void __launch_bounds__(cls::THREADS, 1)
 classifier_argmax_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmW,
                          const __grid_constant__ CUtensorMap tmWtail, const float* __restrict__ bias, int* __restrict__ pred,
-                         RowCount rows, int V, int V_pad, int KB) {
+                         RowCount rows, int V, int V_pad, int KB, SampleArgs sa) {
     const int m0 = blockIdx.x * BM;
     extern __shared__ uint8_t smem_raw[];
     const uint32_t raw = smem_u32(smem_raw);
@@ -2242,7 +2253,7 @@ classifier_argmax_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
             }
             umma_commit(tfull_bar);
         }
-    } else if (live) {  // ===== arg-max: thread = (row, column range) =====
+    } else if (live && EPI == cls::CLS_ARGMAX) {  // ===== arg-max: thread = (row, column range) =====
         const int q = warp & 3, hh = (warp - 2) >> 2;
         const int row = q * 32 + lane;
         const int n32 = V_pad / 32, c_half = (n32 + 1) / 2;
@@ -2270,6 +2281,96 @@ classifier_argmax_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_c
             }
             if (m0 + row < M) pred[m0 + row] = bi;
         }
+    } else if (live) {  // ===== draw of the sampling decoding: thread = (row, column half) =====
+      if constexpr (EPI != cls::CLS_ARGMAX) {
+        const int q = warp & 3, hh = (warp - 2) >> 2;
+        const int row = q * 32 + lane;
+        const int grow = m0 + row;
+        const int n32 = V_pad / 32, c_half = (n32 + 1) / 2;
+        const int c_begin = hh == 0 ? 0 : c_half, c_end = hh == 0 ? c_half : n32;
+        int4 d = make_int4(0, 0, 0, 0);
+        unsigned long long key = 0;
+        if (grow < M) {
+            d = sa.desc[grow];
+            key = sa.keys[d.x / sa.S];
+        }
+        const int t = d.y + 1, smp = d.x % sa.S;
+        const float T = sa.temperature;
+        const uint32_t tm_row = tmem_base + ((uint32_t)(q * 32) << 16);
+        mbar_wait(tfull_bar, 0);
+        tcgen05_fence_after();
+        if constexpr (EPI == cls::CLS_SAMPLE) {
+            float best = -INFINITY;
+            int bi = 0x7fffffff;
+            for (int ch = c_begin; ch < c_end; ++ch) {
+                uint32_t r[32];
+                tmem_ld_32x32(tm_row + (uint32_t)(ch * 32), r);
+#pragma unroll
+                for (int j4 = 0; j4 < 8; ++j4) {
+                    const Philox4 nz = sample_noise_bits(t, smp, ch * 8 + j4, key);
+#pragma unroll
+                    for (int u = 0; u < 4; ++u) {
+                        const int col = ch * 32 + j4 * 4 + u;
+                        const float z = (__uint_as_float(r[j4 * 4 + u]) + bias_sm[col]) / T + gumbel(nz.x[u]);
+                        if (col < V && sample_better(z, col, best, bi)) { best = z; bi = col; }
+                    }
+                }
+            }
+            if (hh == 1) half_best[row] = make_float2(best, __int_as_float(bi));
+            asm volatile("bar.sync 1, 256;" ::: "memory");
+            if (hh == 0) {
+                if (c_end < n32) {   // a strictly larger upper-half z wins (its ids are all above the lower half's)
+                    const float2 o = half_best[row];
+                    if (o.x > best || bi >= V) { best = o.x; bi = __float_as_int(o.y); }
+                }
+                if (grow < M) sa.pred[grow] = bi < V ? bi : 0;   // no candidate only with NaN logits
+            }
+        } else {
+            constexpr int KT = cls::SAMPLE_KT;
+            float* xv = reinterpret_cast<float*>(gen);                    // [2][KT][128] list values (aliases the A tiles)
+            int* xi = reinterpret_cast<int*>(gen + 2 * KT * BM * 4);      // [2][KT][128] list token ids
+            float tv[KT];
+            int ti[KT];
+#pragma unroll
+            for (int i = 0; i < KT; ++i) { tv[i] = -INFINITY; ti[i] = -1; }
+            for (int ch = c_begin; ch < c_end; ++ch) {
+                uint32_t r[32];
+                tmem_ld_32x32(tm_row + (uint32_t)(ch * 32), r);
+#pragma unroll
+                for (int j = 0; j < 32; ++j) {
+                    const int col = ch * 32 + j;
+                    if (col < V) topk_list_insert<KT>(tv, ti, __uint_as_float(r[j]) + bias_sm[col], col);
+                }
+            }
+#pragma unroll
+            for (int i = 0; i < KT; ++i) { xv[(hh * KT + i) * BM + row] = tv[i]; xi[(hh * KT + i) * BM + row] = ti[i]; }
+            asm volatile("bar.sync 1, 256;" ::: "memory");
+            if (hh == 0 && grow < M) {
+                // merge of the two sorted lists (equal values: the lower column half first = lower token id); the first top_k
+                // entries are the candidate set
+                int a = 0, b = 0;
+                float best = -INFINITY;
+                int bi = 0x7fffffff;
+#pragma unroll
+                for (int j = 0; j < KT; ++j) {
+                    const float va = a < KT ? xv[a * BM + row] : -INFINITY;
+                    const float vb = b < KT ? xv[(KT + b) * BM + row] : -INFINITY;
+                    const int ia = a < KT ? xi[a * BM + row] : -1;
+                    const int ib = b < KT ? xi[(KT + b) * BM + row] : -1;
+                    const bool take_a = ia >= 0 && (ib < 0 || va >= vb);
+                    const float mv = take_a ? va : vb;
+                    const int mi = take_a ? ia : ib;
+                    a += take_a ? 1 : 0;
+                    b += take_a ? 0 : 1;
+                    if (j < sa.top_k && mi >= 0) {
+                        const float z = mv / T + gumbel(philox_word(sample_noise_bits(t, smp, mi >> 2, key), mi & 3));
+                        if (sample_better(z, mi, best, bi)) { best = z; bi = mi; }
+                    }
+                }
+                sa.pred[grow] = bi < V ? bi : 0;
+            }
+        }
+      }
     }
     tcgen05_fence_before();
     __syncthreads();
@@ -2394,17 +2495,7 @@ classifier_stats_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_co
                 if (col < V) {
                     mx = fmaxf(mx, v);
                     if (col == tok) { tokval = v; found = 1.f; }
-                    if (v > tv[KT - 1]) {          // enters the list: sift down from the top (equal values stay behind earlier ones)
-                        float cv = v;
-                        int ci = col;
-#pragma unroll
-                        for (int i = 0; i < KT; ++i) {
-                            if (cv > tv[i]) {
-                                const float t0 = tv[i]; tv[i] = cv; cv = t0;
-                                const int t1 = ti[i]; ti[i] = ci; ci = t1;
-                            }
-                        }
-                    }
+                    topk_list_insert<KT>(tv, ti, v, col);   // sift down from the top (equal values stay behind earlier ones)
                 }
             }
         }
@@ -2542,10 +2633,36 @@ int launch_classifier_argmax(const __nv_bfloat16* A, int lda, const __nv_bfloat1
     const int tail_rows = V_pad % 128 ? V_pad % 128 : 128;
     if (int rc = get_tensor_map(W, V, K, K, V_pad >= 128 ? 128 : tail_rows, &tmW)) return rc;
     if (int rc = get_tensor_map(W, V, K, K, tail_rows, &tmWtail)) return rc;
-    if (int rc = ensure_dyn_smem(classifier_argmax_kernel, smem)) return rc;
+    if (int rc = ensure_dyn_smem(classifier_argmax_kernel<cls::CLS_ARGMAX>, smem)) return rc;
     const int tiles = (rows.max_rows + BM - 1) / BM;
-    launch_pdl(classifier_argmax_kernel, dim3(tiles), dim3(cls::THREADS), (size_t)smem, s, tmA, tmW, tmWtail, bias, pred, rows, V, V_pad, KB);
+    launch_pdl(classifier_argmax_kernel<cls::CLS_ARGMAX>, dim3(tiles), dim3(cls::THREADS), (size_t)smem, s, tmA, tmW, tmWtail, bias, pred, rows, V,
+               V_pad, KB, SampleArgs{});
     return 0;
+}
+
+// returns 0 on success, -1 where launch_classifier_argmax would and for top_k > 8 (caller: logits GEMM + launch_sample_rows)
+int launch_classifier_sample(const __nv_bfloat16* A, int lda, const __nv_bfloat16* W, const float* bias, RowCount rows, int V, int K,
+                             const SampleArgs& a, cudaStream_t s) {
+    using namespace tc;
+    if (rows.max_rows <= 0) return 0;
+    const int V_pad = (V + 31) / 32 * 32, KB = K / BK;
+    const int smem = KB * A_BYTES + KB * V_pad * 128 + V_pad * 4 + BM * 8 + 8 * 18 + 64 + 1024;
+    const bool list = a.top_k > 0 && a.top_k < V;   // top_k = V draws from the whole vocabulary like top_k = 0
+    if (K % BK != 0 || KB > 16 || V_pad > 512 || smem > 227 * 1024 || lda % 8 != 0 || (reinterpret_cast<uintptr_t>(A) & 15) ||
+        (reinterpret_cast<uintptr_t>(W) & 15) || (list && (a.top_k > cls::SAMPLE_KT || 2 * 2 * cls::SAMPLE_KT * BM * 4 > KB * A_BYTES)))
+        return -1;
+    CUtensorMap tmA, tmW, tmWtail;
+    if (int rc = get_tensor_map(A, rows.max_rows, K, lda, BM, &tmA)) return rc;
+    const int tail_rows = V_pad % 128 ? V_pad % 128 : 128;
+    if (int rc = get_tensor_map(W, V, K, K, V_pad >= 128 ? 128 : tail_rows, &tmW)) return rc;
+    if (int rc = get_tensor_map(W, V, K, K, tail_rows, &tmWtail)) return rc;
+    const int tiles = (rows.max_rows + BM - 1) / BM;
+    auto launch = [&](auto kernel) -> int {
+        if (int rc = ensure_dyn_smem(kernel, smem)) return rc;
+        launch_pdl(kernel, dim3(tiles), dim3(cls::THREADS), (size_t)smem, s, tmA, tmW, tmWtail, bias, a.pred, rows, V, V_pad, KB, a);
+        return 0;
+    };
+    return list ? launch(classifier_argmax_kernel<cls::CLS_SAMPLE_TOPK>) : launch(classifier_argmax_kernel<cls::CLS_SAMPLE>);
 }
 
 

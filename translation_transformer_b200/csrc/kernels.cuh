@@ -314,6 +314,35 @@ int launch_sbeam_admit(const StdBeamState& st, const SbTable& cb, int grp, int B
 void launch_sbeam_prepare_groups(const StdBeamState& st, const SbTable& cb, cudaStream_t s);
 int launch_sbeam_select_groups(const StdBeamState& st, const SbTable& cb, int max_beam, cudaStream_t s);
 
+// ---- sampling.cu : sampling decoding (the greedy loop with S sample slots per source, slot r = b * S + s) ---------------
+// Per live position of the coming step, beside GreedyState::desc: the source of the slot (cross-attention K/V group of the
+// fp32 kernels) and the cross-attention descriptor {source, -, -, source length} of the tensor-core kernels.
+struct SampleLoop {
+    int S;
+    int* kvsrc;        // [B * S]
+    int4* xdesc;       // [B * S]
+};
+// What a draw reads per live row g: slot and front from desc[g] (column t = front + 1), the source key keys[slot / S].
+struct SampleArgs {
+    const int4* desc;
+    const unsigned long long* keys;
+    int S;
+    float temperature;
+    int top_k;         // 0: whole vocabulary
+    int* pred;         // [rows] drawn token
+};
+// keys[b] = FNV-1a-64(seed bytes, non-PAD tokens of src32[b]) (philox.cuh)
+void launch_sample_keys(const int* src32, int B, int Ls, int pad, unsigned long long seed, unsigned long long* keys, cudaStream_t s);
+void launch_sample_init(const GreedyState& st, const SampleLoop& sl, cudaStream_t s);
+// in place of launch_greedy_std_step: token append, retirement of ended slots into st.out [B * S][max_len], compaction
+void launch_sample_step(const GreedyState& st, const SampleLoop& sl, cudaStream_t s);
+// draw over fp32 logits [rows][ld], any top_k
+void launch_sample_rows(const float* logits, int ld, int V, RowCount rows, const SampleArgs& a, cudaStream_t s);
+// Vocabulary projection fused with the draw (bf16 path): the classifier_argmax_kernel design with a Gumbel-max epilogue.
+// Returns -1 where launch_classifier_argmax would, and for top_k > 8 (caller: logits GEMM + launch_sample_rows).
+int launch_classifier_sample(const __nv_bfloat16* A, int lda, const __nv_bfloat16* W, const float* bias, RowCount rows, int V, int K,
+                             const SampleArgs& a, cudaStream_t s);
+
 // ---- scoring.cu : teacher-forced scoring of given targets (G candidates, Lt columns each, int32 tokens tgt [G][Lt]) -----
 // kvmap[g] = g / K (candidate -> source), row_tok[g * Lt + t] = tgt[g][t + 1] (-1 in the last column)
 void launch_score_prepare(const int* tgt, int G, int Lt, int K, int* kvmap, int* row_tok, cudaStream_t s);

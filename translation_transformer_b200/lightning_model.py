@@ -11,6 +11,7 @@ from pathlib import Path
 from timeit import default_timer as timer
 from typing import Any
 
+from .decoding.sampling import TranslationInferenceSampling
 from .decoding.speculative_decoding import TranslationInferenceBeamSearchSpeculative, TranslationInferenceGreedySpeculative
 from .decoding.standard_decoding import TranslationInferenceBeamSearch, TranslationInferenceGreedy
 from .model import B200Transformer
@@ -29,7 +30,8 @@ class VanillaEncoderDecoderTransformerLightning(_Base):
                  beam_size: int = 0, max_len: int = 0, n_drafts: int = 0, draft_len: int = 0, smart_drafts_mode: bool = True,
                  report_prediction_time: bool = True, report_prediction_file: str | None = None,
                  state_dict: dict | None = None, precision: str = "bf16", device: int = 0, seed: int = 0,
-                 batches_in_flight: int = 1, tgt_test_path: str | None = None, **_unused):
+                 batches_in_flight: int = 1, tgt_test_path: str | None = None, n_samples: int = 1, temperature: float = 1.0,
+                 top_k: int = 0, sampling_seed: int = 0, **_unused):
         if _Base is not object:
             super().__init__()
         assert src_tokenizer is not None, "source tokenizer not provided"
@@ -38,6 +40,8 @@ class VanillaEncoderDecoderTransformerLightning(_Base):
         self.src_tokenizer, self.tgt_tokenizer = src_tokenizer, tgt_tokenizer
         self.generation, self.beam_size, self.max_len = generation, beam_size, max_len
         self.n_drafts, self.draft_len, self.smart_drafts_mode = n_drafts, draft_len, smart_drafts_mode
+        # generation="sampling" only (DESIGN.md section 15)
+        self.n_samples, self.temperature, self.top_k, self.sampling_seed = n_samples, temperature, top_k, sampling_seed
         self.report_prediction_time, self.report_prediction_file = report_prediction_time, report_prediction_file
         self.src_pad_token_i, self.tgt_pad_token_i = src_tokenizer.pad_token_idx, tgt_tokenizer.pad_token_idx
         self.tgt_bos_token_i, self.tgt_eos_token_i = tgt_tokenizer.bos_token_idx, tgt_tokenizer.eos_token_idx
@@ -87,7 +91,11 @@ class VanillaEncoderDecoderTransformerLightning(_Base):
                 draft_len=self.draft_len, n_drafts=self.n_drafts, pad_token=self.tgt_pad_token_i,
                 bos_token=self.tgt_bos_token_i, eos_token=self.tgt_eos_token_i,
                 C_token=self.tgt_tokenizer.encoder_dict["c"], smart_drafts_mode=self.smart_drafts_mode)
-        options = ", ".join(["beam_search", "greedy", "greedy_speculative", "beam_search_speculative"])
+        if self.generation == "sampling":
+            return TranslationInferenceSampling(model, max_len=self.max_len, n_samples=self.n_samples, pad_token=self.tgt_pad_token_i,
+                                                bos_token=self.tgt_bos_token_i, eos_token=self.tgt_eos_token_i,
+                                                temperature=self.temperature, top_k=self.top_k, seed=self.sampling_seed)
+        options = ", ".join(["beam_search", "greedy", "greedy_speculative", "beam_search_speculative", "sampling"])
         raise ValueError(f"Unknown generation option {self.generation}. Options are {options}.")
 
     def predict_step(self, batch: Any, batch_idx: int, dataloader_idx: int = 0) -> Any:
@@ -155,6 +163,9 @@ class VanillaEncoderDecoderTransformerLightning(_Base):
                 accepted = self._counter("accepted_tokens_num")
                 report["accepted_tokens"] = accepted
                 report["acceptance_rate"] = round(accepted / max(self._counter("produced_non_pad_tokens"), 1), 4)
+        if self.generation == "sampling":
+            report["n_samples"], report["temperature"], report["top_k"], report["seed"] = (self.n_samples, self.temperature, self.top_k,
+                                                                                          self.sampling_seed)
         report = json.dumps(report)
         print(report)
         if self.report_prediction_file is not None:
