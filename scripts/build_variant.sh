@@ -4,10 +4,12 @@
 set -e
 NAME=$1; shift
 cd "$(dirname "$0")/../translation_transformer_b200"
+# the sources of the library, as build.py compiles them
+SOURCES=$(python3 -c "from build import SOURCES; print(' '.join(SOURCES))")
 mkdir -p csrc/build_$NAME
 pids=()
-for f in elementwise gemm_simt gemm_tcgen05 attention attention_mma drafting greedy beam std_beam engine; do
-  nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC --expt-relaxed-constexpr "$@" -c csrc/$f.cu -o csrc/build_$NAME/$f.o &
+for f in $SOURCES; do
+  nvcc -gencode arch=compute_100a,code=sm_100a -O3 -lineinfo -std=c++17 -Xcompiler -fPIC --expt-relaxed-constexpr "$@" -c csrc/$f -o csrc/build_$NAME/$f.o &
   pids+=($!)
 done
 for p in "${pids[@]}"; do wait $p; done

@@ -49,10 +49,10 @@ static inline void cpu_relax() {
 #endif
 }
 
-bool pdl_enabled() {
-    static const bool on = [] { const char* v = getenv("TTB_NO_PDL"); return !(v && v[0] == '1'); }();
-    return on;
-}
+// A/B switch: true when the environment variable `name` is set to 1
+static bool env_flag(const char* name) { const char* v = getenv(name); return v && v[0] == '1'; }
+
+bool pdl_enabled() { static const bool on = !env_flag("TTB_NO_PDL"); return on; }
 
 
 struct DevBuf {
@@ -74,6 +74,12 @@ struct DevBuf {
         cap = 0;
     }
     template <typename T> T* as() const { return reinterpret_cast<T*>(p); }
+};
+
+// Layout of several buffers in one allocation: take() returns the offset of the next 256-byte aligned region
+struct Arena {
+    size_t bytes = 0;
+    size_t take(size_t n) { const size_t o = bytes; bytes += (n + 255) / 256 * 256; return o; }
 };
 
 struct Param {
@@ -319,11 +325,7 @@ static int linear(ttb_engine* e, int kc, const __nv_bfloat16* A, int lda, const 
 
 // Sub-layer tail  x <- LN2?(LN1(x + A W^T + b)):  one fused tcgen05 kernel on the bf16 path with E = 256,
 // GEMM (fp32 out) + add_layernorm otherwise.  TTB_NO_FUSED_LN=1 forces the unfused kernels (A/B comparisons).
-static bool fused_ln_enabled() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("TTB_NO_FUSED_LN"); v = (e && e[0] == '1') ? 0 : 1; }
-    return v == 1;
-}
+static bool fused_ln_enabled() { static const bool on = !env_flag("TTB_NO_FUSED_LN"); return on; }
 static int linear_resid_ln(ttb_engine* e, int kc, const float* A, int lda, const Lin& L, const Norm& n1, const Norm* n2,
                            float* x, float* /*xh*/, float* y, float* dst, float* dsth, RowCount rows, cudaStream_t s,
                            const Lin* = nullptr, float* = nullptr, bool* chained = nullptr) {
@@ -335,11 +337,7 @@ static int linear_resid_ln(ttb_engine* e, int kc, const float* A, int lda, const
 }
 // `chain` (optional): a projection of the normalised result that the same kernel computes on the way out
 // (the cross-attention query); *chained tells the caller whether it was taken.
-static bool chain_enabled() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("TTB_NO_CHAIN"); v = (e && e[0] == '1') ? 0 : 1; }
-    return v == 1;
-}
+static bool chain_enabled() { static const bool on = !env_flag("TTB_NO_CHAIN"); return on; }
 static int linear_resid_ln(ttb_engine* e, int kc, const __nv_bfloat16* A, int lda, const Lin& L, const Norm& n1, const Norm* n2,
                            float* x, __nv_bfloat16* xh, float* y, float* dst, __nv_bfloat16* dsth, RowCount rows, cudaStream_t s,
                            const Lin* chain = nullptr, __nv_bfloat16* q2 = nullptr, bool* chained = nullptr) {
@@ -359,11 +357,7 @@ static int linear_resid_ln(ttb_engine* e, int kc, const __nv_bfloat16* A, int ld
 
 // Feed-forward sub-layer  x <- LN2?(LN1(x + relu(x W1^T + b1) W2^T + b2)):  one fused kernel (hidden activations stay
 // on the SM) on the bf16 path with E = 256, FFN1 GEMM + (FFN2 GEMM + LN) otherwise.  TTB_NO_FUSED_FFN=1 disables it.
-static bool fused_ffn_enabled() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("TTB_NO_FUSED_FFN"); v = (e && e[0] == '1') ? 0 : 1; }
-    return v == 1;
-}
+static bool fused_ffn_enabled() { static const bool on = !env_flag("TTB_NO_FUSED_FFN"); return on; }
 static int ffn_block(ttb_engine* e, int kc1, int kc2, const Lin& L1, const Lin& L2, const Norm& n1, const Norm* n2, float* x, float* xh,
                      float* hid, float* y, float* dst, float* dsth, RowCount rows, cudaStream_t s) {
     if (linear<float>(e, kc1, x, L1.K, L1, hid, L1.N, rows, true, s)) return 1;
@@ -390,7 +384,7 @@ static int ffn_block_chained(ttb_engine* e, int kc, const __nv_bfloat16* att, co
     if (!(Lo.N == 256 && Lo.K == 256 && L2.N == 256 && L1.K == 256 && L1.N % 256 == 0 && L1.N <= 4096 && fused_ffn_enabled() && fused_ln_enabled() &&
           chain_enabled() && ffn_pair_available(rows.max_rows)))
         return -1;
-    static const bool off = [] { const char* v = getenv("TTB_NO_FFN_CHAIN"); return v && v[0] == '1'; }();
+    static const bool off = env_flag("TTB_NO_FFN_CHAIN");
     if (off) return -1;
     Scope sc(e, kc, s);
     return launch_ffn_fused(xh, L1.wh, L1.b, L2.wh, L2.b, x, n1.g, n1.b, n2 ? n2->g : nullptr, n2 ? n2->b : nullptr, rows, L1.N, s, att, Lo.wh, Lo.b,
@@ -399,11 +393,7 @@ static int ffn_block_chained(ttb_engine* e, int kc, const __nv_bfloat16* att, co
 
 // Attention dispatch: fp32 path -> SIMT kernels (exact), bf16 path -> tensor-core kernels
 // (TTB_ATTN_SIMT=1 forces the SIMT kernels for A/B comparisons).
-static bool attn_simt_forced() {
-    static int v = -1;
-    if (v < 0) { const char* e = getenv("TTB_ATTN_SIMT"); v = (e && e[0] == '1') ? 1 : 0; }
-    return v == 1;
-}
+static bool attn_simt_forced() { static const bool on = env_flag("TTB_ATTN_SIMT"); return on; }
 static void attn(const float* q, int q_ld, const float* k, const float* v, int kv_ld, float* out, int out_ld, int ng, const int* ng_dev,
                  int Lq, int Lk, long long kvs, const int* kvmap, const int* key_tok, int kts, int pad, bool causal, int H, int HD, cudaStream_t s,
                  const int* lk_dev = nullptr, const int* = nullptr, const int4* = nullptr) {
@@ -461,15 +451,15 @@ static size_t enc_work_bytes(const ttb_engine* e, long long T) {
     const long long E = e->E(), F = e->d.feedforward_dim;
     const long long elems[6] = {T * E * 4, Prec<ActT>::lowp ? T * E * (long long)sizeof(ActT) : 0, T * E * 4, T * 3 * E * (long long)sizeof(ActT),
                                 T * E * (long long)sizeof(ActT), T * F * (long long)sizeof(ActT)};
-    size_t n = 0;
-    for (long long b : elems) n += (size_t)(b + 255) / 256 * 256;
-    return n;
+    Arena a;
+    for (long long b : elems) a.take((size_t)b);
+    return a.bytes;
 }
 template <typename ActT>
 static EncWork<ActT> enc_work_carve(const ttb_engine* e, long long T, void* base) {
     const long long E = e->E(), F = e->d.feedforward_dim;
-    char* p = static_cast<char*>(base);
-    auto take = [&](long long bytes) { char* q = p; p += (bytes + 255) / 256 * 256; return q; };
+    Arena a;
+    auto take = [&](long long bytes) { return static_cast<char*>(base) + a.take((size_t)bytes); };
     EncWork<ActT> w;
     w.x = reinterpret_cast<float*>(take(T * E * 4));
     w.xh = Prec<ActT>::lowp ? reinterpret_cast<ActT*>(take(T * E * sizeof(ActT))) : nullptr;
@@ -639,6 +629,41 @@ static int encode_batch(ttb_engine* e, const int64_t* src, int B, int Ls, int* s
     return cross_kv_impl<ActT>(e, mem, memh, (int)TS, kv, s, kv_layer_stride);
 }
 
+// Buffers of a decoding loop that depend on the source length are sized for a rounded-up capacity: batches of different
+// length must not reallocate (cudaFree synchronises the whole device, i.e. every other engine decoding on this GPU as well)
+// nor invalidate the captured graph.
+static int ls_capacity(int Ls) { return std::max(256, (Ls + 63) / 64 * 64); }
+
+// Buffers of encode_batch: the encoder products of TS_enc source tokens, source lengths of B queries, and the
+// cross-attention K/V of TS_kv source tokens in every decoder layer.
+template <typename ActT>
+static int ensure_encoder(ttb_engine* e, long long TS_enc, int B, long long TS_kv) {
+    const int E = e->E();
+    if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float)) || e->srclen.ensure((size_t)B * sizeof(int))) return 1;
+    if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
+    return e->crosskv.ensure(TS_kv * 2 * E * sizeof(ActT) * e->dec.size());
+}
+
+// Vocabulary projection of the decoder rows and the per-row reduction a loop reads.  bf16 path with `use_fused`:
+// fused_launch(xh), a tcgen05 kernel that keeps the logits in tensor memory (0 taken, < 0 refused, > 0 error).  Otherwise,
+// or when it refuses, the logits GEMM into `logits` and fallback(logits).
+template <typename ActT, typename Fused, typename Fallback>
+static int classifier_head(ttb_engine* e, RowCount rows, bool use_fused, Fused fused_launch, Fallback fallback, float* logits, cudaStream_t s) {
+    if constexpr (Prec<ActT>::lowp) {
+        if (use_fused) {
+            Scope sc(e, KC_GEMM_CLASSIFIER, s);
+            const int rc = fused_launch(e->xh.as<ActT>());
+            if (rc >= 0) return rc > 0 ? 1 : 0;
+            e->launches--;   // refused: nothing was launched
+        }
+    }
+    const ActT* a = a_view<ActT>(e->x.as<float>(), Prec<ActT>::lowp ? e->xh.as<ActT>() : nullptr);
+    if (linear<float>(e, KC_GEMM_CLASSIFIER, a, e->E(), e->classifier, logits, e->d.tgt_vocab_size, rows, false, s)) return 1;
+    Scope sc(e, KC_ARGMAX, s);
+    fallback(logits);
+    return 0;
+}
+
 // The decoding loops run on the engine's own stream (graph capture is not allowed on the legacy default stream), ordered
 // after the caller's stream and drained before they return.
 static int join_caller_stream(ttb_engine* e, cudaStream_t user_stream) {
@@ -702,13 +727,12 @@ struct Staging {
         TTB_CHECK((2 * E * sizeof(ActT)) % 16 == 0, "continuous batching needs 16-byte cross-attention K/V rows");
         slots = B;
         Ls_cap = Ls_cap_;
-        size_t off = 0;
-        auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-        const size_t o_sg = take((size_t)B * 4), o_sq = take((size_t)B * 4), o_as = take((size_t)B * 4), o_gr = take((size_t)cb->n * sizeof(G));
-        const size_t o_sl = take((size_t)B_stage * 4), o_kv = take(e->dec.size() * TS_stage * 2 * E * sizeof(ActT));
+        Arena a;
+        const size_t o_sg = a.take((size_t)B * 4), o_sq = a.take((size_t)B * 4), o_as = a.take((size_t)B * 4), o_gr = a.take((size_t)cb->n * sizeof(G));
+        const size_t o_sl = a.take((size_t)B_stage * 4), o_kv = a.take(e->dec.size() * TS_stage * 2 * E * sizeof(ActT));
         std::vector<size_t> o_extra;
-        for (const auto& x : extra) o_extra.push_back(take(x.second));
-        if (e->cb.ensure(off) || e->cb_work.ensure(enc_work_bytes<ActT>(e, TS_stage)) || e->keytok32.ensure((size_t)B * Ls_cap * sizeof(int))) return 1;
+        for (const auto& x : extra) o_extra.push_back(a.take(x.second));
+        if (e->cb.ensure(a.bytes) || e->cb_work.ensure(enc_work_bytes<ActT>(e, TS_stage)) || e->keytok32.ensure((size_t)B * Ls_cap * sizeof(int))) return 1;
         char* base = e->cb.as<char>();
         t.slots = SlotTable{(int*)(base + o_sg), (int*)(base + o_sq), (int*)(base + o_as)};
         t.groups = (G*)(base + o_gr);
@@ -735,6 +759,17 @@ struct Staging {
         TTB_CHECK(e->alloc_signature() == sig0, "a workspace buffer moved while a continuous decoding loop was running");
         return 0;
     }
+    // Admits the next batches, whole and in list order, while `free_slots` suffice; admit(i) is the loop's admission of
+    // batch i.  Adds the queries admitted to *n_admitted.
+    int next = 0;
+    template <typename Admit>
+    int admit_fitting(int free_slots, int* n_admitted, Admit admit) {
+        while (next < cb->n && free_slots - *n_admitted >= cb->bs[next]) {
+            if (int rc = admit(next)) return rc;
+            *n_admitted += cb->bs[next++];
+        }
+        return 0;
+    }
 };
 
 // Per-batch records of a continuous loop that has drained: every batch must have been admitted whole and closed.
@@ -748,37 +783,37 @@ static int read_groups(const BatchList* cb, const G* dev, std::vector<G>& groups
 }
 
 // Sampling decoding (ttb_sample_generate, DESIGN.md section 15): S sample slots per source, drawn with temperature T from
-// the top_k largest logits (0: all) under the per-source keys of `seed`.
+// the top_k largest logits (0: all) under the per-source keys of `seed`.  The defaults stand for one slot per query.
 struct SampleCfg {
-    int S;
-    float temperature;
-    int top_k;
-    unsigned long long seed;
+    int S = 1;
+    float temperature = 1.f;
+    int top_k = 0;
+    unsigned long long seed = 0;
 };
 
-// Speculative greedy loop, and with `standard` the standard greedy decoding (no drafts).  With `cb` the loop is the
-// continuous one: B is the number of query slots, Ls the longest source of all batches, and the batches of `cb` are
-// admitted into free slots between two graph launches.  With `smp` (and `standard`) the loop is the sampling decoding:
-// B is the number of sample slots (sources x S), slot b * S + s is sample s of source b, and the draw replaces the arg-max.
+// The decodings greedy_api runs: speculative greedy decoding; the standard greedy decoding, the same KV-cached loop with one
+// row per query and no draft tokens (standard_decoding.py); sampling, the standard loop with a draw in place of the arg-max.
+enum class GreedyMode : int { speculative = 0, standard = 1, sampling = 2 };
+
+// With `cb` the loop is the continuous one: B is the number of query slots, Ls the longest source of all batches, and the
+// batches of `cb` are admitted into free slots between two graph launches.  Sampling: B is the number of sample slots
+// (sources x smp.S), slot b * S + s is sample s of source b.
 template <typename ActT>
 static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int max_len, int draft_len, int N,
                       int pad, int bos, int eos, int replace, int tie_break, int64_t* out_dev, int32_t* trace_dev,
-                      ttb_generate_stats* stats, cudaStream_t user_stream, bool standard = false, const BatchList* cb = nullptr,
-                      const SampleCfg* smp = nullptr) {
+                      ttb_generate_stats* stats, cudaStream_t user_stream, GreedyMode mode, const BatchList* cb = nullptr,
+                      const SampleCfg& smp = SampleCfg{}) {
     const int E = e->E(), H = e->d.num_heads, HD = e->HD(), V = e->d.tgt_vocab_size;
     const int n_dec = (int)e->dec.size();
     cudaStream_t s = e->stream;
     if (int rc = join_caller_stream(e, user_stream)) return rc;
-    // speculative: make_drafts(min_draft_len=1, max_draft_len=max_len); standard greedy decoding (standard_decoding.py)
-    // is the same KV-cached loop with one row per query and no draft tokens
+    const bool standard = mode != GreedyMode::speculative, sampling = mode == GreedyMode::sampling;
+    // speculative: make_drafts(min_draft_len=1, max_draft_len=max_len)
     const int D = standard ? 0 : std::min(std::max(1, draft_len), max_len);
     if (standard) N = 1;
-    // buffers that depend on the source length are sized for a rounded-up capacity so that batches of
-    // different length neither reallocate nor invalidate the captured graph
-    const int Ls_cap = std::max(256, (Ls + 63) / 64 * 64);
+    const int Ls_cap = ls_capacity(Ls);
     // sampling: the encoder and the cross-attention K/V run once per source, shared by its S slots
-    const bool sampling = smp != nullptr;
-    const int S = sampling ? smp->S : 1, B_src = B / S;
+    const int S = smp.S, B_src = B / S;
     const long long TS_cap = (long long)B_src * Ls_cap;
     const int per_q = N * (D + 1);
     const long long T = (long long)B * per_q;
@@ -790,12 +825,9 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     // launches ahead of the control words it reads, i.e. a few no-op iterations per admission
     const long long max_iters = cont ? (long long)cb->n * (max_len + 1) + (long long)(cb->n + 1) * 3 * 16 : max_len + 1;
     Staging<ActT> sg(cb);
-    const long long TS_enc = cont ? sg.TS_stage : TS_cap;
 
     // encoder + cross-attention K/V (computed once per query, not once per draft row and iteration)
-    if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float)) || e->srclen.ensure((size_t)B * sizeof(int))) return 1;
-    if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
-    if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
+    if (ensure_encoder<ActT>(e, cont ? sg.TS_stage : TS_cap, B, TS_cap)) return 1;
     const size_t cache_bytes = (size_t)n_dec * B * P * E * sizeof(ActT);
     if (e->kcache.ensure(cache_bytes) || e->vcache.ensure(cache_bytes)) return 1;
     if (e->drafts.ensure((size_t)B * N * D * sizeof(int)) || e->gen.ensure((size_t)B * gen_ld * sizeof(int))) return 1;
@@ -812,9 +844,9 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
         sl.xdesc = reinterpret_cast<int4*>(e->smp.as<char>() + ((size_t)B_src * 8 + 15) / 16 * 16);
         sl.kvsrc = reinterpret_cast<int*>(sl.xdesc + B);
     }
-    // the draw's fused / fallback choice is read per call (part of the graph key), so that one process can compare both
-    const char* nfa = sampling ? getenv("TTB_NO_FUSED_ARGMAX") : nullptr;
-    const bool smp_fused = sampling && Prec<ActT>::lowp && !(nfa && nfa[0] == '1');
+    // the fused / fallback classifier (arg-max or draw) is chosen per call and is part of the graph key, so that one process
+    // can compare both
+    const bool use_fused = Prec<ActT>::lowp && !env_flag("TTB_NO_FUSED_ARGMAX");
     // continuous loop: slot / batch tables, staging of an admitted batch (drafts as well)
     CbTable cbt{};
     int* stage_drafts = nullptr;
@@ -851,16 +883,16 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     if (cont) {
         TTB_CUDA_OK(cudaMemsetAsync(st.ctrl, 0, CTRL_COUNT * sizeof(int), s));
     } else {
-    if (encode_batch<ActT>(e, src_dev, B_src, Ls, e->srclen.as<int>(), crosskv, TS_cap * 2 * E, s)) return 1;
-    // drafts from the source without its BOS column (speculative_decoding.py:64-73)
-    if (!standard) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Ls, B, Ls - 1, D, N, eos, pad, replace, e->drafts.as<int>(), s); }
-    if (sampling) {
-        { Scope sc(e, KC_MISC, s); launch_sample_keys(src32, B_src, Ls, e->d.src_pad_token_idx, smp->seed, smp_keys, s); }
-        { Scope sc(e, KC_MISC, s); launch_sample_init(st, sl, s); }
-    } else {
-        Scope sc(e, KC_MISC, s);
-        launch_greedy_init(st, s);
-    }
+        if (encode_batch<ActT>(e, src_dev, B_src, Ls, e->srclen.as<int>(), crosskv, TS_cap * 2 * E, s)) return 1;
+        // drafts from the source without its BOS column (speculative_decoding.py:64-73)
+        if (!standard) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32 + 1, Ls, B, Ls - 1, D, N, eos, pad, replace, e->drafts.as<int>(), s); }
+        if (sampling) {
+            { Scope sc(e, KC_MISC, s); launch_sample_keys(src32, B_src, Ls, e->d.src_pad_token_idx, smp.seed, smp_keys, s); }
+            { Scope sc(e, KC_MISC, s); launch_sample_init(st, sl, s); }
+        } else {
+            Scope sc(e, KC_MISC, s);
+            launch_greedy_init(st, s);
+        }
     }
 
     float* x = e->x.as<float>();
@@ -882,20 +914,16 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
                                          att, E, Bq, n_active, st.active, st.front, st.gen, gen_ld, e->d.tgt_pad_token_idx,
                                          N, D, H, HD, P, s, st.desc);
     };
+    // cross-attention K/V rows and key tokens: per query, for sampling those of the slot's source (generate()), or slot-major
+    // with Ls_cap (= CTRL_LS) rows per slot (continuous loop)
+    const int kv_ls = cont ? Ls_cap : Ls;
+    const int* kv_map = sampling ? sl.kvsrc : st.active;
+    const int* key_tok = cont ? e->keytok32.as<int>() : src32;
+    const int4* cross_desc = sampling ? sl.xdesc : st.desc;
     auto cross_attn = [&](int l, ActT* q2, ActT* att) {
         const ActT* kv = crosskv + (long long)l * TS_cap * 2 * E;
-        if (cont) {   // slot-major K/V rows and key tokens, row stride Ls_cap (= CTRL_LS) per slot
-            attn(q2, E, kv, kv + E, 2 * E, att, E, Bq, n_active, per_q, Ls_cap, Ls_cap, st.active, e->keytok32.as<int>(), Ls_cap,
-                 e->d.src_pad_token_idx, false, H, HD, s, st.ctrl + CTRL_LS, e->srclen.as<int>(), st.desc);
-            return;
-        }
-        if (sampling) {   // the K/V rows of the slot's source, not of the slot
-            attn(q2, E, kv, kv + E, 2 * E, att, E, Bq, n_active, per_q, Ls, Ls, sl.kvsrc, src32, Ls, e->d.src_pad_token_idx, false, H, HD, s,
-                 st.ctrl + CTRL_LS, e->srclen.as<int>(), sl.xdesc);
-            return;
-        }
-        attn(q2, E, kv, kv + E, 2 * E, att, E, Bq, n_active, per_q, Ls, Ls, st.active,
-             src32, Ls, e->d.src_pad_token_idx, false, H, HD, s, st.ctrl + CTRL_LS, e->srclen.as<int>(), st.desc);
+        attn(q2, E, kv, kv + E, 2 * E, att, E, Bq, n_active, per_q, kv_ls, kv_ls, kv_map, key_tok, kv_ls, e->d.src_pad_token_idx, false, H,
+             HD, s, st.ctrl + CTRL_LS, e->srclen.as<int>(), cross_desc);
     };
 
     auto enqueue_iteration = [&]() -> int {
@@ -909,54 +937,28 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
         }
         if (decoder_stack<ActT>(e, rows, n_dec, qkv_l_stride, self_attn, cross_attn, s)) return 1;
         if (sampling) {
-            const SampleArgs sa{st.desc, smp_keys, S, smp->temperature, smp->top_k, st.pred};
-            bool fused = false;
-            if constexpr (Prec<ActT>::lowp) {
-                if (smp_fused) {
-                    Scope sc(e, KC_GEMM_CLASSIFIER, s);
-                    const int rc = launch_classifier_sample(xh, E, e->classifier.wh, e->classifier.b, rows, V, E, sa, s);
-                    if (rc > 0) return 1;
-                    fused = rc == 0;
-                    if (!fused) e->launches--;
-                }
-            }
-            if (!fused) {
-                if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, e->logits.as<float>(), V, rows, false, s)) return 1;
-                Scope sc(e, KC_ARGMAX, s);
-                launch_sample_rows(e->logits.as<float>(), V, V, rows, sa, s);
-            }
+            const SampleArgs sa{st.desc, smp_keys, S, smp.temperature, smp.top_k, st.pred};
+            auto fused = [&](const auto* a) { return launch_classifier_sample(a, E, e->classifier.wh, e->classifier.b, rows, V, E, sa, s); };
+            auto fallback = [&](const float* lg) { launch_sample_rows(lg, V, V, rows, sa, s); };
+            if (classifier_head<ActT>(e, rows, use_fused, fused, fallback, e->logits.as<float>(), s)) return 1;
             Scope sc(e, KC_ACCEPT, s);
             launch_sample_step(st, sl, s);
             return 0;
         }
-        bool fused_cls = false;
-        if constexpr (Prec<ActT>::lowp) {
-            static const bool off = [] { const char* v = getenv("TTB_NO_FUSED_ARGMAX"); return v && v[0] == '1'; }();
-            if (!off) {
-                Scope sc(e, KC_GEMM_CLASSIFIER, s);
-                const int rc = launch_classifier_argmax(xh, E, e->classifier.wh, e->classifier.b, st.pred, rows, V, E, s);
-                if (rc > 0) return 1;
-                fused_cls = rc == 0;
-                if (!fused_cls) e->launches--;
-            }
-        }
-        if (!fused_cls) {
-            if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, e->logits.as<float>(), V, rows, false, s)) return 1;
-            { Scope sc(e, KC_ARGMAX, s); launch_argmax_rows(e->logits.as<float>(), V, V, st.pred, rows, s); }
-        }
-        {
-            Scope sc(e, KC_ACCEPT, s);
-            if (standard && cont) { if (launch_greedy_std_step_groups(st, cbt, s)) return 1; }
-            else if (standard) launch_greedy_std_step(st, s);
-            else if (cont) launch_greedy_accept_groups(st, cbt, s);
-            else launch_greedy_accept(st, s);
-        }
+        auto fused = [&](const auto* a) { return launch_classifier_argmax(a, E, e->classifier.wh, e->classifier.b, st.pred, rows, V, E, s); };
+        auto fallback = [&](const float* lg) { launch_argmax_rows(lg, V, V, st.pred, rows, s); };
+        if (classifier_head<ActT>(e, rows, use_fused, fused, fallback, e->logits.as<float>(), s)) return 1;
+        Scope sc(e, KC_ACCEPT, s);
+        if (standard && cont) return launch_greedy_std_step_groups(st, cbt, s) ? 1 : 0;
+        if (standard) launch_greedy_std_step(st, s);
+        else if (cont) launch_greedy_accept_groups(st, cbt, s);
+        else launch_greedy_accept(st, s);
         return 0;
     };
 
     // One decoding iteration is a fixed kernel sequence on fixed buffers (all sizes that change while
     // decoding live in device memory), so it is captured once into a CUDA graph and replayed.
-    static const bool no_graph = [] { const char* v = getenv("TTB_NO_GRAPH"); return v && v[0] == '1'; }();
+    static const bool no_graph = env_flag("TTB_NO_GRAPH");
     bool traced = trace_dev != nullptr;
     if (cont && cb->trace)
         for (int i = 0; i < cb->n; ++i) traced |= cb->trace[i] != nullptr;
@@ -970,7 +972,7 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     int bucket_q[ttb_engine::kBuckets];
     int n_buckets = 0;
     {
-        static const bool no_buckets = [] { const char* v = getenv("TTB_NO_BUCKETS"); return v && v[0] == '1'; }();
+        static const bool no_buckets = env_flag("TTB_NO_BUCKETS");
         int cand[ttb_engine::kBuckets];
         for (int i = 0; i < 8; ++i) cand[i] = (B * (8 - i) + 7) / 8;      // B, 7B/8, ... B/8
         cand[8] = (B + 15) / 16;
@@ -978,17 +980,17 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
         for (int i = 0; i < ttb_engine::kBuckets; ++i) {
             // generate() of the standard greedy decoding keeps every row to the end; its continuous loop sheds stopped batches
             // and sampling retires every slot on its own
-            if (i > 0 && (no_buckets || (standard && !cont && !sampling))) break;
+            if (i > 0 && (no_buckets || (mode == GreedyMode::standard && !cont))) break;
             if (n_buckets == 0 || (cand[i] >= 1 && cand[i] < bucket_q[n_buckets - 1])) bucket_q[n_buckets++] = cand[i];
         }
     }
     if (use_graph) {
-        // sampling: everything a call may change that the captured kernels take by value (the keys are in device memory)
+        // everything a call may change that the captured kernels take by value (the sampling keys are in device memory)
         uint32_t t_bits = 0;
-        if (sampling) memcpy(&t_bits, &smp->temperature, 4);
-        const long long key[17] = {B, N, D, (standard ? 1 : 0) + (cont ? 2 : 0) + (sampling ? 4 : 0), max_len, pad, bos, eos, tie_break,
-                                   e->alloc_signature(), (long long)sizeof(ActT) + 16 * K_it, replace, cont ? Ls_cap : 0, sampling ? S : 0,
-                                   (long long)t_bits, sampling ? smp->top_k : -1, smp_fused ? 1 : 0};
+        memcpy(&t_bits, &smp.temperature, 4);
+        const long long key[17] = {B, N, D, (long long)mode + (cont ? 4 : 0), max_len, pad, bos, eos, tie_break,
+                                   e->alloc_signature(), (long long)sizeof(ActT) + 16 * K_it, replace, cont ? Ls_cap : 0, S,
+                                   (long long)t_bits, smp.top_k, use_fused ? 1 : 0};
         if (memcmp(key, e->graph_key, sizeof(key)) != 0) {
             for (auto& gb : e->graph_exec) for (auto& g : gb) if (g) { cudaGraphExecDestroy(g); g = nullptr; }
             memcpy(e->graph_key, key, sizeof(key));
@@ -1024,62 +1026,71 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
     // to `it` are already queued, so the GPU never waits for it.
     constexpr int RING = 4;
     const int LAG = K_it > 1 ? 1 : 2;   // launches (of K_it iterations each) the host stays ahead of the control words it reads
-    if (cont) {
-        // Continuous loop.  `bound` is an upper bound of the live slots of every iteration enqueued from now on: the count of
-        // the newest control words read plus every query admitted after the launch they belong to (the device only retires
-        // queries).  It picks the bucket -- a bucket below the true live count would drop queries -- and B - bound is a
-        // lower bound of the free slots: a batch is admitted at a graph boundary once they suffice.
-        long long admitted = 0, adm_at[RING] = {};
-        long long iters_enq = 0;
-        int next = 0, bound = 0, it = 0;
-        while (true) {
-            while (next < cb->n && B - bound >= cb->bs[next]) {
-                if (admit(next)) return 1;
-                bound += cb->bs[next];
-                admitted += cb->bs[next];
-                ++next;
-            }
-            if (bound == 0) break;   // nothing live and nothing pending (every batch fits the slots)
-            TTB_CHECK(iters_enq < max_iters, "continuous decoding loop did not terminate within max_len + 1 iterations per batch");
-            const int known_live = std::max(1, bound);
-            int bi = 0;
-            while (bi + 1 < n_buckets && bucket_q[bi + 1] >= known_live) ++bi;
-            Bq = bucket_q[bi];
-            if (use_graph) {
-                const int sh = (known_live < B && K_short < K_it) ? 1 : 0;
-                if (graph_for(bi, sh)) return 1;
-                TTB_CUDA_OK(cudaGraphLaunch(e->graph_exec[bi][sh], s));
-                e->launches += e->graph_launches * (sh ? K_short : K_it);
-                iters_enq += sh ? K_short : K_it;
-            } else if (enqueue_iteration()) {
-                return 1;
-            } else {
-                ++iters_enq;
-            }
-            TTB_CUDA_OK(cudaMemcpyAsync(e->h_ctrl + (it % RING) * CTRL_COUNT, st.ctrl, CTRL_COUNT * sizeof(int), cudaMemcpyDeviceToHost, s));
-            TTB_CUDA_OK(cudaEventRecord(e->poll_ev[it % RING], s));
-            adm_at[it % RING] = admitted;
-            if (it >= LAG) {
-                const int j = (it - LAG) % RING;
-                TTB_CUDA_OK(cudaEventSynchronize(e->poll_ev[j]));
-                const int* cj = e->h_ctrl + j * CTRL_COUNT;
-                TTB_CHECK(cj[CTRL_ERROR] != 3, "continuous batching admitted a batch without enough free slots");
-                const int live = cj[CTRL_DONE] ? 0 : cj[CTRL_N_ACTIVE];
-                bound = std::min(bound, live + (int)(admitted - adm_at[j]));
-            }
-            ++it;
+    // `bound` is an upper bound of the live queries of every iteration enqueued from now on: the count of the newest control
+    // words read plus every query admitted after the launch they belong to (the device only retires queries).  It picks the
+    // bucket -- a bucket below the true live count would drop queries.  Continuous loop: B - bound is a lower bound of the
+    // free slots, a batch is admitted at a graph boundary once they suffice.  One batch: nothing is admitted, the loop ends
+    // when the device has raised CTRL_DONE, and a live count of 0 read without it counts as 1.
+    long long admitted = 0, adm_at[RING] = {};
+    long long iters_enq = 0;
+    int bound = cont ? 0 : B, it = 0;
+    while (true) {
+        if (cont) {
+            int n = 0;
+            if (sg.admit_fitting(B - bound, &n, admit)) return 1;
+            bound += n;
+            admitted += n;
         }
-        TTB_CUDA_OK(cudaMemcpyAsync(e->h_ctrl, st.ctrl, CTRL_COUNT * sizeof(int), cudaMemcpyDeviceToHost, s));
-        float ms = 0.f;
-        if (int rc = finish_loop(e, ms)) return rc;
-        const int* c = e->h_ctrl;
+        if (bound == 0) break;   // done, or (continuous) nothing live and nothing pending: every batch fits the slots
+        if (iters_enq >= max_iters) {
+            TTB_CHECK(!cont, "continuous decoding loop did not terminate within max_len + 1 iterations per batch");
+            break;
+        }
+        int bi = 0;
+        while (bi + 1 < n_buckets && bucket_q[bi + 1] >= bound) ++bi;
+        Bq = bucket_q[bi];
+        if (use_graph) {
+            const int sh = (bound < B && K_short < K_it) ? 1 : 0;
+            if (graph_for(bi, sh)) return 1;
+            TTB_CUDA_OK(cudaGraphLaunch(e->graph_exec[bi][sh], s));
+            e->launches += e->graph_launches * (sh ? K_short : K_it);
+            iters_enq += sh ? K_short : K_it;
+        } else if (enqueue_iteration()) {
+            return 1;
+        } else {
+            ++iters_enq;
+        }
+        TTB_CUDA_OK(cudaMemcpyAsync(e->h_ctrl + (it % RING) * CTRL_COUNT, st.ctrl, CTRL_COUNT * sizeof(int), cudaMemcpyDeviceToHost, s));
+        TTB_CUDA_OK(cudaEventRecord(e->poll_ev[it % RING], s));
+        adm_at[it % RING] = admitted;
+        if (it >= LAG) {
+            const int j = (it - LAG) % RING;
+            TTB_CUDA_OK(cudaEventSynchronize(e->poll_ev[j]));
+            const int* cj = e->h_ctrl + j * CTRL_COUNT;
+            TTB_CHECK(cj[CTRL_ERROR] != 3, "continuous batching admitted a batch without enough free slots");
+            const int live = cj[CTRL_DONE] ? 0 : (cont ? cj[CTRL_N_ACTIVE] : std::max(1, cj[CTRL_N_ACTIVE]));
+            bound = std::min(bound, live + (int)(admitted - adm_at[j]));
+        }
+        ++it;
+    }
+    if (!cont) TTB_CUDA_OK(cudaMemcpyAsync(out_dev, st.out, (size_t)B * max_len * sizeof(long long), cudaMemcpyDeviceToDevice, s));
+    TTB_CUDA_OK(cudaMemcpyAsync(e->h_ctrl, st.ctrl, CTRL_COUNT * sizeof(int), cudaMemcpyDeviceToHost, s));
+    float ms = 0.f;
+    if (int rc = finish_loop(e, ms)) return rc;
+    const int* c = e->h_ctrl;
+    std::vector<CbGroup> groups;
+    if (cont) {
         TTB_CHECK(c[CTRL_ERROR] != 3, "continuous batching admitted a batch without enough free slots");
         TTB_CHECK(c[CTRL_DONE] == 1 && c[CTRL_N_ACTIVE] == 0, "continuous decoding loop ended with live queries");
-        std::vector<CbGroup> groups;
         if (int rc = read_groups(cb, cbt.groups, groups)) return rc;
-        e->h_hist.assign((size_t)c[CTRL_ITERS], 0);
-        if (c[CTRL_ITERS] > 0)
-            TTB_CUDA_OK(cudaMemcpy(e->h_hist.data(), st.hist, (size_t)c[CTRL_ITERS] * sizeof(int), cudaMemcpyDeviceToHost));
+    } else {
+        TTB_CHECK(c[CTRL_DONE] == 1, "greedy decoding loop did not terminate within max_len + 1 iterations");
+    }
+    e->h_hist.assign((size_t)c[CTRL_ITERS], 0);
+    if (c[CTRL_ITERS] > 0)
+        TTB_CUDA_OK(cudaMemcpy(e->h_hist.data(), st.hist, (size_t)c[CTRL_ITERS] * sizeof(int), cudaMemcpyDeviceToHost));
+    auto ref_error = [](int err) { return err == 1 ? TTB_ERR_REF_INDEX : (err == 2 ? TTB_ERR_REF_SHAPE : 0); };
+    if (cont) {   // per-batch records
         ttb_generate_stats sum{};
         for (int i = 0; i < cb->n; ++i) {
             const CbGroup& g = groups[(size_t)i];
@@ -1089,7 +1100,7 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
             o.accepted_tokens = g.accepted;
             o.produced_tokens = g.tokens;
             o.unfinished = g.n_left;
-            o.error = g.error == 1 ? TTB_ERR_REF_INDEX : (g.error == 2 ? TTB_ERR_REF_SHAPE : 0);
+            o.error = ref_error(g.error);
             sum.accepted_tokens += g.accepted;
             sum.produced_tokens += g.tokens;
             sum.unfinished += g.n_left;
@@ -1102,49 +1113,12 @@ static int greedy_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int 
         }
         return 0;
     }
-    int it = 0, iters_enq = 0;
-    bool done = false;
-    int known_live = B;                 // live queries in the newest control words read: an upper bound from then on
-    while (!done && iters_enq < max_iters) {
-        int bi = 0;
-        while (bi + 1 < n_buckets && bucket_q[bi + 1] >= known_live) ++bi;
-        Bq = bucket_q[bi];
-        if (use_graph) {
-            const int sh = (known_live < B && K_short < K_it) ? 1 : 0;
-            if (graph_for(bi, sh)) return 1;
-            TTB_CUDA_OK(cudaGraphLaunch(e->graph_exec[bi][sh], s));
-            e->launches += e->graph_launches * (sh ? K_short : K_it);
-            iters_enq += sh ? K_short : K_it;
-        } else if (enqueue_iteration()) {
-            return 1;
-        } else {
-            ++iters_enq;
-        }
-        TTB_CUDA_OK(cudaMemcpyAsync(e->h_ctrl + (it % RING) * CTRL_COUNT, st.ctrl, CTRL_COUNT * sizeof(int), cudaMemcpyDeviceToHost, s));
-        TTB_CUDA_OK(cudaEventRecord(e->poll_ev[it % RING], s));
-        if (it >= LAG) {
-            const int j = (it - LAG) % RING;
-            TTB_CUDA_OK(cudaEventSynchronize(e->poll_ev[j]));
-            if (e->h_ctrl[j * CTRL_COUNT + CTRL_DONE]) done = true;
-            else known_live = std::min(known_live, std::max(1, e->h_ctrl[j * CTRL_COUNT + CTRL_N_ACTIVE]));
-        }
-        ++it;
-    }
-    TTB_CUDA_OK(cudaMemcpyAsync(out_dev, st.out, (size_t)B * max_len * sizeof(long long), cudaMemcpyDeviceToDevice, s));
-    TTB_CUDA_OK(cudaMemcpyAsync(e->h_ctrl, st.ctrl, CTRL_COUNT * sizeof(int), cudaMemcpyDeviceToHost, s));
-    float ms = 0.f;
-    if (int rc = finish_loop(e, ms)) return rc;
-    const int* c = e->h_ctrl;
-    TTB_CHECK(c[CTRL_DONE] == 1, "greedy decoding loop did not terminate within max_len + 1 iterations");
-    e->h_hist.assign((size_t)c[CTRL_ITERS], 0);
-    if (c[CTRL_ITERS] > 0)
-        TTB_CUDA_OK(cudaMemcpy(e->h_hist.data(), st.hist, (size_t)c[CTRL_ITERS] * sizeof(int), cudaMemcpyDeviceToHost));
     if (stats) {
         stats->model_calls = c[CTRL_ITERS];
         stats->accepted_tokens = c[CTRL_ACCEPTED];
         stats->produced_tokens = c[CTRL_TOKENS];
         stats->unfinished = c[CTRL_N_LEFT];
-        stats->error = c[CTRL_ERROR] == 1 ? TTB_ERR_REF_INDEX : (c[CTRL_ERROR] == 2 ? TTB_ERR_REF_SHAPE : 0);
+        stats->error = ref_error(c[CTRL_ERROR]);
         stats->gpu_launches = (int32_t)(e->launches - launches0);
         stats->gpu_ms = ms;
     }
@@ -1214,9 +1188,7 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     const int D_lib = std::min(std::max(5, D0 + 1), 200);
     const int n_lib = Ls - 5;
     if (smart) TTB_CHECK(n_lib > 0, "The number of drafts must be greater than 0");
-    // buffers that depend on the source length are sized for a rounded-up capacity: batches of different length must not
-    // reallocate (cudaFree synchronises the whole device, i.e. every other engine decoding on this GPU as well)
-    const int Ls_cap = std::max(256, (Ls + 63) / 64 * 64);
+    const int Ls_cap = ls_capacity(Ls);
     const long long TS_cap = (long long)B * Ls_cap;
     const int Cmax = B * K, Rmax = Cmax * N;
     const int ldw = max_len + D0 + 4;
@@ -1225,11 +1197,10 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     const bool cont = cb != nullptr;
     Staging<ActT> sg(cb);
     const long long Tc = (long long)Rmax * (D0 + 1);
+    // bf16 path: the statistics the search reads come from the fused classifier (TTB_NO_FUSED_STATS=1: GEMM + beam_stats)
+    const bool use_fused = Prec<ActT>::lowp && !env_flag("TTB_NO_FUSED_STATS");
 
-    const long long TS_enc = cont ? sg.TS_stage : TS_cap;
-    if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float)) || e->srclen.ensure((size_t)B * sizeof(int))) return 1;
-    if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
-    if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
+    if (ensure_encoder<ActT>(e, cont ? sg.TS_stage : TS_cap, B, TS_cap)) return 1;
     if (e->drafts.ensure(smart ? (size_t)B * std::max(n_lib, Ls_cap) * D_lib * sizeof(int) : (size_t)B * N * D0 * sizeof(int))) return 1;
     if (ensure_work<ActT>(e, cont ? Tc : std::max(Tc, TS_cap), n_dec)) return 1;
     const long long cache_c_stride = (long long)ldw * E, cache_l_stride = (long long)Cmax * ldw * E;
@@ -1237,19 +1208,18 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     if (e->kcache.ensure(cbytes) || e->vcache.ensure(cbytes) || e->kcache2.ensure(cbytes) || e->vcache2.ensure(cbytes)) return 1;
     DevBuf& bb = e->beam;
     // one arena for the small beam buffers
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-    const size_t o_cand0 = take((size_t)Cmax * ldw * 4), o_cand1 = take((size_t)Cmax * ldw * 4);
-    const size_t o_lp0 = take(Cmax * 4), o_lp1 = take(Cmax * 4);
-    const size_t o_slot = take(Cmax * 4), o_fin = take(Cmax * 4), o_base = take(Cmax * 4), o_nacc = take((size_t)Cmax * N * 4);
-    const size_t o_pick = take(Cmax * 4), o_acc = take(Cmax * 4), o_ctrl = take(32 * 4);   // control words + loop-control accumulators
+    Arena a;
+    const size_t o_cand0 = a.take((size_t)Cmax * ldw * 4), o_cand1 = a.take((size_t)Cmax * ldw * 4);
+    const size_t o_lp0 = a.take(Cmax * 4), o_lp1 = a.take(Cmax * 4);
+    const size_t o_slot = a.take(Cmax * 4), o_fin = a.take(Cmax * 4), o_base = a.take(Cmax * 4), o_nacc = a.take((size_t)Cmax * N * 4);
+    const size_t o_pick = a.take(Cmax * 4), o_acc = a.take(Cmax * 4), o_ctrl = a.take(32 * 4);   // control words + loop-control accumulators
     const size_t n_rp = (size_t)Rmax * (D0 + 1);
-    const size_t o_topv = take(n_rp * K * 4), o_topi = take(n_rp * K * 4), o_keep = take(n_rp * 4), o_max = take(n_rp * 4), o_sum = take(n_rp * 4);
-    const size_t o_lg = take(n_rp * V * 4), o_rt = take(n_rp * 4), o_tv = take(n_rp * 4);
-    const size_t o_lc = take(Rmax * 4), o_lq = take(Rmax * 4), o_cf = take(Cmax * 4), o_np = take(Cmax * 4), o_nk = take(Cmax * 4), o_nr = take(Cmax * 4);
-    const size_t o_tc = take(smart ? (size_t)B * V * 4 : 4), o_tl = take(smart ? (size_t)B * V * N * 4 : 4), o_cc = take(Cmax * 4),
-                 o_cl = take(Cmax * 4), o_rd = take(Rmax * 4), o_ds = take(Rmax * 16), o_dc = take(Rmax * 16);
-    if (bb.ensure(off)) return 1;
+    const size_t o_topv = a.take(n_rp * K * 4), o_topi = a.take(n_rp * K * 4), o_keep = a.take(n_rp * 4), o_max = a.take(n_rp * 4), o_sum = a.take(n_rp * 4);
+    const size_t o_lg = a.take(n_rp * V * 4), o_rt = a.take(n_rp * 4), o_tv = a.take(n_rp * 4);
+    const size_t o_lc = a.take(Rmax * 4), o_lq = a.take(Rmax * 4), o_cf = a.take(Cmax * 4), o_np = a.take(Cmax * 4), o_nk = a.take(Cmax * 4), o_nr = a.take(Cmax * 4);
+    const size_t o_tc = a.take(smart ? (size_t)B * V * 4 : 4), o_tl = a.take(smart ? (size_t)B * V * N * 4 : 4), o_cc = a.take(Cmax * 4),
+                 o_cl = a.take(Cmax * 4), o_rd = a.take(Rmax * 4), o_ds = a.take(Rmax * 16), o_dc = a.take(Rmax * 16);
+    if (bb.ensure(a.bytes)) return 1;
     char* base = bb.as<char>();
     // continuous loop: slot / batch tables, staging of an admitted batch (drafts or window library as well), smallest draft
     // length of every iteration
@@ -1271,6 +1241,9 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
     int* src32 = e->src32.as<int>();
     ActT* crosskv = e->crosskv.as<ActT>();
     const long long ckv_l_stride = TS_cap * 2 * E;
+    // cross-attention key tokens and K/V rows: per query (generate()) or slot-major with Ls_cap rows per slot (continuous loop)
+    const int kv_ls = cont ? Ls_cap : Ls;
+    const int* key_tok = cont ? e->keytok32.as<int>() : src32;
     if (!cont) {
         if (encode_batch<ActT>(e, src_dev, B, Ls, e->srclen.as<int>(), crosskv, ckv_l_stride, s)) return 1;
         if (smart) { Scope sc(e, KC_MISC, s); launch_make_drafts(src32, Ls, B, Ls, D_lib, n_lib, eos, pad, c_token, e->drafts.as<int>(), s); }
@@ -1343,7 +1316,6 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
         kc_cur = kc_set[parity]; kc_next = kc_set[parity ^ 1];
         vc_cur = vc_set[parity]; vc_next = vc_set[parity ^ 1];
         const int R = (smart && !cont ? C : std::min(C, std::max(1, Cb))) * N;
-        bool fused_stats = false;
         if (cont) { Scope sc(e, KC_MISC, s); launch_beam_prepare_groups(st, cbt, s); }
         else { Scope sc(e, KC_MISC, s); launch_beam_prepare(st, C, beam, dl, s); }
         RowCount rows(R * (dl + 1), n_live, dl + 1);
@@ -1359,29 +1331,17 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
         };
         auto cross_attn = [&](int l, ActT* q2, ActT* att) {
             const ActT* kv = crosskv + (long long)l * ckv_l_stride;
-            if (cont)   // slot-major K/V rows and key tokens, row stride Ls_cap per slot
-                attn(q2, E, kv, kv + E, 2 * E, att, E, G, n_live_cands, n_per_group * (dl + 1), Ls_cap, Ls_cap, st.live_query,
-                     e->keytok32.as<int>(), Ls_cap, e->d.src_pad_token_idx, false, H, HD, s, nullptr, nullptr, st.desc_cross);
-            else
-                attn(q2, E, kv, kv + E, 2 * E, att, E, G, n_live_cands, n_per_group * (dl + 1), Ls, Ls, st.live_query,
-                     src32, Ls, e->d.src_pad_token_idx, false, H, HD, s, nullptr, nullptr, st.desc_cross);
+            attn(q2, E, kv, kv + E, 2 * E, att, E, G, n_live_cands, n_per_group * (dl + 1), kv_ls, kv_ls, st.live_query, key_tok, kv_ls,
+                 e->d.src_pad_token_idx, false, H, HD, s, nullptr, nullptr, st.desc_cross);
         };
         if (decoder_stack<ActT>(e, rows, n_dec, Tc * 3 * E, self_attn, cross_attn, s)) return 1;
-        // every decoder row is a scored position.  bf16 path: the projection is fused with the statistics the search reads
-        // (logits stay in tensor memory); otherwise logits straight from the residual stream + beam_stats below
-        if constexpr (Prec<ActT>::lowp) {
-            const char* nf = getenv("TTB_NO_FUSED_STATS");
-            if (!(nf && nf[0] == '1')) {
-                Scope sc(e, KC_GEMM_CLASSIFIER, s);
-                const int rc = launch_classifier_stats(xh, E, e->classifier.wh, e->classifier.b, rows, V, E, K, st.row_tok, st.tokv, st.lmax, st.lsum,
-                                                       st.nkeep, st.topv, st.topi, s);
-                if (rc > 0) return 1;
-                fused_stats = rc == 0;
-                if (!fused_stats) e->launches--;
-            }
-        }
-        if (!fused_stats && linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, logits, V, rows, false, s)) return 1;
-        if (!fused_stats) { Scope sc(e, KC_ARGMAX, s); launch_beam_stats(st, logits, R, dl, s); }
+        // every decoder row is a scored position: the statistics the search reads (logits in tensor memory when fused)
+        auto fused = [&](const auto* a) {
+            return launch_classifier_stats(a, E, e->classifier.wh, e->classifier.b, rows, V, E, K, st.row_tok, st.tokv, st.lmax, st.lsum,
+                                           st.nkeep, st.topv, st.topi, s);
+        };
+        auto fallback = [&](const float* lg) { launch_beam_stats(st, lg, R, dl, s); };
+        if (classifier_head<ActT>(e, rows, use_fused, fused, fallback, logits, s)) return 1;
         if (cont) { Scope sc(e, KC_ACCEPT, s); launch_beam_choose_groups(st, cbt, dl, s); }
         else { Scope sc(e, KC_ACCEPT, s); launch_beam_choose(st, C, beam, dl, s); }
         // the expand kernel also closes the iteration: its last CTA writes the control words and, last, the iteration's
@@ -1396,7 +1356,7 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
         return 0;
     };
     // wait for the packed word the expand kernel posts for iteration `seq` (sequence | error | all finished | empty columns)
-    static const bool pure_spin = [] { const char* v = getenv("TTB_BEAM_SPIN"); return v && v[0] == '1'; }();
+    static const bool pure_spin = env_flag("TTB_BEAM_SPIN");
     int live_next = B;      // unfinished candidates entering the next iteration, from the newest word read
     int cont_used = 0, cont_dl = 0;   // continuous loop: slots in use and largest draft length of the open batches, idem
     auto wait_word = [&](int seq) -> int {
@@ -1460,21 +1420,18 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
         // every batch takes part in at most max_len iterations
         const long long max_iters = (long long)cb->n * (max_len + 1);
         std::vector<int> hist, hist_dl;
-        int next = 0, it = 0;
+        int it = 0;
         live_next = 0;
         // TTB_BEAM_CB_FULL_DL=1 (read per call): every decoder call runs at the first iteration's draft length, so that
         // every batch near max_len runs with a shorter dl than the call's (a check that results do not depend on it)
-        const char* full_dl = getenv("TTB_BEAM_CB_FULL_DL");
-        const bool force_full_dl = full_dl && full_dl[0] == '1';
+        const bool force_full_dl = env_flag("TTB_BEAM_CB_FULL_DL");
         while (true) {
             int dl_it = force_full_dl ? dl_first : cont_dl;
-            while (next < cb->n && B - cont_used >= cb->bs[next]) {
-                if (admit(next)) return 1;
-                cont_used += cb->bs[next];
-                live_next += cb->bs[next];
-                dl_it = std::max(dl_it, dl_first);
-                ++next;
-            }
+            int n = 0;
+            if (sg.admit_fitting(B - cont_used, &n, admit)) return 1;
+            cont_used += n;
+            live_next += n;
+            if (n > 0) dl_it = std::max(dl_it, dl_first);
             if (cont_used == 0) break;   // nothing open and nothing pending (every batch fits the slots)
             TTB_CHECK(it < max_iters, "continuous beam-search loop did not terminate within max_len iterations per batch");
             hist.push_back(cont_used);
@@ -1515,7 +1472,7 @@ static int beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, int ma
         }
         return 0;
     }
-    static const bool no_ahead = [] { const char* v = getenv("TTB_BEAM_NO_AHEAD"); return v && v[0] == '1'; }();
+    static const bool no_ahead = env_flag("TTB_BEAM_NO_AHEAD");
     const bool ahead_ok = st.host_ctrl && !no_ahead && !trace_nacc && !trace_pick;
     int enq = 0, dl_enq = dl;
     bool ended = false;
@@ -1607,28 +1564,23 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
     const long long launches0 = e->launches;
     const bool cont = cb != nullptr;
     const long long TS = (long long)B * Ls;
-    const int Ls_cap = std::max(256, (Ls + 63) / 64 * 64);
-    const long long TS_cap = (long long)B * Ls_cap;   // no reallocation from one batch length to the next
+    const int Ls_cap = ls_capacity(Ls);
+    const long long TS_cap = (long long)B * Ls_cap;
     const int Cmax = B * K, ldw = max_len;
     Staging<ActT> sg(cb);
-    const long long TS_enc = cont ? sg.TS_stage : TS_cap;
 
-    if (e->src32.ensure(TS_enc * sizeof(int)) || e->memory.ensure(TS_enc * E * sizeof(float))) return 1;
-    if (Prec<ActT>::lowp && e->memh.ensure(TS_enc * E * sizeof(ActT))) return 1;
-    if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
+    if (ensure_encoder<ActT>(e, cont ? sg.TS_stage : TS_cap, B, TS_cap)) return 1;
     if (ensure_work<ActT>(e, cont ? (long long)Cmax : std::max<long long>(Cmax, TS_cap), n_dec)) return 1;
     DevBuf& bb = e->beam;
-    size_t off = 0;
-    auto take = [&](size_t bytes) { size_t o = off; off += (bytes + 255) / 256 * 256; return o; };
-    const size_t o_y0 = take((size_t)Cmax * ldw * 4), o_y1 = take((size_t)Cmax * ldw * 4);
-    const size_t o_s0 = take(Cmax * 4), o_s1 = take(Cmax * 4), o_fin = take(Cmax * 4), o_cr = take(Cmax * 4), o_rc = take(Cmax * 4),
-                 o_rq = take(Cmax * 4), o_tot = take((size_t)Cmax * V * 4), o_ctrl = take(64), o_lg = take((size_t)Cmax * V * 4),
-                 o_cf = take(Cmax * 4), o_par = take(Cmax * 4), o_ds = take(Cmax * 16), o_dc = take(Cmax * 16);
-    if (bb.ensure(off)) return 1;
+    Arena a;
+    const size_t o_y0 = a.take((size_t)Cmax * ldw * 4), o_y1 = a.take((size_t)Cmax * ldw * 4);
+    const size_t o_s0 = a.take(Cmax * 4), o_s1 = a.take(Cmax * 4), o_fin = a.take(Cmax * 4), o_cr = a.take(Cmax * 4), o_rc = a.take(Cmax * 4),
+                 o_rq = a.take(Cmax * 4), o_tot = a.take((size_t)Cmax * V * 4), o_ctrl = a.take(64), o_lg = a.take((size_t)Cmax * V * 4),
+                 o_cf = a.take(Cmax * 4), o_par = a.take(Cmax * 4), o_ds = a.take(Cmax * 16), o_dc = a.take(Cmax * 16);
+    if (bb.ensure(a.bytes)) return 1;
     const long long cache_c_stride = (long long)max_len * E, cache_l_stride = (long long)Cmax * max_len * E;
     const size_t cbytes = (size_t)n_dec * cache_l_stride * sizeof(ActT);
     if (e->kcache.ensure(cbytes) || e->vcache.ensure(cbytes) || e->kcache2.ensure(cbytes) || e->vcache2.ensure(cbytes)) return 1;
-    if (e->srclen.ensure((size_t)B * sizeof(int))) return 1;
     // continuous loop: slot / batch tables, staging of an admitted batch
     SbTable cbt{};
     if (cont)
@@ -1771,14 +1723,12 @@ static int std_beam_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, in
     // every batch takes part in at most max_len - 1 steps
     const long long max_steps = (long long)cb->n * (max_len + 1);
     std::vector<int> hist;
-    int next = 0, step = 0, used = 0, live_next = 0;
+    int step = 0, used = 0, live_next = 0;
     while (true) {
-        while (next < cb->n && B - used >= cb->bs[next]) {
-            if (int rc = admit(next)) return rc;
-            used += cb->bs[next];
-            live_next += cb->bs[next];   // one BOS hypothesis per query
-            ++next;
-        }
+        int n = 0;
+        if (int rc = sg.admit_fitting(B - used, &n, admit)) return rc;
+        used += n;
+        live_next += n;   // one BOS hypothesis per query
         if (used == 0) break;   // nothing open and nothing pending (every batch fits the slots)
         TTB_CHECK(step < max_steps, "continuous beam-search loop did not terminate within max_len steps per batch");
         hist.push_back(used);
@@ -1835,9 +1785,7 @@ static int score_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, const
     const int Bc = std::max(1, std::min(B, kScoreMaxRows / std::max(K * Lt, Ls)));
     const long long T_cap = (long long)Bc * K * Lt, TS_cap = (long long)Bc * Ls;
     if (ensure_work<ActT>(e, std::max(T_cap, TS_cap), 1)) return 1;
-    if (e->src32.ensure(TS_cap * sizeof(int)) || e->memory.ensure(TS_cap * E * sizeof(float)) || e->srclen.ensure((size_t)Bc * sizeof(int))) return 1;
-    if (Prec<ActT>::lowp && e->memh.ensure(TS_cap * E * sizeof(ActT))) return 1;
-    if (e->crosskv.ensure(TS_cap * 2 * E * sizeof(ActT) * n_dec)) return 1;
+    if (ensure_encoder<ActT>(e, TS_cap, Bc, TS_cap)) return 1;
     // kvmap [Bc K], then per row: tokv, lmax, lsum and the top-1 / support outputs of classifier_stats that nothing reads
     const size_t G_cap = (size_t)Bc * K, R = (size_t)T_cap;
     if (e->score.ensure((G_cap + 6 * R) * 4)) return 1;
@@ -1855,8 +1803,7 @@ static int score_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, const
     ActT* crosskv = e->crosskv.as<ActT>();
     float* x = e->x.as<float>();
     ActT* xh = Prec<ActT>::lowp ? e->xh.as<ActT>() : nullptr;
-    const char* nf = getenv("TTB_NO_FUSED_STATS");
-    const bool try_fused = Prec<ActT>::lowp && !(nf && nf[0] == '1');
+    const bool use_fused = Prec<ActT>::lowp && !env_flag("TTB_NO_FUSED_STATS");
     TTB_CUDA_OK(cudaEventRecord(e->t0, s));
 
     for (int b0 = 0; b0 < B; b0 += Bc) {
@@ -1876,22 +1823,11 @@ static int score_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, const
                  nullptr, srclen);
         };
         if (decoder_stack<ActT>(e, rows, 1, 0, self_attn, cross_attn, s)) return 1;
-        bool fused = false;
-        if constexpr (Prec<ActT>::lowp) {
-            if (try_fused) {
-                Scope sc(e, KC_GEMM_CLASSIFIER, s);
-                const int rc = launch_classifier_stats(xh, E, e->classifier.wh, e->classifier.b, rows, V, E, 1, row_tok, tokv, lmax, lsum,
-                                                       nkeep, topv, topi, s);
-                if (rc > 0) return 1;
-                fused = rc == 0;
-                if (!fused) e->launches--;
-            }
-        }
-        if (!fused) {
-            if (linear<float>(e, KC_GEMM_CLASSIFIER, a_view<ActT>(x, xh), E, e->classifier, e->logits.as<float>(), V, rows, false, s)) return 1;
-            Scope sc(e, KC_ARGMAX, s);
-            launch_logprob_stats(e->logits.as<float>(), V, V, row_tok, (int)T, tokv, lmax, lsum, s);
-        }
+        auto fused = [&](const auto* a) {
+            return launch_classifier_stats(a, E, e->classifier.wh, e->classifier.b, rows, V, E, 1, row_tok, tokv, lmax, lsum, nkeep, topv, topi, s);
+        };
+        auto fallback = [&](const float* lg) { launch_logprob_stats(lg, V, V, row_tok, (int)T, tokv, lmax, lsum, s); };
+        if (classifier_head<ActT>(e, rows, use_fused, fused, fallback, e->logits.as<float>(), s)) return 1;
         {
             Scope sc(e, KC_ACCEPT, s);
             launch_score_reduce(tgt32, G, Lt, pad, eos, tokv, lmax, lsum, logp_out + (long long)b0 * K, ntok_out + (long long)b0 * K,
@@ -1901,6 +1837,61 @@ static int score_api(ttb_engine* e, const int64_t* src_dev, int B, int Ls, const
     }
     float ms = 0.f;
     return finish_loop(e, ms);
+}
+
+
+// Calls f(t, stream) on the engine's device, t a value of the engine's activation type: float on the fp32 path,
+// __nv_bfloat16 on the bf16 path.
+template <typename F>
+static int with_act_type(ttb_engine* e, void* stream, F f) {
+    TTB_CUDA_OK(cudaSetDevice(e->device));
+    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
+    return e->d.precision == TTB_PRECISION_FP32 ? f(float{}, s) : f(__nv_bfloat16{}, s);
+}
+
+// Argument rules of the C entry points, each in the order the reference asserts them.  The *_generate_batches entries pass
+// Ls = 0: their source lengths are checked batch by batch.
+static int check_draft_tokens(int n_drafts, int pad, int eos, int replace) {   // drafting.py:38-42
+    TTB_CHECK(n_drafts > 0, "The number of drafts must be greater than 0");
+    TTB_CHECK(pad != replace, "The pad token and the replace token must be different");
+    TTB_CHECK(eos != replace, "The eos token and the replace token must be different");
+    TTB_CHECK(eos != pad, "The eos token and the pad token must be different");
+    return 0;
+}
+static int check_beam(const ttb_engine* e, int Ls, int max_len, int beam_size) {
+    TTB_CHECK(max_len > 1 && beam_size > 0, "max_len must be greater than 1 and beam_size greater than 0");
+    TTB_CHECK(beam_size <= e->d.tgt_vocab_size, "beam_size larger than the vocabulary (the reference's first topk fails as well)");
+    TTB_CHECK(Ls <= e->d.max_positions && max_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
+    return 0;
+}
+static int check_beam_speculative(const ttb_engine* e, int Ls, int max_len, int n_best, int n_drafts, int pad, int eos, int c_token) {
+    TTB_CHECK(n_best >= 1 && n_best <= 32, "n_best must be in [1, 32]");
+    if (int rc = check_draft_tokens(n_drafts, pad, eos, c_token)) return rc;
+    TTB_CHECK(Ls <= e->d.max_positions && max_len + 210 <= e->d.max_positions, "sequence longer than the positional table");
+    TTB_CHECK(e->d.tgt_vocab_size <= 1024, "vocabularies above 1024 tokens are not supported by the beam statistics kernel");
+    return 0;
+}
+
+// The batches of a *_generate_batches call, batch by batch: pointers, B_i > 0 and Ls_i >= min_ls, then B_i <= slots and
+// Ls_i <= max_positions, that pair in the order of `table_first`; with `smart`, last, the Ls_i > 5 that the window library
+// of smart drafts needs.  *Ls_max: the longest source, at least min_ls.
+static int check_batch_list(const ttb_engine* e, int n, const int64_t* const* src, const int32_t* bs, const int32_t* ls, int64_t* const* out,
+                            int slots, int min_ls, bool table_first, bool smart, int* Ls_max) {
+    *Ls_max = min_ls;
+    for (int i = 0; i < n; ++i) {
+        TTB_CHECK(src[i] && out[i] && bs[i] > 0 && ls[i] >= min_ls, "bad arguments");
+        if (table_first) TTB_CHECK(ls[i] <= e->d.max_positions, "sequence longer than the positional table");
+        TTB_CHECK(bs[i] <= slots, "slots must be at least the largest batch size");
+        if (!table_first) TTB_CHECK(ls[i] <= e->d.max_positions, "sequence longer than the positional table");
+        if (smart) TTB_CHECK(ls[i] > 5, "The number of drafts must be greater than 0");
+        *Ls_max = std::max(*Ls_max, (int)ls[i]);
+    }
+    return 0;
+}
+static int check_greedy(const ttb_engine* e, int Ls, int max_len) {
+    TTB_CHECK(max_len > 1, "bad arguments");
+    TTB_CHECK(Ls <= e->d.max_positions && max_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
+    return 0;
 }
 
 }  // namespace ttb
@@ -2067,8 +2058,6 @@ int ttb_make_drafts(const int64_t* src_dev, int64_t src_ld, int32_t B, int32_t L
     return 0;
 }
 
-#define TTB_DISPATCH(e, call_f32, call_bf16) ((e)->d.precision == TTB_PRECISION_FP32 ? (call_f32) : (call_bf16))
-
 // Every exit of a decoding loop leaves the engine's stream drained: kernels still queued there write to the caller's
 // `out` / `trace` buffers, which the caller is free to release as soon as the call returns (error exits included).
 static int drained(ttb_engine* e, int rc) {
@@ -2086,10 +2075,7 @@ int ttb_encode_src(ttb_engine* e, const int64_t* src_dev, const uint8_t* src_pad
     TTB_CHECK(e && e->finalized, "engine not finalized");
     TTB_CHECK(src_dev && memory_out_dev && B > 0 && Ls > 0, "bad arguments");
     TTB_CHECK(Ls <= e->d.max_positions, "source longer than the positional table");
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    return TTB_DISPATCH(e, encode_api<float>(e, src_dev, src_pad_mask_dev, B, Ls, memory_out_dev, s),
-                        encode_api<__nv_bfloat16>(e, src_dev, src_pad_mask_dev, B, Ls, memory_out_dev, s));
+    return with_act_type(e, stream, [&](auto t, cudaStream_t s) { return encode_api<decltype(t)>(e, src_dev, src_pad_mask_dev, B, Ls, memory_out_dev, s); });
 }
 
 int ttb_decode_tgt(ttb_engine* e, const int64_t* tgt_dev, int32_t B, int32_t Lt, const float* memory_dev,
@@ -2097,10 +2083,7 @@ int ttb_decode_tgt(ttb_engine* e, const int64_t* tgt_dev, int32_t B, int32_t Lt,
     TTB_CHECK(e && e->finalized, "engine not finalized");
     TTB_CHECK(tgt_dev && memory_dev && memory_pad_mask_dev && logits_out_dev && B > 0 && Lt > 0 && Ls > 0, "bad arguments");
     TTB_CHECK(Lt <= e->d.max_positions, "target longer than the positional table");
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    return TTB_DISPATCH(e, decode_api<float>(e, tgt_dev, B, Lt, memory_dev, memory_pad_mask_dev, Ls, logits_out_dev, s),
-                        decode_api<__nv_bfloat16>(e, tgt_dev, B, Lt, memory_dev, memory_pad_mask_dev, Ls, logits_out_dev, s));
+    return with_act_type(e, stream, [&](auto t, cudaStream_t s) { return decode_api<decltype(t)>(e, tgt_dev, B, Lt, memory_dev, memory_pad_mask_dev, Ls, logits_out_dev, s); });
 }
 
 int ttb_greedy_speculative_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls,
@@ -2110,17 +2093,12 @@ int ttb_greedy_speculative_generate(ttb_engine* e, const int64_t* src_dev, int32
                                     ttb_generate_stats* stats, void* stream) {
     TTB_CHECK(e && e->finalized, "engine not finalized");
     TTB_CHECK(src_dev && out_dev && B > 0 && Ls > 1 && max_len > 1, "bad arguments");
-    TTB_CHECK(n_drafts > 0, "The number of drafts must be greater than 0");
-    TTB_CHECK(pad_token != replace_token, "The pad token and the replace token must be different");
-    TTB_CHECK(eos_token != replace_token, "The eos token and the replace token must be different");
-    TTB_CHECK(eos_token != pad_token, "The eos token and the pad token must be different");
+    if (int rc = check_draft_tokens(n_drafts, pad_token, eos_token, replace_token)) return rc;
     TTB_CHECK(Ls <= e->d.max_positions && max_len + draft_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    return drained(e, TTB_DISPATCH(e, greedy_api<float>(e, src_dev, B, Ls, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token,
-                                             replace_token, tie_break, out_dev, trace_dev, stats, s),
-                        greedy_api<__nv_bfloat16>(e, src_dev, B, Ls, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token,
-                                                  replace_token, tie_break, out_dev, trace_dev, stats, s)));
+    return drained(e, with_act_type(e, stream, [&](auto t, cudaStream_t s) {
+        return greedy_api<decltype(t)>(e, src_dev, B, Ls, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token, replace_token, tie_break,
+                                       out_dev, trace_dev, stats, s, GreedyMode::speculative);
+    }));
 }
 
 int ttb_greedy_speculative_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs, const int32_t* batch_sizes,
@@ -2131,38 +2109,28 @@ int ttb_greedy_speculative_generate_batches(ttb_engine* e, int32_t n_batches, co
     TTB_CHECK(e && e->finalized, "engine not finalized");
     TTB_CHECK(n_batches >= 0 && max_len > 1 && slots > 0, "bad arguments");
     TTB_CHECK(n_batches == 0 || (src_devs && batch_sizes && src_lens && out_devs && stats), "bad arguments");
-    TTB_CHECK(n_drafts > 0, "The number of drafts must be greater than 0");
-    TTB_CHECK(pad_token != replace_token, "The pad token and the replace token must be different");
-    TTB_CHECK(eos_token != replace_token, "The eos token and the replace token must be different");
-    TTB_CHECK(eos_token != pad_token, "The eos token and the pad token must be different");
+    if (int rc = check_draft_tokens(n_drafts, pad_token, eos_token, replace_token)) return rc;
     TTB_CHECK(max_len + draft_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
-    int Ls_max = 2;
-    for (int i = 0; i < n_batches; ++i) {
-        TTB_CHECK(src_devs[i] && out_devs[i] && batch_sizes[i] > 0 && src_lens[i] > 1, "bad arguments");
-        TTB_CHECK(batch_sizes[i] <= slots, "slots must be at least the largest batch size");
-        TTB_CHECK(src_lens[i] <= e->d.max_positions, "sequence longer than the positional table");
-        Ls_max = std::max(Ls_max, (int)src_lens[i]);
-    }
+    int Ls_max = 0;
+    if (int rc = check_batch_list(e, n_batches, src_devs, batch_sizes, src_lens, out_devs, slots, 2, false, false, &Ls_max)) return rc;
     if (total) *total = ttb_generate_stats{};
     if (n_batches == 0) return 0;
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const BatchList cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, stats, nullptr, trace_devs, nullptr, nullptr};
-    return drained(e, TTB_DISPATCH(e, greedy_api<float>(e, nullptr, slots, Ls_max, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token,
-                                                        replace_token, tie_break, nullptr, nullptr, total, s, false, &cb),
-                                   greedy_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token,
-                                                             replace_token, tie_break, nullptr, nullptr, total, s, false, &cb)));
+    return drained(e, with_act_type(e, stream, [&](auto t, cudaStream_t s) {
+        return greedy_api<decltype(t)>(e, nullptr, slots, Ls_max, max_len, draft_len, n_drafts, pad_token, bos_token, eos_token, replace_token,
+                                       tie_break, nullptr, nullptr, total, s, GreedyMode::speculative, &cb);
+    }));
 }
 
 int ttb_greedy_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len, int32_t pad_token,
                         int32_t bos_token, int32_t eos_token, int64_t* out_dev, ttb_generate_stats* stats, void* stream) {
     TTB_CHECK(e && e->finalized, "engine not finalized");
-    TTB_CHECK(src_dev && out_dev && B > 0 && Ls > 0 && max_len > 1, "bad arguments");
-    TTB_CHECK(Ls <= e->d.max_positions && max_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    return drained(e, TTB_DISPATCH(e, greedy_api<float>(e, src_dev, B, Ls, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, out_dev, nullptr, stats, s, true),
-                        greedy_api<__nv_bfloat16>(e, src_dev, B, Ls, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, out_dev, nullptr, stats, s, true)));
+    TTB_CHECK(src_dev && out_dev && B > 0 && Ls > 0, "bad arguments");
+    if (int rc = check_greedy(e, Ls, max_len)) return rc;
+    return drained(e, with_act_type(e, stream, [&](auto t, cudaStream_t s) {
+        return greedy_api<decltype(t)>(e, src_dev, B, Ls, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, out_dev, nullptr, stats, s,
+                                       GreedyMode::standard);
+    }));
 }
 
 int ttb_greedy_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs, const int32_t* batch_sizes,
@@ -2174,24 +2142,17 @@ int ttb_greedy_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t*
     TTB_CHECK(n_batches == 0 || (src_devs && batch_sizes && src_lens && out_devs && stats), "bad arguments");
     // the rules of ttb_greedy_generate, in its order, before any device work
     for (int i = 0; i < n_batches; ++i) TTB_CHECK(src_devs[i] && out_devs[i] && batch_sizes[i] > 0 && src_lens[i] > 0, "bad arguments");
-    TTB_CHECK(max_len > 1, "bad arguments");
-    TTB_CHECK(max_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
-    int Ls_max = 1;
-    for (int i = 0; i < n_batches; ++i) {
-        TTB_CHECK(src_lens[i] <= e->d.max_positions, "sequence longer than the positional table");
-        TTB_CHECK(batch_sizes[i] <= slots, "slots must be at least the largest batch size");
-        Ls_max = std::max(Ls_max, (int)src_lens[i]);
-    }
+    if (int rc = check_greedy(e, 0, max_len)) return rc;
+    int Ls_max = 0;
+    if (int rc = check_batch_list(e, n_batches, src_devs, batch_sizes, src_lens, out_devs, slots, 1, true, false, &Ls_max)) return rc;
     TTB_CHECK(slots <= 2048, "continuous batching supports at most 2048 slots");
     if (total) *total = ttb_generate_stats{};
     if (n_batches == 0) return 0;
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const BatchList cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, stats, nullptr, nullptr, nullptr, nullptr};
-    return drained(e, TTB_DISPATCH(e, greedy_api<float>(e, nullptr, slots, Ls_max, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1,
-                                                        nullptr, nullptr, total, s, true, &cb),
-                                   greedy_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1,
-                                                             nullptr, nullptr, total, s, true, &cb)));
+    return drained(e, with_act_type(e, stream, [&](auto t, cudaStream_t s) {
+        return greedy_api<decltype(t)>(e, nullptr, slots, Ls_max, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, nullptr, nullptr, total, s,
+                                       GreedyMode::standard, &cb);
+    }));
 }
 
 int ttb_sample_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len, int32_t n_samples, float temperature,
@@ -2206,14 +2167,11 @@ int ttb_sample_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_
     TTB_CHECK(max_len >= 2, "max_len must be at least 2");
     TTB_CHECK(pad_token != eos_token, "The eos token and the pad token must be different");
     TTB_CHECK(Ls <= e->d.max_positions && max_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const SampleCfg smp{n_samples, temperature, top_k, (unsigned long long)seed};
-    const int R = B * n_samples;
-    return drained(e, TTB_DISPATCH(e, greedy_api<float>(e, src_dev, R, Ls, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, out_dev, nullptr,
-                                                        stats, s, true, nullptr, &smp),
-                                   greedy_api<__nv_bfloat16>(e, src_dev, R, Ls, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, out_dev,
-                                                             nullptr, stats, s, true, nullptr, &smp)));
+    return drained(e, with_act_type(e, stream, [&](auto t, cudaStream_t s) {
+        return greedy_api<decltype(t)>(e, src_dev, B * n_samples, Ls, max_len, 0, 1, pad_token, bos_token, eos_token, -1, 1, out_dev, nullptr,
+                                       stats, s, GreedyMode::sampling, nullptr, smp);
+    }));
 }
 
 int ttb_beam_search_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len, int32_t beam_size,
@@ -2221,13 +2179,10 @@ int ttb_beam_search_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, i
                              ttb_generate_stats* stats, void* stream) {
     TTB_CHECK(e && e->finalized, "engine not finalized");
     TTB_CHECK(src_dev && out_dev && B > 0 && Ls > 0, "bad arguments");
-    TTB_CHECK(max_len > 1 && beam_size > 0, "max_len must be greater than 1 and beam_size greater than 0");
-    TTB_CHECK(beam_size <= e->d.tgt_vocab_size, "beam_size larger than the vocabulary (the reference's first topk fails as well)");
-    TTB_CHECK(Ls <= e->d.max_positions && max_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    return drained(e, TTB_DISPATCH(e, std_beam_api<float>(e, src_dev, B, Ls, max_len, beam_size, pad_token, bos_token, eos_token, out_dev, out_width, stats, s),
-                        std_beam_api<__nv_bfloat16>(e, src_dev, B, Ls, max_len, beam_size, pad_token, bos_token, eos_token, out_dev, out_width, stats, s)));
+    if (int rc = check_beam(e, Ls, max_len, beam_size)) return rc;
+    return drained(e, with_act_type(e, stream, [&](auto t, cudaStream_t s) {
+        return std_beam_api<decltype(t)>(e, src_dev, B, Ls, max_len, beam_size, pad_token, bos_token, eos_token, out_dev, out_width, stats, s);
+    }));
 }
 
 int ttb_beam_search_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs, const int32_t* batch_sizes,
@@ -2239,28 +2194,20 @@ int ttb_beam_search_generate_batches(ttb_engine* e, int32_t n_batches, const int
     TTB_CHECK(n_batches == 0 || (src_devs && batch_sizes && src_lens && out_devs && out_widths && stats), "bad arguments");
     for (int i = 0; i < n_batches; ++i) TTB_CHECK(src_devs[i] && out_devs[i] && batch_sizes[i] > 0 && src_lens[i] > 0, "bad arguments");
     // the rules of ttb_beam_search_generate, in its order, before any device work
-    TTB_CHECK(max_len > 1 && beam_size > 0, "max_len must be greater than 1 and beam_size greater than 0");
-    TTB_CHECK(beam_size <= e->d.tgt_vocab_size, "beam_size larger than the vocabulary (the reference's first topk fails as well)");
-    TTB_CHECK(max_len + 2 <= e->d.max_positions, "sequence longer than the positional table");
-    int Ls_max = 1;
-    for (int i = 0; i < n_batches; ++i) {
-        TTB_CHECK(src_lens[i] <= e->d.max_positions, "sequence longer than the positional table");
-        TTB_CHECK(batch_sizes[i] <= slots, "slots must be at least the largest batch size");
-        Ls_max = std::max(Ls_max, (int)src_lens[i]);
-    }
+    if (int rc = check_beam(e, 0, max_len, beam_size)) return rc;
+    int Ls_max = 0;
+    if (int rc = check_batch_list(e, n_batches, src_devs, batch_sizes, src_lens, out_devs, slots, 1, true, false, &Ls_max)) return rc;
     // generate() fails in its first step (one hypothesis per query) or its second (beam_size of them)
     TTB_CHECK(sbeam_select_fits(1, e->d.tgt_vocab_size) && (max_len == 2 || sbeam_select_fits(beam_size, e->d.tgt_vocab_size)),
               "beam_size * vocabulary too large for the selection kernel");
     TTB_CHECK(slots <= 65535 && (long long)slots * beam_size < (1 << 24), "continuous batching supports at most 65535 slots and 2^24 - 1 hypotheses");
     if (total) *total = ttb_generate_stats{};
     if (n_batches == 0) return 0;
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const BatchList cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, stats, out_widths, nullptr, nullptr, nullptr};
-    return drained(e, TTB_DISPATCH(e, std_beam_api<float>(e, nullptr, slots, Ls_max, max_len, beam_size, pad_token, bos_token, eos_token, nullptr, nullptr,
-                                                          total, s, &cb),
-                                   std_beam_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, beam_size, pad_token, bos_token, eos_token, nullptr,
-                                                               nullptr, total, s, &cb)));
+    return drained(e, with_act_type(e, stream, [&](auto t, cudaStream_t s) {
+        return std_beam_api<decltype(t)>(e, nullptr, slots, Ls_max, max_len, beam_size, pad_token, bos_token, eos_token, nullptr, nullptr, total,
+                                         s, &cb);
+    }));
 }
 
 int ttb_beam_speculative_generate(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, int32_t max_len,
@@ -2270,21 +2217,11 @@ int ttb_beam_speculative_generate(ttb_engine* e, const int64_t* src_dev, int32_t
                                   void* stream) {
     TTB_CHECK(e && e->finalized, "engine not finalized");
     TTB_CHECK(src_dev && out_dev && B > 0 && Ls > 1 && max_len > 2, "bad arguments");
-    TTB_CHECK(n_best >= 1 && n_best <= 32, "n_best must be in [1, 32]");
-    TTB_CHECK(n_drafts > 0, "The number of drafts must be greater than 0");
-    TTB_CHECK(pad_token != c_token, "The pad token and the replace token must be different");
-    TTB_CHECK(eos_token != c_token, "The eos token and the replace token must be different");
-    TTB_CHECK(eos_token != pad_token, "The eos token and the pad token must be different");
-    TTB_CHECK(Ls <= e->d.max_positions && max_len + 210 <= e->d.max_positions, "sequence longer than the positional table");
-    TTB_CHECK(e->d.tgt_vocab_size <= 1024, "vocabularies above 1024 tokens are not supported by the beam statistics kernel");
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    return drained(e, TTB_DISPATCH(e, beam_api<float>(e, src_dev, B, Ls, max_len, n_best, draft_len, n_drafts, pad_token, bos_token, eos_token,
-                                           c_token, tie_break, out_dev, out_width, trace_nacc_dev, trace_pick_dev, stats, s,
-                                           smart_drafts_mode != 0),
-                        beam_api<__nv_bfloat16>(e, src_dev, B, Ls, max_len, n_best, draft_len, n_drafts, pad_token, bos_token,
-                                                eos_token, c_token, tie_break, out_dev, out_width, trace_nacc_dev, trace_pick_dev, stats, s,
-                                                smart_drafts_mode != 0)));
+    if (int rc = check_beam_speculative(e, Ls, max_len, n_best, n_drafts, pad_token, eos_token, c_token)) return rc;
+    return drained(e, with_act_type(e, stream, [&](auto t, cudaStream_t s) {
+        return beam_api<decltype(t)>(e, src_dev, B, Ls, max_len, n_best, draft_len, n_drafts, pad_token, bos_token, eos_token, c_token, tie_break,
+                                     out_dev, out_width, trace_nacc_dev, trace_pick_dev, stats, s, smart_drafts_mode != 0);
+    }));
 }
 
 int ttb_beam_speculative_generate_batches(ttb_engine* e, int32_t n_batches, const int64_t* const* src_devs, const int32_t* batch_sizes,
@@ -2296,31 +2233,17 @@ int ttb_beam_speculative_generate_batches(ttb_engine* e, int32_t n_batches, cons
     TTB_CHECK(e && e->finalized, "engine not finalized");
     TTB_CHECK(n_batches >= 0 && max_len > 2 && slots > 0, "bad arguments");
     TTB_CHECK(n_batches == 0 || (src_devs && batch_sizes && src_lens && out_devs && out_widths && stats), "bad arguments");
-    TTB_CHECK(n_best >= 1 && n_best <= 32, "n_best must be in [1, 32]");
-    TTB_CHECK(n_drafts > 0, "The number of drafts must be greater than 0");
-    TTB_CHECK(pad_token != c_token, "The pad token and the replace token must be different");
-    TTB_CHECK(eos_token != c_token, "The eos token and the replace token must be different");
-    TTB_CHECK(eos_token != pad_token, "The eos token and the pad token must be different");
-    TTB_CHECK(max_len + 210 <= e->d.max_positions, "sequence longer than the positional table");
-    TTB_CHECK(e->d.tgt_vocab_size <= 1024, "vocabularies above 1024 tokens are not supported by the beam statistics kernel");
-    int Ls_max = 2;
-    for (int i = 0; i < n_batches; ++i) {
-        TTB_CHECK(src_devs[i] && out_devs[i] && batch_sizes[i] > 0 && src_lens[i] > 1, "bad arguments");
-        TTB_CHECK(batch_sizes[i] <= slots, "slots must be at least the largest batch size");
-        TTB_CHECK(src_lens[i] <= e->d.max_positions, "sequence longer than the positional table");
-        if (smart_drafts_mode) TTB_CHECK(src_lens[i] > 5, "The number of drafts must be greater than 0");
-        Ls_max = std::max(Ls_max, (int)src_lens[i]);
-    }
+    if (int rc = check_beam_speculative(e, 0, max_len, n_best, n_drafts, pad_token, eos_token, c_token)) return rc;
+    int Ls_max = 0;
+    if (int rc = check_batch_list(e, n_batches, src_devs, batch_sizes, src_lens, out_devs, slots, 2, false, smart_drafts_mode != 0, &Ls_max))
+        return rc;
     if (total) *total = ttb_generate_stats{};
     if (n_batches == 0) return 0;
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
     const BatchList cb{n_batches, src_devs, batch_sizes, src_lens, out_devs, stats, out_widths, nullptr, trace_nacc_devs, trace_pick_devs};
-    return drained(e, TTB_DISPATCH(e, beam_api<float>(e, nullptr, slots, Ls_max, max_len, n_best, draft_len, n_drafts, pad_token, bos_token, eos_token,
-                                                      c_token, tie_break, nullptr, nullptr, nullptr, nullptr, total, s, smart_drafts_mode != 0, &cb),
-                                   beam_api<__nv_bfloat16>(e, nullptr, slots, Ls_max, max_len, n_best, draft_len, n_drafts, pad_token, bos_token,
-                                                           eos_token, c_token, tie_break, nullptr, nullptr, nullptr, nullptr, total, s,
-                                                           smart_drafts_mode != 0, &cb)));
+    return drained(e, with_act_type(e, stream, [&](auto t, cudaStream_t s) {
+        return beam_api<decltype(t)>(e, nullptr, slots, Ls_max, max_len, n_best, draft_len, n_drafts, pad_token, bos_token, eos_token, c_token,
+                                     tie_break, nullptr, nullptr, nullptr, nullptr, total, s, smart_drafts_mode != 0, &cb);
+    }));
 }
 
 int ttb_score_targets(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t Ls, const int64_t* tgt_dev, int32_t K, int32_t Lt,
@@ -2332,12 +2255,9 @@ int ttb_score_targets(ttb_engine* e, const int64_t* src_dev, int32_t B, int32_t 
     TTB_CHECK(Ls <= e->d.max_positions && Lt <= e->d.max_positions, "sequence longer than the positional table");
     TTB_CHECK((long long)K * Lt <= kScoreMaxRows, "K * Lt above 32768 decoder rows per source");
     TTB_CHECK(pad_token != eos_token, "The eos token and the pad token must be different");
-    TTB_CUDA_OK(cudaSetDevice(e->device));
-    cudaStream_t s = reinterpret_cast<cudaStream_t>(stream);
-    return drained(e, TTB_DISPATCH(e, score_api<float>(e, src_dev, B, Ls, tgt_dev, K, Lt, pad_token, eos_token, logp_out_dev, ntok_out_dev,
-                                                       token_logp_out_dev, s),
-                                   score_api<__nv_bfloat16>(e, src_dev, B, Ls, tgt_dev, K, Lt, pad_token, eos_token, logp_out_dev, ntok_out_dev,
-                                                            token_logp_out_dev, s)));
+    return drained(e, with_act_type(e, stream, [&](auto t, cudaStream_t s) {
+        return score_api<decltype(t)>(e, src_dev, B, Ls, tgt_dev, K, Lt, pad_token, eos_token, logp_out_dev, ntok_out_dev, token_logp_out_dev, s);
+    }));
 }
 
 int ttb_kernel_class_count(void) { return KC_COUNT; }
